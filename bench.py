@@ -58,6 +58,26 @@ def emit_result(line: dict):
 
 ETA = 3.0  # main.rs:32
 DATA_SEED, PARAM_SEED = 0x5EED, 0xC0FFEE
+# --dump-outputs: at most 4 MiB of float64 per array. At most four training workloads (the main one and the extra ones) write
+# three arrays that can be that large (params, grads, e2e_params) and the feature-stage workload one: under 55 MB in all
+DUMP_MAX_ELEMENTS, DUMP_SEED = 1 << 19, 0xD5
+
+
+def dump_array(a):
+    """float64 numpy copy of ``a`` (numpy array or torch tensor) for --dump-outputs. An array of more than DUMP_MAX_ELEMENTS
+    elements is sampled: its flattened elements at a fixed, seeded set of indices, the same for the same size, so that two
+    builds are compared element for element."""
+    n = int(np.prod(a.shape))
+    if n > DUMP_MAX_ELEMENTS:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n, DUMP_MAX_ELEMENTS, replace=False))
+        if isinstance(a, np.ndarray):
+            a = a.reshape(-1)[idx]
+        else:
+            import torch
+            a = a.reshape(-1)[torch.from_numpy(idx).to(a.device)]
+    if not isinstance(a, np.ndarray):
+        a = a.cpu().numpy()
+    return np.array(a, dtype=np.float64)
 
 
 def feature_len(cfg, H, W):
@@ -453,10 +473,11 @@ def kernel_rooflines(wl, B, shapes, prof, prof_steps, pk, fp64_peak, int8_peak):
     return kernels, top, alg
 
 
-def run_leg(ctx, name, wl, B, steps, warmup, exchange, *, main, steps_per_graph=5, no_graph=False, host_alloc="pinned"):
+def run_leg(ctx, name, wl, B, steps, warmup, exchange, *, main, steps_per_graph=5, no_graph=False, host_alloc="pinned",
+            dump=False):
     """One workload on this rank: device-resident `value` leg (epoch mode, CUDA graph), host-buffer `e2e` leg, eager per-kernel
     profile; the main leg (c2) additionally reads the in-graph device timeline. Collective on every rank; returns a dict
-    (rank 0's view; timings are max over ranks)."""
+    (rank 0's view; timings are max over ranks). ``dump``: rank 0 keeps the outputs of the last timed step in ``_outputs``."""
     torch, dist, dev, rank, world = ctx.torch, ctx.dist, ctx.dev, ctx.rank, ctx.world
     from mercer_research_b200 import RCN, _lib
     from mercer_research_b200.trainer import DataParallelTrainer
@@ -469,7 +490,8 @@ def run_leg(ctx, name, wl, B, steps, warmup, exchange, *, main, steps_per_graph=
     model.load_weights_and_bias(L)
     assert model.layer_shapes == shapes
     scale = 1.0 if L <= 1024 else 1.0 / 64.0        # the 4096-wide layers: N(0,1)/64 keeps the sigmoids out of saturation
-    model.set_params(np.random.default_rng(PARAM_SEED).standard_normal(n_params) * scale)   # same replica on every rank
+    seeded_params = np.random.default_rng(PARAM_SEED).standard_normal(n_params) * scale
+    model.set_params(seeded_params)                 # same replica on every rank
     trainer = DataParallelTrainer(model, eta=ETA, exchange=exchange)
 
     # synthetic dataset resident in HBM, larger than L2 (126 MB) so that consecutive steps never hit in L2
@@ -530,6 +552,11 @@ def run_leg(ctx, name, wl, B, steps, warmup, exchange, *, main, steps_per_graph=
     for i in range(int(extra.item())):
         trainer.epoch_step()
     n_warm += int(extra.item())
+    # the warm-up ran a timing-dependent number of steps: the timed steps start again from the seeded parameters at the first
+    # batch, so that the same arguments give them the same inputs run after run (set_params / epoch_seek copy into the
+    # buffers the captured graph already uses)
+    model.set_params(seeded_params)
+    model.epoch_seek(0)
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     # no cyclic-GC pass between the graph launches of the timed region (what timeit does: at the driver's K = 20 the region is
     # four launches / 0.4 ms long, and a collection landing between two of them stalls the GPU for longer than a step)
@@ -544,6 +571,10 @@ def run_leg(ctx, name, wl, B, steps, warmup, exchange, *, main, steps_per_graph=
     clocks.mark_end()
     gc.enable()
     trainer.check()
+    outputs = None
+    if dump and rank == 0:      # what a caller of the step receives after the last timed step
+        outputs = {"params": dump_array(model.get_params()), "grads": dump_array(model.get_gradients()),
+                   "batch_stats": dump_array(np.array(model.last_batch_stats(), dtype=np.float64))}
     launches = kernels_per_step * steps
     ms_step = _max_over_ranks(ctx, e0.elapsed_time(e1)) / steps
     value = world * B / (ms_step * 1e-3)
@@ -586,7 +617,8 @@ def run_leg(ctx, name, wl, B, steps, warmup, exchange, *, main, steps_per_graph=
     # host-resident dataset; every step's H2D copy and the D2H read of its (cost, hits) are inside the timed region -----
     e2e_steps_n = steps
     n_host = max(2, min(e2e_steps_n, (512 << 20) // (B * H * W)))
-    h_images = torch.randint(0, 256, (n_host * B, H, W), dtype=torch.uint8).pin_memory()
+    hg = torch.Generator(); hg.manual_seed(DATA_SEED + rank)
+    h_images = torch.randint(0, 256, (n_host * B, H, W), dtype=torch.uint8, generator=hg).pin_memory()
     h_labels = (torch.arange(n_host * B) % wl["classes"]).to(torch.int64).pin_memory()
     hi, hl = h_images.numpy(), h_labels.numpy()
     if host_alloc == "wc":
@@ -596,12 +628,14 @@ def run_leg(ctx, name, wl, B, steps, warmup, exchange, *, main, steps_per_graph=
             hi, host_alloc = wc, "pinned, write-combined"
 
     def e2e_run(n, verify):
+        """n steps over the host dataset; returns (cost, hits) of the last step."""
         done = 0
         while done < n:
             m = min(n_host, n - done)
             cost, hits = trainer.train_epoch_host(hi[:m * B], hl[:m * B], B, verify_steps=verify)
             assert len(cost) == m
             done += m
+        return cost[-1], hits[-1]
 
     e2e_run(e2e_steps_n, True)                  # warm-up = the timed call sequence itself: buffers sized, step graphs captured,
                                                 # the per-call step counts agreed on across ranks (not repeated in the timed region)
@@ -618,17 +652,21 @@ def run_leg(ctx, name, wl, B, steps, warmup, exchange, *, main, steps_per_graph=
         dist.broadcast(reps, 0)
     for _ in range(int(reps.item())):
         e2e_run(e2e_steps_n, False)
+    model.set_params(seeded_params)             # as for the device-resident leg: the same inputs run after run
     gc.collect()
     gc.disable()
     _barrier(ctx)
     clocks.mark_begin(expected_s=per_call)
     e0.record(stream)
-    e2e_run(e2e_steps_n, False)
+    e2e_last = e2e_run(e2e_steps_n, False)
     e1.record(stream)
     _barrier(ctx)
     clocks.mark_end()
     gc.enable()
     trainer.check()
+    if outputs is not None:
+        outputs.update({"e2e_params": dump_array(model.get_params()),
+                        "e2e_batch_stats": dump_array(np.array(e2e_last, dtype=np.float64))})
     clk = clocks.stop() if rank == 0 else None
     e2e_ms = _max_over_ranks(ctx, e0.elapsed_time(e1))
     e2e_value = world * B / (e2e_ms / e2e_steps_n * 1e-3)
@@ -681,7 +719,7 @@ def run_leg(ctx, name, wl, B, steps, warmup, exchange, *, main, steps_per_graph=
            "ms_step": ms_step, "steps": steps, "spg": spg, "graph": graph_ok, "n_warm": n_warm * spg, "launches": int(launches),
            "step_desc": step_desc, "clocks": clk, "e2e_value": e2e_value, "e2e_ms_step": e2e_ms / e2e_steps_n, "h2d": h2d, "d2h": d2h,
            "host_alloc": host_alloc, "prof": prof, "prof_steps": prof_steps, "timeline": timeline, "parity": parity,
-           "p2p": trainer.p2p, "scale_set": model.scale_set}
+           "p2p": trainer.p2p, "scale_set": model.scale_set, "_outputs": outputs}
     # leave the group state clean for the next leg
     if world > 1:
         trainer.graph = None
@@ -697,9 +735,10 @@ def run_leg(ctx, name, wl, B, steps, warmup, exchange, *, main, steps_per_graph=
     return out
 
 
-def run_features_leg(ctx, name, wl, B, steps):
+def run_features_leg(ctx, name, wl, B, steps, dump=False):
     """BASELINE configs[3] in reference semantics: throughput of the feature stage alone (rcn_cuda_features) on every rank
-    (independent replicas: the stage has no exchange step). Device-resident inputs; the 1 GiB output per call exceeds L2."""
+    (independent replicas: the stage has no exchange step). Device-resident inputs; the 1 GiB output per call exceeds L2.
+    ``dump``: rank 0 keeps (a sample of) the last timed call's features in ``_outputs``."""
     torch, dev, rank, world = ctx.torch, ctx.dev, ctx.rank, ctx.world
     from mercer_research_b200 import RCN, _lib
     H, W = wl["H"], wl["W"]
@@ -727,6 +766,7 @@ def run_features_leg(ctx, name, wl, B, steps):
     _barrier(ctx)
     clocks.mark_end()
     launches = _lib.kernel_launches() - l0
+    outputs = {"features": dump_array(out)} if dump and rank == 0 else None
     clk = clocks.stop() if rank == 0 else None
     ms_step = _max_over_ranks(ctx, e0.elapsed_time(e1)) / steps
     _lib.profile_enable(True)
@@ -741,7 +781,7 @@ def run_features_leg(ctx, name, wl, B, steps):
     nbytes = B * (H * W + L * 8)
     return {"workload": wl["desc"], "value": world * B / (ms_step * 1e-3), "unit": "images/s", "ms_per_step": ms_step, "steps": steps,
             "scaling": "weak (independent replicas: no exchange step)", "batch_per_gpu": B, "feature_len": L, "gpu_launches": int(launches),
-            "clocks": clk, "_nbytes": nbytes, "_prof": prof, "_prof_steps": min(steps, 10)}
+            "clocks": clk, "_nbytes": nbytes, "_prof": prof, "_prof_steps": min(steps, 10), "_outputs": outputs}
 
 
 def leg_roofline(leg, pk, fp64_peak, int8_peak, int8_how, traffic_all, workload_key):
@@ -889,25 +929,26 @@ def run_gpu(args, wl, rank, world, local_rank):
         dist.init_process_group("nccl", device_id=ctx.dev)
 
     # ---- main leg: BASELINE configs[1] (or --workload), per-GPU batch fixed (weak scaling) --------------------------------
+    dump = args.dump_outputs is not None
     main = run_leg(ctx, args.workload, wl, wl["batch"], args.steps, args.warmup, args.exchange, main=True,
-                   steps_per_graph=args.steps_per_graph, no_graph=args.no_graph, host_alloc=args.host_alloc)
+                   steps_per_graph=args.steps_per_graph, no_graph=args.no_graph, host_alloc=args.host_alloc, dump=dump)
     # ---- extra legs in the same invocation: c3 (STRONG scaling: global batch 4096 split over the ranks, SURVEY 8e) and c5
-    # (weak, NCCL all-reduce of the 268.8 MB gradient buffer at N > 1) -----------------------------------------------------
+    # (weak, NCCL all-reduce of the 268.8 MB gradient buffer at N > 1); every leg times --steps steps ---------------------
     legs = {}
     if args.workload == "c2" and not args.no_extra:
         for key in [k for k in args.extra.split(",") if k]:
             w2 = WORKLOADS[key]
             if key == "c4":
-                legs[key] = run_features_leg(ctx, key, w2, w2["batch"], max(4, min(args.steps, 20)))
+                legs[key] = run_features_leg(ctx, key, w2, w2["batch"], args.steps, dump=dump)
                 continue
             if key == "c3":
                 if w2["batch"] % world:
                     continue
-                B2, st2, ex2, scaling = w2["batch"] // world, max(16, min(args.steps, 320) // 16 * 16), "auto", "strong"
+                B2, ex2, scaling = w2["batch"] // world, "auto", "strong"
             else:
-                B2, st2, ex2, scaling = w2["batch"], max(4, min(args.steps, 12)), ("nccl" if world > 1 else "auto"), "weak"
+                B2, ex2, scaling = w2["batch"], ("nccl" if world > 1 else "auto"), "weak"
             try:
-                leg = run_leg(ctx, key, w2, B2, st2, min(args.warmup, 3), ex2, main=False, steps_per_graph=4)
+                leg = run_leg(ctx, key, w2, B2, args.steps, min(args.warmup, 3), ex2, main=False, steps_per_graph=4, dump=dump)
                 leg["scaling"] = scaling
                 legs[key] = leg
             except Exception as e:  # noqa: BLE001  -- an extra leg must never cost the main line
@@ -924,6 +965,11 @@ def run_gpu(args, wl, rank, world, local_rank):
         return
 
     print("[bench] rank 0: collective phases done", file=sys.stderr, flush=True)
+    if dump:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+    for key, leg in [(args.workload, main)] + list(legs.items()):
+        for name, a in (leg.pop("_outputs", None) or {}).items():
+            np.save(os.path.join(args.dump_outputs, f"{key}_{name}.npy"), a)
     pk = peaks()
     fp64_peak = measure_fp64_peak(torch, ctx.dev)
     int8_peak, int8_how = measure_int8_peak(torch, ctx.dev)
@@ -1049,7 +1095,7 @@ def run_gpu(args, wl, rank, world, local_rank):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=2000)
+    ap.add_argument("--steps", type=int, default=2000, help="timed steps of every workload")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="c2", choices=sorted(WORKLOADS))
@@ -1066,7 +1112,17 @@ def main():
                     help="multi-GPU gradient exchange: fused NVLink peer-memory kernel, NCCL all-reduce, or by size")
     ap.add_argument("--extra", default="c3,c4,c5", help="extra workloads measured after the main one in the same run (parsed.workloads)")
     ap.add_argument("--no-extra", action="store_true", help="main workload only")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what each workload's timed paths computed in their last step to "
+                         "DIR/<workload>_<name>.npy (float64): params, grads and batch_stats ([cost, hits]) of the device-"
+                         "resident leg, e2e_params and e2e_batch_stats of the host-buffer leg, features of the feature-stage "
+                         "workload; arrays of more than 2^19 elements as a fixed, seeded sample. The same arguments give the "
+                         "same inputs, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
     # stdout must carry exactly ONE JSON line: route everything else that writes to fd 1 (e.g. NCCL's version banner)
     # to stderr and keep the real stdout for the result line.
     global _RESULT_FD

@@ -1,7 +1,8 @@
 // C++ host tests above the C ABI (include/rcn.hpp): the reference crate's own unit tests (rcn/src/utils/kernel.rs:352-441,
 // rcn/src/rcn.rs:525-538) restated against the C++ mirror of its API, plus the derived known-answer vectors of SURVEY.md
-// Appendix B.  `host_test cpu` needs no GPU (host-side checks, contract violations, the no-fallback rule);
-// `host_test gpu` runs the compute cases on cuda:0.  Exit code 0 and a final "... ok" line on success.
+// Appendix B.  `host_test cpu [dir]` needs no GPU (host-side checks, contract violations, the no-fallback rule) and writes
+// its scratch files under `dir` (default /tmp); `host_test gpu` runs the compute cases on cuda:0.  Exit code 0 and a final
+// "... ok" line on success.
 #include <cmath>
 #include <cstdio>
 #include <cstring>
@@ -51,7 +52,7 @@ static void validate_padding_calc() {
     EXPECT(m1 - r1 < k1);
 }
 
-static int run_cpu() {
+static int run_cpu(const std::string& dir) {
     verify_separated_sobels();
     validate_padding_calc();
     // no CPU fallback: without a device the model cannot even be created
@@ -78,7 +79,7 @@ static int run_cpu() {
     }
     // the one image format the header decodes itself: binary PGM, comments allowed, 16-bit and truncated files rejected
     {
-        const std::string path = "/tmp/rcn_host_test.pgm";
+        const std::string path = dir + "/rcn_host_test.pgm";
         { std::ofstream f(path, std::ios::binary); f << "P5\n# a comment\n3 2\n255\n"; f.write("\x00\x01\x02\xfd\xfe\xff", 6); }
         std::vector<uint8_t> px;
         size_t h = 0, w = 0;
@@ -89,7 +90,7 @@ static int run_cpu() {
         EXPECT(!rcn::read_pgm(path, &px, &h, &w));
         { std::ofstream f(path, std::ios::binary); f << "P2\n3 2\n255\n1 2 3 4 5 6\n"; }
         EXPECT(!rcn::read_pgm(path, &px, &h, &w));
-        EXPECT(!rcn::read_pgm("/tmp/rcn_host_test_missing.pgm", &px, &h, &w));
+        EXPECT(!rcn::read_pgm(dir + "/rcn_host_test_missing.pgm", &px, &h, &w));
         std::remove(path.c_str());
     }
     if (!g_failed) std::printf("cpu ok\n");
@@ -202,7 +203,7 @@ static int run_gpu() {
 int main(int argc, char** argv) {
     const std::string mode = argc > 1 ? argv[1] : "cpu";
     try {
-        return mode == "gpu" ? run_gpu() : run_cpu();
+        return mode == "gpu" ? run_gpu() : run_cpu(argc > 2 ? argv[2] : "/tmp");
     } catch (const std::exception& e) {
         std::printf("FAILED with exception: %s\n", e.what());
         return 2;

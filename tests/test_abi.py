@@ -54,16 +54,30 @@ def test_version_and_error_string(built_library):
     assert isinstance(built_library.rcn_cuda_last_error(), bytes)
 
 
+NO_DEVICE_SCRIPT = r"""
+import sys
+import numpy as np
+import pytest
+sys.path.insert(0, %(root)r)
+from mercer_research_b200 import RCN, Padding, Pooling, RCNLayer, RcnCudaError, convolve_2d_separated
+with pytest.raises(RcnCudaError) as e:
+    RCN(10, [RCNLayer.Convolve2D(Padding.Same), RCNLayer.Pool2D(Pooling.Max)], [30])
+assert e.value.status == 4 and "no CPU fallback" in e.value.message, e.value
+with pytest.raises(RcnCudaError):
+    convolve_2d_separated(np.zeros((5, 5)), 0, Padding.Same)
+print("ok")
+"""
+
+
 def test_no_cpu_fallback_without_gpu(built_library):
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    from mercer_research_b200 import RCN, Padding, Pooling, RCNLayer, RcnCudaError, convolve_2d_separated
-    with pytest.raises(RcnCudaError) as e:
-        RCN(10, [RCNLayer.Convolve2D(Padding.Same), RCNLayer.Pool2D(Pooling.Max)], [30])
-    assert e.value.status == 4 and "no CPU fallback" in e.value.message
-    with pytest.raises(RcnCudaError):
-        convolve_2d_separated(np.zeros((5, 5)), 0, Padding.Same)
+    """Without a usable device the library refuses to compute. Runs in a process whose devices are hidden, so that a GPU
+    machine checks it too."""
+    import subprocess
+    import sys
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    r = subprocess.run([sys.executable, "-c", NO_DEVICE_SCRIPT % {"root": ROOT}], env=env, capture_output=True, text=True,
+                       timeout=300)
+    assert r.returncode == 0 and "ok" in r.stdout, r.stdout + r.stderr
 
 
 def test_argument_validation_needs_no_gpu(built_library):

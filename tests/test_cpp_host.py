@@ -25,15 +25,18 @@ def host_test(built_library):
     return EXE
 
 
-def run(exe, mode):
-    r = subprocess.run([exe, mode], capture_output=True, text=True, timeout=300)
+def run(exe, mode, *args, env=None):
+    r = subprocess.run([exe, mode, *args], capture_output=True, text=True, timeout=300, env=env)
     assert r.returncode == 0 and f"{mode} ok" in r.stdout, r.stdout + r.stderr
+    return r.stdout
 
 
-def test_cpp_host_cpu(host_test):
+def test_cpp_host_cpu(host_test, tmp_path):
     """Reference unit tests that need no compute, the contract violations (reported before any device work, with the
-    reference's panic classes as status codes) and the no-CPU-fallback rule, through the C++ mirror."""
-    run(host_test, "cpu")
+    reference's panic classes as status codes) and the no-CPU-fallback rule, through the C++ mirror. The devices are
+    hidden, so that the no-fallback rule is checked on a GPU machine too."""
+    out = run(host_test, "cpu", str(tmp_path), env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+    assert "a CUDA device is present" not in out, "the devices were not hidden: the no-CPU-fallback check did not run\n" + out
 
 
 @pytest.mark.gpu

@@ -123,7 +123,7 @@ def test_saturated_units_unscaled_init(api):
     assert_close(model.get_params(), want_params, what="params")
 
 
-def test_dmma_matches_simt_kernels(api):
+def test_dmma_matches_simt_kernels(api, tmp_path):
     """The DMMA tensor path and the plain SIMT cross-check kernels must agree to rounding."""
     import subprocess
     import sys
@@ -139,7 +139,7 @@ np.save(sys.argv[1], model.get_params())
 ''' % os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     outs = []
     for impl in ("dmma", "simt"):
-        path = f"/tmp/rcn_gemm_{impl}.npy"
+        path = str(tmp_path / f"rcn_gemm_{impl}.npy")
         env = dict(os.environ, RCN_CUDA_GEMM=impl)
         subprocess.run([sys.executable, "-c", code, path], check=True, env=env)
         outs.append(np.load(path))
