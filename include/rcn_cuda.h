@@ -160,9 +160,8 @@ int rcn_cuda_epoch_run(rcn_cuda_handle h, double eta, size_t n_steps);
  * train_batch(batch, eta) }` (rcn.rs:147-149). The host->device transfer of chunk k+1 overlaps the kernels of chunk k:
  * with PINNED u8 images and a narrow network the copy engine streams the chunks into a device ring ahead of the steps
  * (the first step starts after one chunk; the training kernel waits on an arrival counter in device memory), the steps
- * are replayed as CUDA graphs of up to 40 steps, and the step's result is written straight into pinned host memory
- * (RCN_CUDA_HOST_COPY=pull: SM-issued zero-copy loads on a graph branch instead); otherwise double-buffered
- * cudaMemcpyAsync on a copy stream. Every step's
+ * are replayed as CUDA graphs of up to 40 steps, and the step's result is written straight into pinned host memory;
+ * otherwise double-buffered cudaMemcpyAsync on a copy stream. Every step's
  * result -- quadratic cost and rcn.rs:153-157 hit count under the pre-update parameters -- lands in cost_out / hits_out
  * (n_samples / B entries each, may be NULL). global_batch = 0 means B x (data-parallel world).
  * In a connected data-parallel group every rank calls this with its own shard of each global minibatch. */

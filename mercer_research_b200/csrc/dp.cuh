@@ -115,19 +115,6 @@ __device__ __forceinline__ double dp_receive_sum(const DpPush& dp, size_t par_of
     return s;
 }
 
-// The last CTA (of `total`) to finish an exchange publishes the step counter; call from ONE thread per CTA after the CTA's
-// receives are done.  `step` is the value dp_push_parity_offset() derived the parity from.
-__device__ __forceinline__ void dp_finish_step(const DpPush& dp, unsigned total_ctas) {
-    DpCtrl* ctrl = reinterpret_cast<DpCtrl*>(dp.peers[dp.rank]);
-    __threadfence();
-    if (atomicAdd(&ctrl->done_ctas, 1u) == total_ctas - 1) {
-        ctrl->done_ctas = 0;
-        const long long step = *reinterpret_cast<volatile long long*>(&ctrl->step) + 1;
-        *reinterpret_cast<volatile long long*>(&ctrl->step) = step;
-        __threadfence();
-    }
-}
-
 // parity offset of the step this rank is about to exchange (reads the device-side step counter of its own block)
 __device__ __forceinline__ size_t dp_push_parity_offset(const DpPush& dp) {
     const long long step = *reinterpret_cast<volatile long long*>(dp.peers[dp.rank]) + 1;

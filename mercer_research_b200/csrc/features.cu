@@ -340,10 +340,12 @@ __global__ void __launch_bounds__(256, 4) conv_same_maps_kernel(const __grid_con
     }
 }
 
-template <int MIN_CTAS>
-__global__ void __launch_bounds__(256, MIN_CTAS) conv_same_final_kernel(const __grid_constant__ Stage st, const int* __restrict__ in,
-                                                             size_t in_stride, double* __restrict__ out, size_t L,
-                                                             const Standardise sc, size_t B, int staged) {
+// 4 CTAs per SM (64 registers).  The 40-register build (6 CTAs per SM) measured slower (351 vs 311 us for the c4 stack): more
+// resident warps do not help a kernel whose stores already cover DRAM's write rate, and the tighter register budget costs
+// instructions.
+__global__ void __launch_bounds__(256, 4) conv_same_final_kernel(const __grid_constant__ Stage st, const int* __restrict__ in,
+                                                      size_t in_stride, double* __restrict__ out, size_t L,
+                                                      const Standardise sc, size_t B, int staged) {
     extern __shared__ __align__(16) int s_map[];
     const int i = blockIdx.x;
     for (size_t img = blockIdx.y; img < B; img += gridDim.y) {
@@ -433,12 +435,7 @@ static int launch_features_t(const FeaturePlan& plan, const TIN* images, size_t 
                                     (reinterpret_cast<uintptr_t>(cin) & 15) == 0) ? 1 : 0;
                 const size_t ssmem = staged ? map_elems * sizeof(int) : 0;
                 if (s == sl.n - 1) {
-                    // RCN_CUDA_CONV_OCC=6: the 40-register build (6 CTAs per SM) instead of the 64-register one (4 per SM).
-                    // Measured SLOWER (351 vs 311 us for the c4 stack): more resident warps do not help a kernel whose
-                    // stores already cover DRAM's write rate, and the tighter register budget costs instructions.
-                    static const bool occ6 = []() { const char* e = getenv("RCN_CUDA_CONV_OCC"); return e && e[0] == '6'; }();
-                    if (occ6) RCN_LAUNCH("conv_same_final_kernel", stream, conv_same_final_kernel<6><<<sgrid, 256, ssmem, stream>>>(st, cin, cur_stride, out, plan.L, sc, B, staged));
-                    else RCN_LAUNCH("conv_same_final_kernel", stream, conv_same_final_kernel<4><<<sgrid, 256, ssmem, stream>>>(st, cin, cur_stride, out, plan.L, sc, B, staged));
+                    RCN_LAUNCH("conv_same_final_kernel", stream, conv_same_final_kernel<<<sgrid, 256, ssmem, stream>>>(st, cin, cur_stride, out, plan.L, sc, B, staged));
                 } else {
                     const size_t out_stride = (size_t)st.n_out * st.h_out * st.w_out;
                     RCN_LAUNCH("conv_same_maps_kernel", stream, conv_same_maps_kernel<<<sgrid, 256, ssmem, stream>>>(st, cin, cur_stride, reinterpret_cast<int*>(nxt), out_stride, B, staged));

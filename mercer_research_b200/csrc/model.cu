@@ -63,45 +63,38 @@ LaunchScope::~LaunchScope() {
 }
 
 // ---- streaming from a pinned HOST dataset (rcn_cuda_train_epoch_host fast path) ---------------------------------------
-// State block in device memory: [0] cursor (samples, advanced by the update), [1] n_steps, [2] host image base,
-// [3] prefetch launches so far, [4] ticket of the running prefetch launch, [5] pad; the step's labels follow.
-// Launch k of the prefetch kernel (its own counter: it runs on a parallel graph branch and must not race with the
-// cursor update at the end of step k) reads chunk k+1 straight from pinned host memory (zero-copy loads over PCIe, 16 B
-// per thread, coalesced) into ring slot (k+1) % 2 while the training kernels of chunk k run on the other branch.
+// State block in device memory: [0] cursor (samples, advanced by the update), [3] images arrived in the ring so far; the
+// other words are padding.  The step's labels follow.
 constexpr int kHsStateSlots = 6;
 // the streamed epoch's cursor never wraps (every call re-initialises the state block), so the captured graphs are independent
 // of the epoch length and serve every later call with the same batch shape
 constexpr long long kHsNoWrap = 1ll << 62;
 // consecutive steps captured into one CUDA graph by rcn_cuda_train_epoch_host (RCN_CUDA_HOST_STEPS_PER_GRAPH overrides)
-// Default: 2 in pull mode (every step joins its prefetch branch anyway), 40 in dma mode -- the steps inside a graph follow each
-// other without the host or the PCIe link in between, while every graph boundary cost 4-5 us (and now and then 27 us) with
-// copies in flight on the link (profiles/r2_e2e_timeline.txt): 24.8 / 23.4 / 22.3 / 21.8 us per step at 5 / 10 / 20 / 40.
-static int hs_steps_per_graph(bool dma) {
+// Default 40: the steps inside a graph follow each other without the host or the PCIe link in between, while every graph
+// boundary cost 4-5 us (and now and then 27 us) with copies in flight on the link (profiles/r2_e2e_timeline.txt): 24.8 / 23.4 /
+// 22.3 / 21.8 us per step at 5 / 10 / 20 / 40.
+static int hs_steps_per_graph() {
     static const int v = []() { const char* e = getenv("RCN_CUDA_HOST_STEPS_PER_GRAPH"); int n = e ? atoi(e) : 0; return n < 1 ? 0 : (n > 64 ? 64 : n); }();
-    return v ? v : (dma ? 40 : 2);
+    return v ? v : 40;
 }
-// How the images of the streamed epoch cross PCIe (RCN_CUDA_HOST_COPY = dma | pull):
-//  dma  (default) the copy engine.  The copy stream walks the dataset with back-to-back cudaMemcpyAsync calls into a ring of
-//       `kHsRingSteps` chunks, an event behind each; a second stream waits for each event and publishes, with an 8-byte copy
-//       from a pinned table, how many images have landed (state[3]).  Kernel A's image-loading lanes wait for their own image on
-//       that counter (wait_arrived), so the compute stream carries nothing but back-to-back graph launches -- no events, no
-//       per-step join.  Once per quarter of the ring the copy stream waits (cuStreamWaitValue64) until the training cursor
-//       (state[0]) has passed the quarter's previous occupants.  Copies ramp 1 ... 2 ... 4 ... 8 chunks: the first step starts
-//       after ONE chunk has crossed the link, later copies run at the link's large-transfer rate.  Measured on a warm link
-//       (profiles/r2_pcie_dma.json): 43.6 GB/s for one 0.8 MB chunk, 48.7 for two, 53.6 for eight, against 38 GB/s for
-//       SM-issued zero-copy loads; and no CTA of the step's kernels shares its SM with a copy kernel.  (Publishing the counter
-//       on the copy stream itself -- cuStreamWriteValue64 or the 8-byte copy -- put ~22 us between consecutive data copies,
-//       which then no longer pipeline: a one-chunk copy took 40 us instead of 18 and the copy stream became the bottleneck.)
-//  pull the prefetch kernel below on a parallel branch of the step's graph (round 1's design; also the fallback when the
-//       driver has no 64-bit stream memory operations or the staged front end is not the one selected).
-static bool hs_dma_env() {
-    static const bool v = []() { const char* e = getenv("RCN_CUDA_HOST_COPY"); return !(e && (e[0] == 'p' || e[0] == 'P')); }();
-    return v;
-}
-constexpr size_t kHsRingSteps = 64;   // dma: chunks the ring holds
-constexpr size_t kHsQuarter = kHsRingSteps / 4;   // dma: granularity of the copy stream's wait for free ring slots
-constexpr size_t kHsMaxCopy = 8;      // dma: chunks per cudaMemcpyAsync once the ramp is over (divides kHsQuarter)
-constexpr int kHsEvents = 64;         // dma: one event behind each copy, reused round robin
+// How the images of the streamed epoch cross PCIe: the copy engine.  The copy stream walks the dataset with back-to-back
+// cudaMemcpyAsync calls into a ring of `kHsRingSteps` chunks, an event behind each; a second stream waits for each event and
+// publishes, with an 8-byte copy from a pinned table, how many images have landed (state[3]).  Kernel A's image-loading lanes
+// wait for their own image on that counter (wait_arrived), so the compute stream carries nothing but back-to-back graph
+// launches -- no events, no per-step join.  Once per quarter of the ring the copy stream waits (cuStreamWaitValue64) until the
+// training cursor (state[0]) has passed the quarter's previous occupants.  Copies ramp 1 ... 2 ... 4 ... 8 chunks: the first
+// step starts after ONE chunk has crossed the link, later copies run at the link's large-transfer rate.  Measured on a warm
+// link (profiles/r2_pcie_dma.json): 43.6 GB/s for one 0.8 MB chunk, 48.7 for two, 53.6 for eight, against 38 GB/s for
+// SM-issued zero-copy loads; and no CTA of the step's kernels shares its SM with a copy kernel.  (Publishing the counter on
+// the copy stream itself -- cuStreamWriteValue64 or the 8-byte copy -- put ~22 us between consecutive data copies, which then
+// no longer pipeline: a one-chunk copy took 40 us instead of 18 and the copy stream became the bottleneck.)  Round 1's
+// design -- a prefetch kernel pulling each chunk with zero-copy loads on a parallel graph branch -- measured slower end to
+// end (42.8-43.9 M against 48.5-49.5 M images/s) and was removed; without stream memory operations or the staged front end
+// the call takes the general double-buffered loop.
+constexpr size_t kHsRingSteps = 64;   // chunks the ring holds
+constexpr size_t kHsQuarter = kHsRingSteps / 4;   // granularity of the copy stream's wait for free ring slots
+constexpr size_t kHsMaxCopy = 8;      // chunks per cudaMemcpyAsync once the ramp is over (divides kHsQuarter)
+constexpr int kHsEvents = 64;         // one event behind each copy, reused round robin
 struct StreamMemOps {
     CUresult (*wait64)(CUstream, CUdeviceptr, cuuint64_t, unsigned int) = nullptr;
 
@@ -125,59 +118,6 @@ static const StreamMemOps& stream_mem_ops(int device) {
     }();
     return ops;
 }
-// PCIe pulls are latency-bound per request: every thread first issues ALL the 16-byte loads of its round (U independent
-// zero-copy reads in flight, the whole 0.8 MB chunk of the canonical config in one round trip) and only then stores them.
-// (Written as `d4[i] = s4[i]` the compiler must keep load/store pairs in order -- source and ring may alias as far as it
-// knows -- which leaves ONE load in flight per thread and costs a PCIe round trip per 128 KB.)
-template <int U>
-__global__ void __launch_bounds__(256) host_prefetch_kernel(long long* __restrict__ state, unsigned char* __restrict__ ring,
-                                                            long long B, long long img_bytes) {
-    const long long k1 = *reinterpret_cast<volatile long long*>(state + 3) + 1;
-    if (k1 < state[1]) {
-        const unsigned char* src = reinterpret_cast<const unsigned char*>(state[2]) + k1 * B * img_bytes;
-        unsigned char* dst = ring + ((k1 * B) % (2 * B)) * img_bytes;
-        const long long n16 = B * img_bytes / 16;
-        const uint4* s4 = reinterpret_cast<const uint4*>(src);
-        uint4* d4 = reinterpret_cast<uint4*>(dst);
-        const long long stride = (long long)gridDim.x * blockDim.x;
-        for (long long base = blockIdx.x * (long long)blockDim.x + threadIdx.x; base < n16; base += stride * U) {
-            uint4 v[U];
-#pragma unroll
-            for (int u = 0; u < U; ++u)
-                if (base + u * stride < n16) v[u] = s4[base + u * stride];
-#pragma unroll
-            for (int u = 0; u < U; ++u)
-                if (base + u * stride < n16) d4[base + u * stride] = v[u];
-        }
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {   // the last CTA to finish publishes the counter: every CTA has read it by then
-        __threadfence();
-        if (atomicAdd(reinterpret_cast<unsigned long long*>(state + 4), 1ull) == gridDim.x - 1) {
-            state[4] = 0;
-            *reinterpret_cast<volatile long long*>(state + 3) = k1;
-        }
-    }
-}
-// RCN_CUDA_PREFETCH_UNROLL = loads in flight per thread (1 = the load/store-paired loop, default 8);
-// RCN_CUDA_PREFETCH_CTAS = grid size (default 32: the SMs the 128-CTA step kernels leave free, and then some)
-static int prefetch_unroll() {
-    static const int v = []() { const char* e = getenv("RCN_CUDA_PREFETCH_UNROLL"); int n = e ? atoi(e) : 8; return n <= 1 ? 1 : (n <= 4 ? 4 : 8); }();
-    return v;
-}
-static int prefetch_ctas() {
-    static const int v = []() { const char* e = getenv("RCN_CUDA_PREFETCH_CTAS"); int n = e ? atoi(e) : 32; return n < 1 ? 1 : (n > 1024 ? 1024 : n); }();
-    return v;
-}
-static void launch_host_prefetch(long long* state, unsigned char* ring, long long B, long long img_bytes, cudaStream_t s) {
-    const int g = prefetch_ctas();
-    switch (prefetch_unroll()) {
-        case 1: host_prefetch_kernel<1><<<g, 256, 0, s>>>(state, ring, B, img_bytes); break;
-        case 4: host_prefetch_kernel<4><<<g, 256, 0, s>>>(state, ring, B, img_bytes); break;
-        default: host_prefetch_kernel<8><<<g, 256, 0, s>>>(state, ring, B, img_bytes); break;
-    }
-}
-
 bool is_pinned_host_ptr(const void* p) {
     cudaPointerAttributes a;
     if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
@@ -243,14 +183,14 @@ struct rcn_cuda_model {
     DevBuf host_slot[2];
     double* stats_host = nullptr;   // pinned, 2 doubles per step
     size_t stats_host_cap = 0;
-    // streaming variant: the GPU pulls chunk k+1 from pinned host memory while it trains on chunk k; one graph per step
+    // streaming variant: the copy engine fills a device ring from pinned host memory while the GPU trains on earlier chunks
     DevBuf hs_ring, hs_state;
-    cudaStream_t flag_stream = nullptr;     // dma mode: publishes the arrival counter behind each copy
+    cudaStream_t flag_stream = nullptr;     // publishes the arrival counter behind each copy
     cudaEvent_t hs_ev[kHsEvents] = {};
-    long long* hs_counts = nullptr;         // pinned: "images arrived" value behind each copy of the streamed epoch (dma mode)
+    long long* hs_counts = nullptr;         // pinned: "images arrived" value behind each copy of the streamed epoch
     size_t hs_counts_cap = 0;
     std::map<int, cudaGraphExec_t> hs_graphs;   // streamed epoch: g consecutive steps per graph, captured on first use
-    cudaEvent_t hs_fork = nullptr, hs_join = nullptr;
+    cudaEvent_t hs_fork = nullptr;
     struct HsKey {
         size_t B = 0, H = 0, W = 0, n_steps = 0;
         unsigned long long alloc_gen = 0;   // no device buffer has moved since the capture (common.cuh)
@@ -390,9 +330,9 @@ int accumulate_dev(rcn_cuda_model* h, const double* feats, const double* onehot,
                                          labels, h->acts.as<double>(), h->deltas.as<double>(), h->grads,
                                          h->small.as<double>(), h->gemm_ws, front, h->stream, fuse_push ? &push : nullptr,
                                          ((upd.params || upd.cursor) && (!h->dp.connected || fuse_push)) ? &upd : nullptr));
-        h->upd_fused = upd.params && (!h->dp.connected || fuse_push);
+        h->upd_fused = upd.params != nullptr;   // (armed on one GPU only)
         h->cursor_fused = upd.cursor && (!h->dp.connected || fuse_push);
-        h->dp_pushed = fuse_push && !h->upd_fused;   // pushed but not yet received: the exchange kernel must follow
+        h->dp_pushed = fuse_push;   // pushed but not yet received: the exchange kernel must follow
         h->stats_valid = true;
         h->last_B = B;
         return RCN_OK;
@@ -417,16 +357,6 @@ int accumulate_dev(rcn_cuda_model* h, const double* feats, const double* onehot,
 // images (DEVICE) -> gradient sums.  The canonical narrow network with u8 pixels runs the convpool stack inside
 // kernel A (smallnet.cu); everything else runs the feature kernel(s) first.  `bi` (optional) is the epoch-mode
 // device-side batch selection; without it `labels` are this batch's labels.
-// How far the single-GPU prewait goes (kernel A's front end ahead of griddepcontrol.wait, under the previous kernel B's tail;
-// RCN_CUDA_PREWAIT): 0 = nowhere, 1 = in the streamed host epoch only (default), 2 = in every training step.  Measured: the host
-// epoch gains 3-6 % (the arrival-counter wait and the ring loads move under kernel B); the device-resident step does not (kernel
-// A needs a whole SM's registers, so all but ~26 of its CTAs start only when kernel B's CTAs leave, and its parameter loads are
-// no longer hidden behind the front end).
-static int prewait_mode() {
-    static const int v = []() { const char* e = getenv("RCN_CUDA_PREWAIT"); return e ? atoi(e) : 1; }();
-    return v;
-}
-
 static bool fused_front_enabled() {
     static const bool v = []() { const char* e = getenv("RCN_CUDA_FUSED_FRONT"); return !(e && e[0] == '0'); }();
     return v;
@@ -448,17 +378,20 @@ int accumulate_images_dev(rcn_cuda_model* h, const void* images, int fmt, const 
         smallnet_front_select(h->plan, &fr);
         // Data-parallel step behind the exchange kernel: kernel A may run its front end ahead of griddepcontrol.wait
         // (smallnet.cu) when this step's kernel B pushes to the peers (so the exchange kernel X precedes the next kernel
-        // A), the update is not folded into kernel B, and any device-side cursor it reads is advanced by kernel B -- this
-        // step's and the previous one's (x_owns_cursor) -- not by X, which may still be running then.
+        // A) and any device-side cursor it reads is advanced by kernel B -- this step's and the previous one's
+        // (x_owns_cursor) -- not by X, which may still be running then.
         static const bool prewait_env = []() { const char* e = getenv("RCN_CUDA_DP_PREWAIT"); return !(e && e[0] == '0'); }();
         const bool fuse_push = h->dp.connected && dp_fused_push_enabled() && !h->dp_push_suppress;
-        fr.prewait = (prewait_env && fr.use_cp && fuse_push && !h->pending_upd.params && !h->x_owns_cursor &&
+        fr.prewait = (prewait_env && fr.use_cp && fuse_push && !h->x_owns_cursor &&
                       (!fr.bi.cursor || h->pending_upd.cursor == fr.bi.cursor)) ? 1 : 0;
-        // One GPU: the same front end under the tail of the previous step's kernel B (which triggers its dependents early).
-        // Safe whatever precedes this launch: a kernel that does not trigger early has completed before kernel A starts; kernel B
-        // advances a device-side cursor before it triggers, and the only buffer both touch -- the features -- is written by
-        // this kernel A after its wait.
-        if (!h->dp.connected && fr.use_cp && (prewait_mode() == 2 || (prewait_mode() == 1 && fr.bi.window != 0))) fr.prewait = 2;
+        // One GPU, streamed host epoch: the same front end under the tail of the previous step's kernel B (which triggers its
+        // dependents early).  Safe whatever precedes this launch: a kernel that does not trigger early has completed before
+        // kernel A starts; kernel B advances a device-side cursor before it triggers, and the only buffer both touch -- the
+        // features -- is written by this kernel A after its wait.  Measured: the host epoch gains 3-6 % (the arrival-counter
+        // wait and the ring loads move under kernel B).  Prewaiting nowhere, or in every training step, measured slower and
+        // was removed: in the device-resident step kernel A needs a whole SM's registers, so all but ~26 of its CTAs start
+        // only when kernel B's CTAs leave, and its parameter loads are no longer hidden behind the front end.
+        if (!h->dp.connected && fr.use_cp && fr.bi.window != 0) fr.prewait = 2;
         if (smallnet_front_fits(h->small_desc, fr))
             return accumulate_dev(h, h->feats.as<double>(), nullptr, step_labels, B, &fr);
     }
@@ -547,7 +480,6 @@ int rcn_cuda_destroy(rcn_cuda_handle h) {
     if (h->stats_host) cudaFreeHost(h->stats_host);
     for (auto& kv : h->hs_graphs) cudaGraphExecDestroy(kv.second);
     if (h->hs_fork) cudaEventDestroy(h->hs_fork);
-    if (h->hs_join) cudaEventDestroy(h->hs_join);
 
     h->hs_ring.release(); h->hs_state.release();
     if (h->hs_counts) cudaFreeHost(h->hs_counts);
@@ -930,19 +862,17 @@ static void arm_fused_update(rcn_cuda_model* h, double scale, long long* cursor,
     static const bool on = []() { const char* e = getenv("RCN_CUDA_FUSED_UPDATE"); return !(e && e[0] == '0'); }();
     h->pending_upd = SnUpdate{};
     if (!on || !h || !h->params_ready || !h->use_small) return;
-    // Data-parallel groups: receiving inside the weight-gradient kernel (MODE 3) was measured SLOWER than the separate
-    // exchange kernel (2 GPUs, c2: 30.8 vs 28.4 us/step) -- the NVLink round trip is then exposed inside the kernel
-    // instead of overlapping the next launch -- so it is opt-in (RCN_CUDA_DP_FUSED_UPDATE=1).  By default kernel B only
-    // takes over the cursor / result ring there (params stays null) and the exchange kernel applies the update.
-    static const bool dp_on = []() { const char* e = getenv("RCN_CUDA_DP_FUSED_UPDATE"); return e && e[0] == '1'; }();
+    // Data-parallel groups: kernel B only takes over the cursor / result ring (params stays null) and the exchange kernel
+    // applies the update.  (Receiving inside kernel B as well was measured slower, 2 GPUs, c2: 30.8 vs 28.4 us/step -- the
+    // NVLink round trip is then exposed inside the kernel instead of overlapping the next launch -- and was removed.)
     if (h->dp.connected && (!dp_fused_push_enabled() || h->dp_push_suppress)) return;
-    if (!h->dp.connected || dp_on) h->pending_upd.params = h->params.as<double>();
+    if (!h->dp.connected) h->pending_upd.params = h->params.as<double>();
     h->pending_upd.scale = scale;
     h->pending_upd.cursor = cursor;
     h->pending_upd.batch = batch;
     h->pending_upd.n_samples = n_samples;
     h->pending_upd.stats_ring = stats_ring;
-    h->pending_upd.early_cursor = (!h->dp.connected && (prewait_mode() == 2 || (prewait_mode() == 1 && streamed))) ? 1 : 0;
+    h->pending_upd.early_cursor = (!h->dp.connected && streamed) ? 1 : 0;   // kernel A of the streamed epoch prewaits
 }
 // What the accumulate did with the armed update: bit 0 = parameters updated, bit 1 = cursor advanced / result ring written.
 static int take_upd_fused(rcn_cuda_model* h) {
@@ -1113,7 +1043,6 @@ int rcn_cuda_train_epoch_host(rcn_cuda_handle h, const void* images, int pixel_f
             RCN_CUDA_TRY(cudaEventCreateWithFlags(&h->ev_consumed[i], cudaEventDisableTiming));
         }
         RCN_CUDA_TRY(cudaEventCreateWithFlags(&h->hs_fork, cudaEventDisableTiming));
-        RCN_CUDA_TRY(cudaEventCreateWithFlags(&h->hs_join, cudaEventDisableTiming));
     }
     if (h->stats_host_cap < n_steps) {
         if (h->stats_host) cudaFreeHost(h->stats_host);
@@ -1121,17 +1050,22 @@ int rcn_cuda_train_epoch_host(rcn_cuda_handle h, const void* images, int pixel_f
         RCN_CUDA_TRY(cudaHostAlloc((void**)&h->stats_host, n_steps * 2 * sizeof(double), cudaHostAllocDefault));
         h->stats_host_cap = n_steps;
     }
-    // ---- streaming fast path: pinned u8 dataset + fused small-network kernels: the GPU pulls chunk k+1 over PCIe itself
-    // (zero-copy loads) while chunk k trains; per-step results are written straight into pinned host memory; the host
-    // launches ONE CUDA graph per step and nothing else.
+    // ---- streaming fast path: pinned u8 dataset + fused small-network kernels: the copy engine streams the images into a
+    // device ring while earlier chunks train; per-step results are written straight into pinned host memory; the host
+    // launches CUDA graphs of several steps each and queues the copies.  It needs the staged front end (its image-loading
+    // lanes wait for the arrival counter) and 64-bit stream memory operations (the copy stream's wait for free ring slots).
     static const bool stream_env = []() { const char* e = getenv("RCN_CUDA_HOST_STREAMING"); return !(e && e[0] == '0'); }();
     if (stream_env && pixel_format == RCN_PIXELS_U8_ROWMAJOR && h->use_small && B <= smallnet_max_batch() && img_bytes % 16 == 0 &&
-        (reinterpret_cast<uintptr_t>(images) & 15) == 0 && is_pinned_host_ptr(images) && h->plan.L > 0 && h->plan.n_conv <= 10) {
+        (reinterpret_cast<uintptr_t>(images) & 15) == 0 && is_pinned_host_ptr(images) && h->plan.L > 0 && h->plan.n_conv <= 10 &&
+        fused_front_enabled() && kHsRingSteps * B < (1ull << 31) && stream_mem_ops(h->device).ok) {
         SmallNetFront probe{};
         probe.H = (int)H; probe.W = (int)W; probe.max_elems = (int)h->plan.max_elems; probe.stages = h->plan.stages;
         cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
         RCN_CUDA_TRY(cudaStreamIsCapturing(h->stream, &cs));
-        if (smallnet_front_fits(h->small_desc, probe) && cs == cudaStreamCaptureStatusNone) {
+        const bool fits = smallnet_front_fits(h->small_desc, probe);
+        probe.images = static_cast<const uint8_t*>(images);   // 16-byte aligned, as the ring the steps will read is
+        smallnet_front_select(h->plan, &probe);
+        if (fits && probe.use_cp && cs == cudaStreamCaptureStatusNone) {
             // The legacy default stream cannot be captured: run the loop on the model's own stream, ordered after whatever
             // the caller has enqueued on the legacy stream; the call drains that stream before it returns.
             struct StreamSwap {
@@ -1145,16 +1079,8 @@ int rcn_cuda_train_epoch_host(rcn_cuda_handle h, const void* images, int pixel_f
                 h->stream = h->own_stream;
             }
             RCN_TRY(h->hs_ring.reserve(kHsRingSteps * img_bytes));
-            // copy-engine mode needs the staged front end (its image-loading lanes do the waiting) and stream memory operations
-            bool dma = hs_dma_env() && fused_front_enabled() && kHsRingSteps * B < (1ull << 31) && stream_mem_ops(h->device).ok;
-            if (dma) {
-                probe.images = h->hs_ring.as<uint8_t>();
-                smallnet_front_select(h->plan, &probe);
-                dma = probe.use_cp != 0;
-            }
-            const size_t spg = (size_t)hs_steps_per_graph(dma);
-            const size_t ring_steps = dma ? kHsRingSteps : 2;
-            // The epoch as a sequence of graph launches: as many `spg`-step graphs as fit, then (dma) the largest of 20 / 10 / 5 / 2 /
+            const size_t spg = (size_t)hs_steps_per_graph();
+            // The epoch as a sequence of graph launches: as many `spg`-step graphs as fit, then the largest of 20 / 10 / 5 / 2 /
             // 1 steps that still fits -- as few launches as possible: with copies on the link a graph boundary costs 4-5 us and
             // now and then 27 us (a short FIRST graph to get going sooner measured worse for that reason: 507-519 us against 479
             // for a 20-step epoch; its launch latency passes while the first chunk crosses the link anyway).
@@ -1162,7 +1088,7 @@ int rcn_cuda_train_epoch_host(rcn_cuda_handle h, const void* images, int pixel_f
             for (size_t left = n_steps; left;) {
                 size_t g = 1;
                 if (left >= spg) g = spg;
-                else if (dma)
+                else
                     for (size_t c : {(size_t)20, (size_t)10, (size_t)5, (size_t)2})
                         if (c < spg && left >= c) { g = c; break; }
                 plan_g.push_back((int)g);
@@ -1177,13 +1103,12 @@ int rcn_cuda_train_epoch_host(rcn_cuda_handle h, const void* images, int pixel_f
             bi.cursor = st;
             bi.labels_all = h->tgt_stage.as<long long>();
             bi.labels_batch = st + kHsStateSlots;
-            bi.window = (long long)(ring_steps * B);
-            bi.arrived = dma ? st + 3 : nullptr;
-            // state, labels of the whole epoch (and, pull mode, chunk 0) go up with plain copies; after that graph replays
-            const long long init[kHsStateSlots] = {0, (long long)n_steps, (long long)reinterpret_cast<uintptr_t>(images), 0, 0, 0};
+            bi.window = (long long)(kHsRingSteps * B);
+            bi.arrived = st + 3;
+            // cursor and arrival counter start at zero, the labels of the whole epoch go up in one copy; after that graph replays
+            const long long init[kHsStateSlots] = {};
             RCN_CUDA_TRY(cudaMemcpyAsync(st, init, sizeof(init), cudaMemcpyHostToDevice, h->stream));
             RCN_CUDA_TRY(cudaMemcpyAsync(h->tgt_stage.p, labels, n_steps * B * sizeof(int64_t), cudaMemcpyHostToDevice, h->stream));
-            if (!dma) RCN_CUDA_TRY(cudaMemcpyAsync(h->hs_ring.p, images, img_bytes, cudaMemcpyHostToDevice, h->stream));
             rcn_cuda_model::HsKey key;
             key.B = B; key.H = H; key.W = W; key.n_steps = 0; key.scale = scale_s;   // the graphs do not depend on the epoch length
             key.labels = h->tgt_stage.p;   // (grows with the epoch length: a longer epoch than any before re-captures)
@@ -1192,7 +1117,7 @@ int rcn_cuda_train_epoch_host(rcn_cuda_handle h, const void* images, int pixel_f
             memcpy(&key.sd_bits, &h->sd, sizeof(double));
             key.stats = h->stats_host; key.ring = h->hs_ring.p; key.state = st; key.grads = h->grads; key.stream = h->stream;
             key.dp = h->dp.connected;
-            key.window = dma ? -bi.window : bi.window;   // (sign: the pull graphs carry the prefetch branch, the dma graphs do not)
+            key.window = bi.window;
             if (h->hs_graphs.empty() || !(key == h->hs_key)) {
                 for (auto& kv : h->hs_graphs) cudaGraphExecDestroy(kv.second);
                 h->hs_graphs.clear();
@@ -1215,24 +1140,11 @@ int rcn_cuda_train_epoch_host(rcn_cuda_handle h, const void* images, int pixel_f
                     RCN_CUDA_TRY(cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal));
                     int rc = RCN_OK;
                     for (int q = 0; q < g && rc == RCN_OK; ++q) {
-                        if (!dma) {
-                        if (cudaEventRecord(h->hs_fork, h->stream) != cudaSuccess || cudaStreamWaitEvent(h->copy_stream, h->hs_fork, 0) != cudaSuccess) { rc = fail(RCN_ERR_CUDA, "graph fork failed"); break; }
-                        {
-                            LaunchScope ls("host_prefetch_kernel", h->copy_stream);
-                            launch_host_prefetch(st, h->hs_ring.as<unsigned char>(), (long long)B, (long long)(H * W), h->copy_stream);
-                        }
-                        if (cudaPeekAtLastError() != cudaSuccess) { rc = fail(RCN_ERR_CUDA, "prefetch kernel launch failed: %s", cudaGetErrorString(cudaGetLastError())); break; }
-                        if (cudaEventRecord(h->hs_join, h->copy_stream) != cudaSuccess) { rc = fail(RCN_ERR_CUDA, "graph join failed"); break; }
-                        }
                         arm_fused_update(h, scale_s, st, (long long)B, kHsNoWrap, h->stats_host, true);
                         rc = accumulate_images_dev(h, h->hs_ring.p, pixel_format, nullptr, B, H, W, &bi);
                         const int fused = take_upd_fused(h);
                         if (rc != RCN_OK) break;
-                        if (fused & 1) {   // the weight-gradient kernel applied the update, advanced the cursor, wrote the result
-                            // the prefetch branch joins at the end of its step: the next step starts after both
-                            if (!dma && cudaStreamWaitEvent(h->stream, h->hs_join, 0) != cudaSuccess) { rc = fail(RCN_ERR_CUDA, "graph join failed"); break; }
-                            continue;
-                        }
+                        if (fused & 1) continue;   // the weight-gradient kernel applied the update, advanced the cursor, wrote the result
                         // (fused & 2: kernel B advanced the cursor and wrote the result; the update kernel gets no cursor)
                         long long* cur = (fused & 2) ? nullptr : st;
                         if (h->dp.connected) {
@@ -1243,11 +1155,6 @@ int rcn_cuda_train_epoch_host(rcn_cuda_handle h, const void* images, int pixel_f
                             rc = launch_sgd_update(h->params.as<double>(), h->grads, h->n_params, scale_s, h->stream, cur, (long long)B,
                                                    kHsNoWrap, h->small.as<double>(), h->stats_host);
                         }
-                        if (rc != RCN_OK) break;
-                        // the prefetch branch joins AFTER the exchange / update kernel was enqueued: the next step's kernel A
-                        // then directly follows that kernel in the stream (its programmatic dependent) and also waits for
-                        // the prefetched chunk
-                        if (!dma && cudaStreamWaitEvent(h->stream, h->hs_join, 0) != cudaSuccess) { rc = fail(RCN_ERR_CUDA, "graph join failed"); break; }
                     }
                     cudaError_t ce = cudaStreamEndCapture(h->stream, &graph);
                     if (rc != RCN_OK) { if (graph) cudaGraphDestroy(graph); cudaGetLastError(); return rc; }
@@ -1264,9 +1171,7 @@ int rcn_cuda_train_epoch_host(rcn_cuda_handle h, const void* images, int pixel_f
                     h->hs_graphs[g] = ge;
                 }
             }
-            if (!dma) {
-                for (int g : plan_g) RCN_CUDA_TRY(cudaGraphLaunch(h->hs_graphs[g], h->stream));
-            } else {
+            {
                 // Copies first (the driver queues them; each waits on the device for its ring slots), then the graph launches.
                 const StreamMemOps& mo = stream_mem_ops(h->device);
                 const CUdeviceptr cursor_dev = (CUdeviceptr)reinterpret_cast<uintptr_t>(st);
@@ -1291,12 +1196,12 @@ int rcn_cuda_train_epoch_host(rcn_cuda_handle h, const void* images, int pixel_f
                     size_t g = a < 2 ? 1 : (a < 16 ? 2 : (a < 32 ? 4 : kHsMaxCopy));
                     g = std::min(g, n_steps - a);
                     g = std::min(g, kHsQuarter - a % kHsQuarter);                      // never across a quarter of the ring
-                    if (a >= ring_steps && a % kHsQuarter == 0) {
+                    if (a >= kHsRingSteps && a % kHsQuarter == 0) {
                         // entering a quarter whose slots held steps [a - ring, a + quarter - ring): all of them must have trained
-                        if (mo.wait64(h->copy_stream, cursor_dev, (cuuint64_t)((a + kHsQuarter - ring_steps) * B), CU_STREAM_WAIT_VALUE_GEQ) != CUDA_SUCCESS)
+                        if (mo.wait64(h->copy_stream, cursor_dev, (cuuint64_t)((a + kHsQuarter - kHsRingSteps) * B), CU_STREAM_WAIT_VALUE_GEQ) != CUDA_SUCCESS)
                             return fail(RCN_ERR_CUDA, "cuStreamWaitValue64 failed");
                     }
-                    RCN_CUDA_TRY(cudaMemcpyAsync(h->hs_ring.as<char>() + (a % ring_steps) * img_bytes, src + a * img_bytes, g * img_bytes,
+                    RCN_CUDA_TRY(cudaMemcpyAsync(h->hs_ring.as<char>() + (a % kHsRingSteps) * img_bytes, src + a * img_bytes, g * img_bytes,
                                                  cudaMemcpyHostToDevice, h->copy_stream));
                     a += g;
                     h->hs_counts[n_copy] = (long long)(a * B);
@@ -1315,11 +1220,11 @@ int rcn_cuda_train_epoch_host(rcn_cuda_handle h, const void* images, int pixel_f
                 for (int g : plan_g) {
                     RCN_CUDA_TRY(cudaGraphLaunch(h->hs_graphs[g], h->stream));
                     k += (size_t)g;
-                    while (a < n_steps && a < k + ring_steps / 2) RCN_TRY(enqueue_copy());
+                    while (a < n_steps && a < k + kHsRingSteps / 2) RCN_TRY(enqueue_copy());
                 }
             }
-            // (pull: prefetch +) A + B (+ exchange/update) per replayed step
-            g_launches.fetch_add((unsigned long long)n_steps * ((dma ? 2 : 3) + (h->dp.connected ? 1 : 0)), std::memory_order_relaxed);
+            // A + B (+ exchange/update) per replayed step
+            g_launches.fetch_add((unsigned long long)n_steps * (2 + (h->dp.connected ? 1 : 0)), std::memory_order_relaxed);
             RCN_CUDA_TRY(cudaStreamSynchronize(h->stream));
             stream_drained(h);
             for (size_t k = 0; k < n_steps; ++k) {

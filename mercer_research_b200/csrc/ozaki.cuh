@@ -125,27 +125,6 @@ __device__ __forceinline__ void tma_load_3d(void* smem_dst, const CUtensorMap* m
         "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
         ::"r"(smem_u32(smem_dst)), "l"(map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2) : "memory");
 }
-// Multicast variant: the box lands at the same CTA-relative offset in every CTA of `cta_mask`, and so does the
-// complete_tx on the mbarrier at the same CTA-relative offset.
-__device__ __forceinline__ void tma_load_3d_mc(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2,
-                                               uint16_t cta_mask) {
-    asm volatile(
-        "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%4, %5, %6}], [%2], %3;"
-        ::"r"(smem_u32(smem_dst)), "l"(map), "r"(smem_u32(bar)), "h"(cta_mask), "r"(c0), "r"(c1), "r"(c2) : "memory");
-}
-// Arrives (once the issuing thread's earlier MMAs have completed) on the mbarrier at this offset in every CTA of the mask.
-__device__ __forceinline__ void tc_commit_mc(uint64_t* bar, uint16_t cta_mask) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-                 ::"r"(smem_u32(bar)), "h"(cta_mask) : "memory");
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
 __device__ __forceinline__ void tma_load_5d(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2, int c3,
                                             int c4) {
     asm volatile(
@@ -193,10 +172,9 @@ __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.
 }  // namespace oz
 
 // C(m, n) = sum_k A(m, k) B(n, k), delivered to epi(m, n, value).  Tile (blockIdx.x, blockIdx.y) = (m-tile, n-tile).
-// CLUSTER == 2: the two CTAs of a cluster own the SAME m-tile and neighbouring n-tiles; each loads half of the A slice
-// rows and TMA-multicasts it into both CTAs' shared memory (A traffic from L2 halves; the kernel is L2 -> SM bound),
-// and a stage is released only when BOTH CTAs' MMAs have consumed it (multicast tcgen05.commit, empty count 2).
-template <typename Epi, int CLUSTER>
+// (2-CTA clusters that TMA-multicast halves of the A slice into both CTAs were measured neutral -- the kernel is bound by
+// shared memory, not by L2 -> SM traffic -- and were removed.)
+template <typename Epi>
 __global__ void __launch_bounds__(OZ_THREADS, 1) ozaki_gemm_kernel(const __grid_constant__ CUtensorMap map_a,
                                                                     const __grid_constant__ CUtensorMap map_b,
                                                                     const double* __restrict__ scale_a,
@@ -211,25 +189,22 @@ __global__ void __launch_bounds__(OZ_THREADS, 1) ozaki_gemm_kernel(const __grid_
     uint32_t* tmem_base_slot = reinterpret_cast<uint32_t*>(tmem_full_bar + 1);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    // rasterisation: groups of 8 m-tiles sweep all n-tiles, so concurrently resident CTAs share operand tiles in L2;
-    // with CLUSTER == 2 the unit is a PAIR of n-tiles (n_tiles is the padded, even count)
-    const uint32_t crank = CLUSTER > 1 ? oz::cluster_ctarank() : 0;
-    const int tile = blockIdx.x / CLUSTER;
-    const int n_units = n_tiles / CLUSTER;
-    const int group = 8 * n_units;
+    // rasterisation: groups of 8 m-tiles sweep all n-tiles, so concurrently resident CTAs share operand tiles in L2
+    const int tile = blockIdx.x;
+    const int group = 8 * n_tiles;
     const int g = tile / group;
     const int g_m0 = g * 8;
     const int g_rows = min(8, m_tiles - g_m0);
     const int in_g = tile - g * group;
     const int m_tile = g_m0 + in_g % g_rows;
-    const int n_tile = (in_g / g_rows) * CLUSTER + (int)crank;
+    const int n_tile = in_g / g_rows;
     const int m0 = m_tile * OZ_BM, n0 = n_tile * OZ_BN;
     // split-K: blockIdx.y owns k-blocks [kb0, kb0 + n_kb); the epilogue functor sees blockIdx.y and stores a partial
     const int kb0 = blockIdx.y * kb_per_split;
     const int n_kb = min(Kp / OZ_BK - kb0, kb_per_split);
 
     if (threadIdx.x == 0) {
-        for (int s = 0; s < OZ_STAGES; ++s) { oz::mbar_init(full_bar + s, 1); oz::mbar_init(empty_bar + s, CLUSTER); }
+        for (int s = 0; s < OZ_STAGES; ++s) { oz::mbar_init(full_bar + s, 1); oz::mbar_init(empty_bar + s, 1); }
         oz::mbar_init(tmem_full_bar, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
@@ -239,7 +214,6 @@ __global__ void __launch_bounds__(OZ_THREADS, 1) ozaki_gemm_kernel(const __grid_
     }
     oz::tc_fence_before();
     __syncthreads();
-    if (CLUSTER > 1) oz::cluster_sync_all();      // the peer's barriers exist before anything is multicast at them
     oz::tc_fence_after();
     const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(tmem_base_slot);
 
@@ -255,13 +229,7 @@ __global__ void __launch_bounds__(OZ_THREADS, 1) ozaki_gemm_kernel(const __grid_
                 oz::mbar_expect_tx(full_bar + stage, OZ_STAGE_BYTES);
                 unsigned char* sa = smem + stage * OZ_STAGE_BYTES;
                 unsigned char* sb = sa + OZ_S * OZ_A_TILE;
-                if (CLUSTER > 1) {
-                    constexpr int HALF = OZ_BM / 2;          // my half of the A rows, delivered to both CTAs
-#pragma unroll
-                    for (int s = 0; s < OZ_S; ++s)
-                        oz::tma_load_3d_mc(sa + s * OZ_A_TILE + crank * (HALF * OZ_BK), &map_a, full_bar + stage, (kb0 + kb) * OZ_BK,
-                                           m0 + (int)crank * HALF, s, (uint16_t)0x3);
-                } else if (conv.enabled) {
+                if (conv.enabled) {
                     // k-block -> (tap, channel block); tile -> (image, first row, first column) of its pixel patch
                     const int kk = (kb0 + kb) * OZ_BK;
                     const int tap = kk / conv.C, c0 = kk - tap * conv.C;
@@ -303,9 +271,7 @@ __global__ void __launch_bounds__(OZ_THREADS, 1) ozaki_gemm_kernel(const __grid_
                         }
                     }
                 }
-                // frees the smem slot once these MMAs have read it -- in BOTH CTAs when the A halves are multicast
-                if (CLUSTER > 1) oz::tc_commit_mc(empty_bar + stage, (uint16_t)0x3);
-                else oz::tc_commit(empty_bar + stage);
+                oz::tc_commit(empty_bar + stage);   // frees the smem slot once these MMAs have read it
             }
             oz::tc_commit(tmem_full_bar);               // accumulators complete
         }
@@ -348,7 +314,6 @@ __global__ void __launch_bounds__(OZ_THREADS, 1) ozaki_gemm_kernel(const __grid_
         oz::tc_fence_before();
     }
     __syncthreads();
-    if (CLUSTER > 1) oz::cluster_sync_all();      // nobody leaves while the peer may still multicast into this CTA
     if (warp == 1) {
         oz::tc_fence_after();
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(OZ_TMEM_COLS) : "memory");
@@ -390,38 +355,16 @@ static int launch_gemm_ozaki(const char* name, const OzOperand& A, const OzOpera
     RCN_TRY(ws.b_scale.reserve((size_t)2 * N * sizeof(double)));
     RCN_TRY(ozaki_slice(A, M, K, Kp, ws.a_slices.as<int8_t>(), ws.a_scale.as<double>(), ws.a_scale.as<double>() + M, stream));
     RCN_TRY(ozaki_slice(B, N, K, Kp, ws.b_slices.as<int8_t>(), ws.b_scale.as<double>(), ws.b_scale.as<double>() + N, stream));
-    static const int cluster = []() { const char* e = getenv("RCN_CUDA_TC_CLUSTER"); return (e && e[0] == '2') ? 2 : 1; }();   // 2 = A halves multicast across a CTA pair (measured: no gain, the kernel is smem-bound)
-    const int m_tiles = (M + OZ_BM - 1) / OZ_BM;
-    int n_tiles = (N + OZ_BN - 1) / OZ_BN;
+    const int m_tiles = (M + OZ_BM - 1) / OZ_BM, n_tiles = (N + OZ_BN - 1) / OZ_BN;
     CUtensorMap map_a, map_b;
-    RCN_TRY(ozaki_make_tensor_map(&map_a, ws.a_slices.as<int8_t>(), M, Kp, cluster == 2 ? OZ_BM / 2 : OZ_BM));
+    RCN_TRY(ozaki_make_tensor_map(&map_a, ws.a_slices.as<int8_t>(), M, Kp, OZ_BM));
     RCN_TRY(ozaki_make_tensor_map(&map_b, ws.b_slices.as<int8_t>(), N, Kp, OZ_BN));
-    if (cluster == 2) {
-        n_tiles = (n_tiles + 1) & ~1;             // pad to whole pairs: the odd partner computes a tile nobody stores
-        auto kern = ozaki_gemm_kernel<Epi, 2>;
-        static SmemAttrCache attr;
-        if (attr.need(OZ_SMEM_BYTES)) RCN_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_SMEM_BYTES));
-        cudaLaunchConfig_t cfg{};
-        cfg.gridDim = dim3((unsigned)(m_tiles * n_tiles), (unsigned)splits, 1);
-        cfg.blockDim = dim3(OZ_THREADS, 1, 1);
-        cfg.dynamicSmemBytes = OZ_SMEM_BYTES;
-        cfg.stream = stream;
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeClusterDimension;
-        at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-        cfg.attrs = at; cfg.numAttrs = 1;
-        const double* sa = ws.a_scale.as<double>();
-        const double* sb = ws.b_scale.as<double>();
-        const OzConvA no_conv{};
-        RCN_LAUNCH(name, stream, cudaLaunchKernelEx(&cfg, kern, map_a, map_b, sa, sb, M, N, Kp, m_tiles, n_tiles, kb_per_split, no_conv, epi));
-    } else {
-        auto kern = ozaki_gemm_kernel<Epi, 1>;
-        static SmemAttrCache attr;
-        if (attr.need(OZ_SMEM_BYTES)) RCN_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_SMEM_BYTES));
-        RCN_LAUNCH(name, stream,
-                   kern<<<dim3((unsigned)(m_tiles * n_tiles), (unsigned)splits), OZ_THREADS, OZ_SMEM_BYTES, stream>>>(
-                       map_a, map_b, ws.a_scale.as<double>(), ws.b_scale.as<double>(), M, N, Kp, m_tiles, n_tiles, kb_per_split, OzConvA{}, epi));
-    }
+    auto kern = ozaki_gemm_kernel<Epi>;
+    static SmemAttrCache attr;
+    if (attr.need(OZ_SMEM_BYTES)) RCN_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_SMEM_BYTES));
+    RCN_LAUNCH(name, stream,
+               kern<<<dim3((unsigned)(m_tiles * n_tiles), (unsigned)splits), OZ_THREADS, OZ_SMEM_BYTES, stream>>>(
+                   map_a, map_b, ws.a_scale.as<double>(), ws.b_scale.as<double>(), M, N, Kp, m_tiles, n_tiles, kb_per_split, OzConvA{}, epi));
     return RCN_OK;
 }
 
@@ -450,7 +393,7 @@ static int launch_conv_ozaki(const char* name, const ConvGeom& g, int B, const d
     CUtensorMap map_a, map_b;
     RCN_TRY(ozaki_make_conv_tensor_map(&map_a, ws.a_slices.as<int8_t>(), B, g.Hi, g.Wi, g.C, tw, th));
     RCN_TRY(ozaki_make_tensor_map(&map_b, ws.b_slices.as<int8_t>(), N, K, OZ_BN));
-    auto kern = ozaki_gemm_kernel<Epi, 1>;
+    auto kern = ozaki_gemm_kernel<Epi>;
     static SmemAttrCache attr;
     if (attr.need(OZ_SMEM_BYTES)) RCN_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, OZ_SMEM_BYTES));
     const int m_tiles = M / OZ_BM, n_tiles = (N + OZ_BN - 1) / OZ_BN;

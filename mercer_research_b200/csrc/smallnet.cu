@@ -555,17 +555,14 @@ constexpr int SNB_TILE = 32 * 64;   // padded partial tile: 32 rows x 64 columns
 
 // MODE 0: gradients only.  MODE 1: also push the final values into the data-parallel peers' receive slots (dp.cu
 // protocol; the update kernel then only receives).  MODE 2: single GPU, apply the SGD update to the finished elements
-// right here (SnUpdate).  MODE 3: data-parallel AND fused update: every thread pushes its finished element to the peers,
-// waits for theirs, adds the ranks in rank order and applies the update -- the whole exchange + update of rcn.rs:190-222
-// inside this kernel's epilogue, so a multi-GPU step is two launches as well.
+// right here (SnUpdate).
 // Whatever the mode, when `upd.cursor` is set the statistics thread also advances the epoch cursor and writes the per-step
 // result ring (on a data-parallel group that makes the cursor final BEFORE the exchange kernel runs, which is what lets the
 // next step's kernel A read it ahead of its griddepcontrol.wait).
 // (Measured and dropped, round 2: 48 columns per CTA = 17 column groups x 8 K-splits + 8 = 144 CTAs "one per SM" ran 11.2 us
 // instead of 6.1 -- B200 co-schedules only ~15 clusters of 8 CTAs, so 18 clusters take two waves.)
-// CW: columns of dW0 per CTA: 64 (one warp per 8 columns) or 32 (two warps per 8 columns, each taking half of every
-// 64-sample chunk; their two partial tiles are added, in order, by the reduction).
-template <int MODE, int CW>
+// Each column CTA owns 64 columns of dW0, one warp per 8 columns.
+template <int MODE>
 __device__ __forceinline__ void sn_phase_b(const SmallNetDesc& d, const double* __restrict__ feats,
                                            const double* __restrict__ acts, const double* __restrict__ deltas,
                                            int B, int ksplit, int col_groups, double* __restrict__ grads,
@@ -573,10 +570,10 @@ __device__ __forceinline__ void sn_phase_b(const SmallNetDesc& d, const double* 
                                            const DpPush& dp, const SnUpdate& upd, const int chunk /* samples per staging pass of the small CTA */,
                                            const int cg_idx, const int rank, const int S,
                                            double* sP, double* sD /* [2][64 * SN_DPITCH]: double-buffered 64-sample delta_0 chunk */,
-                                           const unsigned total_ctas, const long long cur0_early /* >= 0: the cursor was advanced at the top */) {
-    constexpr bool DP = MODE == 1 || MODE == 3;
-    constexpr bool UPD = MODE == 2 || MODE == 3;
-    constexpr bool DPX = MODE == 3;
+                                           const long long cur0_early /* >= 0: the cursor was advanced at the top */) {
+    constexpr bool DP = MODE == 1;
+    constexpr bool UPD = MODE == 2;
+    constexpr int CW = 64;                                   // columns of dW0 per CTA
     namespace cg = cooperative_groups;
     cg::cluster_group cluster = cg::this_cluster();
     RCN_TL_BEGIN(d.tl, 1);
@@ -761,27 +758,18 @@ __device__ __forceinline__ void sn_phase_b(const SmallNetDesc& d, const double* 
         double pold = 0.0;
         if (UPD && gi >= 0) pold = upd.params[gi];
         // all S remote reads are issued before the first add (one DSMEM round trip, not S dependent ones; S <= 8)
-        double rv[8], rw[8];
+        double rv[8];
 #pragma unroll
         for (int q = 0; q < 8; ++q) {
-            rv[q] = 0.0; rw[q] = 0.0;
-            if (q < S) {
-                const double* remote = cluster.map_shared_rank(sP, q);
-                rv[q] = remote[o];
-                if (is_col && CW == 32) rw[q] = remote[CW * 32 + o];   // the second warp's half of every chunk
-            }
+            rv[q] = 0.0;
+            if (q < S) rv[q] = cluster.map_shared_rank(sP, q)[o];
         }
         double s = 0.0;
 #pragma unroll
-        for (int q = 0; q < 8; ++q) {
-            if (q < S) {
-                s += rv[q];
-                if (is_col && CW == 32) s += rw[q];
-            }
-        }
+        for (int q = 0; q < 8; ++q)
+            if (q < S) s += rv[q];
         if (gi >= 0) {
             if (DP) dp_push_value(dp, dp_par, (size_t)gi, s);
-            if (DPX) s = dp_receive_sum<0>(dp, dp_par, (size_t)gi, s);   // the global sum, identical on every rank
             grads[gi] = s;
             if (UPD) upd.params[gi] = sgd_apply(pold, upd.scale, s);
         }
@@ -823,11 +811,10 @@ __device__ __forceinline__ void sn_phase_b(const SmallNetDesc& d, const double* 
     // the release fence of cluster.sync() does (ncu: 9 % of the kernel's samples sat in that membar).
     asm volatile("barrier.cluster.arrive.relaxed.aligned;" ::: "memory");
     asm volatile("barrier.cluster.wait.aligned;" ::: "memory");
-    if (DPX && tid == 0) dp_finish_step(dp, total_ctas);
     RCN_TL_END(d.tl, 1);
 }
 
-template <int MODE, int CW>
+template <int MODE>
 __global__ void __launch_bounds__(SNB_THREADS) smallnet_wgrad_kernel(const __grid_constant__ SmallNetDesc d,
                                                                      const double* __restrict__ feats,
                                                                      const double* __restrict__ acts,
@@ -867,8 +854,8 @@ __global__ void __launch_bounds__(SNB_THREADS) smallnet_wgrad_kernel(const __gri
         if (dp.world <= 1 || MODE == 1) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
         asm volatile("griddepcontrol.wait;" ::: "memory");
     }
-    sn_phase_b<MODE, CW>(d, feats, acts, deltas, B, ksplit, col_groups, grads, stats_partial, n_stat, stats, dp, upd, chunk,
-                         (int)blockIdx.x, (int)blockIdx.y, (int)gridDim.y, sP_dyn, sD_static, gridDim.x * gridDim.y, cur0_early);
+    sn_phase_b<MODE>(d, feats, acts, deltas, B, ksplit, col_groups, grads, stats_partial, n_stat, stats, dp, upd, chunk,
+                     (int)blockIdx.x, (int)blockIdx.y, (int)gridDim.y, sP_dyn, sD_static, cur0_early);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -901,8 +888,9 @@ static bool sn_pdl_enabled() {
     return on;
 }
 
-// Highest launch priority for the training kernels: pending CTAs of kernels A / B must win the SMs (kernel A needs a whole
-// SM per CTA) against anything a parallel branch runs (the host-dataset loop's prefetch kernel).
+// Highest launch priority for the training kernels: pending CTAs of kernels A / B win the SMs (kernel A needs a whole SM
+// per CTA) against lower-priority work queued on the same device.  (It was added against the SM-issued prefetch kernel of
+// the host-dataset loop, which no longer exists; whether it still pays has not been measured.)
 static int sn_high_priority() {
     static const int prio = []() {
         const char* e = getenv("RCN_CUDA_LAUNCH_PRIORITY");
@@ -1017,16 +1005,13 @@ int launch_smallnet_backprop(const SmallNetDesc& d, const double* params, double
     const bool with_push = push.world > 1;
     SnUpdate upd{};
     if (update) upd = *update;
-    const int mode = with_push ? (upd.params ? 3 : 1) : (upd.params ? 2 : 0);
+    const int mode = with_push ? 1 : (upd.params ? 2 : 0);
     static SmemAttrCache attr_b;
     if (attr_b.need(smem_b)) {  // static 36 KB + dynamic tile exceeds the 48 KB default; all variants at once (a later
                                 // launch of another variant may happen inside a stream capture)
-        RCN_CUDA_TRY(cudaFuncSetAttribute(smallnet_wgrad_kernel<0, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
-        RCN_CUDA_TRY(cudaFuncSetAttribute(smallnet_wgrad_kernel<1, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
-        RCN_CUDA_TRY(cudaFuncSetAttribute(smallnet_wgrad_kernel<2, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
-        RCN_CUDA_TRY(cudaFuncSetAttribute(smallnet_wgrad_kernel<3, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
-
-
+        RCN_CUDA_TRY(cudaFuncSetAttribute(smallnet_wgrad_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
+        RCN_CUDA_TRY(cudaFuncSetAttribute(smallnet_wgrad_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
+        RCN_CUDA_TRY(cudaFuncSetAttribute(smallnet_wgrad_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_b));
     }
     cudaLaunchConfig_t cfg{};
     // one or two "small" column groups (db_l, dW_l of the narrow layers): two when there are more entries than threads and the
@@ -1048,8 +1033,8 @@ int launch_smallnet_backprop(const SmallNetDesc& d, const double* params, double
     cfg.attrs = attr;
     cfg.numAttrs = sn_pdl_enabled() ? 3 : 2;
     const int Bi = (int)B;
-    auto kern = mode == 1 ? smallnet_wgrad_kernel<1, 64> : mode == 2 ? smallnet_wgrad_kernel<2, 64> : mode == 3 ? smallnet_wgrad_kernel<3, 64> : smallnet_wgrad_kernel<0, 64>;
-    RCN_LAUNCH(mode == 2 ? "smallnet_wgrad_kernel(+SGD update)" : mode == 3 ? "smallnet_wgrad_kernel(+exchange+SGD update)" : "smallnet_wgrad_kernel", stream,
+    auto kern = mode == 1 ? smallnet_wgrad_kernel<1> : mode == 2 ? smallnet_wgrad_kernel<2> : smallnet_wgrad_kernel<0>;
+    RCN_LAUNCH(mode == 2 ? "smallnet_wgrad_kernel(+SGD update)" : "smallnet_wgrad_kernel", stream,
                cudaLaunchKernelEx(&cfg, kern, d, (const double*)feats, (const double*)acts, (const double*)deltas, Bi,
                                   ksplit, col_groups, grads, (const double*)stats_partial, n_tiles, stats, push, upd, chunk));
     return RCN_OK;

@@ -24,9 +24,8 @@ M = ["gpu__time_duration.sum", "dram__bytes_read.sum", "dram__bytes_write.sum", 
 NAMES = {"smallnet_fwd_bwd_kernel<1, 0>": "smallnet_fwd_bwd_kernel(fused features)", "smallnet_fwd_bwd_kernel<2, 0>": "smallnet_fwd_bwd_kernel(fused features)",
          # (ncu runs on one GPU only: the <2, 1> instance seen there is the single-GPU prewait, not the data-parallel one)
          "smallnet_fwd_bwd_kernel<2, 1>": "smallnet_fwd_bwd_kernel(fused features, front end ahead of the wait)",
-         "smallnet_fwd_bwd_kernel<0, 0>": "smallnet_fwd_bwd_kernel", "smallnet_wgrad_kernel<2, 64>": "smallnet_wgrad_kernel(+SGD update)",
-         "smallnet_wgrad_kernel<0, 64>": "smallnet_wgrad_kernel", "smallnet_wgrad_kernel<1, 64>": "smallnet_wgrad_kernel",
-         "smallnet_wgrad_kernel<3, 64>": "smallnet_wgrad_kernel(+exchange+SGD update)"}
+         "smallnet_fwd_bwd_kernel<0, 0>": "smallnet_fwd_bwd_kernel", "smallnet_wgrad_kernel<2>": "smallnet_wgrad_kernel(+SGD update)",
+         "smallnet_wgrad_kernel<0>": "smallnet_wgrad_kernel", "smallnet_wgrad_kernel<1>": "smallnet_wgrad_kernel"}
 
 
 def to_bytes(v, unit):

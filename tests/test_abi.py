@@ -116,8 +116,8 @@ def test_layer_codes_and_enums():
 
 def test_built_library_carries_the_blackwell_instructions(built_library):
     """The shipped library is sm_100a machine code that really uses the units DESIGN.md names (no GPU needed to see it):
-    tcgen05 integer MMA + TMEM loads + their mbarrier commits (Ozaki GEMM / conv), TMA tensor loads incl. multicast and the
-    5-D im2col boxes, bulk-async copies (staged feature kernel), FP64 tensor-core DMMA, cp.async rings."""
+    tcgen05 integer MMA + TMEM loads + their mbarrier commits (Ozaki GEMM / conv), TMA tensor loads and the 5-D
+    im2col boxes, bulk-async copies (staged feature kernel), FP64 tensor-core DMMA, cp.async rings."""
     import shutil
     import subprocess
     cuobjdump = shutil.which("cuobjdump") or "/usr/local/cuda/bin/cuobjdump"
@@ -127,5 +127,5 @@ def test_built_library_carries_the_blackwell_instructions(built_library):
     elf = subprocess.run([cuobjdump, "-lelf", so], capture_output=True, text=True, check=True).stdout
     assert "sm_100a" in elf and not re.search(r"sm_(?!100a)\d+", elf), elf      # one target, no multi-arch fatbin
     sass = subprocess.run([cuobjdump, "-sass", so], capture_output=True, text=True, check=True).stdout
-    for mnemonic in ("UTCIMMA", "LDTM", "UTCBAR", "UTMALDG.3D", "UTMALDG.3D.MULTICAST", "UTMALDG.5D", "UBLKCP", "DMMA", "LDGSTS"):
+    for mnemonic in ("UTCIMMA", "LDTM", "UTCBAR", "UTMALDG.3D", "UTMALDG.5D", "UBLKCP", "DMMA", "LDGSTS"):
         assert mnemonic in sass, f"{mnemonic} not found in the library's SASS"

@@ -8,21 +8,18 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SRC = os.path.join(ROOT, "tests", "cpp", "host_test.cpp")
-BUILD = os.path.join(ROOT, "tests", "cpp", "_build")
-EXE = os.path.join(BUILD, "host_test")
+LIB_DIR = os.path.join(ROOT, "mercer_research_b200")
 
 
 @pytest.fixture(scope="module")
-def host_test(built_library):
-    deps = [SRC, os.path.join(ROOT, "include", "rcn.hpp"), os.path.join(ROOT, "include", "rcn_cuda.h")]
-    if not os.path.exists(EXE) or any(os.path.getmtime(d) > os.path.getmtime(EXE) for d in deps):
-        os.makedirs(BUILD, exist_ok=True)
-        cmd = ["g++", "-std=c++17", "-O1", "-Wall", "-Wextra", "-I", os.path.join(ROOT, "include"), SRC,
-               "-L", os.path.join(ROOT, "mercer_research_b200"), "-lrcn_cuda",
-               "-Wl,-rpath,$ORIGIN/../../../mercer_research_b200", "-o", EXE]
-        r = subprocess.run(cmd, capture_output=True, text=True)
-        assert r.returncode == 0, r.stderr
-    return EXE
+def host_test(built_library, tmp_path_factory):
+    # built in pytest's temporary directory: the suite also runs from a checkout it cannot write to
+    exe = str(tmp_path_factory.mktemp("cpp_host") / "host_test")
+    cmd = ["g++", "-std=c++17", "-O1", "-Wall", "-Wextra", "-I", os.path.join(ROOT, "include"), SRC,
+           "-L", LIB_DIR, "-lrcn_cuda", "-Wl,-rpath," + LIB_DIR, "-o", exe]
+    r = subprocess.run(cmd, capture_output=True, text=True)
+    assert r.returncode == 0, r.stderr
+    return exe
 
 
 def run(exe, mode, *args, env=None):

@@ -397,7 +397,7 @@ def test_train_epoch_host_equals_step_by_step(api):
     params = None
     results = []
     import torch
-    pinned = torch.from_numpy(images).pin_memory()       # pinned host memory takes the streaming (zero-copy prefetch) path
+    pinned = torch.from_numpy(images).pin_memory()       # pinned host memory takes the streaming (copy-engine ring) path
     pinned_labels = torch.from_numpy(labels).pin_memory()
     for mode in ("loop", "epoch", "epoch-pinned", "epoch-pinned-again"):
         model = api.RCN(10, cfg, [30])
@@ -428,8 +428,8 @@ def test_train_epoch_host_equals_step_by_step(api):
 
 
 def test_train_epoch_host_streaming_large_chunks(api):
-    """Same equality at a chunk size where every prefetch thread carries several 16-byte loads and the last round is
-    ragged (B=1000: 49 000 uint4 per chunk over 8192 threads)."""
+    """Same equality at a large chunk (B=1000: 784 000 bytes per step, each copied into its own ring slot), four steps
+    and a ragged remainder of 123 samples that is dropped."""
     import torch
     rng = np.random.default_rng(23)
     B, N = 1000, 1000 * 4 + 123
@@ -490,16 +490,21 @@ print("ok")
 '''
 
 
-@pytest.mark.parametrize("copy_mode,spg", [("dma", "0"), ("dma", "1"), ("dma", "7"), ("pull", "0"), ("pull", "3")])
-def test_train_epoch_host_copy_modes(api, copy_mode, spg):
-    """Both ways the streamed epoch moves its images over PCIe (copy engine into a 64-chunk ring with an arrival counter
-    kernel A waits on / SM-issued zero-copy loads on a graph branch), at several steps per graph ("0" = the mode's default:
-    40 / 2): 151 steps wrap the ring twice and leave a remainder of 20-, 10- and single-step launches; bit-identical to train_batch_images chunk by chunk
-    (rcn.rs:147-149)."""
+@pytest.mark.parametrize("extra_env", [
+    {"RCN_CUDA_HOST_STEPS_PER_GRAPH": "0"},
+    {"RCN_CUDA_HOST_STEPS_PER_GRAPH": "1"},
+    {"RCN_CUDA_HOST_STEPS_PER_GRAPH": "7"},
+    {"RCN_CUDA_FEATURES_STAGED": "0"},
+], ids=["dma-0", "dma-1", "dma-7", "general-loop"])
+def test_train_epoch_host_copy_modes(api, extra_env):
+    """The streamed epoch (copy engine into a 64-chunk ring with an arrival counter kernel A waits on) at several steps
+    per graph ("0" = the default, 40): 151 steps wrap the ring twice and leave a remainder of 20-, 10- and single-step
+    launches.  Without the staged front end the call takes the general double-buffered loop instead.  Every case is
+    bit-identical to train_batch_images chunk by chunk (rcn.rs:147-149)."""
     import subprocess
     import sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    env = dict(os.environ, RCN_CUDA_HOST_COPY=copy_mode, RCN_CUDA_HOST_STEPS_PER_GRAPH=spg)
+    env = dict(os.environ, **extra_env)
     r = subprocess.run([sys.executable, "-c", HOST_COPY_SCRIPT % {"root": root}], env=env, capture_output=True, text=True, timeout=300)
     assert r.returncode == 0 and "ok" in r.stdout, r.stdout[-2000:] + r.stderr[-2000:]
 
