@@ -277,11 +277,6 @@ bool conv_wgrad_use_tc(size_t Co, size_t n_k, size_t n_pix) {
     return Co >= 64 && n_k >= 256 && n_pix >= 4096 && (double)Co * (double)n_k * (double)n_pix >= 2.0e9;
 }
 
-bool conv_tma_enabled() {
-    static const bool on = []() { const char* e = getenv("RCN_CUDA_CONV_TMA"); return !(e && e[0] == '0'); }();
-    return on;
-}
-
 OzakiWorkspace& conv_tc_workspace() {
     static thread_local OzakiWorkspace ws[64];   // one per device this thread drives
     int dev = 0;
@@ -319,7 +314,7 @@ int launch_conv2d_forward(const double* x, const double* w, const double* bias, 
     const ConvGeom geom{x, (int)s.H, (int)s.W, (int)s.Ci, (int)s.Ho, (int)s.Wo, (int)s.kh, (int)s.kw, s.ph, s.pw, N, K};
     if (conv_use_tc((size_t)N, (size_t)M, (size_t)K)) {
         const EpiConvForwardT epi{bias, y, M, act};
-        if (conv_tma_enabled() && ozaki_conv_tma_ok(geom))   // im2col by TMA: the tensor is sliced once, taps are shifted boxes
+        if (ozaki_conv_tma_ok(geom))   // im2col by TMA: the tensor is sliced once, taps are shifted boxes
             return launch_conv_ozaki("conv2d_forward_igemm(tcgen05 int8 slices, TMA im2col)", geom, (int)s.B, w, M, epi,
                                      conv_tc_workspace(), stream);
         OzOperand oa{x, 0, true};                 // im2col rows gathered straight into int8 digit planes
@@ -350,7 +345,7 @@ int launch_conv2d_backward_data(const double* dz, const double* w, const ConvSha
                         (int)s.kh - 1 - s.ph, (int)s.kw - 1 - s.pw, N, K};
     if (conv_use_tc((size_t)N, (size_t)M, (size_t)K)) {
         const EpiConvBackDataT epi{y_prev, dx, M, act_prev};
-        if (conv_tma_enabled() && ozaki_conv_tma_ok(geom))
+        if (ozaki_conv_tma_ok(geom))
             return launch_conv_ozaki("conv2d_backward_data_igemm(tcgen05 int8 slices, TMA im2col)", geom, (int)s.B, ws.as<double>(), M,
                                      epi, conv_tc_workspace(), stream);
         OzOperand oa{dz, 0, true};

@@ -299,8 +299,7 @@ __global__ void __launch_bounds__(256) skinny_backward_weight_kernel(const doubl
 }
 
 static bool skinny_layer(size_t M, size_t K) {
-    static const bool off = []() { const char* e = getenv("RCN_CUDA_SKINNY"); return e && e[0] == '0'; }();
-    return !off && gemm_impl() == GEMM_AUTO && M >= 1 && M <= (size_t)SK_MAX_ROWS && K >= 512 && K % 128 == 0;
+    return gemm_impl() == GEMM_AUTO && M >= 1 && M <= (size_t)SK_MAX_ROWS && K >= 512 && K % 128 == 0;
 }
 
 template <int MR>
@@ -552,8 +551,7 @@ int launch_dense_backward_weight(const double* delta, const double* A_prev, size
         // with the batch split floor(148 / tiles) ways beats two waves of 64 x 64 tiles (ncu, c3: 20 % warps active, 0.52 of peak).
         // launch_gemm_tiles takes the big tile when tiles x splits covers at least 7/8 of the SMs.
         const size_t big = M > 32 ? (size_t)cdiv(M, 128) * cdiv(N, 128) : 0;
-        static const bool big_on = []() { const char* e = getenv("RCN_CUDA_WGRAD_BIG_TILE"); return !(e && e[0] == '0'); }();
-        if (big_on && big > 0 && big < (size_t)kNumSMs) {
+        if (big > 0 && big < (size_t)kNumSMs) {
             const int s_big = (int)((size_t)kNumSMs / big);
             if (s_big >= 2 && Kb / (size_t)s_big >= 256 && big * (size_t)s_big >= (size_t)kNumSMs * 7 / 8) splits = s_big;
         }

@@ -157,7 +157,6 @@ int launch_dp_allreduce_sgd(const DpState& st, double* params, double* grads, do
     unsigned grid = cdiv(st.n, kDpThreads);
     if (grid <= 2u * kDpMaxCtas) { if (grid > (unsigned)kDpMaxCtas) grid = kDpMaxCtas; }
     else if (grid > 2u * kNumSMs) grid = 2u * kNumSMs;
-    static const bool pdl = []() { const char* e = getenv("RCN_CUDA_PDL"); return !(e && e[0] == '0'); }();
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = dim3(grid, 1, 1);
     cfg.blockDim = dim3(kDpThreads, 1, 1);
@@ -166,7 +165,7 @@ int launch_dp_allreduce_sgd(const DpState& st, double* params, double* grads, do
     at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     at[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = at;
-    cfg.numAttrs = pdl ? 1 : 0;
+    cfg.numAttrs = 1;
     const int pushed_i = already_pushed ? 1 : 0;
 #define RCN_DP_LAUNCH(W)                                                                                                       \
     RCN_LAUNCH("dp_allreduce_sgd_kernel", stream,                                                                              \

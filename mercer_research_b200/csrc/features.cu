@@ -425,25 +425,22 @@ static int launch_features_t(const FeaturePlan& plan, const TIN* images, size_t 
         dim3 grid(cdiv(items, 256), (unsigned)(B > 32768 ? 32768 : B));
         if (grid.x > 1024) grid.x = 1024;
         if (std::is_same<T, int>::value && st.kind == 0 && st.same && st.h_in >= 2) {   // streaming strip kernels (see above)
-            static const bool strips = []() { const char* e = getenv("RCN_CUDA_CONV_STRIPS"); return !(e && e[0] == '0'); }();
-            if (strips) {
-                const dim3 sgrid((unsigned)st.n_in, grid.y);
-                const int* cin = reinterpret_cast<const int*>(cur);
-                // the map goes through shared memory when it fits the default 48 KB and 16-byte loads are possible
-                const size_t map_elems = (size_t)st.h_in * st.w_in;
-                const int staged = (map_elems * sizeof(int) <= 48 * 1024 && map_elems % 4 == 0 && cur_stride % 4 == 0 &&
-                                    (reinterpret_cast<uintptr_t>(cin) & 15) == 0) ? 1 : 0;
-                const size_t ssmem = staged ? map_elems * sizeof(int) : 0;
-                if (s == sl.n - 1) {
-                    RCN_LAUNCH("conv_same_final_kernel", stream, conv_same_final_kernel<<<sgrid, 256, ssmem, stream>>>(st, cin, cur_stride, out, plan.L, sc, B, staged));
-                } else {
-                    const size_t out_stride = (size_t)st.n_out * st.h_out * st.w_out;
-                    RCN_LAUNCH("conv_same_maps_kernel", stream, conv_same_maps_kernel<<<sgrid, 256, ssmem, stream>>>(st, cin, cur_stride, reinterpret_cast<int*>(nxt), out_stride, B, staged));
-                    T* tmp = cur; cur = nxt; nxt = tmp;
-                    cur_stride = out_stride;
-                }
-                continue;
+            const dim3 sgrid((unsigned)st.n_in, grid.y);
+            const int* cin = reinterpret_cast<const int*>(cur);
+            // the map goes through shared memory when it fits the default 48 KB and 16-byte loads are possible
+            const size_t map_elems = (size_t)st.h_in * st.w_in;
+            const int staged = (map_elems * sizeof(int) <= 48 * 1024 && map_elems % 4 == 0 && cur_stride % 4 == 0 &&
+                                (reinterpret_cast<uintptr_t>(cin) & 15) == 0) ? 1 : 0;
+            const size_t ssmem = staged ? map_elems * sizeof(int) : 0;
+            if (s == sl.n - 1) {
+                RCN_LAUNCH("conv_same_final_kernel", stream, conv_same_final_kernel<<<sgrid, 256, ssmem, stream>>>(st, cin, cur_stride, out, plan.L, sc, B, staged));
+            } else {
+                const size_t out_stride = (size_t)st.n_out * st.h_out * st.w_out;
+                RCN_LAUNCH("conv_same_maps_kernel", stream, conv_same_maps_kernel<<<sgrid, 256, ssmem, stream>>>(st, cin, cur_stride, reinterpret_cast<int*>(nxt), out_stride, B, staged));
+                T* tmp = cur; cur = nxt; nxt = tmp;
+                cur_stride = out_stride;
             }
+            continue;
         }
         if (s == sl.n - 1) {
             RCN_LAUNCH("stage_final_kernel", stream, stage_final_kernel<T><<<grid, 256, 0, stream>>>(st, cur, cur_stride, out, plan.L, sc, B));

@@ -168,13 +168,9 @@ struct rcn_cuda_model {
     bool stats_valid = false;
     // data-parallel group (dp.cu) and the pipelined host-dataset loop (rcn_cuda_train_epoch_host)
     DpState dp;
-    SnUpdate pending_upd{};         // set by the step entry points: the next small-network accumulate applies the update itself
-    bool upd_fused = false;         // ... and did (the standalone update kernel is then skipped)
-    bool cursor_fused = false;      // ... or at least advanced the cursor / wrote the result ring (data-parallel groups)
     bool x_owns_cursor = false;     // an exchange kernel that advances a cursor may be in flight: kernel A must not read the
                                     // cursor ahead of its griddepcontrol.wait (cleared wherever the stream is drained)
     bool dp_pushed = false;         // the last accumulate pushed its gradients to the peers itself (kernel B epilogue)
-    bool dp_push_suppress = false;  // warm-up launches must not push (a push is consumed by exactly one receive)
     DevBuf timeline;                // device-side launch timeline (timeline.cuh), allocated by rcn_cuda_timeline_enable
     bool tl_on = false;
     OzakiWorkspace oz;              // tcgen05 integer-slice GEMM scratch (wide dense layers)
@@ -235,11 +231,6 @@ struct DeviceGuard {
     if (!(h)) return fail(RCN_ERR_INVALID, "null model handle");                         \
     DeviceGuard _guard((h)->device);                                                     \
     if (!_guard.ok) return fail(RCN_ERR_CUDA, "cudaSetDevice(%d) failed", (h)->device);
-
-bool dp_fused_push_enabled() {
-    static const bool on = []() { const char* e = getenv("RCN_CUDA_DP_FUSED_PUSH"); return !(e && e[0] == '0'); }();
-    return on;
-}
 
 // Consumes the "already pushed" flag of the last accumulate: every push is matched by exactly one receive.
 bool take_dp_pushed(rcn_cuda_model* h) {
@@ -306,12 +297,59 @@ int forward_dev(rcn_cuda_model* h, const double* feats, size_t B, const double* 
     return RCN_OK;
 }
 
+// What a training step asks of the accumulate.  On the fused small-network path kernel B applies `upd` itself: on one GPU
+// the whole update, on a data-parallel group (`upd.params` null) only the cursor / result ring, and the exchange kernel
+// updates.  `push`: on a connected group kernel B pushes its gradients to the peers -- not in a warm-up, as every push is
+// consumed by exactly one receive.  The default request arms nothing.
+struct StepRequest {
+    SnUpdate upd{};
+    bool push = true;
+};
+
+// What kernel B did with the request's update; finish_step launches the rest.
+enum class StepDone {
+    nothing,   // the generic path, an over-size batch, or no update armed
+    cursor,    // advanced the cursor and wrote the result ring (data-parallel group)
+    update,    // updated the parameters (one GPU): the step is complete
+};
+
+// The update of a training step: `scale` = eta / global batch; the optional device-side cursor advances by `batch` over
+// `n_samples`, and `stats_ring` receives each step's {cost, hits}.  `streamed`: kernel A of the streamed host epoch reads
+// the cursor ahead of its wait (one GPU).
+SnUpdate step_update(rcn_cuda_model* h, double scale, long long* cursor = nullptr, long long batch = 0, long long n_samples = 0,
+                     double* stats_ring = nullptr, bool streamed = false) {
+    SnUpdate u{};
+    // (Receiving inside kernel B on a group as well was measured slower, 2 GPUs, c2: 30.8 vs 28.4 us/step -- the NVLink
+    // round trip is then exposed inside the kernel instead of overlapping the next launch -- and was removed.)
+    if (!h->dp.connected) u.params = h->params.as<double>();
+    u.scale = scale;
+    u.cursor = cursor;
+    u.batch = batch;
+    u.n_samples = n_samples;
+    u.stats_ring = stats_ring;
+    u.early_cursor = (!h->dp.connected && streamed) ? 1 : 0;
+    return u;
+}
+
+// Launches what kernel B left of a step: on a data-parallel group the exchange kernel (receive, sum, update), otherwise the
+// update kernel; either advances the cursor and writes the result ring unless kernel B already did.
+int finish_step(rcn_cuda_model* h, const SnUpdate& u, StepDone done) {
+    if (done == StepDone::update) return RCN_OK;
+    long long* cursor = done == StepDone::cursor ? nullptr : u.cursor;
+    const double* stats = u.stats_ring ? h->small.as<double>() : nullptr;   // the step's {cost, hits}, written by the accumulate
+    if (h->dp.connected) {
+        if (cursor) h->x_owns_cursor = true;
+        return launch_dp_allreduce_sgd(h->dp, h->params.as<double>(), h->grads, u.scale, h->stream, cursor, u.batch, u.n_samples,
+                                       stats, u.stats_ring, take_dp_pushed(h), h->small_desc.tl);
+    }
+    return launch_sgd_update(h->params.as<double>(), h->grads, h->n_params, u.scale, h->stream, cursor, u.batch, u.n_samples, stats,
+                             u.stats_ring);
+}
+
 int accumulate_dev(rcn_cuda_model* h, const double* feats, const double* onehot, const int64_t* labels, size_t B,
-                   const SmallNetFront* front = nullptr) {
+                   const SmallNetFront* front, const StepRequest& req, StepDone* done) {
     const size_t n = h->rows.size();
-    const SnUpdate upd = h->pending_upd;   // consumed by this call whichever path it takes
-    h->pending_upd = SnUpdate{};
-    h->upd_fused = false;
+    if (done) *done = StepDone::nothing;
     if (h->dp_pushed)   // a pushed gradient must be received by the group's update before the next one is produced
         return fail(RCN_ERR_STATE, "data-parallel group: the previous gradients were pushed to the peers but never applied "
                                    "(every accumulate needs exactly one apply on every rank)");
@@ -324,14 +362,15 @@ int accumulate_dev(rcn_cuda_model* h, const double* feats, const double* onehot,
         RCN_TRY(h->deltas.reserve(h->sum_rows * B * sizeof(double)));
         RCN_TRY(h->small.reserve(64));
         DpPush push{};
-        const bool fuse_push = h->dp.connected && dp_fused_push_enabled() && !h->dp_push_suppress;
+        const bool fuse_push = h->dp.connected && req.push;
         if (fuse_push) push = dp_push_desc(h->dp);
+        const SnUpdate& upd = req.upd;
+        const bool armed = (upd.params || upd.cursor) && (!h->dp.connected || fuse_push);
         RCN_TRY(launch_smallnet_backprop(h->small_desc, h->params.as<double>(), const_cast<double*>(feats), B, onehot,
                                          labels, h->acts.as<double>(), h->deltas.as<double>(), h->grads,
                                          h->small.as<double>(), h->gemm_ws, front, h->stream, fuse_push ? &push : nullptr,
-                                         ((upd.params || upd.cursor) && (!h->dp.connected || fuse_push)) ? &upd : nullptr));
-        h->upd_fused = upd.params != nullptr;   // (armed on one GPU only)
-        h->cursor_fused = upd.cursor && (!h->dp.connected || fuse_push);
+                                         armed ? &upd : nullptr));
+        if (done) *done = upd.params ? StepDone::update : (armed && upd.cursor) ? StepDone::cursor : StepDone::nothing;
         h->dp_pushed = fuse_push;   // pushed but not yet received: the exchange kernel must follow
         h->stats_valid = true;
         h->last_B = B;
@@ -357,16 +396,11 @@ int accumulate_dev(rcn_cuda_model* h, const double* feats, const double* onehot,
 // images (DEVICE) -> gradient sums.  The canonical narrow network with u8 pixels runs the convpool stack inside
 // kernel A (smallnet.cu); everything else runs the feature kernel(s) first.  `bi` (optional) is the epoch-mode
 // device-side batch selection; without it `labels` are this batch's labels.
-static bool fused_front_enabled() {
-    static const bool v = []() { const char* e = getenv("RCN_CUDA_FUSED_FRONT"); return !(e && e[0] == '0'); }();
-    return v;
-}
-
 int accumulate_images_dev(rcn_cuda_model* h, const void* images, int fmt, const int64_t* labels, size_t B, size_t H,
-                          size_t W, const BatchIndex* bi) {
+                          size_t W, const BatchIndex* bi, const StepRequest& req = {}, StepDone* done = nullptr) {
     RCN_TRY(h->feats.reserve(h->plan.L * B * sizeof(double)));
     const int64_t* step_labels = bi ? (const int64_t*)bi->labels_batch : labels;
-    if (fused_front_enabled() && h->use_small && B <= smallnet_max_batch() && fmt == RCN_PIXELS_U8_ROWMAJOR && h->plan.n_conv <= 10 &&
+    if (h->use_small && B <= smallnet_max_batch() && fmt == RCN_PIXELS_U8_ROWMAJOR && h->plan.n_conv <= 10 &&
         h->plan.L > 0) {
         SmallNetFront fr{};
         fr.images = (const uint8_t*)images;
@@ -380,10 +414,8 @@ int accumulate_images_dev(rcn_cuda_model* h, const void* images, int fmt, const 
         // (smallnet.cu) when this step's kernel B pushes to the peers (so the exchange kernel X precedes the next kernel
         // A) and any device-side cursor it reads is advanced by kernel B -- this step's and the previous one's
         // (x_owns_cursor) -- not by X, which may still be running then.
-        static const bool prewait_env = []() { const char* e = getenv("RCN_CUDA_DP_PREWAIT"); return !(e && e[0] == '0'); }();
-        const bool fuse_push = h->dp.connected && dp_fused_push_enabled() && !h->dp_push_suppress;
-        fr.prewait = (prewait_env && fr.use_cp && fuse_push && !h->x_owns_cursor &&
-                      (!fr.bi.cursor || h->pending_upd.cursor == fr.bi.cursor)) ? 1 : 0;
+        fr.prewait = (fr.use_cp && h->dp.connected && req.push && !h->x_owns_cursor &&
+                      (!fr.bi.cursor || req.upd.cursor == fr.bi.cursor)) ? 1 : 0;
         // One GPU, streamed host epoch: the same front end under the tail of the previous step's kernel B (which triggers its
         // dependents early).  Safe whatever precedes this launch: a kernel that does not trigger early has completed before
         // kernel A starts; kernel B advances a device-side cursor before it triggers, and the only buffer both touch -- the
@@ -393,11 +425,11 @@ int accumulate_images_dev(rcn_cuda_model* h, const void* images, int fmt, const 
         // only when kernel B's CTAs leave, and its parameter loads are no longer hidden behind the front end.
         if (!h->dp.connected && fr.use_cp && fr.bi.window != 0) fr.prewait = 2;
         if (smallnet_front_fits(h->small_desc, fr))
-            return accumulate_dev(h, h->feats.as<double>(), nullptr, step_labels, B, &fr);
+            return accumulate_dev(h, h->feats.as<double>(), nullptr, step_labels, B, &fr, req, done);
     }
     RCN_TRY(launch_features(h->plan, images, fmt, B, H, W, true, h->mean, h->sd, h->feats.as<double>(), h->fscratch,
                             h->stream, bi));
-    return accumulate_dev(h, h->feats.as<double>(), nullptr, step_labels, B);
+    return accumulate_dev(h, h->feats.as<double>(), nullptr, step_labels, B, nullptr, req, done);
 }
 
 // stage targets (exactly one of onehot / labels)
@@ -798,9 +830,10 @@ int rcn_cuda_evaluate(rcn_cuda_handle h, const double* feats, const int64_t* lab
     return RCN_OK;
 }
 
-int rcn_cuda_accumulate_gradients(rcn_cuda_handle h, const double* feats, const double* onehot, const int64_t* labels,
-                                  size_t B) {
-    RCN_ENTER(h);
+// The accumulate entry points behind the public ones, which pass the default (unarmed) request; the training steps arm
+// their update.
+static int accumulate_gradients(rcn_cuda_model* h, const double* feats, const double* onehot, const int64_t* labels, size_t B,
+                                const StepRequest& req, StepDone* done) {
     RCN_TRY(require_params(h));
     const double* oh = nullptr; const int64_t* lb = nullptr;
     const double* f_dev = nullptr;
@@ -812,15 +845,14 @@ int rcn_cuda_accumulate_gradients(rcn_cuda_handle h, const double* feats, const 
         RCN_TRY(in.stage(feats, h->cols[0] * B * sizeof(double), h->in_stage, h->stream, &host_in));
         f_dev = (const double*)in.dev;
     }
-    RCN_TRY(accumulate_dev(h, f_dev, oh, lb, B));
+    RCN_TRY(accumulate_dev(h, f_dev, oh, lb, B, nullptr, req, done));
     if (host_in || (onehot && !is_device_ptr(onehot)) || (labels && !is_device_ptr(labels)))
         RCN_CUDA_TRY(cudaStreamSynchronize(h->stream));  // caller may reuse host buffers
     return RCN_OK;
 }
 
-int rcn_cuda_accumulate_gradients_images(rcn_cuda_handle h, const void* images, int pixel_format, const int64_t* labels,
-                                         size_t B, size_t H, size_t W) {
-    RCN_ENTER(h);
+static int accumulate_gradients_images(rcn_cuda_model* h, const void* images, int pixel_format, const int64_t* labels, size_t B,
+                                       size_t H, size_t W, const StepRequest& req, StepDone* done) {
     RCN_TRY(require_params(h));
     RCN_TRY(ensure_plan(h, H, W));
     RCN_TRY(check_feature_width(h, h->plan.L));
@@ -833,75 +865,58 @@ int rcn_cuda_accumulate_gradients_images(rcn_cuda_handle h, const void* images, 
         if (!images) return fail(RCN_ERR_INVALID, "null images");
         StagedIn in;
         RCN_TRY(in.stage(images, B * H * W * pixel_bytes(pixel_format), h->in_stage, h->stream, nullptr));
-        RCN_TRY(accumulate_images_dev(h, in.dev, pixel_format, lb, B, H, W, nullptr));
+        RCN_TRY(accumulate_images_dev(h, in.dev, pixel_format, lb, B, H, W, nullptr, req, done));
     } else {
-        RCN_TRY(accumulate_dev(h, nullptr, nullptr, nullptr, 0));
+        RCN_TRY(accumulate_dev(h, nullptr, nullptr, nullptr, 0, nullptr, req, done));
     }
     if (B && (!is_device_ptr(images) || !is_device_ptr(labels))) RCN_CUDA_TRY(cudaStreamSynchronize(h->stream));
     return RCN_OK;
+}
+
+int rcn_cuda_accumulate_gradients(rcn_cuda_handle h, const double* feats, const double* onehot, const int64_t* labels,
+                                  size_t B) {
+    RCN_ENTER(h);
+    return accumulate_gradients(h, feats, onehot, labels, B, StepRequest{}, nullptr);
+}
+
+int rcn_cuda_accumulate_gradients_images(rcn_cuda_handle h, const void* images, int pixel_format, const int64_t* labels,
+                                         size_t B, size_t H, size_t W) {
+    RCN_ENTER(h);
+    return accumulate_gradients_images(h, images, pixel_format, labels, B, H, W, StepRequest{}, nullptr);
 }
 
 int rcn_cuda_apply_gradients(rcn_cuda_handle h, double eta, size_t batch) {
     RCN_ENTER(h);
     RCN_TRY(require_params(h));
     if (batch == 0) return RCN_OK;  // chunks_exact never yields an empty batch (rcn.rs:147)
-    const double scale = eta / (double)batch;  // (eta / batch.len() as f64)  (rcn.rs:214)
-    if (h->dp.connected)   // exchange over NVLink peer memory fused with the update (dp.cu)
-        return launch_dp_allreduce_sgd(h->dp, h->params.as<double>(), h->grads, scale, h->stream, nullptr, 0, 0, nullptr, nullptr,
-                                       take_dp_pushed(h), h->small_desc.tl);
-    return launch_sgd_update(h->params.as<double>(), h->grads, h->n_params, scale, h->stream);
+    // (eta / batch.len() as f64)  (rcn.rs:214); on a group the exchange over NVLink peer memory fused with the update (dp.cu)
+    return finish_step(h, step_update(h, eta / (double)batch), StepDone::nothing);
 }
 
 // Every entry point that drains the model's stream ends the hazard x_owns_cursor guards against.
 static void stream_drained(rcn_cuda_model* h) { h->x_owns_cursor = false; }
 
-// Single-GPU steps of the fused small-network path let the weight-gradient kernel apply the update (SnUpdate): arm it
-// before the accumulate; if that accumulate took another path the standalone update kernel runs as before.
-static void arm_fused_update(rcn_cuda_model* h, double scale, long long* cursor, long long batch, long long n_samples,
-                             double* stats_ring, bool streamed = false) {
-    static const bool on = []() { const char* e = getenv("RCN_CUDA_FUSED_UPDATE"); return !(e && e[0] == '0'); }();
-    h->pending_upd = SnUpdate{};
-    if (!on || !h || !h->params_ready || !h->use_small) return;
-    // Data-parallel groups: kernel B only takes over the cursor / result ring (params stays null) and the exchange kernel
-    // applies the update.  (Receiving inside kernel B as well was measured slower, 2 GPUs, c2: 30.8 vs 28.4 us/step -- the
-    // NVLink round trip is then exposed inside the kernel instead of overlapping the next launch -- and was removed.)
-    if (h->dp.connected && (!dp_fused_push_enabled() || h->dp_push_suppress)) return;
-    if (!h->dp.connected) h->pending_upd.params = h->params.as<double>();
-    h->pending_upd.scale = scale;
-    h->pending_upd.cursor = cursor;
-    h->pending_upd.batch = batch;
-    h->pending_upd.n_samples = n_samples;
-    h->pending_upd.stats_ring = stats_ring;
-    h->pending_upd.early_cursor = (!h->dp.connected && streamed) ? 1 : 0;   // kernel A of the streamed epoch prewaits
-}
-// What the accumulate did with the armed update: bit 0 = parameters updated, bit 1 = cursor advanced / result ring written.
-static int take_upd_fused(rcn_cuda_model* h) {
-    const int f = (h->upd_fused ? 1 : 0) | (h->cursor_fused ? 2 : 0);
-    h->upd_fused = false;
-    h->cursor_fused = false;
-    h->pending_upd = SnUpdate{};
-    return f;
-}
-
+// One training step: the fused small-network path lets kernel B apply the update (one GPU) or push the gradients to the
+// peers; finish_step launches whatever it left.  On a connected data-parallel group B is this rank's shard and the update
+// uses the global batch (rcn.rs:214).
 int rcn_cuda_train_batch(rcn_cuda_handle h, const double* feats, const double* onehot, const int64_t* labels, size_t B,
                          double eta) {
-    // on a connected data-parallel group B is this rank's shard and the update uses the global batch (rcn.rs:214)
-    const size_t global = h ? B * (size_t)(h->dp.connected ? h->dp.world : 1) : B;
-    if (h && B) arm_fused_update(h, eta / (double)global, nullptr, 0, 0, nullptr);
-    const int rc = rcn_cuda_accumulate_gradients(h, feats, onehot, labels, B);
-    if (rc != RCN_OK) { if (h) take_upd_fused(h); return rc; }
-    if (take_upd_fused(h) & 1) return RCN_OK;
-    return rcn_cuda_apply_gradients(h, eta, global);
+    RCN_ENTER(h);
+    if (B == 0) return accumulate_gradients(h, feats, onehot, labels, 0, StepRequest{}, nullptr);
+    const StepRequest req{step_update(h, eta / (double)(B * (size_t)(h->dp.connected ? h->dp.world : 1)))};
+    StepDone done;
+    RCN_TRY(accumulate_gradients(h, feats, onehot, labels, B, req, &done));
+    return finish_step(h, req.upd, done);
 }
 
 int rcn_cuda_train_batch_images(rcn_cuda_handle h, const void* images, int pixel_format, const int64_t* labels, size_t B,
                                 size_t H, size_t W, double eta) {
-    const size_t global = h ? B * (size_t)(h->dp.connected ? h->dp.world : 1) : B;
-    if (h && B) arm_fused_update(h, eta / (double)global, nullptr, 0, 0, nullptr);
-    const int rc = rcn_cuda_accumulate_gradients_images(h, images, pixel_format, labels, B, H, W);
-    if (rc != RCN_OK) { if (h) take_upd_fused(h); return rc; }
-    if (take_upd_fused(h) & 1) return RCN_OK;
-    return rcn_cuda_apply_gradients(h, eta, global);
+    RCN_ENTER(h);
+    if (B == 0) return accumulate_gradients_images(h, images, pixel_format, labels, 0, H, W, StepRequest{}, nullptr);
+    const StepRequest req{step_update(h, eta / (double)(B * (size_t)(h->dp.connected ? h->dp.world : 1)))};
+    StepDone done;
+    RCN_TRY(accumulate_gradients_images(h, images, pixel_format, labels, B, H, W, req, &done));
+    return finish_step(h, req.upd, done);
 }
 
 int rcn_cuda_last_batch_stats(rcn_cuda_handle h, double* cost, uint64_t* hits) {
@@ -959,8 +974,12 @@ int rcn_cuda_epoch_position(rcn_cuda_handle h, size_t* position) {
     return RCN_OK;
 }
 
-int rcn_cuda_epoch_accumulate(rcn_cuda_handle h) {
-    RCN_ENTER(h);
+// The update of a step over the bound dataset: it also advances the device-side cursor.
+static SnUpdate epoch_update(rcn_cuda_model* h, double scale) {
+    return step_update(h, scale, h->ep_state.as<long long>(), (long long)h->ep_B, (long long)h->ep_n);
+}
+
+static int epoch_accumulate(rcn_cuda_model* h, const StepRequest& req, StepDone* done) {
     RCN_TRY(require_params(h));
     if (!h->ep_images) return fail(RCN_ERR_STATE, "no dataset bound: call rcn_cuda_epoch_bind first");
     BatchIndex bi;
@@ -968,44 +987,32 @@ int rcn_cuda_epoch_accumulate(rcn_cuda_handle h) {
     bi.perm = (const long long*)h->ep_perm;
     bi.labels_all = (const long long*)h->ep_labels;
     bi.labels_batch = h->ep_state.as<long long>() + kEpSlots;
-    static const bool l2_prefetch = []() { const char* e = getenv("RCN_CUDA_L2_PREFETCH"); return !(e && e[0] == '0'); }();
-    if (l2_prefetch) {   // lets kernel A ask L2 for the next step's images (smallnet.cu)
-        bi.batch = (long long)h->ep_B;
-        bi.n_samples = (long long)h->ep_n;
-    }
-    return accumulate_images_dev(h, h->ep_images, h->ep_fmt, nullptr, h->ep_B, h->ep_H, h->ep_W, &bi);
+    bi.batch = (long long)h->ep_B;   // lets kernel A ask L2 for the next step's images (smallnet.cu)
+    bi.n_samples = (long long)h->ep_n;
+    return accumulate_images_dev(h, h->ep_images, h->ep_fmt, nullptr, h->ep_B, h->ep_H, h->ep_W, &bi, req, done);
 }
 
-static int epoch_apply_impl(rcn_cuda_model* h, double eta, size_t global_batch, bool cursor_done) {
-    if (global_batch == 0) return fail(RCN_ERR_INVALID, "global batch is zero");
-    const double scale = eta / (double)global_batch;
-    long long* cursor = cursor_done ? nullptr : h->ep_state.as<long long>();   // kernel B already advanced it
-    if (h->dp.connected) {
-        if (cursor) h->x_owns_cursor = true;
-        return launch_dp_allreduce_sgd(h->dp, h->params.as<double>(), h->grads, scale, h->stream, cursor, (long long)h->ep_B,
-                                       (long long)h->ep_n, nullptr, nullptr, take_dp_pushed(h), h->small_desc.tl);
-    }
-    return launch_sgd_update(h->params.as<double>(), h->grads, h->n_params, scale, h->stream, cursor, (long long)h->ep_B,
-                             (long long)h->ep_n, nullptr, nullptr);
+int rcn_cuda_epoch_accumulate(rcn_cuda_handle h) {
+    RCN_ENTER(h);
+    return epoch_accumulate(h, StepRequest{}, nullptr);
 }
 
 int rcn_cuda_epoch_apply(rcn_cuda_handle h, double eta, size_t global_batch) {
     RCN_ENTER(h);
     RCN_TRY(require_params(h));
     if (!h->ep_images) return fail(RCN_ERR_STATE, "no dataset bound: call rcn_cuda_epoch_bind first");
-    return epoch_apply_impl(h, eta, global_batch, false);
+    if (global_batch == 0) return fail(RCN_ERR_INVALID, "global batch is zero");
+    return finish_step(h, epoch_update(h, eta / (double)global_batch), StepDone::nothing);
 }
 
 int rcn_cuda_epoch_step(rcn_cuda_handle h, double eta) {
-    const size_t global = h ? h->ep_B * (size_t)(h->dp.connected ? h->dp.world : 1) : 0;
-    if (h && h->ep_images && h->ep_B)
-        arm_fused_update(h, eta / (double)global, h->ep_state.as<long long>(), (long long)h->ep_B, (long long)h->ep_n, nullptr);
-    const int rc = rcn_cuda_epoch_accumulate(h);
-    if (rc != RCN_OK) { if (h) take_upd_fused(h); return rc; }
-    const int fused = take_upd_fused(h);
-    if (fused & 1) return RCN_OK;
     RCN_ENTER(h);
-    return epoch_apply_impl(h, eta, global, (fused & 2) != 0);
+    RCN_TRY(require_params(h));
+    if (!h->ep_images) return fail(RCN_ERR_STATE, "no dataset bound: call rcn_cuda_epoch_bind first");
+    const StepRequest req{epoch_update(h, eta / (double)(h->ep_B * (size_t)(h->dp.connected ? h->dp.world : 1)))};
+    StepDone done;
+    RCN_TRY(epoch_accumulate(h, req, &done));
+    return finish_step(h, req.upd, done);
 }
 
 int rcn_cuda_epoch_run(rcn_cuda_handle h, double eta, size_t n_steps) {
@@ -1054,10 +1061,9 @@ int rcn_cuda_train_epoch_host(rcn_cuda_handle h, const void* images, int pixel_f
     // device ring while earlier chunks train; per-step results are written straight into pinned host memory; the host
     // launches CUDA graphs of several steps each and queues the copies.  It needs the staged front end (its image-loading
     // lanes wait for the arrival counter) and 64-bit stream memory operations (the copy stream's wait for free ring slots).
-    static const bool stream_env = []() { const char* e = getenv("RCN_CUDA_HOST_STREAMING"); return !(e && e[0] == '0'); }();
-    if (stream_env && pixel_format == RCN_PIXELS_U8_ROWMAJOR && h->use_small && B <= smallnet_max_batch() && img_bytes % 16 == 0 &&
+    if (pixel_format == RCN_PIXELS_U8_ROWMAJOR && h->use_small && B <= smallnet_max_batch() && img_bytes % 16 == 0 &&
         (reinterpret_cast<uintptr_t>(images) & 15) == 0 && is_pinned_host_ptr(images) && h->plan.L > 0 && h->plan.n_conv <= 10 &&
-        fused_front_enabled() && kHsRingSteps * B < (1ull << 31) && stream_mem_ops(h->device).ok) {
+        kHsRingSteps * B < (1ull << 31) && stream_mem_ops(h->device).ok) {
         SmallNetFront probe{};
         probe.H = (int)H; probe.W = (int)W; probe.max_elems = (int)h->plan.max_elems; probe.stages = h->plan.stages;
         cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
@@ -1121,13 +1127,13 @@ int rcn_cuda_train_epoch_host(rcn_cuda_handle h, const void* images, int pixel_f
             if (h->hs_graphs.empty() || !(key == h->hs_key)) {
                 for (auto& kv : h->hs_graphs) cudaGraphExecDestroy(kv.second);
                 h->hs_graphs.clear();
-                // warm-up outside capture: reserves every scratch buffer and sets kernel attributes (no parameter update)
-                h->dp_push_suppress = true;
+                // warm-up outside capture: reserves every scratch buffer and sets kernel attributes (no parameter update, no
+                // push to the peers)
                 BatchIndex bi_warm = bi;
                 bi_warm.arrived = nullptr;   // nothing has been copied yet: the warm-up trains on whatever the ring holds
-                const int wrc = accumulate_images_dev(h, h->hs_ring.p, pixel_format, nullptr, B, H, W, &bi_warm);
-                h->dp_push_suppress = false;
-                RCN_TRY(wrc);
+                StepRequest warm;
+                warm.push = false;
+                RCN_TRY(accumulate_images_dev(h, h->hs_ring.p, pixel_format, nullptr, B, H, W, &bi_warm, warm));
                 RCN_CUDA_TRY(cudaStreamSynchronize(h->stream));
                 key.alloc_gen = alloc_generation().load(std::memory_order_relaxed);   // the warm-up may have grown scratch buffers
                 h->hs_key = key;
@@ -1139,22 +1145,11 @@ int rcn_cuda_train_epoch_host(rcn_cuda_handle h, const void* images, int pixel_f
                     cudaGraph_t graph = nullptr;
                     RCN_CUDA_TRY(cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal));
                     int rc = RCN_OK;
+                    const StepRequest req{step_update(h, scale_s, st, (long long)B, kHsNoWrap, h->stats_host, true)};
                     for (int q = 0; q < g && rc == RCN_OK; ++q) {
-                        arm_fused_update(h, scale_s, st, (long long)B, kHsNoWrap, h->stats_host, true);
-                        rc = accumulate_images_dev(h, h->hs_ring.p, pixel_format, nullptr, B, H, W, &bi);
-                        const int fused = take_upd_fused(h);
-                        if (rc != RCN_OK) break;
-                        if (fused & 1) continue;   // the weight-gradient kernel applied the update, advanced the cursor, wrote the result
-                        // (fused & 2: kernel B advanced the cursor and wrote the result; the update kernel gets no cursor)
-                        long long* cur = (fused & 2) ? nullptr : st;
-                        if (h->dp.connected) {
-                            if (cur) h->x_owns_cursor = true;
-                            rc = launch_dp_allreduce_sgd(h->dp, h->params.as<double>(), h->grads, scale_s, h->stream, cur, (long long)B,
-                                                         kHsNoWrap, h->small.as<double>(), h->stats_host, take_dp_pushed(h), h->small_desc.tl);
-                        } else {
-                            rc = launch_sgd_update(h->params.as<double>(), h->grads, h->n_params, scale_s, h->stream, cur, (long long)B,
-                                                   kHsNoWrap, h->small.as<double>(), h->stats_host);
-                        }
+                        StepDone done;
+                        rc = accumulate_images_dev(h, h->hs_ring.p, pixel_format, nullptr, B, H, W, &bi, req, &done);
+                        if (rc == RCN_OK) rc = finish_step(h, req.upd, done);
                     }
                     cudaError_t ce = cudaStreamEndCapture(h->stream, &graph);
                     if (rc != RCN_OK) { if (graph) cudaGraphDestroy(graph); cudaGetLastError(); return rc; }
@@ -1246,7 +1241,8 @@ int rcn_cuda_train_epoch_host(rcn_cuda_handle h, const void* images, int pixel_f
     // everything the previous user of the staging slots enqueued on the compute stream must be finished first
     RCN_CUDA_TRY(cudaEventRecord(h->ev_consumed[0], h->stream));
     RCN_CUDA_TRY(cudaEventRecord(h->ev_consumed[1], h->stream));
-    const double scale = eta / (double)global_batch;   // (eta / batch.len() as f64)  (rcn.rs:214)
+    // unarmed: kernel B leaves the update to the update kernel (or the exchange kernel)
+    const SnUpdate update = step_update(h, eta / (double)global_batch);   // (eta / batch.len() as f64)  (rcn.rs:214)
     const char* img = (const char*)images;
     for (size_t k = 0; k < n_steps; ++k) {
         const int slot = (int)(k & 1);
@@ -1258,11 +1254,7 @@ int rcn_cuda_train_epoch_host(rcn_cuda_handle h, const void* images, int pixel_f
         RCN_CUDA_TRY(cudaStreamWaitEvent(h->stream, h->ev_copied[slot], 0));
         RCN_TRY(accumulate_images_dev(h, dst, pixel_format, labels_dev + k * B, B, H, W, nullptr));
         RCN_CUDA_TRY(cudaEventRecord(h->ev_consumed[slot], h->stream));
-        if (h->dp.connected)
-            RCN_TRY(launch_dp_allreduce_sgd(h->dp, h->params.as<double>(), h->grads, scale, h->stream, nullptr, 0, 0, nullptr, nullptr,
-                                            take_dp_pushed(h), h->small_desc.tl));
-        else
-            RCN_TRY(launch_sgd_update(h->params.as<double>(), h->grads, h->n_params, scale, h->stream));
+        RCN_TRY(finish_step(h, update, StepDone::nothing));
         // D2H of this step's result (cost, hits evaluated with the pre-update parameters)
         RCN_CUDA_TRY(cudaMemcpyAsync(h->stats_host + 2 * k, h->small.p, 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
     }

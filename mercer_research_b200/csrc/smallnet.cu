@@ -881,20 +881,11 @@ static void smallnet_splits(size_t B, int* splits, int* ksplit) {
 
 size_t smallnet_max_batch() { return (size_t)1 << 22; }
 
-// Programmatic dependent launch between the step's kernels: the launch latency of kernel N+1 overlaps kernel N
-// (RCN_CUDA_PDL=0 turns it off; measured on c2: gap A->B 2.9 -> 1.8 us, B->A 2.3 -> 1.95 us, step 22.25 -> 21.77 us).
-static bool sn_pdl_enabled() {
-    static const bool on = []() { const char* e = getenv("RCN_CUDA_PDL"); return !(e && e[0] == '0'); }();
-    return on;
-}
-
 // Highest launch priority for the training kernels: pending CTAs of kernels A / B win the SMs (kernel A needs a whole SM
 // per CTA) against lower-priority work queued on the same device.  (It was added against the SM-issued prefetch kernel of
 // the host-dataset loop, which no longer exists; whether it still pays has not been measured.)
 static int sn_high_priority() {
     static const int prio = []() {
-        const char* e = getenv("RCN_CUDA_LAUNCH_PRIORITY");
-        if (e && e[0] == '0') return 0;
         int least = 0, greatest = 0;
         if (cudaDeviceGetStreamPriorityRange(&least, &greatest) != cudaSuccess) { cudaGetLastError(); return 0; }
         return greatest;
@@ -937,18 +928,20 @@ static int launch_kernel_a(const SmallNetDesc& d, const double* params, double* 
         cfg.blockDim = dim3(SNA_THREADS, 1, 1);
         cfg.dynamicSmemBytes = smem;
         cfg.stream = stream;
+        // Programmatic dependent launch between the step's kernels: the launch latency of kernel N+1 overlaps kernel N
+        // (measured on c2 against launches without it: gap A->B 2.9 -> 1.8 us, B->A 2.3 -> 1.95 us, step 22.25 -> 21.77 us).
         cudaLaunchAttribute at[2];
         at[0].id = cudaLaunchAttributePriority;
         at[0].val.priority = sn_high_priority();
         at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
         at[1].val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = at;
-        cfg.numAttrs = sn_pdl_enabled() ? 2 : 1;
+        cfg.numAttrs = 2;
         RCN_LAUNCH(name, stream, cudaLaunchKernelEx(&cfg, kern, d, params, feats, Bi, onehot, labels, acts, deltas, stats_partial,
                                                     backward, front));
         return RCN_OK;
     };
-    if (fr && fr->use_cp && fr->prewait && backward && sn_pdl_enabled()) {
+    if (fr && fr->use_cp && fr->prewait && backward) {
         static SmemAttrCache attr;
         RCN_TRY(launch(smallnet_fwd_bwd_kernel<2, true>, attr,
                        fr->prewait == 2 ? "smallnet_fwd_bwd_kernel(fused features, front end ahead of the wait)"
@@ -1031,7 +1024,7 @@ int launch_smallnet_backprop(const SmallNetDesc& d, const double* params, double
     attr[2].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[2].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = sn_pdl_enabled() ? 3 : 2;
+    cfg.numAttrs = 3;
     const int Bi = (int)B;
     auto kern = mode == 1 ? smallnet_wgrad_kernel<1> : mode == 2 ? smallnet_wgrad_kernel<2> : smallnet_wgrad_kernel<0>;
     RCN_LAUNCH(mode == 2 ? "smallnet_wgrad_kernel(+SGD update)" : "smallnet_wgrad_kernel", stream,
