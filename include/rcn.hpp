@@ -305,6 +305,15 @@ class RCN {
         if (set.n) check(rcn_cuda_classify(h_, set.pixels.data(), RCN_PIXELS_U8_ROWMAJOR, set.n, set.h, set.w, labels.data()));
         return labels;
     }
+    /// Test-set evaluation (rcn.rs:152-157) of a decoded set standardised with scale_set: {accept, quadratic cost
+    /// sum_b 0.5*|a - y|^2}, with the exact-one-hot hit rule of the reference's epoch loop.
+    std::pair<uint64_t, double> evaluate_images(const GraySet& set) const {
+        uint64_t accept = 0;
+        double cost = 0.0;
+        check(rcn_cuda_evaluate_images(h_, set.pixels.data(), RCN_PIXELS_U8_ROWMAJOR, set.labels.data(), set.n, set.h, set.w,
+                                       &cost, &accept, nullptr));
+        return {accept, cost};
+    }
     /// classify(img_path) for a binary PGM; an unreadable file is an error value like the reference's `?` (rcn.rs:83).
     size_t classify_pgm(const std::string& img_path) const {
         std::vector<uint8_t> px;

@@ -115,6 +115,19 @@ int rcn_cuda_classify(rcn_cuda_handle h, const void* images, int pixel_format, s
                       int64_t* labels_out);
 /* Number of samples whose {i : a_i == max a} equals {label} exactly (rcn.rs:153-157). */
 int rcn_cuda_evaluate(rcn_cuda_handle h, const double* feats, const int64_t* labels, size_t B, uint64_t* accept);
+/* Test-set evaluation (rcn.rs:152-157) straight from images: features + standardise with scale_set
+ * (rcn.rs:84-89), forward, and per batch the quadratic cost sum_b 0.5*|a_L - y|^2 and the hit count of
+ * rcn_cuda_evaluate. labels_out (optional, may be NULL) receives the rcn.rs:92-97 argmax of every sample.
+ * images / labels / outputs may be host or device pointers. When images, labels, cost_out, accept_out and (if
+ * given) labels_out are all in device memory the call does not synchronise; it can then be captured into a CUDA
+ * graph once a call with at least as many images has run outside the capture (that call sizes the scratch
+ * buffers, see rcn_cuda_allocation_generation). A host pointer among them makes the call synchronise.
+ * Networks without the fused inference kernel (f64 pixels, a layer wider than 32, more than 4 layers) keep
+ * features and activations of the whole batch in the model's grow-only scratch buffers after the call.
+ * Leaves the gradient buffer, the epoch state and rcn_cuda_last_batch_stats untouched. */
+int rcn_cuda_evaluate_images(rcn_cuda_handle h, const void* images, int pixel_format, const int64_t* labels,
+                             size_t B, size_t H, size_t W, double* cost_out, uint64_t* accept_out,
+                             int64_t* labels_out);
 
 /* ---- training: backprop (rcn.rs:260-314) + train_batch (rcn.rs:176-223) ------------------------ */
 /* Targets: exactly one of `onehot` (classes x B, the reference's `y`) and `labels` (class index per sample,

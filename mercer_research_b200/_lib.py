@@ -51,6 +51,7 @@ SIGNATURES = {
     "rcn_cuda_classify_features": [_vp, _vp, _sz, _vp],
     "rcn_cuda_classify": [_vp, _vp, _i, _sz, _sz, _sz, _vp],
     "rcn_cuda_evaluate": [_vp, _vp, _vp, _sz, C.POINTER(C.c_uint64)],
+    "rcn_cuda_evaluate_images": [_vp, _vp, _i, _vp, _sz, _sz, _sz, _vp, _vp, _vp],
     "rcn_cuda_accumulate_gradients": [_vp, _vp, _vp, _vp, _sz],
     "rcn_cuda_accumulate_gradients_images": [_vp, _vp, _i, _vp, _sz, _sz, _sz],
     "rcn_cuda_apply_gradients": [_vp, _d, _sz],

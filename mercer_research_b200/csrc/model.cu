@@ -157,6 +157,7 @@ struct rcn_cuda_model {
     // scratch (grow-only)
     DevBuf in_stage, tgt_stage, feats, acts, deltas, gemm_ws, out_stage, small, red_ws;
     ReduceScratch rs;           // deterministic two-stage reductions (bias gradient, batch statistics)
+    ReduceScratch eval_rs;      // per-tile partials + ticket of the inference kernel (rcn_cuda_evaluate_images)
     // epoch mode (rcn.rs:144-149 on a resident dataset)
     const void* ep_images = nullptr;
     const int64_t* ep_labels = nullptr;
@@ -393,6 +394,24 @@ int accumulate_dev(rcn_cuda_model* h, const double* feats, const double* onehot,
     return RCN_OK;
 }
 
+// Can kernel A run the convpool stack of these images itself (narrow network, u8 pixels, a stack it implements)?
+bool fused_front_possible(const rcn_cuda_model* h, int fmt) {
+    return h->use_small && fmt == RCN_PIXELS_U8_ROWMAJOR && h->plan.n_conv <= 10 && h->plan.L > 0;
+}
+
+// Kernel A's front end for u8 DEVICE images (standardised with scale_set); `bi` optional, see below.
+SmallNetFront make_front(const rcn_cuda_model* h, const void* images, size_t H, size_t W, const BatchIndex* bi) {
+    SmallNetFront fr{};
+    fr.images = (const uint8_t*)images;
+    fr.H = (int)H; fr.W = (int)W;
+    fr.max_elems = (int)h->plan.max_elems;
+    fr.stages = h->plan.stages;
+    fr.sc = make_standardise(h->plan, RCN_PIXELS_U8_ROWMAJOR, true, h->mean, h->sd);
+    if (bi) fr.bi = *bi;
+    smallnet_front_select(h->plan, &fr);
+    return fr;
+}
+
 // images (DEVICE) -> gradient sums.  The canonical narrow network with u8 pixels runs the convpool stack inside
 // kernel A (smallnet.cu); everything else runs the feature kernel(s) first.  `bi` (optional) is the epoch-mode
 // device-side batch selection; without it `labels` are this batch's labels.
@@ -400,16 +419,8 @@ int accumulate_images_dev(rcn_cuda_model* h, const void* images, int fmt, const 
                           size_t W, const BatchIndex* bi, const StepRequest& req = {}, StepDone* done = nullptr) {
     RCN_TRY(h->feats.reserve(h->plan.L * B * sizeof(double)));
     const int64_t* step_labels = bi ? (const int64_t*)bi->labels_batch : labels;
-    if (h->use_small && B <= smallnet_max_batch() && fmt == RCN_PIXELS_U8_ROWMAJOR && h->plan.n_conv <= 10 &&
-        h->plan.L > 0) {
-        SmallNetFront fr{};
-        fr.images = (const uint8_t*)images;
-        fr.H = (int)H; fr.W = (int)W;
-        fr.max_elems = (int)h->plan.max_elems;
-        fr.stages = h->plan.stages;
-        fr.sc = make_standardise(h->plan, fmt, true, h->mean, h->sd);
-        if (bi) fr.bi = *bi;
-        smallnet_front_select(h->plan, &fr);
+    if (B <= smallnet_max_batch() && fused_front_possible(h, fmt)) {
+        SmallNetFront fr = make_front(h, images, H, W, bi);
         // Data-parallel step behind the exchange kernel: kernel A may run its front end ahead of griddepcontrol.wait
         // (smallnet.cu) when this step's kernel B pushes to the peers (so the exchange kernel X precedes the next kernel
         // A) and any device-side cursor it reads is advanced by kernel B -- this step's and the previous one's
@@ -522,7 +533,8 @@ int rcn_cuda_destroy(rcn_cuda_handle h) {
     dp_release(h->dp);
     h->oz.release();
     DevBuf* bufs[] = {&h->params, &h->grads_own, &h->in_stage, &h->tgt_stage, &h->feats, &h->acts, &h->deltas,
-                      &h->gemm_ws, &h->out_stage, &h->small, &h->red_ws, &h->ep_state, &h->fscratch.a, &h->fscratch.b, &h->rs.buf};
+                      &h->gemm_ws, &h->out_stage, &h->small, &h->red_ws, &h->ep_state, &h->fscratch.a, &h->fscratch.b, &h->rs.buf,
+                      &h->eval_rs.buf};
     for (DevBuf* b : bufs) b->release();
     delete h;
     return RCN_OK;
@@ -827,6 +839,59 @@ int rcn_cuda_evaluate(rcn_cuda_handle h, const double* feats, const int64_t* lab
     RCN_CUDA_TRY(cudaMemcpyAsync(host, st, sizeof(host), cudaMemcpyDeviceToHost, h->stream));
     RCN_CUDA_TRY(cudaStreamSynchronize(h->stream));
     *accept = host[1];
+    return RCN_OK;
+}
+
+int rcn_cuda_evaluate_images(rcn_cuda_handle h, const void* images, int pixel_format, const int64_t* labels, size_t B, size_t H,
+                             size_t W, double* cost_out, uint64_t* accept_out, int64_t* labels_out) {
+    RCN_ENTER(h);
+    RCN_TRY(require_params(h));
+    if (pixel_format != RCN_PIXELS_U8_ROWMAJOR && pixel_format != RCN_PIXELS_F64_COLMAJOR)
+        return fail(RCN_ERR_INVALID, "unknown pixel format %d", pixel_format);
+    if (B == 0) {
+        if (cost_out && is_device_ptr(cost_out)) RCN_CUDA_TRY(cudaMemsetAsync(cost_out, 0, sizeof(double), h->stream));
+        else if (cost_out) *cost_out = 0.0;
+        if (accept_out && is_device_ptr(accept_out)) RCN_CUDA_TRY(cudaMemsetAsync(accept_out, 0, sizeof(uint64_t), h->stream));
+        else if (accept_out) *accept_out = 0;
+        return RCN_OK;
+    }
+    if (!images || !labels || !cost_out || !accept_out) return fail(RCN_ERR_INVALID, "null images / labels / cost / accept");
+    RCN_TRY(ensure_plan(h, H, W));
+    RCN_TRY(check_feature_width(h, h->plan.L));
+    bool host_in = false;
+    StagedIn in, lb;
+    RCN_TRY(in.stage(images, B * H * W * pixel_bytes(pixel_format), h->in_stage, h->stream, &host_in));
+    RCN_TRY(lb.stage(labels, B * sizeof(int64_t), h->tgt_stage, h->stream, &host_in));
+    const int64_t* lab_in = (const int64_t*)lb.dev;
+    RCN_TRY(h->small.reserve(64));
+    double* st = h->small.as<double>() + 6;   // {cost, hits}: not the words behind rcn_cuda_last_batch_stats (0, 1)
+    int64_t* lab_dev = labels_out;
+    const bool lab_host = labels_out && !is_device_ptr(labels_out);
+    if (lab_host) { RCN_TRY(h->out_stage.reserve(B * sizeof(int64_t))); lab_dev = h->out_stage.as<int64_t>(); }
+    bool done = false;
+    if (fused_front_possible(h, pixel_format)) {
+        // One launch, the front end inside the inference kernel.  Measured against the feature kernel followed by the
+        // inference kernel on the features (profiles/eval_routes_b200.txt, B200 at 1000 W) it was faster from 64 to
+        // 1 048 576 images (9.42 against 9.69 ms at 1 048 576) and equal at 1, so that route was not kept.
+        const SmallNetFront fr = make_front(h, in.dev, H, W, nullptr);
+        if (smallnet_front_fits(h->small_desc, fr)) {
+            RCN_TRY(launch_smallnet_infer(h->small_desc, h->params.as<double>(), B, lab_in, lab_dev, st, h->eval_rs, fr, h->stream));
+            done = true;
+        }
+    }
+    if (!done) {   // the existing kernels: features + standardise, forward, batch statistics, argmax
+        RCN_TRY(h->feats.reserve(h->plan.L * B * sizeof(double)));
+        RCN_TRY(launch_features(h->plan, in.dev, pixel_format, B, H, W, true, h->mean, h->sd, h->feats.as<double>(), h->fscratch,
+                                h->stream));
+        RCN_TRY(forward_dev(h, h->feats.as<double>(), B, nullptr, nullptr, false));
+        const size_t n = h->rows.size();
+        RCN_TRY(launch_batch_stats(h->act(n - 1, B), h->rows[n - 1], B, nullptr, lab_in, st, h->rs, h->stream));
+        if (labels_out) RCN_TRY(launch_argmax_last(h->act(n - 1, B), h->rows[n - 1], B, lab_dev, h->stream));
+    }
+    if (lab_host) RCN_TRY(deliver(h, labels_out, lab_dev, B * sizeof(int64_t)));
+    RCN_TRY(deliver(h, cost_out, st, sizeof(double)));
+    RCN_TRY(deliver(h, accept_out, st + 1, sizeof(uint64_t)));
+    if (host_in) RCN_CUDA_TRY(cudaStreamSynchronize(h->stream));   // the caller may reuse its host buffers
     return RCN_OK;
 }
 

@@ -83,7 +83,8 @@ constexpr int SN_U = 7;           // k-steps of W0 fragments a warp keeps in reg
 constexpr int SN_ZPITCH = 36;     // layer-0 partial sums [warp][sample][36]: conflict-free for the DMMA C fragments and the row reads
 constexpr int SN_MAX_SMALL = 32 + (kSmallNetMaxLayers - 1) * (32 * 32 + 32);  // params after W0
 
-// final-stage emit of the fused front end: standardised feature -> shared tile + HBM
+// final-stage emit of the fused front end: standardised feature -> shared tile + HBM (TO_HBM = false: the tile only)
+template <bool TO_HBM>
 struct EmitTile {
     double* tile; double* gout; int h, hw; Standardise sc;
     __device__ __forceinline__ void operator()(int slot, int y, int x, int v) const {
@@ -100,7 +101,7 @@ struct EmitTile {
         }
         const int idx = slot * hw + x * h + y;
         tile[idx] = d;
-        gout[idx] = d;
+        if (TO_HBM) gout[idx] = d;
     }
 };
 
@@ -123,19 +124,29 @@ __device__ __forceinline__ unsigned char* sn_align128(void* p) {
     return reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(p) + 127) & ~(uintptr_t)127);
 }
 
+// What the inference variant of kernel A (smallnet_infer_kernel) writes besides its per-tile {cost, hits} partials.
+struct SnInfer {
+    int64_t* labels_out;     // optional: argmax of every sample (argmax_last_kernel's rule)
+    unsigned* ticket;        // zero before the launch; the last CTA resets it
+    double* stats;           // {cost, hits as uint64 bits} of the launch
+    int accumulate;          // add to stats instead of overwriting them (the chunks of a batch above smallnet_max_batch())
+};
+
 // ------------------------------------------------------------------------------------------------
 // Kernel A
 // ------------------------------------------------------------------------------------------------
 // FUSED 0: features are an input; 1: generic fused front end; 2: staged front end (CpPlan).
 // PREWAIT (FUSED == 2, data-parallel groups): the whole front end runs before griddepcontrol.wait -- under the previous
 // step's exchange kernel -- and only the parameter loads wait for it (see the file header for why that is safe).
-template <int FUSED, bool PREWAIT>
+// INFER (smallnet_infer_kernel, backward == 0): forward only, nothing but the statistics partials, `inf.stats` and
+// `inf.labels_out` goes to global memory -- the features stay in the shared tile and the activations on chip.
+template <int FUSED, bool PREWAIT, bool INFER>
 __device__ __forceinline__ void sn_phase_a(const SmallNetDesc& d, const double* __restrict__ params,
                                            double* __restrict__ feats, int B, const double* __restrict__ onehot,
                                            const int64_t* __restrict__ labels, double* __restrict__ acts,
                                            double* __restrict__ deltas, double* __restrict__ stats_partial,
                                            int backward, const SmallNetFront& fr,
-                                           const int tile_idx, unsigned char* sn_smem) {
+                                           const int tile_idx, unsigned char* sn_smem, const SnInfer& inf) {
     double* zpart = reinterpret_cast<double*>(sn_smem);                 // [16][8][36]
     double* s_small = zpart + SNA_WARPS * SN_TB * SN_ZPITCH;                   // params after W0: b0 | W1 | b1 | ...
     double* tile = s_small + SN_MAX_SMALL;                              // FUSED: [8][n_in + 4]
@@ -260,7 +271,8 @@ __device__ __forceinline__ void sn_phase_a(const SmallNetDesc& d, const double* 
                 const int itl = it - gi * items;
                 const int* in = tiles + gi * fr.cp.tile_ints + st.off;
                 int* nxt = tiles + gi * fr.cp.tile_ints + nx.off;
-                CpSinkTile<PREWAIT> sink{tile + (size_t)gi * pitch, (PREWAIT && fr.prewait == 2) ? nullptr : feats + (size_t)(s0 + gi) * L, fr.sc};
+                CpSinkTile<PREWAIT || INFER> sink{tile + (size_t)gi * pitch,
+                                                  (INFER || (PREWAIT && fr.prewait == 2)) ? nullptr : feats + (size_t)(s0 + gi) * L, fr.sc};
                 if (last) {
                     if (q == 0) cp_item<true, true>(st, in, itl, nullptr, 0, 0, sink);
                     else cp_item<true, false>(st, in, itl, nullptr, 0, 0, sink);
@@ -299,7 +311,7 @@ __device__ __forceinline__ void sn_phase_a(const SmallNetDesc& d, const double* 
             const Stage& st = fr.stages.s[s];
             if (live) {
                 if (s == fr.stages.n - 1) {
-                    EmitTile e{trow, feats + (size_t)sample * L, st.h_out, st.h_out * st.w_out, fr.sc};
+                    EmitTile<!INFER> e{trow, INFER ? nullptr : feats + (size_t)sample * L, st.h_out, st.h_out * st.w_out, fr.sc};
                     run_stage<int>(st, cur, e, lt, 64);
                 } else {
                     EmitMaps<int> e{nxt, st.h_out, st.h_out * st.w_out};
@@ -434,7 +446,7 @@ __device__ __forceinline__ void sn_phase_a(const SmallNetDesc& d, const double* 
         }
         SN_PHASE(5);
         // ---- activations out ---------------------------------------------------------------------------------------
-        {
+        if constexpr (!INFER) {
             int off = 0;
 #pragma unroll
             for (int l = 0; l < kSmallNetMaxLayers; ++l) {
@@ -446,13 +458,15 @@ __device__ __forceinline__ void sn_phase_a(const SmallNetDesc& d, const double* 
             }
         }
         SN_PHASE(18);
-        if (backward) {
+        if (INFER || backward) {
             // ---- output delta (rcn.rs:299) and batch statistics (rcn.rs:152-157) ---------------------------------------
             const bool out = m < RL;
             double y = 0.0;
             if (out && live) y = onehot ? onehot[(size_t)sample * RL + m] : ((s_label[n] == (long long)m) ? 1.0 : 0.0);
             const double a = out ? s_act[last][n][m] : 0.0;
-            if (out) s_del[last][n][m] = (a - y) * (a * (1.0 - a));
+            if constexpr (!INFER) {
+                if (out) s_del[last][n][m] = (a - y) * (a * (1.0 - a));
+            }
             {
                 double mx = out ? a : -1.0;                        // activations are in (0, 1)
                 const double df = a - y;                           // 0 for lanes beyond the output layer
@@ -468,6 +482,19 @@ __device__ __forceinline__ void sn_phase_a(const SmallNetDesc& d, const double* 
                     s_hit[n] = (live && ok) ? 1ull : 0ull;
                 }
             }
+            if constexpr (INFER) {
+                // the class label with argmax_last_kernel's sequential scan: last maximal element wins (rcn.rs:92-97), and a
+                // NaN output gives the label classify gives
+                if (inf.labels_out && live && m == 0) {
+                    int best = 0;
+                    double bv = s_act[last][n][0];
+                    for (int i = 1; i < RL; ++i) {
+                        const double v = s_act[last][n][i];
+                        if (!(v < bv)) { bv = v; best = i; }
+                    }
+                    inf.labels_out[sample] = best;
+                }
+            } else {
             SN_PHASE(19);
             __syncwarp();
             // ---- backward-data chain (rcn.rs:305-309) -------------------------------------------------------------------
@@ -504,10 +531,11 @@ __device__ __forceinline__ void sn_phase_a(const SmallNetDesc& d, const double* 
                     off += R;
                 }
             }
+            }   // !INFER
         }
     }
     SN_PHASE(21);
-    if (!backward) { RCN_TL_END(d.tl, 0); return; }
+    if (!INFER && !backward) { RCN_TL_END(d.tl, 0); return; }
     __syncthreads();
     SN_PHASE(6);
     if (tid == SNA_THREADS - 32) {
@@ -517,6 +545,78 @@ __device__ __forceinline__ void sn_phase_a(const SmallNetDesc& d, const double* 
         for (int i = 0; i < SN_TB; ++i) { c += s_cost[i]; h += s_hit[i]; }
         stats_partial[2 * tile_idx] = c;
         reinterpret_cast<unsigned long long*>(stats_partial)[2 * tile_idx + 1] = h;
+    }
+    if constexpr (INFER) {
+        // ---- the last CTA to finish (ticket after a fence, as batch_stats_kernel) adds the partials in exactly the order of
+        // kernel B's statistics CTA: same partials, same order, so the result is bit-identical to the training step's
+        // {cost, hits} on the same batch.  It resets the ticket, so a captured launch can be replayed.
+        __shared__ bool s_last;
+        if (tid == SNA_THREADS - 32) {
+            __threadfence();
+            const unsigned t = atomicAdd(inf.ticket, 1u);
+            s_last = (t == gridDim.x - 1);
+            if (s_last) *inf.ticket = 0;
+        }
+        __syncthreads();
+        if (s_last) {   // uniform across the CTA
+            const int n_stat = (int)gridDim.x;
+            const int per_l = (n_stat + 31) / 32;
+            // Lane l of warp 0 adds partials l*per_l, l*per_l + 1, ... in order.  Up to SN_RJ partials per lane it loads them
+            // itself; above that (B > 16 384) the loads are not left to one warp, a chain of dependent L2 round trips that
+            // grows with B: all 16 warps stage SN_RJ consecutive partials of every lane's range into shared memory (the layer-0
+            // partial-sum area, free by now) and warp 0 folds them, in the same order.  Measured with profiles/eval_bench.py on
+            // B200s at 1000 W (separate runs), staging at every size against the warp-0 loop: 9.42 against 9.53 ms at
+            // B = 1 048 576, equal at 10 000, 16.4 against 14.4 us at B = 1.
+            constexpr int SN_RJ = 64, SN_RPITCH = SN_RJ + 1;       // odd pitch: lane l's row starts in bank 2l mod 32
+            double c = 0.0;
+            unsigned long long h = 0;
+            if (per_l <= SN_RJ) {
+                if (warp != 0) return;
+                __threadfence();
+                for (int i = lane * per_l; i < min(n_stat, (lane + 1) * per_l); ++i) {
+                    c += __ldcg(stats_partial + 2 * i);
+                    h += __ldcg(reinterpret_cast<const unsigned long long*>(stats_partial) + 2 * i + 1);
+                }
+            } else {
+                __threadfence();
+                double* rc = zpart;
+                unsigned long long* rh = reinterpret_cast<unsigned long long*>(zpart + 32 * SN_RPITCH);
+                for (int j0 = 0; j0 < per_l; j0 += SN_RJ) {
+                    for (int e = tid; e < 32 * SN_RJ; e += SNA_THREADS) {
+                        const int l = e / SN_RJ, jj = e - l * SN_RJ;
+                        const int i = l * per_l + j0 + jj;
+                        if (j0 + jj < per_l && i < n_stat) {
+                            rc[l * SN_RPITCH + jj] = __ldcg(stats_partial + 2 * i);
+                            rh[l * SN_RPITCH + jj] = __ldcg(reinterpret_cast<const unsigned long long*>(stats_partial) + 2 * i + 1);
+                        }
+                    }
+                    __syncthreads();
+                    if (warp == 0) {
+                        const int n_j = min(SN_RJ, min(per_l, n_stat - lane * per_l) - j0);
+                        for (int jj = 0; jj < n_j; ++jj) {
+                            c += rc[lane * SN_RPITCH + jj];
+                            h += rh[lane * SN_RPITCH + jj];
+                        }
+                    }
+                    __syncthreads();
+                }
+                if (warp != 0) return;
+            }
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) {
+                c += __shfl_down_sync(0xffffffffu, c, o);
+                h += __shfl_down_sync(0xffffffffu, h, o);
+            }
+            if (lane == 0) {
+                if (inf.accumulate) {   // chunks in order: ((c0 + c1) + c2) ...
+                    c = inf.stats[0] + c;
+                    h += reinterpret_cast<const unsigned long long*>(inf.stats)[1];
+                }
+                inf.stats[0] = c;
+                reinterpret_cast<unsigned long long*>(inf.stats)[1] = h;
+            }
+        }
+        return;
     }
     // ---- epoch mode: ask L2 for the images this tile will load in the NEXT step (same tile index, cursor advanced like the
     // update does, rcn.rs:147): 20 us from now their bulk loads hit L2 instead of paying an HBM round trip at the head of
@@ -540,8 +640,22 @@ smallnet_fwd_bwd_kernel(const __grid_constant__ SmallNetDesc d, const double* __
                         const int64_t* __restrict__ labels, double* __restrict__ acts, double* __restrict__ deltas,
                         double* __restrict__ stats_partial, int backward, const __grid_constant__ SmallNetFront fr) {
     extern __shared__ __align__(128) unsigned char sn_smem[];
-    sn_phase_a<FUSED, PREWAIT>(d, params, feats, B, onehot, labels, acts, deltas, stats_partial, backward, fr,
-                               (int)blockIdx.x, sn_smem);
+    sn_phase_a<FUSED, PREWAIT, false>(d, params, feats, B, onehot, labels, acts, deltas, stats_partial, backward, fr,
+                                      (int)blockIdx.x, sn_smem, SnInfer{});
+}
+
+// Inference variant of kernel A (test-set evaluation): the same front end and forward pass per tile of 8 samples, then the
+// cost and hit rule of the training epilogue, the optional argmax labels, and one {cost, hits} for the whole launch.
+// FUSED 1 / 2: the features are computed from `fr.images` and stay in shared memory.
+template <int FUSED>
+__global__ void __launch_bounds__(SNA_THREADS, 1)
+smallnet_infer_kernel(const __grid_constant__ SmallNetDesc d, const double* __restrict__ params, int B,
+                      const int64_t* __restrict__ labels, double* __restrict__ stats_partial, const __grid_constant__ SnInfer inf,
+                      const __grid_constant__ SmallNetFront fr) {
+    static_assert(FUSED == 1 || FUSED == 2, "the inference kernel runs the fused front end");
+    extern __shared__ __align__(128) unsigned char sn_smem[];
+    sn_phase_a<FUSED, false, true>(d, params, nullptr, B, nullptr, labels, nullptr, nullptr, stats_partial, 0,
+                                   fr, (int)blockIdx.x, sn_smem, inf);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -963,6 +1077,46 @@ int launch_smallnet_forward(const SmallNetDesc& d, const double* params, double*
                             const SmallNetFront* front, cudaStream_t stream) {
     if (B == 0) return RCN_OK;
     return launch_kernel_a(d, params, feats, B, nullptr, nullptr, acts, nullptr, nullptr, 0, front, stream);
+}
+
+int launch_smallnet_infer(const SmallNetDesc& d, const double* params, size_t B, const int64_t* labels, int64_t* labels_out,
+                          double* stats, ReduceScratch& ws, const SmallNetFront& front, cudaStream_t stream) {
+    if (B == 0) return RCN_OK;
+    const size_t chunk_max = smallnet_max_batch();
+    RCN_TRY(ws.ensure(2 * (size_t)cdiv(B < chunk_max ? B : chunk_max, SN_TB) * sizeof(double), stream));
+    SmallNetDesc di = d;
+    di.tl = nullptr;                     // the launch timeline records the training kernels only
+    const size_t smem = kernel_a_smem(d, &front);
+    for (size_t c0 = 0; c0 < B; c0 += chunk_max) {
+        const size_t n = B - c0 < chunk_max ? B - c0 : chunk_max;
+        SnInfer inf{labels_out ? labels_out + c0 : nullptr, ws.tickets(), stats, c0 > 0 ? 1 : 0};
+        SmallNetFront fr = front;
+        fr.images += c0 * (size_t)fr.H * fr.W;
+        auto launch = [&](auto kern, SmemAttrCache& attr, const char* name) -> int {
+            if (attr.need(smem)) RCN_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            cudaLaunchConfig_t cfg{};
+            cfg.gridDim = dim3(cdiv(n, SN_TB), 1, 1);
+            cfg.blockDim = dim3(SNA_THREADS, 1, 1);
+            cfg.dynamicSmemBytes = smem;
+            cfg.stream = stream;
+            // as the forward-only launch of kernel A: griddepcontrol.wait before any memory access, no early trigger
+            cudaLaunchAttribute at[1];
+            at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+            at[0].val.programmaticStreamSerializationAllowed = 1;
+            cfg.attrs = at;
+            cfg.numAttrs = 1;
+            RCN_LAUNCH(name, stream, cudaLaunchKernelEx(&cfg, kern, di, params, (int)n, labels + c0, ws.partials(), inf, fr));
+            return RCN_OK;
+        };
+        if (front.use_cp) {
+            static SmemAttrCache attr;
+            RCN_TRY(launch(smallnet_infer_kernel<2>, attr, "smallnet_infer_kernel(fused features)"));
+        } else {
+            static SmemAttrCache attr;
+            RCN_TRY(launch(smallnet_infer_kernel<1>, attr, "smallnet_infer_kernel(fused features, generic front end)"));
+        }
+    }
+    return RCN_OK;
 }
 
 int launch_smallnet_backprop(const SmallNetDesc& d, const double* params, double* feats, size_t B, const double* onehot,

@@ -61,6 +61,12 @@ bool smallnet_front_fits(const SmallNetDesc& d, const SmallNetFront& fr);
 // With a front end, `feats` (n_in x B) is an OUTPUT (kernel B and the parity taps read it); without, an input.
 int launch_smallnet_forward(const SmallNetDesc& d, const double* params, double* feats, size_t B, double* acts,
                             const SmallNetFront* front, cudaStream_t stream);
+// Test-set evaluation (rcn.rs:152-157) in the inference variant of kernel A, from the u8 images of `front`: stats[0..1] =
+// quadratic cost and hit count (uint64 bits) of the whole batch, bit-identical to what launch_smallnet_backprop reports for
+// it; labels_out (optional) the argmax of every sample.  The features never leave shared memory.  Batches above
+// smallnet_max_batch() run as consecutive launches of that size.  Writes nothing else but `ws`.
+int launch_smallnet_infer(const SmallNetDesc& d, const double* params, size_t B, const int64_t* labels, int64_t* labels_out,
+                          double* stats, ReduceScratch& ws, const SmallNetFront& front, cudaStream_t stream);
 // Full backprop of a minibatch: fills acts, deltas, the flat gradient buffer (batch sums) and stats[0..1]
 // (quadratic cost, hit count as uint64 bits).
 int launch_smallnet_backprop(const SmallNetDesc& d, const double* params, double* feats, size_t B, const double* onehot,

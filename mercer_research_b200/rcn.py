@@ -336,6 +336,30 @@ class RCN:
         _lib.check(self._lib.rcn_cuda_evaluate(self._h, f.ptr, l.ptr, f.shape[0], C.byref(acc)))
         return acc.value
 
+    def evaluate_images(self, images, labels, want_labels: bool = False):
+        """Test-set evaluation (rcn.rs:152-157) of a batch of decoded grayscale images, standardised with ``scale_set``:
+        ``(accept, cost)`` -- the exact-one-hot hit count of ``evaluate`` and the quadratic cost sum_b 0.5*|a - y|^2 --
+        and with ``want_labels`` also the ``classify_images`` labels, ``(accept, cost, labels)``."""
+        self._require_params()
+        buf, fmt, (B, H, W) = self._images(images)
+        lb = _Buf(labels, np.int64)
+        self._use_torch_stream(buf, lb)
+        cost, acc = C.c_double(), C.c_uint64()
+        o, optr = None, None
+        if want_labels:
+            if buf.torch:
+                import torch
+                o = torch.empty((B,), dtype=torch.int64, device=buf.device)
+                optr = o.data_ptr()
+            else:
+                o = np.zeros(B, dtype=np.int64)
+                optr = o.ctypes.data
+        _lib.check(self._lib.rcn_cuda_evaluate_images(self._h, buf.ptr, fmt, lb.ptr, B, H, W, C.addressof(cost),
+                                                      C.addressof(acc), optr))
+        if want_labels:
+            return acc.value, cost.value, o
+        return acc.value, cost.value
+
     # -- training ---------------------------------------------------------------------------------------------
     def _targets(self, onehot, labels):
         oh = _Buf(onehot, np.float64) if onehot is not None else None
@@ -587,10 +611,7 @@ class RCN:
                     else:
                         self.epoch_step(eta)
             self.scale_set = te_stats
-            accept = 0
-            for i in range(0, int(te.shape[0]), 16384):
-                feats = self.flatten_feature_set(te[i:i + 16384], standardise=True)
-                accept += self.evaluate(feats, te_y[i:i + 16384])
+            accept, _ = self.evaluate_images(te, te_y)
             history.append(accept)
             if log:
                 log("Epoch {}: {}/{} [{:.2f}%]".format(e, accept, int(te.shape[0]), accept / max(1, int(te.shape[0])) * 100.0))

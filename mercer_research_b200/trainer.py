@@ -8,7 +8,8 @@ identical ``W -= (eta / B_global) * g`` (rcn.rs:210-222), so replicas stay bit-i
 the single-GPU result only by summation order (SURVEY.md 8e). No other collective is on the data path.
 
 The compute backend is any object with ``n_params``, ``bind_gradient_buffer(t)``, ``accumulate_gradients_images``,
-``accumulate_gradients``, ``apply_gradients`` and ``last_batch_stats`` -- in the product that is ``RCN`` (CUDA);
+``accumulate_gradients``, ``apply_gradients`` and ``last_batch_stats`` (``evaluate`` also needs ``evaluate_images``) --
+in the product that is ``RCN`` (CUDA);
 the gloo CPU tests plug in a checker-backed stand-in to exercise exactly this host logic without a GPU.
 
 Stream discipline: the library launches on the stream bound with ``set_stream``; the NCCL collective is ordered against
@@ -71,7 +72,8 @@ class DataParallelTrainer:
         import torch
         self.model.set_stream(torch.cuda.current_stream(self.device).cuda_stream)
 
-    def _same_on_all_ranks(self, value: int, what: str):
+    def _same_on_all_ranks(self, value: int, what: str,
+                           rule: str = "every rank must run the same number of steps per epoch"):
         """Every rank must run the same number of exchanges: a rank with fewer steps would leave its peers waiting for
         gradients that never come (the peer-memory receive would time out, the NCCL all-reduce would hang)."""
         if self.world == 1:
@@ -82,8 +84,7 @@ class DataParallelTrainer:
         self.dist.all_reduce(t, op=self.dist.ReduceOp.MIN, group=self.group)
         lo, hi = int(t[0].item()), -int(t[1].item())
         if lo != hi:
-            raise ValueError(f"{what} differs across ranks (min {lo}, max {hi}; this rank {int(value)}): "
-                             "every rank must run the same number of steps per epoch")
+            raise ValueError(f"{what} differs across ranks (min {lo}, max {hi}; this rank {int(value)}): {rule}")
 
     def check(self):
         """Synchronises; raises if a peer-memory exchange timed out (dead or desynchronised rank)."""
@@ -140,6 +141,32 @@ class DataParallelTrainer:
         """Convenience: every rank passes the same GLOBAL batch and trains on its own contiguous shard of it."""
         lo, hi = shard_bounds(int(images.shape[0]), self.rank, self.world)
         self.step_images(images[lo:hi], labels[lo:hi])
+
+    def evaluate(self, images, labels) -> Tuple[int, float]:
+        """Test-set evaluation (rcn.rs:152-157) across the group: every rank passes the same GLOBAL set and evaluates a
+        contiguous near-equal shard of it (the first ``n % world`` ranks take one sample more; a shard may be empty).
+        Returns ``(accept, cost)`` of the whole set, identical on every rank: the hit counts are all-reduced, the costs
+        gathered and added in rank order."""
+        n = int(images.shape[0])
+        self._same_on_all_ranks(n, "the evaluation set size", "every rank must pass the same global set")
+        per, extra = divmod(n, self.world)
+        lo = self.rank * per + min(self.rank, extra)
+        hi = lo + per + (1 if self.rank < extra else 0)
+        self._bind_stream()
+        accept, cost = self.model.evaluate_images(images[lo:hi], labels[lo:hi])
+        if self.world == 1:
+            return int(accept), float(cost)
+        import torch
+        dev = self.device if self.device.type == "cuda" else torch.device("cpu")
+        acc = torch.tensor([int(accept)], dtype=torch.int64, device=dev)
+        self.dist.all_reduce(acc, op=self.dist.ReduceOp.SUM, group=self.group)
+        mine = torch.tensor([float(cost)], dtype=torch.float64, device=dev)
+        costs = [torch.zeros_like(mine) for _ in range(self.world)]
+        self.dist.all_gather(costs, mine, group=self.group)
+        total = 0.0
+        for c in costs:          # rank order: every rank adds the same values in the same order
+            total += float(c.item())
+        return int(acc.item()), total
 
     # -- epoch mode: device-resident dataset, device-side batch cursor, one CUDA graph per step shape ---------------
     def bind_dataset(self, images, labels, batch: int, perm=None):

@@ -45,6 +45,9 @@ extern "C" {
                              labels_out: *mut i64) -> c_int;
     pub fn rcn_cuda_evaluate(h: rcn_cuda_handle, feats: *const c_double, labels: *const i64, B: usize,
                              accept: *mut u64) -> c_int;
+    pub fn rcn_cuda_evaluate_images(h: rcn_cuda_handle, images: *const c_void, pixel_format: c_int, labels: *const i64,
+                                    B: usize, H: usize, W: usize, cost_out: *mut c_double, accept_out: *mut u64,
+                                    labels_out: *mut i64) -> c_int;
     pub fn rcn_cuda_train_batch(h: rcn_cuda_handle, feats: *const c_double, onehot: *const c_double, labels: *const i64,
                                 B: usize, eta: c_double) -> c_int;
     pub fn rcn_cuda_train_batch_images(h: rcn_cuda_handle, images: *const c_void, pixel_format: c_int, labels: *const i64,

@@ -231,6 +231,18 @@ pub mod rcn {
             Ok(label as usize)
         }
 
+        /// rcn.rs:152-157 on `n` decoded h x w Luma8 images (row-major, back to back) standardised with scale_set:
+        /// (accept, quadratic cost sum_b 0.5*|a - y|^2) in one call, without materialising the features.
+        pub fn evaluate_images(&self, pixels: &[u8], labels: &[i64], n: usize, h: usize, w: usize) -> (u64, f64) {
+            assert!(pixels.len() == n * h * w && labels.len() == n, "evaluate_images: {} images of {}x{} expected", n, h, w);
+            let (mut accept, mut cost) = (0u64, 0f64);
+            let _one_at_a_time = self.gate.lock().unwrap();
+            check(unsafe { ffi::rcn_cuda_evaluate_images(self.handle, pixels.as_ptr() as *const c_void,
+                                                         ffi::RCN_PIXELS_U8_ROWMAJOR, labels.as_ptr(), n, h, w, &mut cost,
+                                                         &mut accept, ptr::null_mut()) });
+            (accept, cost)
+        }
+
         /// rcn.rs:126-167. Host: directory walk, sampling, PNG decode, shuffle. GPU: everything else -- the feature
         /// stage and the statistics of each set, the `chunks_exact` loop (one call per epoch, the next chunk is pulled
         /// over PCIe while the current one trains) and the per-epoch evaluation on the HBM-resident test features.
