@@ -8,6 +8,7 @@
 #include <memory>
 #include <mutex>
 #include <new>
+#include <tuple>
 #include <vector>
 
 #include "dense.cuh"
@@ -89,8 +90,9 @@ static int hs_steps_per_graph() {
 // the copy stream itself -- cuStreamWriteValue64 or the 8-byte copy -- put ~22 us between consecutive data copies, which then
 // no longer pipeline: a one-chunk copy took 40 us instead of 18 and the copy stream became the bottleneck.)  Round 1's
 // design -- a prefetch kernel pulling each chunk with zero-copy loads on a parallel graph branch -- measured slower end to
-// end (42.8-43.9 M against 48.5-49.5 M images/s) and was removed; without stream memory operations or the staged front end
-// the call takes the general double-buffered loop.
+// end (42.8-43.9 M against 48.5-49.5 M images/s) and was removed.  The call streams only when the steps on the ring run
+// kernel A with the staged front end (fused_front, the rule of every training step) and the device has 64-bit stream
+// memory operations; otherwise it takes the general double-buffered loop.
 constexpr size_t kHsRingSteps = 64;   // chunks the ring holds
 constexpr size_t kHsQuarter = kHsRingSteps / 4;   // granularity of the copy stream's wait for free ring slots
 constexpr size_t kHsMaxCopy = 8;      // chunks per cudaMemcpyAsync once the ramp is over (divides kHsQuarter)
@@ -124,6 +126,69 @@ bool is_pinned_host_ptr(const void* p) {
     return a.type == cudaMemoryTypeHost && a.devicePointer != nullptr;
 }
 
+// Grow-only pinned host table of `T`: the host-side counterpart of DevBuf.
+template <typename T> struct PinnedBuf {
+    T* p = nullptr;
+    size_t cap = 0;
+    int reserve(size_t n) {
+        if (n <= cap) return RCN_OK;
+        release();
+        RCN_CUDA_TRY(cudaHostAlloc((void**)&p, n * sizeof(T), cudaHostAllocDefault));
+        cap = n;
+        return RCN_OK;
+    }
+    void release() { if (p) cudaFreeHost(p); p = nullptr; cap = 0; }
+};
+
+// What rcn_cuda_train_epoch_host keeps between calls: two streams beside the model's, their events, the device buffers and
+// pinned tables of both loops, and the streamed loop's step graphs with the key they were captured under.
+struct HostEpoch {
+    cudaStream_t copy_stream = nullptr;        // the H2D copies of the images
+    cudaStream_t flag_stream = nullptr;        // streamed loop: publishes the arrival counter behind each copy
+    cudaEvent_t fork = nullptr;                // orders another stream after the compute stream
+    cudaEvent_t ev_copied[2] = {}, ev_consumed[2] = {};   // double-buffered loop: one pair per staging slot
+    cudaEvent_t ev_arrived[kHsEvents] = {};    // streamed loop: one behind each copy, reused round robin
+    DevBuf host_slot[2];                       // double-buffered loop: the staging slots
+    DevBuf ring, state;                        // streamed loop: kHsRingSteps chunks; state block (kHsStateSlots) | step labels
+    PinnedBuf<double> stats;                   // {cost, hits} of every step
+    PinnedBuf<long long> counts;               // streamed loop: the "images arrived" value behind each copy
+    std::map<int, cudaGraphExec_t> graphs;     // streamed loop: g consecutive steps per graph, captured on first use
+    struct Key {
+        size_t B = 0, H = 0, W = 0;
+        unsigned long long alloc_gen = 0;      // no device buffer has moved since the capture (common.cuh)
+        uint64_t mean_bits = 0, sd_bits = 0;   // scale_set travels BY VALUE in the captured kernel arguments
+        double scale = 0.0;
+        const void *labels = nullptr, *stats = nullptr, *ring = nullptr, *state = nullptr, *grads = nullptr;
+        cudaStream_t stream = nullptr;
+        bool dp = false;
+        long long window = 0;                  // ring size in images (captured in kernel A's arguments)
+        auto fields() const { return std::tie(B, H, W, alloc_gen, mean_bits, sd_bits, scale, labels, stats, ring, state, grads, stream, dp, window); }
+        bool operator==(const Key& o) const { return fields() == o.fields(); }
+    } key;
+
+    int setup() {
+        for (cudaStream_t* s : {&copy_stream, &flag_stream})
+            if (!*s) RCN_CUDA_TRY(cudaStreamCreateWithFlags(s, cudaStreamNonBlocking));
+        for (cudaEvent_t* e : {&fork, &ev_copied[0], &ev_copied[1], &ev_consumed[0], &ev_consumed[1]})
+            if (!*e) RCN_CUDA_TRY(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
+        for (cudaEvent_t& e : ev_arrived)
+            if (!e) RCN_CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+        return RCN_OK;
+    }
+    void release() {
+        if (copy_stream) { cudaStreamSynchronize(copy_stream); cudaStreamDestroy(copy_stream); }
+        if (flag_stream) cudaStreamDestroy(flag_stream);
+        for (cudaEvent_t e : {fork, ev_copied[0], ev_copied[1], ev_consumed[0], ev_consumed[1]})
+            if (e) cudaEventDestroy(e);
+        for (cudaEvent_t e : ev_arrived)
+            if (e) cudaEventDestroy(e);
+        for (auto& kv : graphs) cudaGraphExecDestroy(kv.second);
+        for (DevBuf* b : {&host_slot[0], &host_slot[1], &ring, &state}) b->release();
+        stats.release();
+        counts.release();
+        *this = HostEpoch{};
+    }
+};
 
 }  // namespace rcn
 
@@ -175,34 +240,7 @@ struct rcn_cuda_model {
     DevBuf timeline;                // device-side launch timeline (timeline.cuh), allocated by rcn_cuda_timeline_enable
     bool tl_on = false;
     OzakiWorkspace oz;              // tcgen05 integer-slice GEMM scratch (wide dense layers)
-    cudaStream_t copy_stream = nullptr;
-    cudaEvent_t ev_copied[2] = {nullptr, nullptr}, ev_consumed[2] = {nullptr, nullptr};
-    DevBuf host_slot[2];
-    double* stats_host = nullptr;   // pinned, 2 doubles per step
-    size_t stats_host_cap = 0;
-    // streaming variant: the copy engine fills a device ring from pinned host memory while the GPU trains on earlier chunks
-    DevBuf hs_ring, hs_state;
-    cudaStream_t flag_stream = nullptr;     // publishes the arrival counter behind each copy
-    cudaEvent_t hs_ev[kHsEvents] = {};
-    long long* hs_counts = nullptr;         // pinned: "images arrived" value behind each copy of the streamed epoch
-    size_t hs_counts_cap = 0;
-    std::map<int, cudaGraphExec_t> hs_graphs;   // streamed epoch: g consecutive steps per graph, captured on first use
-    cudaEvent_t hs_fork = nullptr;
-    struct HsKey {
-        size_t B = 0, H = 0, W = 0, n_steps = 0;
-        unsigned long long alloc_gen = 0;   // no device buffer has moved since the capture (common.cuh)
-        uint64_t mean_bits = 0, sd_bits = 0; // scale_set travels BY VALUE in the captured kernel arguments
-        double scale = 0.0;
-        const void *labels = nullptr, *stats = nullptr, *ring = nullptr, *state = nullptr, *grads = nullptr;
-        cudaStream_t stream = nullptr;
-        bool dp = false;
-        long long window = 0;               // ring size in images (captured in kernel A's arguments)
-        bool operator==(const HsKey& o) const {
-            return B == o.B && H == o.H && W == o.W && n_steps == o.n_steps && alloc_gen == o.alloc_gen && mean_bits == o.mean_bits &&
-                   sd_bits == o.sd_bits && scale == o.scale && labels == o.labels &&
-                   stats == o.stats && ring == o.ring && state == o.state && grads == o.grads && stream == o.stream && dp == o.dp && window == o.window;
-        }
-    } hs_key;
+    HostEpoch host_epoch;           // rcn_cuda_train_epoch_host
 
     double* act(size_t l, size_t B) const {
         size_t off = 0;
@@ -394,22 +432,21 @@ int accumulate_dev(rcn_cuda_model* h, const double* feats, const double* onehot,
     return RCN_OK;
 }
 
-// Can kernel A run the convpool stack of these images itself (narrow network, u8 pixels, a stack it implements)?
-bool fused_front_possible(const rcn_cuda_model* h, int fmt) {
-    return h->use_small && fmt == RCN_PIXELS_U8_ROWMAJOR && h->plan.n_conv <= 10 && h->plan.L > 0;
-}
-
-// Kernel A's front end for u8 DEVICE images (standardised with scale_set); `bi` optional, see below.
-SmallNetFront make_front(const rcn_cuda_model* h, const void* images, size_t H, size_t W, const BatchIndex* bi) {
-    SmallNetFront fr{};
-    fr.images = (const uint8_t*)images;
-    fr.H = (int)H; fr.W = (int)W;
-    fr.max_elems = (int)h->plan.max_elems;
-    fr.stages = h->plan.stages;
-    fr.sc = make_standardise(h->plan, RCN_PIXELS_U8_ROWMAJOR, true, h->mean, h->sd);
-    if (bi) fr.bi = *bi;
-    smallnet_front_select(h->plan, &fr);
-    return fr;
+// Does kernel A run the convpool stack of these DEVICE images itself?  It does for a narrow network, u8 pixels and a stack
+// it implements, when the front end selected for these images (the staged one where it qualifies, else the generic one)
+// fits its shared memory.  Fills `fr` with that front end, standardised with scale_set; `bi` optional, see below.
+bool fused_front(const rcn_cuda_model* h, const void* images, int fmt, size_t H, size_t W, const BatchIndex* bi,
+                 SmallNetFront* fr) {
+    if (!h->use_small || fmt != RCN_PIXELS_U8_ROWMAJOR || h->plan.n_conv > 10 || h->plan.L == 0) return false;
+    *fr = SmallNetFront{};
+    fr->images = (const uint8_t*)images;
+    fr->H = (int)H; fr->W = (int)W;
+    fr->max_elems = (int)h->plan.max_elems;
+    fr->stages = h->plan.stages;
+    fr->sc = make_standardise(h->plan, RCN_PIXELS_U8_ROWMAJOR, true, h->mean, h->sd);
+    if (bi) fr->bi = *bi;
+    smallnet_front_select(h->plan, fr);
+    return smallnet_front_fits(h->small_desc, *fr);
 }
 
 // images (DEVICE) -> gradient sums.  The canonical narrow network with u8 pixels runs the convpool stack inside
@@ -419,8 +456,8 @@ int accumulate_images_dev(rcn_cuda_model* h, const void* images, int fmt, const 
                           size_t W, const BatchIndex* bi, const StepRequest& req = {}, StepDone* done = nullptr) {
     RCN_TRY(h->feats.reserve(h->plan.L * B * sizeof(double)));
     const int64_t* step_labels = bi ? (const int64_t*)bi->labels_batch : labels;
-    if (B <= smallnet_max_batch() && fused_front_possible(h, fmt)) {
-        SmallNetFront fr = make_front(h, images, H, W, bi);
+    SmallNetFront fr;
+    if (B <= smallnet_max_batch() && fused_front(h, images, fmt, H, W, bi, &fr)) {
         // Data-parallel step behind the exchange kernel: kernel A may run its front end ahead of griddepcontrol.wait
         // (smallnet.cu) when this step's kernel B pushes to the peers (so the exchange kernel X precedes the next kernel
         // A) and any device-side cursor it reads is advanced by kernel B -- this step's and the previous one's
@@ -435,8 +472,7 @@ int accumulate_images_dev(rcn_cuda_model* h, const void* images, int fmt, const 
         // was removed: in the device-resident step kernel A needs a whole SM's registers, so all but ~26 of its CTAs start
         // only when kernel B's CTAs leave, and its parameter loads are no longer hidden behind the front end.
         if (!h->dp.connected && fr.use_cp && fr.bi.window != 0) fr.prewait = 2;
-        if (smallnet_front_fits(h->small_desc, fr))
-            return accumulate_dev(h, h->feats.as<double>(), nullptr, step_labels, B, &fr, req, done);
+        return accumulate_dev(h, h->feats.as<double>(), nullptr, step_labels, B, &fr, req, done);
     }
     RCN_TRY(launch_features(h->plan, images, fmt, B, H, W, true, h->mean, h->sd, h->feats.as<double>(), h->fscratch,
                             h->stream, bi));
@@ -514,22 +550,7 @@ int rcn_cuda_destroy(rcn_cuda_handle h) {
     cudaSetDevice(h->device);
     cudaStreamSynchronize(h->stream);
     if (h->own_stream) { cudaStreamSynchronize(h->own_stream); cudaStreamDestroy(h->own_stream); }
-    if (h->copy_stream) { cudaStreamSynchronize(h->copy_stream); cudaStreamDestroy(h->copy_stream); }
-    for (int i = 0; i < 2; ++i) {
-        if (h->ev_copied[i]) cudaEventDestroy(h->ev_copied[i]);
-        if (h->ev_consumed[i]) cudaEventDestroy(h->ev_consumed[i]);
-        h->host_slot[i].release();
-    }
-    if (h->stats_host) cudaFreeHost(h->stats_host);
-    for (auto& kv : h->hs_graphs) cudaGraphExecDestroy(kv.second);
-    if (h->hs_fork) cudaEventDestroy(h->hs_fork);
-
-    h->hs_ring.release(); h->hs_state.release();
-    if (h->hs_counts) cudaFreeHost(h->hs_counts);
-    if (h->flag_stream) cudaStreamDestroy(h->flag_stream);
-    for (int i = 0; i < kHsEvents; ++i)
-        if (h->hs_ev[i]) cudaEventDestroy(h->hs_ev[i]);
-
+    h->host_epoch.release();
     dp_release(h->dp);
     h->oz.release();
     DevBuf* bufs[] = {&h->params, &h->grads_own, &h->in_stage, &h->tgt_stage, &h->feats, &h->acts, &h->deltas,
@@ -868,18 +889,13 @@ int rcn_cuda_evaluate_images(rcn_cuda_handle h, const void* images, int pixel_fo
     int64_t* lab_dev = labels_out;
     const bool lab_host = labels_out && !is_device_ptr(labels_out);
     if (lab_host) { RCN_TRY(h->out_stage.reserve(B * sizeof(int64_t))); lab_dev = h->out_stage.as<int64_t>(); }
-    bool done = false;
-    if (fused_front_possible(h, pixel_format)) {
+    SmallNetFront fr;
+    if (fused_front(h, in.dev, pixel_format, H, W, nullptr, &fr)) {
         // One launch, the front end inside the inference kernel.  Measured against the feature kernel followed by the
         // inference kernel on the features (profiles/eval_routes_b200.txt, B200 at 1000 W) it was faster from 64 to
         // 1 048 576 images (9.42 against 9.69 ms at 1 048 576) and equal at 1, so that route was not kept.
-        const SmallNetFront fr = make_front(h, in.dev, H, W, nullptr);
-        if (smallnet_front_fits(h->small_desc, fr)) {
-            RCN_TRY(launch_smallnet_infer(h->small_desc, h->params.as<double>(), B, lab_in, lab_dev, st, h->eval_rs, fr, h->stream));
-            done = true;
-        }
-    }
-    if (!done) {   // the existing kernels: features + standardise, forward, batch statistics, argmax
+        RCN_TRY(launch_smallnet_infer(h->small_desc, h->params.as<double>(), B, lab_in, lab_dev, st, h->eval_rs, fr, h->stream));
+    } else {   // the existing kernels: features + standardise, forward, batch statistics, argmax
         RCN_TRY(h->feats.reserve(h->plan.L * B * sizeof(double)));
         RCN_TRY(launch_features(h->plan, in.dev, pixel_format, B, H, W, true, h->mean, h->sd, h->feats.as<double>(), h->fscratch,
                                 h->stream));
@@ -1090,6 +1106,165 @@ int rcn_cuda_epoch_run(rcn_cuda_handle h, double eta, size_t n_steps) {
 }
 
 // ---- pipelined loop over a HOST-resident dataset: rcn.rs:147-149 ------------------------------------------------------
+// Streamed loop over the epoch's labels in tgt_stage: the copy engine streams the pinned u8 images into the device ring while
+// earlier chunks train, kernel B writes each step's result into pinned host memory, and the host launches CUDA graphs of
+// several steps each and queues the copies.
+static int train_epoch_streamed(rcn_cuda_model* h, const void* images, size_t n_steps, size_t H, size_t W, size_t B, double scale) {
+    HostEpoch& ep = h->host_epoch;
+    const size_t img_bytes = B * H * W;
+    const size_t spg = (size_t)hs_steps_per_graph();
+    // The epoch as a sequence of graph launches: as many `spg`-step graphs as fit, then the largest of 20 / 10 / 5 / 2 / 1 steps
+    // that still fits -- as few launches as possible: with copies on the link a graph boundary costs 4-5 us and now and then
+    // 27 us (a short FIRST graph to get going sooner measured worse for that reason: 507-519 us against 479 for a 20-step
+    // epoch; its launch latency passes while the first chunk crosses the link anyway).
+    std::vector<int> plan_g;
+    for (size_t left = n_steps; left;) {
+        size_t g = 1;
+        if (left >= spg) g = spg;
+        else
+            for (size_t c : {(size_t)20, (size_t)10, (size_t)5, (size_t)2})
+                if (c < spg && left >= c) { g = c; break; }
+        plan_g.push_back((int)g);
+        left -= g;
+    }
+    RCN_TRY(ep.state.reserve((kHsStateSlots + B) * sizeof(long long)));
+    RCN_TRY(h->feats.reserve(h->plan.L * B * sizeof(double)));
+    long long* st = ep.state.as<long long>();
+    BatchIndex bi;
+    bi.cursor = st;
+    bi.labels_all = h->tgt_stage.as<long long>();
+    bi.labels_batch = st + kHsStateSlots;
+    bi.window = (long long)(kHsRingSteps * B);
+    bi.arrived = st + 3;
+    // cursor and arrival counter start at zero; after that graph replays
+    const long long init[kHsStateSlots] = {};
+    RCN_CUDA_TRY(cudaMemcpyAsync(st, init, sizeof(init), cudaMemcpyHostToDevice, h->stream));
+    HostEpoch::Key key;   // the graphs do not depend on the epoch length
+    key.B = B; key.H = H; key.W = W; key.scale = scale;
+    key.labels = h->tgt_stage.p;   // (grows with the epoch length: a longer epoch than any before re-captures)
+    key.alloc_gen = alloc_generation().load(std::memory_order_relaxed);
+    memcpy(&key.mean_bits, &h->mean, sizeof(double));   // a set_scale / gen_scales since the capture re-captures
+    memcpy(&key.sd_bits, &h->sd, sizeof(double));
+    key.stats = ep.stats.p; key.ring = ep.ring.p; key.state = st; key.grads = h->grads; key.stream = h->stream;
+    key.dp = h->dp.connected;
+    key.window = bi.window;
+    if (ep.graphs.empty() || !(key == ep.key)) {
+        for (auto& kv : ep.graphs) cudaGraphExecDestroy(kv.second);
+        ep.graphs.clear();
+        // warm-up outside capture: reserves every scratch buffer and sets kernel attributes (no parameter update, no push to
+        // the peers)
+        BatchIndex bi_warm = bi;
+        bi_warm.arrived = nullptr;   // nothing has been copied yet: the warm-up trains on whatever the ring holds
+        StepRequest warm;
+        warm.push = false;
+        RCN_TRY(accumulate_images_dev(h, ep.ring.p, RCN_PIXELS_U8_ROWMAJOR, nullptr, B, H, W, &bi_warm, warm));
+        RCN_CUDA_TRY(cudaStreamSynchronize(h->stream));
+        key.alloc_gen = alloc_generation().load(std::memory_order_relaxed);   // the warm-up may have grown scratch buffers
+        ep.key = key;
+    }
+    // `g` consecutive steps in ONE graph: a step is only tens of microseconds long, so the host's per-launch cost is spread
+    // over several of them; the remainder of the epoch replays the one-step graph.
+    auto capture_steps = [&](int g, cudaGraphExec_t* out) -> int {
+        cudaGraph_t graph = nullptr;
+        RCN_CUDA_TRY(cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal));
+        int rc = RCN_OK;
+        const StepRequest req{step_update(h, scale, st, (long long)B, kHsNoWrap, ep.stats.p, true)};
+        for (int q = 0; q < g && rc == RCN_OK; ++q) {
+            StepDone done;
+            rc = accumulate_images_dev(h, ep.ring.p, RCN_PIXELS_U8_ROWMAJOR, nullptr, B, H, W, &bi, req, &done);
+            if (rc == RCN_OK) rc = finish_step(h, req.upd, done);
+        }
+        cudaError_t ce = cudaStreamEndCapture(h->stream, &graph);
+        if (rc != RCN_OK) { if (graph) cudaGraphDestroy(graph); cudaGetLastError(); return rc; }
+        if (ce != cudaSuccess || !graph) return fail(RCN_ERR_CUDA, "stream capture of the training step failed: %s", cudaGetErrorString(ce));
+        ce = cudaGraphInstantiate(out, graph, 0);
+        cudaGraphDestroy(graph);
+        if (ce != cudaSuccess) { *out = nullptr; return fail(RCN_ERR_CUDA, "cudaGraphInstantiate failed: %s", cudaGetErrorString(ce)); }
+        return RCN_OK;
+    };
+    for (int g : plan_g) {
+        if (ep.graphs.count(g)) continue;
+        cudaGraphExec_t ge = nullptr;
+        RCN_TRY(capture_steps(g, &ge));
+        ep.graphs[g] = ge;
+    }
+    // Copies first (the driver queues them; each waits on the device for its ring slots), then the graph launches.
+    const StreamMemOps& mo = stream_mem_ops(h->device);
+    const CUdeviceptr cursor_dev = (CUdeviceptr)reinterpret_cast<uintptr_t>(st);
+    const char* src = static_cast<const char*>(images);
+    RCN_TRY(ep.counts.reserve(n_steps));
+    // the state block (cursor 0, arrived 0) must be in place before the first counter copy can land
+    RCN_CUDA_TRY(cudaEventRecord(ep.fork, h->stream));
+    RCN_CUDA_TRY(cudaStreamWaitEvent(ep.flag_stream, ep.fork, 0));
+    size_t a = 0, k = 0, n_copy = 0;
+    auto enqueue_copy = [&]() -> int {
+        // ramp: while the copies are only a few chunks ahead of the training steps a long copy would hold back the steps
+        // waiting for its first chunk (the counter moves when a copy has landed completely)
+        size_t g = a < 2 ? 1 : (a < 16 ? 2 : (a < 32 ? 4 : kHsMaxCopy));
+        g = std::min(g, n_steps - a);
+        g = std::min(g, kHsQuarter - a % kHsQuarter);                      // never across a quarter of the ring
+        if (a >= kHsRingSteps && a % kHsQuarter == 0) {
+            // entering a quarter whose slots held steps [a - ring, a + quarter - ring): all of them must have trained
+            if (mo.wait64(ep.copy_stream, cursor_dev, (cuuint64_t)((a + kHsQuarter - kHsRingSteps) * B), CU_STREAM_WAIT_VALUE_GEQ) != CUDA_SUCCESS)
+                return fail(RCN_ERR_CUDA, "cuStreamWaitValue64 failed");
+        }
+        RCN_CUDA_TRY(cudaMemcpyAsync(ep.ring.as<char>() + (a % kHsRingSteps) * img_bytes, src + a * img_bytes, g * img_bytes,
+                                     cudaMemcpyHostToDevice, ep.copy_stream));
+        a += g;
+        ep.counts.p[n_copy] = (long long)(a * B);
+        cudaEvent_t ev = ep.ev_arrived[n_copy % kHsEvents];
+        RCN_CUDA_TRY(cudaEventRecord(ev, ep.copy_stream));
+        RCN_CUDA_TRY(cudaStreamWaitEvent(ep.flag_stream, ev, 0));
+        // (cuStreamWriteValue64 here instead measured the same: 476 vs 478 us for a 20-step epoch)
+        RCN_CUDA_TRY(cudaMemcpyAsync(st + 3, ep.counts.p + n_copy, sizeof(long long), cudaMemcpyHostToDevice, ep.flag_stream));
+        ++n_copy;
+        return RCN_OK;
+    };
+    // One chunk's copy, then the first graph launch (its launch latency passes while the chunk crosses the link; kernel A
+    // waits on the device for whatever has not arrived yet), then copies and launches interleaved, the copies enqueued half a
+    // ring ahead of the launches.
+    RCN_TRY(enqueue_copy());
+    for (int g : plan_g) {
+        RCN_CUDA_TRY(cudaGraphLaunch(ep.graphs[g], h->stream));
+        k += (size_t)g;
+        while (a < n_steps && a < k + kHsRingSteps / 2) RCN_TRY(enqueue_copy());
+    }
+    // A + B (+ exchange/update) per replayed step
+    g_launches.fetch_add((unsigned long long)n_steps * (2 + (h->dp.connected ? 1 : 0)), std::memory_order_relaxed);
+    return RCN_OK;
+}
+
+// General loop over the epoch's labels in tgt_stage: double-buffered cudaMemcpyAsync of each step's images on the copy stream.
+static int train_epoch_buffered(rcn_cuda_model* h, const void* images, int pixel_format, size_t n_steps, size_t H, size_t W,
+                                size_t B, double scale) {
+    HostEpoch& ep = h->host_epoch;
+    const size_t img_bytes = B * H * W * pixel_bytes(pixel_format);
+    for (DevBuf& buf : ep.host_slot) RCN_TRY(buf.reserve(img_bytes));
+    const int64_t* labels_dev = h->tgt_stage.as<int64_t>();
+    // everything the previous user of the staging slots enqueued on the compute stream must be finished first
+    RCN_CUDA_TRY(cudaEventRecord(ep.ev_consumed[0], h->stream));
+    RCN_CUDA_TRY(cudaEventRecord(ep.ev_consumed[1], h->stream));
+    // unarmed: kernel B leaves the update to the update kernel (or the exchange kernel)
+    const SnUpdate update = step_update(h, scale);
+    const char* img = (const char*)images;
+    for (size_t k = 0; k < n_steps; ++k) {
+        const int slot = (int)(k & 1);
+        char* dst = ep.host_slot[slot].as<char>();
+        // H2D of chunk k on the copy stream: overlaps the kernels of chunk k-1
+        RCN_CUDA_TRY(cudaStreamWaitEvent(ep.copy_stream, ep.ev_consumed[slot], 0));
+        RCN_CUDA_TRY(cudaMemcpyAsync(dst, img + k * img_bytes, img_bytes, cudaMemcpyHostToDevice, ep.copy_stream));
+        RCN_CUDA_TRY(cudaEventRecord(ep.ev_copied[slot], ep.copy_stream));
+        RCN_CUDA_TRY(cudaStreamWaitEvent(h->stream, ep.ev_copied[slot], 0));
+        RCN_TRY(accumulate_images_dev(h, dst, pixel_format, labels_dev + k * B, B, H, W, nullptr));
+        RCN_CUDA_TRY(cudaEventRecord(ep.ev_consumed[slot], h->stream));
+        RCN_TRY(finish_step(h, update, StepDone::nothing));
+        // D2H of this step's result (cost, hits evaluated with the pre-update parameters)
+        RCN_CUDA_TRY(cudaMemcpyAsync(ep.stats.p + 2 * k, h->small.p, 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    }
+    RCN_CUDA_TRY(cudaStreamSynchronize(ep.copy_stream));
+    return RCN_OK;
+}
+
 int rcn_cuda_train_epoch_host(rcn_cuda_handle h, const void* images, int pixel_format, const int64_t* labels,
                               size_t n_samples, size_t H, size_t W, size_t B, double eta, size_t global_batch,
                               double* cost_out, uint64_t* hits_out, size_t* n_steps_out) {
@@ -1108,227 +1283,50 @@ int rcn_cuda_train_epoch_host(rcn_cuda_handle h, const void* images, int pixel_f
     RCN_TRY(check_feature_width(h, h->plan.L));
     if (global_batch == 0) global_batch = B * (size_t)(h->dp.connected ? h->dp.world : 1);
     const size_t img_bytes = B * H * W * pixel_bytes(pixel_format);
-    if (!h->copy_stream) RCN_CUDA_TRY(cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking));
-    if (!h->hs_fork) {
-        for (int i = 0; i < 2; ++i) {
-            RCN_CUDA_TRY(cudaEventCreateWithFlags(&h->ev_copied[i], cudaEventDisableTiming));
-            RCN_CUDA_TRY(cudaEventCreateWithFlags(&h->ev_consumed[i], cudaEventDisableTiming));
-        }
-        RCN_CUDA_TRY(cudaEventCreateWithFlags(&h->hs_fork, cudaEventDisableTiming));
-    }
-    if (h->stats_host_cap < n_steps) {
-        if (h->stats_host) cudaFreeHost(h->stats_host);
-        h->stats_host = nullptr; h->stats_host_cap = 0;
-        RCN_CUDA_TRY(cudaHostAlloc((void**)&h->stats_host, n_steps * 2 * sizeof(double), cudaHostAllocDefault));
-        h->stats_host_cap = n_steps;
-    }
-    // ---- streaming fast path: pinned u8 dataset + fused small-network kernels: the copy engine streams the images into a
-    // device ring while earlier chunks train; per-step results are written straight into pinned host memory; the host
-    // launches CUDA graphs of several steps each and queues the copies.  It needs the staged front end (its image-loading
-    // lanes wait for the arrival counter) and 64-bit stream memory operations (the copy stream's wait for free ring slots).
+    HostEpoch& ep = h->host_epoch;
+    RCN_TRY(ep.setup());
+    RCN_TRY(ep.stats.reserve(2 * n_steps));
+    // The streamed loop needs a pinned, 16-byte aligned u8 dataset, steps that run kernel A with the staged front end on the
+    // ring (its image-loading lanes wait for the arrival counter), 64-bit stream memory operations (the copy stream's wait for
+    // free ring slots) and a compute stream that is not being captured.  (No ring for a network kernel A does not train.)
+    bool streamed = false;
     if (pixel_format == RCN_PIXELS_U8_ROWMAJOR && h->use_small && B <= smallnet_max_batch() && img_bytes % 16 == 0 &&
-        (reinterpret_cast<uintptr_t>(images) & 15) == 0 && is_pinned_host_ptr(images) && h->plan.L > 0 && h->plan.n_conv <= 10 &&
-        kHsRingSteps * B < (1ull << 31) && stream_mem_ops(h->device).ok) {
-        SmallNetFront probe{};
-        probe.H = (int)H; probe.W = (int)W; probe.max_elems = (int)h->plan.max_elems; probe.stages = h->plan.stages;
+        (reinterpret_cast<uintptr_t>(images) & 15) == 0 && is_pinned_host_ptr(images) && kHsRingSteps * B < (1ull << 31) &&
+        stream_mem_ops(h->device).ok) {
         cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
         RCN_CUDA_TRY(cudaStreamIsCapturing(h->stream, &cs));
-        const bool fits = smallnet_front_fits(h->small_desc, probe);
-        probe.images = static_cast<const uint8_t*>(images);   // 16-byte aligned, as the ring the steps will read is
-        smallnet_front_select(h->plan, &probe);
-        if (fits && probe.use_cp && cs == cudaStreamCaptureStatusNone) {
-            // The legacy default stream cannot be captured: run the loop on the model's own stream, ordered after whatever
-            // the caller has enqueued on the legacy stream; the call drains that stream before it returns.
-            struct StreamSwap {
-                rcn_cuda_model* m; cudaStream_t saved;
-                StreamSwap(rcn_cuda_model* m_) : m(m_), saved(m_->stream) {}
-                ~StreamSwap() { m->stream = saved; }
-            } swap_guard(h);
-            if (h->stream == nullptr) {
-                RCN_CUDA_TRY(cudaEventRecord(h->hs_fork, nullptr));
-                RCN_CUDA_TRY(cudaStreamWaitEvent(h->own_stream, h->hs_fork, 0));
-                h->stream = h->own_stream;
-            }
-            RCN_TRY(h->hs_ring.reserve(kHsRingSteps * img_bytes));
-            const size_t spg = (size_t)hs_steps_per_graph();
-            // The epoch as a sequence of graph launches: as many `spg`-step graphs as fit, then the largest of 20 / 10 / 5 / 2 /
-            // 1 steps that still fits -- as few launches as possible: with copies on the link a graph boundary costs 4-5 us and
-            // now and then 27 us (a short FIRST graph to get going sooner measured worse for that reason: 507-519 us against 479
-            // for a 20-step epoch; its launch latency passes while the first chunk crosses the link anyway).
-            std::vector<int> plan_g;
-            for (size_t left = n_steps; left;) {
-                size_t g = 1;
-                if (left >= spg) g = spg;
-                else
-                    for (size_t c : {(size_t)20, (size_t)10, (size_t)5, (size_t)2})
-                        if (c < spg && left >= c) { g = c; break; }
-                plan_g.push_back((int)g);
-                left -= g;
-            }
-            RCN_TRY(h->hs_state.reserve((kHsStateSlots + B) * sizeof(long long)));
-            RCN_TRY(h->tgt_stage.reserve(n_steps * B * sizeof(int64_t)));
-            RCN_TRY(h->feats.reserve(h->plan.L * B * sizeof(double)));
-            const double scale_s = eta / (double)global_batch;
-            long long* st = h->hs_state.as<long long>();
-            BatchIndex bi;
-            bi.cursor = st;
-            bi.labels_all = h->tgt_stage.as<long long>();
-            bi.labels_batch = st + kHsStateSlots;
-            bi.window = (long long)(kHsRingSteps * B);
-            bi.arrived = st + 3;
-            // cursor and arrival counter start at zero, the labels of the whole epoch go up in one copy; after that graph replays
-            const long long init[kHsStateSlots] = {};
-            RCN_CUDA_TRY(cudaMemcpyAsync(st, init, sizeof(init), cudaMemcpyHostToDevice, h->stream));
-            RCN_CUDA_TRY(cudaMemcpyAsync(h->tgt_stage.p, labels, n_steps * B * sizeof(int64_t), cudaMemcpyHostToDevice, h->stream));
-            rcn_cuda_model::HsKey key;
-            key.B = B; key.H = H; key.W = W; key.n_steps = 0; key.scale = scale_s;   // the graphs do not depend on the epoch length
-            key.labels = h->tgt_stage.p;   // (grows with the epoch length: a longer epoch than any before re-captures)
-            key.alloc_gen = alloc_generation().load(std::memory_order_relaxed);
-            memcpy(&key.mean_bits, &h->mean, sizeof(double));   // a set_scale / gen_scales since the capture re-captures
-            memcpy(&key.sd_bits, &h->sd, sizeof(double));
-            key.stats = h->stats_host; key.ring = h->hs_ring.p; key.state = st; key.grads = h->grads; key.stream = h->stream;
-            key.dp = h->dp.connected;
-            key.window = bi.window;
-            if (h->hs_graphs.empty() || !(key == h->hs_key)) {
-                for (auto& kv : h->hs_graphs) cudaGraphExecDestroy(kv.second);
-                h->hs_graphs.clear();
-                // warm-up outside capture: reserves every scratch buffer and sets kernel attributes (no parameter update, no
-                // push to the peers)
-                BatchIndex bi_warm = bi;
-                bi_warm.arrived = nullptr;   // nothing has been copied yet: the warm-up trains on whatever the ring holds
-                StepRequest warm;
-                warm.push = false;
-                RCN_TRY(accumulate_images_dev(h, h->hs_ring.p, pixel_format, nullptr, B, H, W, &bi_warm, warm));
-                RCN_CUDA_TRY(cudaStreamSynchronize(h->stream));
-                key.alloc_gen = alloc_generation().load(std::memory_order_relaxed);   // the warm-up may have grown scratch buffers
-                h->hs_key = key;
-            }
-            {
-                // `g` consecutive steps in ONE graph: a step is only tens of microseconds long, so the host's per-launch cost
-                // is spread over several of them; the remainder of the epoch replays the one-step graph.
-                auto capture_steps = [&](int g, cudaGraphExec_t* out) -> int {
-                    cudaGraph_t graph = nullptr;
-                    RCN_CUDA_TRY(cudaStreamBeginCapture(h->stream, cudaStreamCaptureModeThreadLocal));
-                    int rc = RCN_OK;
-                    const StepRequest req{step_update(h, scale_s, st, (long long)B, kHsNoWrap, h->stats_host, true)};
-                    for (int q = 0; q < g && rc == RCN_OK; ++q) {
-                        StepDone done;
-                        rc = accumulate_images_dev(h, h->hs_ring.p, pixel_format, nullptr, B, H, W, &bi, req, &done);
-                        if (rc == RCN_OK) rc = finish_step(h, req.upd, done);
-                    }
-                    cudaError_t ce = cudaStreamEndCapture(h->stream, &graph);
-                    if (rc != RCN_OK) { if (graph) cudaGraphDestroy(graph); cudaGetLastError(); return rc; }
-                    if (ce != cudaSuccess || !graph) return fail(RCN_ERR_CUDA, "stream capture of the training step failed: %s", cudaGetErrorString(ce));
-                    ce = cudaGraphInstantiate(out, graph, 0);
-                    cudaGraphDestroy(graph);
-                    if (ce != cudaSuccess) { *out = nullptr; return fail(RCN_ERR_CUDA, "cudaGraphInstantiate failed: %s", cudaGetErrorString(ce)); }
-                    return RCN_OK;
-                };
-                for (int g : plan_g) {
-                    if (h->hs_graphs.count(g)) continue;
-                    cudaGraphExec_t ge = nullptr;
-                    RCN_TRY(capture_steps(g, &ge));
-                    h->hs_graphs[g] = ge;
-                }
-            }
-            {
-                // Copies first (the driver queues them; each waits on the device for its ring slots), then the graph launches.
-                const StreamMemOps& mo = stream_mem_ops(h->device);
-                const CUdeviceptr cursor_dev = (CUdeviceptr)reinterpret_cast<uintptr_t>(st);
-                const char* src = static_cast<const char*>(images);
-                if (h->hs_counts_cap < n_steps) {   // pinned table of the counter values, one per copy
-                    if (h->hs_counts) cudaFreeHost(h->hs_counts);
-                    h->hs_counts = nullptr; h->hs_counts_cap = 0;
-                    RCN_CUDA_TRY(cudaHostAlloc((void**)&h->hs_counts, n_steps * sizeof(long long), cudaHostAllocDefault));
-                    h->hs_counts_cap = n_steps;
-                }
-                if (!h->flag_stream) {
-                    RCN_CUDA_TRY(cudaStreamCreateWithFlags(&h->flag_stream, cudaStreamNonBlocking));
-                    for (int i = 0; i < kHsEvents; ++i) RCN_CUDA_TRY(cudaEventCreateWithFlags(&h->hs_ev[i], cudaEventDisableTiming));
-                }
-                // the state block (cursor 0, arrived 0) must be in place before the first counter copy can land
-                RCN_CUDA_TRY(cudaEventRecord(h->hs_fork, h->stream));
-                RCN_CUDA_TRY(cudaStreamWaitEvent(h->flag_stream, h->hs_fork, 0));
-                size_t a = 0, k = 0, n_copy = 0;
-                auto enqueue_copy = [&]() -> int {
-                    // ramp: while the copies are only a few chunks ahead of the training steps a long copy would hold back the
-                    // steps waiting for its first chunk (the counter moves when a copy has landed completely)
-                    size_t g = a < 2 ? 1 : (a < 16 ? 2 : (a < 32 ? 4 : kHsMaxCopy));
-                    g = std::min(g, n_steps - a);
-                    g = std::min(g, kHsQuarter - a % kHsQuarter);                      // never across a quarter of the ring
-                    if (a >= kHsRingSteps && a % kHsQuarter == 0) {
-                        // entering a quarter whose slots held steps [a - ring, a + quarter - ring): all of them must have trained
-                        if (mo.wait64(h->copy_stream, cursor_dev, (cuuint64_t)((a + kHsQuarter - kHsRingSteps) * B), CU_STREAM_WAIT_VALUE_GEQ) != CUDA_SUCCESS)
-                            return fail(RCN_ERR_CUDA, "cuStreamWaitValue64 failed");
-                    }
-                    RCN_CUDA_TRY(cudaMemcpyAsync(h->hs_ring.as<char>() + (a % kHsRingSteps) * img_bytes, src + a * img_bytes, g * img_bytes,
-                                                 cudaMemcpyHostToDevice, h->copy_stream));
-                    a += g;
-                    h->hs_counts[n_copy] = (long long)(a * B);
-                    cudaEvent_t ev = h->hs_ev[n_copy % kHsEvents];
-                    RCN_CUDA_TRY(cudaEventRecord(ev, h->copy_stream));
-                    RCN_CUDA_TRY(cudaStreamWaitEvent(h->flag_stream, ev, 0));
-                    // (cuStreamWriteValue64 here instead measured the same: 476 vs 478 us for a 20-step epoch)
-                    RCN_CUDA_TRY(cudaMemcpyAsync(st + 3, h->hs_counts + n_copy, sizeof(long long), cudaMemcpyHostToDevice, h->flag_stream));
-                    ++n_copy;
-                    return RCN_OK;
-                };
-                // One chunk's copy, then the first graph launch (its launch latency passes while the chunk crosses the link; kernel
-                // A waits on the device for whatever has not arrived yet), then copies and launches interleaved, the copies
-                // enqueued half a ring ahead of the launches.
-                RCN_TRY(enqueue_copy());
-                for (int g : plan_g) {
-                    RCN_CUDA_TRY(cudaGraphLaunch(h->hs_graphs[g], h->stream));
-                    k += (size_t)g;
-                    while (a < n_steps && a < k + kHsRingSteps / 2) RCN_TRY(enqueue_copy());
-                }
-            }
-            // A + B (+ exchange/update) per replayed step
-            g_launches.fetch_add((unsigned long long)n_steps * (2 + (h->dp.connected ? 1 : 0)), std::memory_order_relaxed);
-            RCN_CUDA_TRY(cudaStreamSynchronize(h->stream));
-            stream_drained(h);
-            for (size_t k = 0; k < n_steps; ++k) {
-                if (cost_out) cost_out[k] = h->stats_host[2 * k];
-                if (hits_out) memcpy(&hits_out[k], &h->stats_host[2 * k + 1], sizeof(uint64_t));
-            }
-            h->stats_valid = true;
-            h->last_B = B;
-            if (n_steps_out) *n_steps_out = n_steps;
-            return RCN_OK;
+        if (cs == cudaStreamCaptureStatusNone) {
+            RCN_TRY(ep.ring.reserve(kHsRingSteps * img_bytes));
+            SmallNetFront fr;
+            streamed = fused_front(h, ep.ring.p, pixel_format, H, W, nullptr, &fr) && fr.use_cp;
         }
     }
-    // ---- general path: double-buffered cudaMemcpyAsync on the copy stream -----------------------------------------------
-    for (int i = 0; i < 2; ++i) RCN_TRY(h->host_slot[i].reserve(img_bytes));
+    // The legacy default stream cannot be captured: the streamed loop runs on the model's own stream, ordered after whatever
+    // the caller has enqueued on the legacy stream; the call drains that stream before it returns.
+    struct StreamSwap {
+        rcn_cuda_model* m; cudaStream_t saved;
+        StreamSwap(rcn_cuda_model* m_) : m(m_), saved(m_->stream) {}
+        ~StreamSwap() { m->stream = saved; }
+    } swap_guard(h);
+    if (streamed && h->stream == nullptr) {
+        RCN_CUDA_TRY(cudaEventRecord(ep.fork, nullptr));
+        RCN_CUDA_TRY(cudaStreamWaitEvent(h->own_stream, ep.fork, 0));
+        h->stream = h->own_stream;
+    }
     // the labels of the whole epoch go up in ONE copy (one driver call per step less); images stream chunk by chunk
     RCN_TRY(h->tgt_stage.reserve(n_steps * B * sizeof(int64_t)));
     RCN_CUDA_TRY(cudaMemcpyAsync(h->tgt_stage.p, labels, n_steps * B * sizeof(int64_t), cudaMemcpyHostToDevice, h->stream));
-    const int64_t* labels_dev = h->tgt_stage.as<int64_t>();
-    // everything the previous user of the staging slots enqueued on the compute stream must be finished first
-    RCN_CUDA_TRY(cudaEventRecord(h->ev_consumed[0], h->stream));
-    RCN_CUDA_TRY(cudaEventRecord(h->ev_consumed[1], h->stream));
-    // unarmed: kernel B leaves the update to the update kernel (or the exchange kernel)
-    const SnUpdate update = step_update(h, eta / (double)global_batch);   // (eta / batch.len() as f64)  (rcn.rs:214)
-    const char* img = (const char*)images;
-    for (size_t k = 0; k < n_steps; ++k) {
-        const int slot = (int)(k & 1);
-        char* dst = h->host_slot[slot].as<char>();
-        // H2D of chunk k on the copy stream: overlaps the kernels of chunk k-1
-        RCN_CUDA_TRY(cudaStreamWaitEvent(h->copy_stream, h->ev_consumed[slot], 0));
-        RCN_CUDA_TRY(cudaMemcpyAsync(dst, img + k * img_bytes, img_bytes, cudaMemcpyHostToDevice, h->copy_stream));
-        RCN_CUDA_TRY(cudaEventRecord(h->ev_copied[slot], h->copy_stream));
-        RCN_CUDA_TRY(cudaStreamWaitEvent(h->stream, h->ev_copied[slot], 0));
-        RCN_TRY(accumulate_images_dev(h, dst, pixel_format, labels_dev + k * B, B, H, W, nullptr));
-        RCN_CUDA_TRY(cudaEventRecord(h->ev_consumed[slot], h->stream));
-        RCN_TRY(finish_step(h, update, StepDone::nothing));
-        // D2H of this step's result (cost, hits evaluated with the pre-update parameters)
-        RCN_CUDA_TRY(cudaMemcpyAsync(h->stats_host + 2 * k, h->small.p, 2 * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-    }
+    const double scale = eta / (double)global_batch;   // (eta / batch.len() as f64)  (rcn.rs:214)
+    RCN_TRY(streamed ? train_epoch_streamed(h, images, n_steps, H, W, B, scale)
+                     : train_epoch_buffered(h, images, pixel_format, n_steps, H, W, B, scale));
     RCN_CUDA_TRY(cudaStreamSynchronize(h->stream));
-    RCN_CUDA_TRY(cudaStreamSynchronize(h->copy_stream));
+    stream_drained(h);
     for (size_t k = 0; k < n_steps; ++k) {
-        if (cost_out) cost_out[k] = h->stats_host[2 * k];
-        if (hits_out) memcpy(&hits_out[k], &h->stats_host[2 * k + 1], sizeof(uint64_t));
+        if (cost_out) cost_out[k] = ep.stats.p[2 * k];
+        if (hits_out) memcpy(&hits_out[k], &ep.stats.p[2 * k + 1], sizeof(uint64_t));
     }
+    h->stats_valid = true;
+    h->last_B = B;
     if (n_steps_out) *n_steps_out = n_steps;
     return RCN_OK;
 }

@@ -386,22 +386,37 @@ def test_epoch_run_equals_steps_and_oracle(api, B, N, n_steps):
     assert_close(run.get_params(), p, rtol=1e-9, what="params vs oracle epoch loop")
 
 
+HOST_EPOCH_SHAPES = [
+    # (convpool stack, (H, W), whether pinned images stream through the copy-engine ring)
+    ([1, 3], (28, 28), True),         # 784-30-10, the canonical network
+    ([1, 3, 1, 3], (8, 96), False),   # 768-30-10: kernel A cannot run this front end, the steps run the feature kernels
+    ([1, 3], (12, 96), True),         # 1152-30-10: only the staged front end fits kernel A
+]
+
+
 def test_train_epoch_host_equals_step_by_step(api):
-    """The pipelined host-dataset loop (double-buffered H2D on a copy stream) == train_batch_images chunk by chunk,
-    remainder dropped like chunks_exact (rcn.rs:147-149); per-step (cost, hits) equal last_batch_stats."""
+    """The pipelined host-dataset loop == train_batch_images chunk by chunk, remainder dropped like chunks_exact
+    (rcn.rs:147-149); per-step (cost, hits) equal last_batch_stats.  Pinned images stream through the copy-engine ring
+    exactly when the steps on it run kernel A with the staged front end, otherwise they take the double-buffered loop."""
+    for stack, hw, streams in HOST_EPOCH_SHAPES:
+        check_train_epoch_host(api, stack, hw, streams)
+
+
+def check_train_epoch_host(api, stack, hw, streams):
+    from mercer_research_b200 import _lib
     rng = np.random.default_rng(21)
     B, N = 64, 64 * 5 + 17
-    images = rng.integers(0, 256, size=(N, 28, 28), dtype=np.uint8)
+    images = rng.integers(0, 256, size=(N,) + hw, dtype=np.uint8)
     labels = rng.integers(0, 10, size=N).astype(np.int64)
-    cfg = [api.RCNLayer.Convolve2D(api.Padding.Same), api.RCNLayer.Pool2D(api.Pooling.Max)]
+    cfg = [api.RCNLayer.Convolve2D(api.Padding.Same) if c == 1 else api.RCNLayer.Pool2D(api.Pooling.Max) for c in stack]
     params = None
     results = []
     import torch
-    pinned = torch.from_numpy(images).pin_memory()       # pinned host memory takes the streaming (copy-engine ring) path
+    pinned = torch.from_numpy(images).pin_memory()
     pinned_labels = torch.from_numpy(labels).pin_memory()
     for mode in ("loop", "epoch", "epoch-pinned", "epoch-pinned-again"):
         model = api.RCN(10, cfg, [30])
-        model.load_weights_and_bias(784)
+        model.load_weights_and_bias(model.feature_len(*hw))
         if params is None:
             params = np.random.default_rng(22).standard_normal(model.n_params)
         model.set_params(params)
@@ -415,16 +430,26 @@ def test_train_epoch_host_equals_step_by_step(api):
         elif mode == "epoch":
             cost, hits = model.train_epoch_host(images, labels, B, 3.0)
             assert len(cost) == N // B
-        else:
-            if mode.endswith("again"):                   # second epoch on the same handle replays the cached graph
-                model.train_epoch_host(pinned.numpy(), pinned_labels.numpy(), B, 3.0)
-                model.set_params(params)
+        elif mode == "epoch-pinned":
+            # the double-buffered loop launches the update kernel every step; the streamed loop updates inside kernel B in its
+            # graphs, and only its warm-up (no update) runs eagerly
+            _lib.profile_enable(True)
+            try:
+                cost, hits = model.train_epoch_host(pinned.numpy(), pinned_labels.numpy(), B, 3.0)
+                names = list(_lib.profile_report())
+            finally:
+                _lib.profile_enable(False)
+            assert len(cost) == N // B
+        else:                                            # a second epoch on the same handle (the ring replays its graphs)
+            model.train_epoch_host(pinned.numpy(), pinned_labels.numpy(), B, 3.0)
+            model.set_params(params)
             cost, hits = model.train_epoch_host(pinned.numpy(), pinned_labels.numpy(), B, 3.0)
             assert len(cost) == N // B
         results.append((model.get_params(), cost, hits))
     for other in results[1:]:
-        assert np.array_equal(results[0][0], other[0]), "same kernels, same order: parameters must be bit-identical"
-        assert np.array_equal(results[0][1], other[1]) and np.array_equal(results[0][2], other[2])
+        assert np.array_equal(results[0][0], other[0]), f"{stack} {hw}: same kernels, same order: parameters must be bit-identical"
+        assert np.array_equal(results[0][1], other[1]) and np.array_equal(results[0][2], other[2]), f"{stack} {hw}"
+    assert ("sgd_update_kernel" in names) != streams, (stack, hw, names)
 
 
 def test_train_epoch_host_streaming_large_chunks(api):
