@@ -231,30 +231,44 @@ __global__ void __launch_bounds__(256) ozaki_slice_rmajor_kernel(const OzOperand
     }
 }
 
-// ---- whole-tensor slicing (one scale): convolution inputs whose im2col is done by TMA -------------------------------
-__global__ void __launch_bounds__(256) ozaki_amax_tensor_kernel(const double* __restrict__ x, size_t n, unsigned long long* __restrict__ amax_bits) {
-    double amax = 0.0;
-    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) amax = amax_fold(amax, x[i]);
+// ---- per-image slicing (one scale per image): convolution inputs whose im2col is done by TMA -----------------------
+// x is [B][per_img]; blockIdx.y strides over the images, so a warp's maximum never mixes two images.  One scale per image
+// keeps every output's truncation relative to its own image (a 128-pixel tile never crosses an image, see
+// ozaki_conv_tma_ok), and a non-finite element poisons only its own image.
+__global__ void __launch_bounds__(256) ozaki_amax_tensor_kernel(const double* __restrict__ x, int B, size_t per_img,
+                                                                unsigned long long* __restrict__ amax_bits) {
+    for (int img = blockIdx.y; img < B; img += gridDim.y) {
+        const double* xi = x + (size_t)img * per_img;
+        double amax = 0.0;
+        for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < per_img; i += (size_t)gridDim.x * blockDim.x)
+            amax = amax_fold(amax, xi[i]);
 #pragma unroll
-    for (int o = 16; o > 0; o >>= 1) amax = fmax(amax, __shfl_xor_sync(0xffffffffu, amax, o));
-    if ((threadIdx.x & 31) == 0) atomicMax(amax_bits, (unsigned long long)__double_as_longlong(amax_finish(amax)));
+        for (int o = 16; o > 0; o >>= 1) amax = fmax(amax, __shfl_xor_sync(0xffffffffu, amax, o));
+        if ((threadIdx.x & 31) == 0) atomicMax(amax_bits + img, (unsigned long long)__double_as_longlong(amax_finish(amax)));
+    }
 }
 
-__global__ void __launch_bounds__(256) ozaki_slice_tensor_kernel(const double* __restrict__ x, size_t n, const unsigned long long* __restrict__ amax_bits,
+__global__ void __launch_bounds__(256) ozaki_slice_tensor_kernel(const double* __restrict__ x, int B, size_t per_img,
+                                                                 const unsigned long long* __restrict__ amax_bits,
                                                                  int8_t* __restrict__ planes, double* __restrict__ scale_out) {
-    double inv, sc;
-    row_scale(__longlong_as_double((long long)*amax_bits), inv, sc);
-    if (blockIdx.x == 0 && threadIdx.x == 0) scale_out[0] = sc;
-    const size_t n4 = n / 4;       // n is a multiple of 64 (C % 64 == 0)
-    for (size_t i4 = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i4 < n4; i4 += (size_t)gridDim.x * blockDim.x) {
-        const double2 a = reinterpret_cast<const double2*>(x)[2 * i4], b = reinterpret_cast<const double2*>(x)[2 * i4 + 1];
-        int8_t q[4][OZ_S];
-        slice6(a.x, inv, q[0]); slice6(a.y, inv, q[1]); slice6(b.x, inv, q[2]); slice6(b.y, inv, q[3]);
+    const size_t n = (size_t)B * per_img;
+    const size_t n4 = per_img / 4;   // per_img is a multiple of 64 (C % 64 == 0)
+    for (int img = blockIdx.y; img < B; img += gridDim.y) {
+        double inv, sc;
+        row_scale(__longlong_as_double((long long)amax_bits[img]), inv, sc);
+        if (blockIdx.x == 0 && threadIdx.x == 0) scale_out[img] = sc;
+        const double2* xi = reinterpret_cast<const double2*>(x + (size_t)img * per_img);
+        uint32_t* pi = reinterpret_cast<uint32_t*>(planes + (size_t)img * per_img);
+        for (size_t i4 = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i4 < n4; i4 += (size_t)gridDim.x * blockDim.x) {
+            const double2 a = xi[2 * i4], b = xi[2 * i4 + 1];
+            int8_t q[4][OZ_S];
+            slice6(a.x, inv, q[0]); slice6(a.y, inv, q[1]); slice6(b.x, inv, q[2]); slice6(b.y, inv, q[3]);
 #pragma unroll
-        for (int j = 0; j < OZ_S; ++j) {
-            const uint32_t w = (uint32_t)(uint8_t)q[0][j] | ((uint32_t)(uint8_t)q[1][j] << 8) | ((uint32_t)(uint8_t)q[2][j] << 16) |
-                               ((uint32_t)(uint8_t)q[3][j] << 24);
-            reinterpret_cast<uint32_t*>(planes + (size_t)j * n)[i4] = w;
+            for (int j = 0; j < OZ_S; ++j) {
+                const uint32_t w = (uint32_t)(uint8_t)q[0][j] | ((uint32_t)(uint8_t)q[1][j] << 8) | ((uint32_t)(uint8_t)q[2][j] << 16) |
+                                   ((uint32_t)(uint8_t)q[3][j] << 24);
+                pi[(size_t)j * (n / 4) + i4] = w;
+            }
         }
     }
 }
@@ -311,15 +325,21 @@ int ozaki_slice(const OzOperand& op, int rows, int K, int Kp, int8_t* planes, do
     return RCN_OK;
 }
 
-int ozaki_slice_tensor(const double* x, size_t n, int8_t* planes, double* scale_out, cudaStream_t stream) {
-    if (n == 0) return RCN_OK;
-    if (n % 64 || (reinterpret_cast<uintptr_t>(x) & 15)) return fail(RCN_ERR_INVALID, "tensor slicing needs a 16-byte aligned tensor of a multiple of 64 elements");
-    unsigned long long* amax_bits = reinterpret_cast<unsigned long long*>(scale_out + 1);
-    RCN_CUDA_TRY(cudaMemsetAsync(amax_bits, 0, sizeof(unsigned long long), stream));
-    unsigned grid = cdiv(n, 256 * 8);
-    if (grid > kNumSMs * 8) grid = kNumSMs * 8;
-    RCN_LAUNCH("ozaki_amax_tensor_kernel", stream, ozaki_amax_tensor_kernel<<<grid, 256, 0, stream>>>(x, n, amax_bits));
-    RCN_LAUNCH("ozaki_slice_tensor_kernel", stream, ozaki_slice_tensor_kernel<<<grid, 256, 0, stream>>>(x, n, amax_bits, planes, scale_out));
+int ozaki_slice_tensor(const double* x, int B, size_t per_image, int8_t* planes, double* scale_out, cudaStream_t stream) {
+    if (B <= 0 || per_image == 0) return RCN_OK;
+    if (per_image % 64 || (reinterpret_cast<uintptr_t>(x) & 15))
+        return fail(RCN_ERR_INVALID, "tensor slicing needs a 16-byte aligned tensor of a multiple of 64 elements per image");
+    unsigned long long* amax_bits = reinterpret_cast<unsigned long long*>(scale_out + B);
+    RCN_CUDA_TRY(cudaMemsetAsync(amax_bits, 0, (size_t)B * sizeof(unsigned long long), stream));
+    // about as many CTAs as the one-scale version launched: up to 8 per SM over the whole tensor
+    const unsigned gy = B < 65535 ? (unsigned)B : 65535u;
+    unsigned gx = cdiv(per_image, 256 * 8);
+    const unsigned gx_max = cdiv((size_t)kNumSMs * 8, gy);
+    if (gx > gx_max) gx = gx_max;
+    const dim3 grid(gx, gy);
+    RCN_LAUNCH("ozaki_amax_tensor_kernel", stream, ozaki_amax_tensor_kernel<<<grid, 256, 0, stream>>>(x, B, per_image, amax_bits));
+    RCN_LAUNCH("ozaki_slice_tensor_kernel", stream,
+               ozaki_slice_tensor_kernel<<<grid, 256, 0, stream>>>(x, B, per_image, amax_bits, planes, scale_out));
     return RCN_OK;
 }
 

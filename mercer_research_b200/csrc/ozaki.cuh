@@ -84,9 +84,10 @@ struct OzConvA {
     int C, kw, ph, pw, Ho, Wo;
 };
 
-// One power-of-two scale for a whole tensor (all pixels of a convolution input share the contraction scale):
-// planes[s][i] for i < n, scale_out[0] = scale.
-int ozaki_slice_tensor(const double* x, size_t n, int8_t* planes, double* scale_out, cudaStream_t stream);
+// One power-of-two scale per image of a convolution input x [B][per_image] (every pixel of an image, so every im2col row
+// the image feeds, shares that image's scale): planes[s][i] for i < B * per_image, scale_out[b] = scale of image b.
+// scale_out holds 2 * B doubles (the upper half is scratch for the image maxima).
+int ozaki_slice_tensor(const double* x, int B, size_t per_image, int8_t* planes, double* scale_out, cudaStream_t stream);
 // 5-D tensor map over planes [OZ_S][B][Hi][Wi][C], box = (64 channels, tw, th, 1, 1), SWIZZLE_64B.
 int ozaki_make_conv_tensor_map(CUtensorMap* map, const int8_t* planes, int B, int Hi, int Wi, int C, int tw, int th);
 
@@ -280,9 +281,12 @@ __global__ void __launch_bounds__(OZ_THREADS, 1) ozaki_gemm_kernel(const __grid_
         const int quad = warp & 3;
         const int col_half = (warp - 2) >> 2;
         const int m = m0 + quad * 32 + lane;
+        // read while the main loop runs: the slicing kernels that write the scales precede this launch in plain stream
+        // order (this kernel is never launched as a programmatic dependent, which would make the read race with them).
+        // A TMA-gathered tensor has one scale per image, and a 128-pixel tile never crosses an image (ozaki_conv_tma_ok).
+        const double sa = (m < M) ? scale_a[conv.enabled ? m0 / (conv.Ho * conv.Wo) : m] : 0.0;
         oz::mbar_wait(tmem_full_bar, 0);
         oz::tc_fence_after();
-        const double sa = (m < M) ? scale_a[conv.enabled ? 0 : m] : 0.0;   // a TMA-gathered tensor has ONE scale
         const uint32_t lane_addr = tmem_base + ((uint32_t)(quad * 32) << 16);
         constexpr double kW = 1.0 / 256.0;   // 2^-8 between neighbouring diagonals
 #pragma unroll 1
@@ -370,10 +374,11 @@ static int launch_gemm_ozaki(const char* name, const OzOperand& A, const OzOpera
 
 // Convolution forward / backward-data with the im2col done by TMA: C(pix, n) = sum_{tap, c} T[pix + tap, c] * Wk(n, (tap, c)).
 // `g` describes the gather (ConvGeom); wk is the dense [N][kh*kw*C] weight matrix (k-contiguous).  The tensor is sliced
-// ONCE, element-wise (5 B written per element instead of 45 for a materialised im2col), under one tensor-wide scale.
+// ONCE, element-wise (5 B written per element instead of 45 for a materialised im2col), under one scale per image.
+// The slicing kernel reads the tensor in 16-byte vectors; a misaligned tensor takes the per-row gather path instead.
 inline bool ozaki_conv_tma_ok(const ConvGeom& g) {
     const bool tiles_ok = (g.Wo <= OZ_BM && OZ_BM % g.Wo == 0 && g.Ho % (OZ_BM / g.Wo) == 0) || (g.Wo % OZ_BM == 0);
-    return g.C % OZ_BK == 0 && tiles_ok && g.n_k <= OZ_MAX_K;
+    return g.C % OZ_BK == 0 && tiles_ok && g.n_k <= OZ_MAX_K && (reinterpret_cast<uintptr_t>(g.t) & 15) == 0;
 }
 
 template <typename Epi>
@@ -381,12 +386,12 @@ static int launch_conv_ozaki(const char* name, const ConvGeom& g, int B, const d
                              cudaStream_t stream) {
     const int M = g.n_pix, K = g.n_k;            // K is a multiple of 64 because C is
     if (M <= 0 || N <= 0) return RCN_OK;
-    const size_t n_elems = (size_t)B * g.Hi * g.Wi * g.C;
-    RCN_TRY(ws.a_slices.reserve((size_t)OZ_S * n_elems));
+    const size_t per_image = (size_t)g.Hi * g.Wi * g.C;
+    RCN_TRY(ws.a_slices.reserve((size_t)OZ_S * B * per_image));
     RCN_TRY(ws.b_slices.reserve((size_t)OZ_S * N * K));
-    RCN_TRY(ws.a_scale.reserve(2 * sizeof(double)));
+    RCN_TRY(ws.a_scale.reserve((size_t)2 * B * sizeof(double)));
     RCN_TRY(ws.b_scale.reserve((size_t)2 * N * sizeof(double)));
-    RCN_TRY(ozaki_slice_tensor(g.t, n_elems, ws.a_slices.as<int8_t>(), ws.a_scale.as<double>(), stream));
+    RCN_TRY(ozaki_slice_tensor(g.t, B, per_image, ws.a_slices.as<int8_t>(), ws.a_scale.as<double>(), stream));
     const OzOperand ob{wk, (size_t)K, true};
     RCN_TRY(ozaki_slice(ob, N, K, K, ws.b_slices.as<int8_t>(), ws.b_scale.as<double>(), ws.b_scale.as<double>() + N, stream));
     const int tw = g.Wo < OZ_BM ? g.Wo : OZ_BM, th = OZ_BM / tw;
