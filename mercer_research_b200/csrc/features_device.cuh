@@ -7,11 +7,12 @@
 namespace rcn {
 
 // ------------------------------------------------------------------------------------------------
-// Device arithmetic.  mac(a, k, c) = c + a*k.  The taps are in {0, +-1, +-2}, so a*k is exact in f64 and a
-// fused multiply-add rounds exactly like the reference's separate multiply and add (kernel.rs:164).  Zero
-// taps are kept (inf*0 must stay NaN as in the reference); for T = int the compiler folds them away.
+// Device arithmetic.  mac(a, k, c) = c + a*k, the product rounded before the add like the reference's separate
+// multiply and add (kernel.rs:164).  The taps are in {0, +-1, +-2}, so a*k is exact -- except that 2*a overflows for
+// |a| > DBL_MAX / 2: the reference then adds +-Inf, where a fused multiply-add would round the exact sum to a finite
+// value.  Zero taps are kept (inf*0 must stay NaN as in the reference); for T = int the compiler folds them away.
 // ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ double mac(double a, double k, double c) { return fma(a, k, c); }
+__device__ __forceinline__ double mac(double a, double k, double c) { return __dadd_rn(c, __dmul_rn(a, k)); }
 __device__ __forceinline__ int mac(int a, int k, int c) { return a * k + c; }
 
 template <typename T>
