@@ -399,4 +399,76 @@ class RCN {
     int device_ = 0;
 };
 
+/// Learned conv / pool layers in front of the reference's dense stack (rcn_cuda_cnn_* in rcn_cuda.h): a thin owner of the
+/// handle.  Images are u8 (B, H, W) row-major or f64 (B, H, W, C) NHWC, host or device memory.
+class ConvNet {
+  public:
+    struct Layer {
+        static Layer conv(size_t co, size_t kh, size_t kw, Padding p) {
+            return Layer{{RCN_CNN_CONV, (int32_t)co, (int32_t)kh, (int32_t)kw, (int32_t)p}};
+        }
+        static Layer pool(Pooling pooling, Padding p) { return Layer{{RCN_CNN_POOL, (int32_t)pooling, (int32_t)p, 0, 0}}; }
+        int32_t spec[RCN_CNN_LAYER_INTS];
+    };
+
+    ConvNet(size_t H, size_t W, size_t in_channels, const std::vector<Layer>& layers, const std::vector<size_t>& feedforward,
+            size_t classes, int device = 0) {
+        std::vector<int32_t> spec;
+        for (const Layer& l : layers) spec.insert(spec.end(), l.spec, l.spec + RCN_CNN_LAYER_INTS);
+        check(rcn_cuda_cnn_create(device, H, W, in_channels, spec.data(), layers.size(), feedforward.data(), feedforward.size(),
+                                  classes, &h_));
+    }
+    ~ConvNet() { rcn_cuda_cnn_destroy(h_); }
+    ConvNet(const ConvNet&) = delete;
+    ConvNet& operator=(const ConvNet&) = delete;
+
+    size_t n_params() const {
+        size_t n = 0;
+        check(rcn_cuda_cnn_param_count(h_, &n));
+        return n;
+    }
+    void set_params(const std::vector<double>& flat) { check(rcn_cuda_cnn_set_params(h_, flat.data(), flat.size())); }
+    std::vector<double> get_params() const {
+        std::vector<double> p(n_params());
+        check(rcn_cuda_cnn_get_params(h_, p.data(), p.size()));
+        return p;
+    }
+    std::vector<double> get_gradients() const {
+        std::vector<double> g(n_params());
+        check(rcn_cuda_cnn_get_gradients(h_, g.data(), g.size()));
+        return g;
+    }
+    void train_batch(const void* images, int pixel_format, const int64_t* labels, size_t B, size_t H, size_t W, double eta) {
+        check(rcn_cuda_cnn_train_batch(h_, images, pixel_format, labels, B, H, W, eta));
+    }
+    void accumulate(const void* images, int pixel_format, const int64_t* labels, size_t B, size_t H, size_t W) {
+        check(rcn_cuda_cnn_accumulate(h_, images, pixel_format, labels, B, H, W));
+    }
+    void apply(double eta, size_t global_batch) { check(rcn_cuda_cnn_apply(h_, eta, global_batch)); }
+    /// (quadratic cost, hit count) of the last accumulated batch under the pre-update parameters.
+    std::pair<double, uint64_t> last_batch_stats() const {
+        double c = 0.0;
+        uint64_t hits = 0;
+        check(rcn_cuda_cnn_last_batch_stats(h_, &c, &hits));
+        return {c, hits};
+    }
+    /// (accept, cost) of a labelled batch (rcn.rs:152-157 rule); labels_out (optional) receives the predictions.
+    std::pair<uint64_t, double> evaluate(const void* images, int pixel_format, const int64_t* labels, size_t B, size_t H, size_t W,
+                                         int64_t* labels_out = nullptr) {
+        double c = 0.0;
+        uint64_t acc = 0;
+        check(rcn_cuda_cnn_evaluate_images(h_, images, pixel_format, labels, B, H, W, &c, &acc, labels_out));
+        return {acc, c};
+    }
+    std::vector<int64_t> classify(const void* images, int pixel_format, size_t B, size_t H, size_t W) {
+        std::vector<int64_t> out(B);
+        check(rcn_cuda_cnn_classify_images(h_, images, pixel_format, B, H, W, out.data()));
+        return out;
+    }
+    rcn_cuda_cnn_handle handle() const { return h_; }
+
+  private:
+    rcn_cuda_cnn_handle h_ = nullptr;
+};
+
 }  // namespace rcn

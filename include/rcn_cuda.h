@@ -30,6 +30,7 @@ extern "C" {
 #endif
 
 typedef struct rcn_cuda_model* rcn_cuda_handle;
+typedef struct rcn_cuda_cnn* rcn_cuda_cnn_handle;
 
 typedef enum rcn_status {
     RCN_OK = 0,
@@ -52,7 +53,8 @@ enum { RCN_LAYER_CONV_NONE = 0, RCN_LAYER_CONV_SAME = 1, RCN_LAYER_POOL_AVERAGE 
 /* Pixel formats accepted by the image entry points. */
 enum {
     RCN_PIXELS_U8_ROWMAJOR = 0,  /* `image` crate GrayImage buffer, before get_pixel_matrix (lib.rs:27-33) */
-    RCN_PIXELS_F64_COLMAJOR = 1  /* DMatrix<f64> H x W as get_pixel_matrix returns it */
+    RCN_PIXELS_F64_COLMAJOR = 1, /* DMatrix<f64> H x W as get_pixel_matrix returns it */
+    RCN_PIXELS_F64_NHWC = 2      /* f64 (B, H, W, C) channels-last; only the rcn_cuda_cnn_* entry points accept it */
 };
 
 const char* rcn_cuda_last_error(void);
@@ -302,6 +304,67 @@ int rcn_cuda_ext_softmax_xent(int device, void* cuda_stream, const double* z, si
  * The dense layers pick impl 1 automatically for large shapes (env RCN_CUDA_GEMM = dmma | tc | simt overrides). */
 int rcn_cuda_ext_gemm_f64(int device, void* cuda_stream, const double* A, size_t lda, int a_kcontig, const double* B,
                           size_t ldb, int b_kcontig, size_t M, size_t N, size_t K, int impl, double* C);
+
+/* ---- convolutional network: learned conv / pool layers in front of the dense stack ---------------------------------
+ * EXTENSION (BASELINE.json north_star configs 3 and 4; the reference has no learned convolution).  The network is
+ *   input (B, H, W, C)  ->  conv / pool stack (NHWC)  ->  flatten  ->  the reference's dense stack (sigmoid layers,
+ *   quadratic cost, W -= (eta/B) * sum dW).
+ * layer_spec: n_layers records of RCN_CNN_LAYER_INTS int32 each:
+ *   {RCN_CNN_CONV, Co, kh, kw, padding}   learned cross-correlation with bias, ALWAYS followed by ReLU; conventions and
+ *                                         contract errors of rcn_cuda_ext_conv2d_forward (odd kernels for Same)
+ *   {RCN_CNN_POOL, pooling, padding, 0, 0} 2x2 / stride 2 as rcn_cuda_ext_pool2d_forward (last maximal element wins, Same
+ *                                         pads the bottom row / right column)
+ * Flatten: the last stack output [B][Hp][Wp][C] IS the L x B column-major feature matrix of the dense stack,
+ * L = Hp*Wp*C (sample-major NHWC order).  The dense stack is feedforward[0..n_ff) then `classes`; its features are NOT
+ * standardised.
+ * Parameters and gradients are one flat buffer [w0 (Co,kh,kw,Ci) | b0 (Co) | w1 | b1 | ... | W0 | b0 | W1 | b1 | ...]: the
+ * conv layers in stack order, then the dense layers in the layout of rcn_cuda_set_params.
+ * Images: RCN_PIXELS_U8_ROWMAJOR (B, H, W) with in_channels == 1, or RCN_PIXELS_F64_NHWC (B, H, W, in_channels); the shape
+ * is fixed at creation (it fixes L and so the parameter count): other H, W fail with RCN_ERR_SHAPE.
+ * Pointers may be host or device memory as elsewhere; with device images, labels and outputs nothing synchronises, and
+ * once a call with at least as many images has sized the buffers (rcn_cuda_allocation_generation), accumulate + apply can
+ * be captured into a CUDA graph.  A NaN reaching a max pool is not reported (the cost turns NaN instead). */
+enum { RCN_CNN_CONV = 0, RCN_CNN_POOL = 1 };
+#define RCN_CNN_LAYER_INTS 5
+/* Validates the whole spec before any device work (status codes and messages of the ext ops; a zero-width dense layer or
+ * zero classes is RCN_ERR_INVALID).  Parameters start at zero: set them with rcn_cuda_cnn_set_params. */
+int rcn_cuda_cnn_create(int device, size_t H, size_t W, size_t in_channels, const int32_t* layer_spec, size_t n_layers,
+                        const size_t* feedforward, size_t n_ff, size_t classes, rcn_cuda_cnn_handle* out);
+int rcn_cuda_cnn_destroy(rcn_cuda_cnn_handle h);
+/* As rcn_cuda_set_stream: NULL is the legacy default stream, RCN_STREAM_OWN the handle's own stream. */
+int rcn_cuda_cnn_set_stream(rcn_cuda_cnn_handle h, void* cuda_stream);
+int rcn_cuda_cnn_synchronize(rcn_cuda_cnn_handle h);
+/* Output shape of stack layer `layer` (n_layers - 1: the flattened features, L = H*W*C). */
+int rcn_cuda_cnn_layer_shape(rcn_cuda_cnn_handle h, size_t layer, size_t* H, size_t* W, size_t* C);
+int rcn_cuda_cnn_param_count(rcn_cuda_cnn_handle h, size_t* n);
+int rcn_cuda_cnn_set_params(rcn_cuda_cnn_handle h, const double* flat, size_t n);
+int rcn_cuda_cnn_get_params(rcn_cuda_cnn_handle h, double* flat, size_t n);
+/* Gradient sums of the batch into the flat gradient buffer, no update.  Per step: conv (+bias+ReLU) and pool forward, the
+ * dense stack's accumulate on the stack output, dX = W0^T delta0 with the pre-update W0, then down the stack pool
+ * backward, ReLU', conv weight and bias gradients, and conv input gradients except for the first conv layer. */
+int rcn_cuda_cnn_accumulate(rcn_cuda_cnn_handle h, const void* images, int pixel_format, const int64_t* labels, size_t B,
+                            size_t H, size_t W);
+/* p <- p - (eta / global_batch) * g over every parameter (rcn.rs:210-222 rounding). */
+int rcn_cuda_cnn_apply(rcn_cuda_cnn_handle h, double eta, size_t global_batch);
+/* accumulate + apply(eta, B) */
+int rcn_cuda_cnn_train_batch(rcn_cuda_cnn_handle h, const void* images, int pixel_format, const int64_t* labels, size_t B,
+                             size_t H, size_t W, double eta);
+/* Quadratic cost and rcn.rs:153-157 hit count of the last accumulate, under the pre-update parameters. */
+int rcn_cuda_cnn_last_batch_stats(rcn_cuda_cnn_handle h, double* cost, uint64_t* hits);
+/* Forward pass only: cost_out, accept_out as rcn_cuda_evaluate_images; labels_out (optional) the rcn.rs:92-97 argmax.
+ * Leaves the gradients and the last-batch statistics untouched (the layer-output tap then shows this batch). */
+int rcn_cuda_cnn_evaluate_images(rcn_cuda_cnn_handle h, const void* images, int pixel_format, const int64_t* labels, size_t B,
+                                 size_t H, size_t W, double* cost_out, uint64_t* accept_out, int64_t* labels_out);
+int rcn_cuda_cnn_classify_images(rcn_cuda_cnn_handle h, const void* images, int pixel_format, size_t B, size_t H, size_t W,
+                                 int64_t* labels_out);
+/* As rcn_cuda_bind_gradient_buffer / rcn_cuda_gradient_buffer / rcn_cuda_get_gradients, over the whole flat buffer. */
+int rcn_cuda_cnn_bind_gradient_buffer(rcn_cuda_cnn_handle h, double* device_ptr, size_t n);
+int rcn_cuda_cnn_gradient_buffer(rcn_cuda_cnn_handle h, double** device_ptr, size_t* n);
+int rcn_cuda_cnn_get_gradients(rcn_cuda_cnn_handle h, double* flat, size_t n);
+/* Debug / parity taps: the output of stack layer `layer` of the last accumulate or evaluate (post-ReLU for a conv, pooled
+ * for a pool; B x H x W x C), and the dense stack's input gradient dX (L x B) of the last accumulate. */
+int rcn_cuda_cnn_get_layer_output(rcn_cuda_cnn_handle h, size_t layer, double* out);
+int rcn_cuda_cnn_get_input_gradient(rcn_cuda_cnn_handle h, double* out);
 
 #ifdef __cplusplus
 }

@@ -19,6 +19,7 @@ STATUS_NAMES = {
 
 PIXELS_U8_ROWMAJOR = 0
 PIXELS_F64_COLMAJOR = 1
+PIXELS_F64_NHWC = 2
 
 # name -> argtypes; every function returns int (rcn_status) unless listed in _RESTYPES.
 _vp, _sz, _i, _d = C.c_void_p, C.c_size_t, C.c_int, C.c_double
@@ -95,6 +96,26 @@ SIGNATURES = {
     "rcn_cuda_ext_pool2d_backward": [_i, _vp, _vp, _vp, _sz, _sz, _sz, _sz, _i, _i, _vp],
     "rcn_cuda_ext_softmax_xent": [_i, _vp, _vp, _sz, _sz, _vp, _vp, _vp, _vp, _vp],
     "rcn_cuda_ext_gemm_f64": [_i, _vp, _vp, _sz, _i, _vp, _sz, _i, _sz, _sz, _sz, _i, _vp],
+    # convolutional network handle (learned conv / pool layers + the dense stack)
+    "rcn_cuda_cnn_create": [_i, _sz, _sz, _sz, _vp, _sz, _vp, _sz, _sz, C.POINTER(_vp)],
+    "rcn_cuda_cnn_destroy": [_vp],
+    "rcn_cuda_cnn_set_stream": [_vp, _vp],
+    "rcn_cuda_cnn_synchronize": [_vp],
+    "rcn_cuda_cnn_layer_shape": [_vp, _sz, _szp, _szp, _szp],
+    "rcn_cuda_cnn_param_count": [_vp, _szp],
+    "rcn_cuda_cnn_set_params": [_vp, _vp, _sz],
+    "rcn_cuda_cnn_get_params": [_vp, _vp, _sz],
+    "rcn_cuda_cnn_accumulate": [_vp, _vp, _i, _vp, _sz, _sz, _sz],
+    "rcn_cuda_cnn_apply": [_vp, _d, _sz],
+    "rcn_cuda_cnn_train_batch": [_vp, _vp, _i, _vp, _sz, _sz, _sz, _d],
+    "rcn_cuda_cnn_last_batch_stats": [_vp, C.POINTER(_d), C.POINTER(C.c_uint64)],
+    "rcn_cuda_cnn_evaluate_images": [_vp, _vp, _i, _vp, _sz, _sz, _sz, _vp, _vp, _vp],
+    "rcn_cuda_cnn_classify_images": [_vp, _vp, _i, _sz, _sz, _sz, _vp],
+    "rcn_cuda_cnn_bind_gradient_buffer": [_vp, _vp, _sz],
+    "rcn_cuda_cnn_gradient_buffer": [_vp, C.POINTER(_vp), _szp],
+    "rcn_cuda_cnn_get_gradients": [_vp, _vp, _sz],
+    "rcn_cuda_cnn_get_layer_output": [_vp, _sz, _vp],
+    "rcn_cuda_cnn_get_input_gradient": [_vp, _vp],
 }
 _RESTYPES = {"rcn_cuda_last_error": C.c_char_p}
 

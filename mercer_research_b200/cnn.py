@@ -1,0 +1,258 @@
+"""A trainable convolutional network: learned conv / pool layers in front of the reference's dense stack (sigmoid layers,
+quadratic cost, ``W -= (eta/B) * sum dW``), driving the ``rcn_cuda_cnn_*`` entry points of librcn_cuda.so.
+
+Images are numpy arrays (staged through the device) or torch CUDA tensors (used in place, on torch's current stream):
+``(B, H, W)`` uint8 (one channel) or ``(B, H, W, C)`` float64 channels-last.  Labels are ``(B,)`` int64.  The flat
+parameter and gradient layout is ``[w0 (Co,kh,kw,Ci) | b0 | w1 | b1 | ... | W0 | b0 | W1 | b1 | ...]`` -- the conv layers
+in stack order, then the dense layers exactly as ``RCN.get_params`` lays them out.  The method names are the ones
+``DataParallelTrainer`` calls, so the trainer's NCCL exchange drives this network unchanged.
+"""
+from __future__ import annotations
+
+import ctypes as C
+from dataclasses import dataclass
+from typing import List, Sequence, Tuple
+
+import numpy as np
+
+from . import _lib
+from .kernel import Padding, Pooling, _is_torch
+from .rcn import _Buf
+
+CNN_CONV, CNN_POOL, LAYER_INTS = 0, 1, 5
+
+
+@dataclass(frozen=True)
+class Conv:
+    """Learned cross-correlation with bias, always followed by ReLU (odd kernels for ``Padding.Same``)."""
+    out_channels: int
+    kh: int = 3
+    kw: int = 3
+    padding: Padding = Padding.Same
+
+    def spec(self):
+        return [CNN_CONV, int(self.out_channels), int(self.kh), int(self.kw), int(Padding(self.padding))]
+
+
+@dataclass(frozen=True)
+class Pool:
+    """2x2 / stride-2 pooling; ``Padding.Same`` pads the bottom row / right column of odd maps."""
+    pooling: Pooling = Pooling.Max
+    padding: Padding = Padding.Same
+
+    def spec(self):
+        return [CNN_POOL, int(Pooling(self.pooling)), int(Padding(self.padding)), 0, 0]
+
+
+class ConvNet:
+    """``ConvNet((H, W, C), [Conv(16), Pool(), ...], feedforward=[64], classes=10)``."""
+
+    def __init__(self, input_shape: Sequence[int], layers: Sequence, feedforward: Sequence[int], classes: int, device: int = 0):
+        self._lib = _lib.load()
+        H, W, Cin = (int(x) for x in input_shape)
+        self.input_shape = (H, W, Cin)
+        self.layers = list(layers)
+        self.feedforward = [int(x) for x in feedforward]
+        self.classes = int(classes)
+        self.device = int(device)
+        spec = [v for l in self.layers for v in l.spec()]
+        arr = (C.c_int32 * max(1, len(spec)))(*spec)
+        ff = (C.c_size_t * max(1, len(self.feedforward)))(*self.feedforward)
+        h = C.c_void_p()
+        _lib.check(self._lib.rcn_cuda_cnn_create(self.device, H, W, Cin, arr, len(self.layers), ff, len(self.feedforward),
+                                                 self.classes, C.byref(h)))
+        self._h = h
+        self._shapes = []
+        for i in range(len(self.layers)):
+            a, b, c = C.c_size_t(), C.c_size_t(), C.c_size_t()
+            _lib.check(self._lib.rcn_cuda_cnn_layer_shape(self._h, i, C.byref(a), C.byref(b), C.byref(c)))
+            self._shapes.append((a.value, b.value, c.value))
+        self._B_out = self._B_grad = 0
+
+    # -- lifetime -----------------------------------------------------------------------------------------------------
+    def close(self):
+        if getattr(self, "_h", None):
+            self._lib.rcn_cuda_cnn_destroy(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def set_stream(self, cuda_stream):
+        """Run on an existing cudaStream_t (int handle); ``-1`` restores the handle's own stream."""
+        if cuda_stream is not None and cuda_stream < 0:
+            cuda_stream = C.c_void_p(-1).value
+        _lib.check(self._lib.rcn_cuda_cnn_set_stream(self._h, cuda_stream))
+
+    def synchronize(self):
+        _lib.check(self._lib.rcn_cuda_cnn_synchronize(self._h))
+
+    def _use_torch_stream(self, *bufs):
+        for b in bufs:
+            if b is not None and b.torch:
+                import torch
+                self.set_stream(torch.cuda.current_stream(b.device).cuda_stream)
+                return
+
+    # -- shapes / parameters ------------------------------------------------------------------------------------------
+    def layer_shape(self, layer: int) -> Tuple[int, int, int]:
+        """(H, W, C) output of stack layer ``layer``."""
+        return self._shapes[layer]
+
+    @property
+    def feature_len(self) -> int:
+        h, w, c = self._shapes[-1]
+        return h * w * c
+
+    @property
+    def n_params(self) -> int:
+        n = C.c_size_t()
+        _lib.check(self._lib.rcn_cuda_cnn_param_count(self._h, C.byref(n)))
+        return n.value
+
+    def param_slices(self) -> List[Tuple[str, slice, tuple]]:
+        """(name, slice of the flat buffer, shape) of every parameter tensor, conv layers first."""
+        out, off, cin = [], 0, self.input_shape[2]
+        for i, l in enumerate(self.layers):
+            if isinstance(l, Conv):
+                shp = (l.out_channels, l.kh, l.kw, cin)
+                n = int(np.prod(shp))
+                out.append((f"conv{i}.w", slice(off, off + n), shp))
+                off += n
+                out.append((f"conv{i}.b", slice(off, off + l.out_channels), (l.out_channels,)))
+                off += l.out_channels
+            cin = self._shapes[i][2]
+        cols = self.feature_len
+        for j, rows in enumerate(self.feedforward + [self.classes]):
+            out.append((f"dense{j}.W", slice(off, off + rows * cols), (rows, cols)))   # column-major rows x cols
+            off += rows * cols
+            out.append((f"dense{j}.b", slice(off, off + rows), (rows,)))
+            off += rows
+            cols = rows
+        return out
+
+    def init_params(self, rng: np.random.Generator) -> np.ndarray:
+        """He-scaled N(0, 2/fan_in) conv weights, zero conv biases, and the reference's unscaled N(0, 1) for every dense
+        weight and bias (rcn.rs:500-523).  Sets and returns the flat parameters."""
+        p = np.zeros(self.n_params)
+        for name, sl, shp in self.param_slices():
+            if name.startswith("conv") and name.endswith(".w"):
+                fan_in = shp[1] * shp[2] * shp[3]
+                p[sl] = rng.standard_normal(sl.stop - sl.start) * np.sqrt(2.0 / fan_in)
+            elif name.startswith("dense"):
+                p[sl] = rng.standard_normal(sl.stop - sl.start)
+        self.set_params(p)
+        return p
+
+    def set_params(self, flat):
+        flat = np.ascontiguousarray(flat, dtype=np.float64).ravel()
+        _lib.check(self._lib.rcn_cuda_cnn_set_params(self._h, flat.ctypes.data, flat.size))
+
+    def get_params(self) -> np.ndarray:
+        buf = np.zeros(self.n_params)
+        _lib.check(self._lib.rcn_cuda_cnn_get_params(self._h, buf.ctypes.data, buf.size))
+        return buf
+
+    def get_gradients(self) -> np.ndarray:
+        buf = np.zeros(self.n_params)
+        _lib.check(self._lib.rcn_cuda_cnn_get_gradients(self._h, buf.ctypes.data, buf.size))
+        return buf
+
+    def bind_gradient_buffer(self, tensor):
+        """Use a caller-owned torch CUDA float64 tensor (n_params) as the flat gradient buffer (all-reduce target)."""
+        if tensor is None:
+            _lib.check(self._lib.rcn_cuda_cnn_bind_gradient_buffer(self._h, None, 0))
+            self._grad_keepalive = None
+            return
+        self._grad_keepalive = tensor
+        _lib.check(self._lib.rcn_cuda_cnn_bind_gradient_buffer(self._h, tensor.data_ptr(), tensor.numel()))
+
+    # -- batches --------------------------------------------------------------------------------------------------------
+    def _images(self, images):
+        if _is_torch(images):
+            import torch
+            if images.dtype == torch.uint8:
+                b = _Buf(images, np.uint8)
+                return b, _lib.PIXELS_U8_ROWMAJOR, b.shape[:3]
+            b = _Buf(images, np.float64)
+            return b, _lib.PIXELS_F64_NHWC, b.shape[:3]
+        a = np.asarray(images)
+        if a.dtype == np.uint8:
+            if a.ndim != 3:
+                raise ValueError("u8 images must be (B, H, W)")
+            return _Buf(a, np.uint8), _lib.PIXELS_U8_ROWMAJOR, a.shape
+        if a.ndim != 4:
+            raise ValueError("float images must be (B, H, W, C)")
+        return _Buf(a, np.float64), _lib.PIXELS_F64_NHWC, a.shape[:3]
+
+    def accumulate_gradients_images(self, images, labels):
+        """Gradient sums of the batch into the flat gradient buffer; no update."""
+        buf, fmt, (B, H, W) = self._images(images)
+        lb = _Buf(labels, np.int64)
+        self._use_torch_stream(buf, lb)
+        _lib.check(self._lib.rcn_cuda_cnn_accumulate(self._h, buf.ptr, fmt, lb.ptr, B, H, W))
+        self._B_out = self._B_grad = B
+
+    def apply_gradients(self, eta: float, batch: int):
+        """p <- p - (eta / batch) * g over every parameter; ``batch`` is the global minibatch."""
+        _lib.check(self._lib.rcn_cuda_cnn_apply(self._h, float(eta), int(batch)))
+
+    def train_batch_images(self, images, labels, eta: float):
+        buf, fmt, (B, H, W) = self._images(images)
+        lb = _Buf(labels, np.int64)
+        self._use_torch_stream(buf, lb)
+        _lib.check(self._lib.rcn_cuda_cnn_train_batch(self._h, buf.ptr, fmt, lb.ptr, B, H, W, float(eta)))
+        self._B_out = self._B_grad = B
+
+    def last_batch_stats(self) -> Tuple[float, int]:
+        """(quadratic cost, hits) of the last accumulated batch, evaluated with the pre-update parameters."""
+        c, h = C.c_double(), C.c_uint64()
+        _lib.check(self._lib.rcn_cuda_cnn_last_batch_stats(self._h, C.byref(c), C.byref(h)))
+        return c.value, h.value
+
+    def _labels_out(self, buf, B):
+        if buf.torch:
+            import torch
+            o = torch.empty((B,), dtype=torch.int64, device=buf.device)
+            return o, o.data_ptr()
+        o = np.zeros(B, dtype=np.int64)
+        return o, o.ctypes.data
+
+    def evaluate_images(self, images, labels, want_labels: bool = False):
+        """``(accept, cost)`` of a labelled batch -- the rcn.rs:153-157 hit count and the quadratic cost -- and with
+        ``want_labels`` also the predicted labels, ``(accept, cost, labels)``.  Leaves the gradients untouched."""
+        buf, fmt, (B, H, W) = self._images(images)
+        lb = _Buf(labels, np.int64)
+        self._use_torch_stream(buf, lb)
+        cost, acc = C.c_double(), C.c_uint64()
+        o, optr = self._labels_out(buf, B) if want_labels else (None, None)
+        _lib.check(self._lib.rcn_cuda_cnn_evaluate_images(self._h, buf.ptr, fmt, lb.ptr, B, H, W, C.addressof(cost),
+                                                          C.addressof(acc), optr))
+        if B:
+            self._B_out = B
+        return (acc.value, cost.value, o) if want_labels else (acc.value, cost.value)
+
+    def classify_images(self, images):
+        buf, fmt, (B, H, W) = self._images(images)
+        self._use_torch_stream(buf)
+        o, optr = self._labels_out(buf, B)
+        _lib.check(self._lib.rcn_cuda_cnn_classify_images(self._h, buf.ptr, fmt, B, H, W, optr))
+        if B:
+            self._B_out = B
+        return o
+
+    # -- taps -----------------------------------------------------------------------------------------------------------
+    def layer_output(self, layer: int) -> np.ndarray:
+        """Output of stack layer ``layer`` of the last batch run through the network, (B, H, W, C)."""
+        out = np.zeros((self._B_out,) + tuple(self._shapes[layer]))
+        _lib.check(self._lib.rcn_cuda_cnn_get_layer_output(self._h, int(layer), out.ctypes.data))
+        return out
+
+    def input_gradient(self) -> np.ndarray:
+        """dX = W0^T delta0 of the last accumulate: (B, L), sample b's gradient with respect to its flattened features."""
+        out = np.zeros((self._B_grad, self.feature_len))
+        _lib.check(self._lib.rcn_cuda_cnn_get_input_gradient(self._h, out.ctypes.data))
+        return out

@@ -18,14 +18,13 @@
 // layers (Ci*kh*kw <= 64, e.g. 1- or 3-channel images) are not dense contractions: they run a direct kernel that
 // stages the input halo tile and the weights in shared memory (north_star: "small-channel first layers ... run as
 // coalesced, vectorised, shared-memory-staged kernels").
+#include "conv.cuh"
 #include "dense.cuh"
 #include "gemm_f64.cuh"
 #include "opctx.cuh"
 #include "ozaki.cuh"
 
 namespace rcn {
-
-enum { ACT_NONE = 0, ACT_RELU = 1, ACT_SIGMOID = 2 };
 
 __device__ __forceinline__ double act_forward(double z, int act) {
     if (act == ACT_RELU) return z >= 0.0 ? z : 0.0;              // kernel.rs:209-216 rule
@@ -182,11 +181,12 @@ __global__ void activation_backward_kernel(const double* __restrict__ y, const d
 // One CTA = a 16 x 16 tile of output pixels of one image, all output channels.  The input halo tile
 // ((16+kh-1) x (16+kw-1) x Ci) and the whole weight tensor are staged in shared memory (coalesced row runs); each
 // thread owns one pixel and produces the output channels eight at a time (weights are warp-uniform broadcasts).
+// The pixel type is a template parameter: u8 images (one channel) are read as they are stored.
 constexpr int DT = 16;
-__global__ void __launch_bounds__(DT * DT) conv2d_direct_small_kernel(const double* __restrict__ x, int H, int W, int Ci,
-                                                                       const double* __restrict__ w, const double* __restrict__ bias,
-                                                                       int Co, int kh, int kw, int ph, int pw, int Ho, int Wo,
-                                                                       int act, double* __restrict__ y) {
+template <typename Px>
+__device__ __forceinline__ void conv2d_direct_small(const Px* __restrict__ x, int H, int W, int Ci, const double* __restrict__ w,
+                                                    const double* __restrict__ bias, int Co, int kh, int kw, int ph, int pw, int Ho,
+                                                    int Wo, int act, double* __restrict__ y) {
     extern __shared__ __align__(16) double sm_direct[];
     const int th = DT + kh - 1, tw = DT + kw - 1;
     const int kk = kh * kw * Ci;
@@ -202,7 +202,7 @@ __global__ void __launch_bounds__(DT * DT) conv2d_direct_small_kernel(const doub
         const int iy = oy0 + ry - ph;
         const int ix = ox0 - pw + rx / Ci;
         const bool ok = (unsigned)iy < (unsigned)H && (unsigned)ix < (unsigned)W;
-        sx[i] = ok ? __ldg(x + (((long long)b * H + iy) * W + (ox0 - pw)) * Ci + rx) : 0.0;
+        sx[i] = ok ? (double)__ldg(x + (((long long)b * H + iy) * W + (ox0 - pw)) * Ci + rx) : 0.0;
     }
     __syncthreads();
     const int ty = tid / DT, tx = tid % DT;
@@ -230,17 +230,20 @@ __global__ void __launch_bounds__(DT * DT) conv2d_direct_small_kernel(const doub
             }
     }
 }
+__global__ void __launch_bounds__(DT * DT) conv2d_direct_small_kernel(const double* __restrict__ x, int H, int W, int Ci,
+                                                                       const double* __restrict__ w, const double* __restrict__ bias,
+                                                                       int Co, int kh, int kw, int ph, int pw, int Ho, int Wo,
+                                                                       int act, double* __restrict__ y) {
+    conv2d_direct_small(x, H, W, Ci, w, bias, Co, kh, kw, ph, pw, Ho, Wo, act, y);
+}
+__global__ void __launch_bounds__(DT * DT) conv2d_direct_small_u8_kernel(const uint8_t* __restrict__ x, int H, int W, int Ci,
+                                                                          const double* __restrict__ w, const double* __restrict__ bias,
+                                                                          int Co, int kh, int kw, int ph, int pw, int Ho, int Wo,
+                                                                          int act, double* __restrict__ y) {
+    conv2d_direct_small(x, H, W, Ci, w, bias, Co, kh, kw, ph, pw, Ho, Wo, act, y);
+}
 
 // ---- host side --------------------------------------------------------------------------------------------------------
-namespace {
-
-struct ConvShape {
-    size_t B, H, W, Ci, Co, kh, kw;
-    int padding;
-    size_t Ho = 0, Wo = 0;
-    int ph, pw;
-};
-
 int check_conv_shape(size_t B, size_t H, size_t W, size_t Ci, size_t Co, size_t kh, size_t kw, int padding, ConvShape* s) {
     if (padding != RCN_PADDING_NONE && padding != RCN_PADDING_SAME) return fail(RCN_ERR_INVALID, "unknown padding %d", padding);
     if (Ci == 0 || Co == 0) return fail(RCN_ERR_INVALID, "zero channels");
@@ -258,6 +261,8 @@ int check_conv_shape(size_t B, size_t H, size_t W, size_t Ci, size_t Co, size_t 
         return fail(RCN_ERR_INVALID, "convolution problem too large for 32-bit pixel indices");
     return RCN_OK;
 }
+
+namespace {
 
 // tcgen05 integer-slice implicit GEMM when the contraction is really dense (wide-channel layers: BASELINE config 4):
 // >= half the SMs worth of 128-pixel x 96-channel tiles, K = kh*kw*C deep enough, enough work to amortise the gather.
@@ -293,8 +298,36 @@ bool use_direct(const ConvShape& s) {
 
 }  // namespace
 
+bool conv_direct_ok(const ConvShape& s) { return use_direct(s); }
+
+int launch_conv2d_forward_u8(const uint8_t* x, const double* w, const double* bias, const ConvShape& s, int act, double* y,
+                             cudaStream_t stream) {
+    if (s.B == 0) return RCN_OK;
+    if (!use_direct(s) || s.Ci != 1) return fail(RCN_ERR_STATE, "internal: u8 convolution outside the direct kernel");
+    if (s.B > 65535) return fail(RCN_ERR_INVALID, "batch too large for the direct convolution kernel");
+    const size_t smem = ((DT + s.kh - 1) * (DT + s.kw - 1) * s.Ci + s.Co * s.kh * s.kw * s.Ci) * sizeof(double);
+    static SmemAttrCache attr;
+    if (smem > 48 * 1024 && attr.need(smem))
+        RCN_CUDA_TRY(cudaFuncSetAttribute(conv2d_direct_small_u8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    dim3 grid(cdiv(s.Wo, DT), cdiv(s.Ho, DT), (unsigned)s.B);
+    RCN_LAUNCH("conv2d_direct_small_u8_kernel", stream,
+               conv2d_direct_small_u8_kernel<<<grid, DT * DT, smem, stream>>>(x, (int)s.H, (int)s.W, (int)s.Ci, w, bias, (int)s.Co,
+                                                                             (int)s.kh, (int)s.kw, s.ph, s.pw, (int)s.Ho, (int)s.Wo,
+                                                                             act, y));
+    return RCN_OK;
+}
+
+int launch_activation_backward(const double* y, const double* dy, size_t n, int act, double* dz, cudaStream_t stream) {
+    if (n == 0) return RCN_OK;
+    unsigned grid = cdiv(n, 256);
+    if (grid > kNumSMs * 8) grid = kNumSMs * 8;
+    RCN_LAUNCH("activation_backward_kernel", stream,
+               activation_backward_kernel<<<grid, 256, 0, stream>>>(y, dy, n, act, dz));
+    return RCN_OK;
+}
+
 int launch_conv2d_forward(const double* x, const double* w, const double* bias, const ConvShape& s, int act, double* y,
-                          cudaStream_t stream) {
+                          cudaStream_t stream, OzakiWorkspace* tw) {
     if (s.B == 0) return RCN_OK;
     if (use_direct(s)) {
         const size_t kk = s.kh * s.kw * s.Ci;
@@ -313,14 +346,15 @@ int launch_conv2d_forward(const double* x, const double* w, const double* bias, 
     const int M = (int)s.Co, N = (int)(s.B * s.Ho * s.Wo), K = (int)(s.kh * s.kw * s.Ci);
     const ConvGeom geom{x, (int)s.H, (int)s.W, (int)s.Ci, (int)s.Ho, (int)s.Wo, (int)s.kh, (int)s.kw, s.ph, s.pw, N, K};
     if (conv_use_tc((size_t)N, (size_t)M, (size_t)K)) {
+        OzakiWorkspace& ows = tw ? *tw : conv_tc_workspace();
         const EpiConvForwardT epi{bias, y, M, act};
         if (ozaki_conv_tma_ok(geom))   // im2col by TMA: the tensor is sliced once, taps are shifted boxes
             return launch_conv_ozaki("conv2d_forward_igemm(tcgen05 int8 slices, TMA im2col)", geom, (int)s.B, w, M, epi,
-                                     conv_tc_workspace(), stream);
+                                     ows, stream);
         OzOperand oa{x, 0, true};                 // im2col rows gathered straight into int8 digit planes
         oa.gather = 1; oa.g = geom;
         const OzOperand ob{w, (size_t)K, true};   // w[co][k]
-        return launch_gemm_ozaki("conv2d_forward_igemm(tcgen05 int8 slices)", oa, ob, N, M, K, epi, conv_tc_workspace(), stream);
+        return launch_gemm_ozaki("conv2d_forward_igemm(tcgen05 int8 slices)", oa, ob, N, M, K, epi, ows, stream);
     }
     const DenseLoader<true> la{w, K, M};
     const Im2colPixelRows lb{geom};
@@ -331,7 +365,7 @@ int launch_conv2d_forward(const double* x, const double* w, const double* bias, 
 }
 
 int launch_conv2d_backward_data(const double* dz, const double* w, const ConvShape& s, const double* y_prev, int act_prev,
-                                double* dx, DevBuf& ws, cudaStream_t stream) {
+                                double* dx, DevBuf& ws, cudaStream_t stream, OzakiWorkspace* tw) {
     if (s.B == 0) return RCN_OK;
     const size_t nw = s.Co * s.kh * s.kw * s.Ci;
     RCN_TRY(ws.reserve(nw * sizeof(double)));
@@ -344,14 +378,15 @@ int launch_conv2d_backward_data(const double* dz, const double* w, const ConvSha
     const ConvGeom geom{dz, (int)s.Ho, (int)s.Wo, (int)s.Co, (int)s.H, (int)s.W, (int)s.kh, (int)s.kw,
                         (int)s.kh - 1 - s.ph, (int)s.kw - 1 - s.pw, N, K};
     if (conv_use_tc((size_t)N, (size_t)M, (size_t)K)) {
+        OzakiWorkspace& ows = tw ? *tw : conv_tc_workspace();
         const EpiConvBackDataT epi{y_prev, dx, M, act_prev};
         if (ozaki_conv_tma_ok(geom))
             return launch_conv_ozaki("conv2d_backward_data_igemm(tcgen05 int8 slices, TMA im2col)", geom, (int)s.B, ws.as<double>(), M,
-                                     epi, conv_tc_workspace(), stream);
+                                     epi, ows, stream);
         OzOperand oa{dz, 0, true};
         oa.gather = 1; oa.g = geom;
         const OzOperand ob{ws.as<double>(), (size_t)K, true};   // w'[ci][k]
-        return launch_gemm_ozaki("conv2d_backward_data_igemm(tcgen05 int8 slices)", oa, ob, N, M, K, epi, conv_tc_workspace(), stream);
+        return launch_gemm_ozaki("conv2d_backward_data_igemm(tcgen05 int8 slices)", oa, ob, N, M, K, epi, ows, stream);
     }
     const DenseLoader<true> la{ws.as<double>(), K, M};
     const Im2colPixelRows lb{geom};
@@ -362,7 +397,7 @@ int launch_conv2d_backward_data(const double* dz, const double* w, const ConvSha
 }
 
 int launch_conv2d_backward_weight(const double* x, const double* dz, const ConvShape& s, double* dw, double* db, DevBuf& ws,
-                                  cudaStream_t stream) {
+                                  cudaStream_t stream, OzakiWorkspace* tw_in, ReduceScratch* rs) {
     const int M = (int)s.Co, N = (int)(s.kh * s.kw * s.Ci), Kc = (int)(s.B * s.Ho * s.Wo);
     if (Kc == 0) {
         RCN_CUDA_TRY(cudaMemsetAsync(dw, 0, (size_t)M * N * sizeof(double), stream));
@@ -373,7 +408,7 @@ int launch_conv2d_backward_weight(const double* x, const double* dz, const ConvS
         // contraction over the grid pixels: dz columns (co) x im2col columns (ky, kx, ci), both gathered straight into
         // digit planes with per-row scales over ALL pixels; split-K keeps each CTA's contraction inside the exact int32
         // range and fills the machine; partials are combined in split order (deterministic)
-        OzakiWorkspace& tw = conv_tc_workspace();
+        OzakiWorkspace& tw = tw_in ? *tw_in : conv_tc_workspace();
         const int splits = ozaki_plan_splits(M, N, Kc);
         OzOperand oa{dz, (size_t)M, false};                      // element (co, pix) at dz[pix*Co + co]
         OzOperand ob{x, 0, false};
@@ -388,7 +423,8 @@ int launch_conv2d_backward_weight(const double* x, const double* dz, const ConvS
             RCN_TRY(launch_gemm_ozaki("conv2d_backward_weight_igemm(tcgen05 int8 slices)", oa, ob, M, N, Kc, epi, tw, stream, splits));
             RCN_TRY(launch_reduce_splits(tw.partials.as<double>(), splits, (size_t)M * N, dw, stream));
         }
-        if (db) {
+        if (db && rs) RCN_TRY(launch_bias_grad(dz, (size_t)M, (size_t)Kc, db, *rs, stream));
+        else if (db) {
             static thread_local ReduceScratch tl_rs2[64];
             int dev = 0;
             RCN_CUDA_TRY(cudaGetDevice(&dev));
@@ -423,7 +459,8 @@ int launch_conv2d_backward_weight(const double* x, const double* dz, const ConvS
         RCN_TRY(launch_gemm_tiles("conv2d_backward_weight_igemm", la, lb, M, N, Kc, splits, kps, epi, stream));
         RCN_TRY(launch_reduce_splits(ws.as<double>(), splits, (size_t)M * N, dw, stream));
     }
-    if (db) {
+    if (db && rs) RCN_TRY(launch_bias_grad(dz, (size_t)M, (size_t)Kc, db, *rs, stream));
+    else if (db) {
         static thread_local ReduceScratch tl_rs[64];   // one per device this thread drives
         int dev = 0;
         RCN_CUDA_TRY(cudaGetDevice(&dev));
@@ -468,10 +505,7 @@ int rcn_cuda_ext_activation_backward(int device, void* cuda_stream, const double
     RCN_TRY(c.in(y, n * 8, tl_op_in, &y_dev));
     RCN_TRY(c.in(dy, n * 8, tl_op_in2, &dy_dev));
     RCN_TRY(c.out(dz, n * 8, tl_op_out, &o_dev, &host));
-    unsigned grid = cdiv(n, 256);
-    if (grid > kNumSMs * 8) grid = kNumSMs * 8;
-    RCN_LAUNCH("activation_backward_kernel", c.stream,
-               activation_backward_kernel<<<grid, 256, 0, c.stream>>>((const double*)y_dev, (const double*)dy_dev, n, activation, (double*)o_dev));
+    RCN_TRY(launch_activation_backward((const double*)y_dev, (const double*)dy_dev, n, activation, (double*)o_dev, c.stream));
     return c.finish(dz, o_dev, n * 8, host);
 }
 

@@ -71,6 +71,10 @@ struct EpiBackData {
         delta_out[o] = v * (s * (1.0 - s));                  // (W^T delta) .* sigmoid_prime(z)  (rcn.rs:306-308)
     }
 };
+struct EpiInputGrad {  // dX = W^T delta with no activation derivative: the input gradient of the dense stack
+    double* dx; int M;
+    __device__ __forceinline__ void operator()(int m, int n, double v) const { dx[(size_t)n * M + m] = v; }
+};
 struct EpiStore {  // split-K partial (or final) store, column-major M x N
     double* out; int M; size_t split_stride;
     __device__ __forceinline__ void operator()(int m, int n, double v) const {
@@ -345,6 +349,14 @@ int launch_dense_backward_data(const double* W_up, const double* delta_up, const
     const bool tc = use_tensor_cores(M, N, K, oz);
     return launch_gemm<true, true, EpiBackData>(tc ? "dense_backward_data_gemm(tcgen05 int8 slices)" : "dense_backward_data_gemm", W_up,
                                                 (int)K, delta_up, (int)K, M, N, K, 1, epi, stream, oz);
+}
+
+int launch_dense_input_grad(const double* W0, const double* delta0, size_t M, size_t K, size_t N, double* dx, cudaStream_t stream,
+                            OzakiWorkspace* oz) {
+    EpiInputGrad epi{dx, (int)M};
+    const bool tc = use_tensor_cores(M, N, K, oz);   // the engine choice of launch_dense_backward_data
+    return launch_gemm<true, true, EpiInputGrad>(tc ? "dense_input_grad_gemm(tcgen05 int8 slices)" : "dense_input_grad_gemm", W0,
+                                                 (int)K, delta0, (int)K, M, N, K, 1, epi, stream, oz);
 }
 
 __global__ void reduce_splits_kernel(const double* __restrict__ part, int splits, size_t n, double* __restrict__ out) {

@@ -24,6 +24,11 @@ int launch_dense_forward(const double* W, const double* b, const double* A_in, s
 int launch_dense_backward_data(const double* W_up, const double* delta_up, const double* A, size_t M, size_t K,
                                size_t N, double* delta_out, cudaStream_t stream, OzakiWorkspace* oz = nullptr);
 
+// dx (M x N) = W0^T (M x K) * delta0 (K x N): the gradient of the cost with respect to the dense stack's input (no
+// activation derivative); W0 is stored K x M.  Same DMMA / tcgen05 choice as launch_dense_backward_data.
+int launch_dense_input_grad(const double* W0, const double* delta0, size_t M, size_t K, size_t N, double* dx, cudaStream_t stream,
+                            OzakiWorkspace* oz = nullptr);
+
 // dW (M x N) = delta (M x Kb) * A_prev (N x Kb)^T, db (M) = delta * 1                 rcn.rs:302-303,309-310 summed
 // over the batch (rcn.rs:190-205).  workspace: split-K partials.
 int launch_dense_backward_weight(const double* delta, const double* A_prev, size_t M, size_t N, size_t Kb, double* dW,

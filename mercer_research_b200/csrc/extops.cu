@@ -9,6 +9,7 @@
 // argmax byte is 2*dy+dx.  Average divides by 4 always.  All are HBM-bound element-wise kernels: one thread per
 // output element with the channel index fastest, so every warp access is a contiguous run.  Checked against
 // oracle/ext_oracle.cpp ("parity unpinned").
+#include "conv.cuh"
 #include "opctx.cuh"
 
 namespace rcn {
@@ -101,8 +102,7 @@ __global__ void __launch_bounds__(256) ext_softmax_xent_kernel(const double* __r
     }
 }
 
-namespace {
-int pool_shape(size_t H, size_t W, int padding, int pooling, size_t* Ho, size_t* Wo) {
+int pool2d_shape(size_t H, size_t W, int padding, int pooling, size_t* Ho, size_t* Wo) {
     if (padding != RCN_PADDING_NONE && padding != RCN_PADDING_SAME) return fail(RCN_ERR_INVALID, "unknown padding %d", padding);
     if (pooling != RCN_POOLING_AVERAGE && pooling != RCN_POOLING_MAX) return fail(RCN_ERR_INVALID, "unknown pooling %d", pooling);
     if (H < 2 || W < 2)  // kernel.rs:246-251
@@ -113,11 +113,32 @@ int pool_shape(size_t H, size_t W, int padding, int pooling, size_t* Ho, size_t*
     *Wo = same ? (W + 1) / 2 : W / 2;
     return RCN_OK;
 }
+namespace {
 unsigned ew_grid(size_t n) {
     unsigned g = cdiv(n, 256);
     return g > kNumSMs * 16 ? kNumSMs * 16 : (g ? g : 1);
 }
 }  // namespace
+
+int launch_pool2d_forward(const double* x, size_t B, size_t H, size_t W, size_t C, size_t Ho, size_t Wo, int pooling, double* y,
+                          uint8_t* argmax, int* nan_flag, cudaStream_t stream) {
+    const size_t n_out = B * Ho * Wo * C;
+    if (n_out == 0) return RCN_OK;
+    RCN_LAUNCH("ext_pool_forward_kernel", stream,
+               ext_pool_forward_kernel<<<ew_grid(n_out), 256, 0, stream>>>(x, (int)H, (int)W, (int)C, (int)Ho, (int)Wo, n_out, pooling,
+                                                                           y, argmax, nan_flag));
+    return RCN_OK;
+}
+
+int launch_pool2d_backward(const double* dy, const uint8_t* argmax, size_t B, size_t H, size_t W, size_t C, size_t Ho, size_t Wo,
+                           int pooling, double* dx, cudaStream_t stream) {
+    const size_t n_in = B * H * W * C;
+    if (n_in == 0) return RCN_OK;
+    RCN_LAUNCH("ext_pool_backward_kernel", stream,
+               ext_pool_backward_kernel<<<ew_grid(n_in), 256, 0, stream>>>(dy, argmax, (int)H, (int)W, (int)C, (int)Ho, (int)Wo, n_in,
+                                                                           pooling, dx));
+    return RCN_OK;
+}
 
 }  // namespace rcn
 
@@ -129,7 +150,7 @@ int rcn_cuda_ext_pool2d_forward(int device, void* cuda_stream, const double* x, 
                                 int padding, int pooling, double* y, uint8_t* argmax_out) {
     if (!x || !y) return fail(RCN_ERR_INVALID, "null pointer");
     size_t Ho = 0, Wo = 0;
-    RCN_TRY(pool_shape(H, W, padding, pooling, &Ho, &Wo));
+    RCN_TRY(pool2d_shape(H, W, padding, pooling, &Ho, &Wo));
     const size_t n_out = B * Ho * Wo * C;
     if (n_out == 0) return RCN_OK;
     OpCtx c;
@@ -146,9 +167,7 @@ int rcn_cuda_ext_pool2d_forward(int device, void* cuda_stream, const double* x, 
         if (is_device_ptr(argmax_out)) am_dev = argmax_out;
         else { am_dev = tl_op_aux.as<uint8_t>() + 16; am_host = true; }
     }
-    RCN_LAUNCH("ext_pool_forward_kernel", c.stream,
-               ext_pool_forward_kernel<<<ew_grid(n_out), 256, 0, c.stream>>>((const double*)x_dev, (int)H, (int)W, (int)C, (int)Ho,
-                                                                             (int)Wo, n_out, pooling, (double*)y_dev, am_dev, flag));
+    RCN_TRY(launch_pool2d_forward((const double*)x_dev, B, H, W, C, Ho, Wo, pooling, (double*)y_dev, am_dev, flag, c.stream));
     int nan = 0;
     RCN_CUDA_TRY(cudaMemcpyAsync(&nan, flag, sizeof(int), cudaMemcpyDeviceToHost, c.stream));
     if (am_host) RCN_CUDA_TRY(cudaMemcpyAsync(argmax_out, am_dev, n_out, cudaMemcpyDeviceToHost, c.stream));
@@ -162,7 +181,7 @@ int rcn_cuda_ext_pool2d_backward(int device, void* cuda_stream, const double* dy
                                  size_t W, size_t C, int padding, int pooling, double* dx) {
     if (!dy || !dx) return fail(RCN_ERR_INVALID, "null pointer");
     size_t Ho = 0, Wo = 0;
-    RCN_TRY(pool_shape(H, W, padding, pooling, &Ho, &Wo));
+    RCN_TRY(pool2d_shape(H, W, padding, pooling, &Ho, &Wo));
     if (pooling == RCN_POOLING_MAX && !argmax) return fail(RCN_ERR_INVALID, "max-pool backward needs the forward pass's argmax");
     const size_t n_in = B * H * W * C, n_out = B * Ho * Wo * C;
     if (n_in == 0) return RCN_OK;
@@ -172,10 +191,8 @@ int rcn_cuda_ext_pool2d_backward(int device, void* cuda_stream, const double* dy
     RCN_TRY(c.in(dy, n_out * 8, tl_op_in, &dy_dev));
     if (pooling == RCN_POOLING_MAX) RCN_TRY(c.in(argmax, n_out, tl_op_in2, &am_dev));
     RCN_TRY(c.out(dx, n_in * 8, tl_op_out, &dx_dev, &host));
-    RCN_LAUNCH("ext_pool_backward_kernel", c.stream,
-               ext_pool_backward_kernel<<<ew_grid(n_in), 256, 0, c.stream>>>((const double*)dy_dev, (const uint8_t*)am_dev, (int)H,
-                                                                             (int)W, (int)C, (int)Ho, (int)Wo, n_in, pooling,
-                                                                             (double*)dx_dev));
+    RCN_TRY(launch_pool2d_backward((const double*)dy_dev, (const uint8_t*)am_dev, B, H, W, C, Ho, Wo, pooling, (double*)dx_dev,
+                                   c.stream));
     return c.finish(dx, dx_dev, n_in * 8, host);
 }
 

@@ -11,6 +11,7 @@
 #include <tuple>
 #include <vector>
 
+#include "cnn.cuh"
 #include "dense.cuh"
 #include "features.cuh"
 #include "smallnet.cuh"
@@ -1639,3 +1640,28 @@ int rcn_cuda_pool_2d(int device, void* cuda_stream, const double* m, size_t H, s
 }
 
 }  // extern "C"
+
+// ---- the dense stack of the convolutional network handle (cnn.cuh) ------------------------------------------------
+namespace rcn {
+
+int model_evaluate_features(rcn_cuda_model* h, const double* feats, const int64_t* labels, size_t B, double* stats,
+                            int64_t* labels_out) {
+    RCN_TRY(require_params(h));
+    if (B == 0) return RCN_OK;
+    RCN_TRY(forward_dev(h, feats, B, nullptr, nullptr, false));
+    const size_t n = h->rows.size();
+    if (labels) RCN_TRY(launch_batch_stats(h->act(n - 1, B), h->rows[n - 1], B, nullptr, labels, stats, h->rs, h->stream));
+    if (labels_out) RCN_TRY(launch_argmax_last(h->act(n - 1, B), h->rows[n - 1], B, labels_out, h->stream));
+    return RCN_OK;
+}
+
+int model_first_layer(rcn_cuda_model* h, const double** W0, const double** delta0, size_t* rows0, size_t* cols0) {
+    RCN_TRY(require_params(h));
+    *W0 = h->params.as<double>() + h->w_off[0];
+    *delta0 = h->deltas.as<double>();
+    *rows0 = h->rows[0];
+    *cols0 = h->cols[0];
+    return RCN_OK;
+}
+
+}  // namespace rcn

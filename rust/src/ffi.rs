@@ -7,6 +7,11 @@ pub struct rcn_cuda_model {
     _private: [u8; 0],
 }
 pub type rcn_cuda_handle = *mut rcn_cuda_model;
+#[repr(C)]
+pub struct rcn_cuda_cnn {
+    _private: [u8; 0],
+}
+pub type rcn_cuda_cnn_handle = *mut rcn_cuda_cnn;
 
 pub const RCN_OK: c_int = 0;
 pub const RCN_ERR_INVALID: c_int = 1;
@@ -18,6 +23,10 @@ pub const RCN_ERR_OUT_OF_BOUNDS: c_int = 6;
 pub const RCN_ERR_NAN: c_int = 7;
 pub const RCN_PIXELS_U8_ROWMAJOR: c_int = 0;
 pub const RCN_PIXELS_F64_COLMAJOR: c_int = 1;
+pub const RCN_PIXELS_F64_NHWC: c_int = 2;
+pub const RCN_CNN_CONV: i32 = 0;
+pub const RCN_CNN_POOL: i32 = 1;
+pub const RCN_CNN_LAYER_INTS: usize = 5;
 
 extern "C" {
     pub fn rcn_cuda_last_error() -> *const c_char;
@@ -131,4 +140,30 @@ extern "C" {
     pub fn rcn_cuda_relu(device: c_int, stream: *mut c_void, m: *const c_double, n: usize, out: *mut c_double) -> c_int;
     pub fn rcn_cuda_pool_2d(device: c_int, stream: *mut c_void, m: *const c_double, H: usize, W: usize, padding: c_int,
                             pooling: c_int, out: *mut c_double, argmax_out: *mut u8) -> c_int;
+    // ---- convolutional network handle (learned conv / pool layers + the dense stack) -------------------------------
+    pub fn rcn_cuda_cnn_create(device: c_int, H: usize, W: usize, in_channels: usize, layer_spec: *const i32, n_layers: usize,
+                               feedforward: *const usize, n_ff: usize, classes: usize, out: *mut rcn_cuda_cnn_handle) -> c_int;
+    pub fn rcn_cuda_cnn_destroy(h: rcn_cuda_cnn_handle) -> c_int;
+    pub fn rcn_cuda_cnn_set_stream(h: rcn_cuda_cnn_handle, stream: *mut c_void) -> c_int;
+    pub fn rcn_cuda_cnn_synchronize(h: rcn_cuda_cnn_handle) -> c_int;
+    pub fn rcn_cuda_cnn_layer_shape(h: rcn_cuda_cnn_handle, layer: usize, H: *mut usize, W: *mut usize, C: *mut usize) -> c_int;
+    pub fn rcn_cuda_cnn_param_count(h: rcn_cuda_cnn_handle, n: *mut usize) -> c_int;
+    pub fn rcn_cuda_cnn_set_params(h: rcn_cuda_cnn_handle, flat: *const c_double, n: usize) -> c_int;
+    pub fn rcn_cuda_cnn_get_params(h: rcn_cuda_cnn_handle, flat: *mut c_double, n: usize) -> c_int;
+    pub fn rcn_cuda_cnn_accumulate(h: rcn_cuda_cnn_handle, images: *const c_void, pixel_format: c_int, labels: *const i64,
+                                   B: usize, H: usize, W: usize) -> c_int;
+    pub fn rcn_cuda_cnn_apply(h: rcn_cuda_cnn_handle, eta: c_double, global_batch: usize) -> c_int;
+    pub fn rcn_cuda_cnn_train_batch(h: rcn_cuda_cnn_handle, images: *const c_void, pixel_format: c_int, labels: *const i64,
+                                    B: usize, H: usize, W: usize, eta: c_double) -> c_int;
+    pub fn rcn_cuda_cnn_last_batch_stats(h: rcn_cuda_cnn_handle, cost: *mut c_double, hits: *mut u64) -> c_int;
+    pub fn rcn_cuda_cnn_evaluate_images(h: rcn_cuda_cnn_handle, images: *const c_void, pixel_format: c_int, labels: *const i64,
+                                        B: usize, H: usize, W: usize, cost_out: *mut c_double, accept_out: *mut u64,
+                                        labels_out: *mut i64) -> c_int;
+    pub fn rcn_cuda_cnn_classify_images(h: rcn_cuda_cnn_handle, images: *const c_void, pixel_format: c_int, B: usize, H: usize,
+                                        W: usize, labels_out: *mut i64) -> c_int;
+    pub fn rcn_cuda_cnn_bind_gradient_buffer(h: rcn_cuda_cnn_handle, device_ptr: *mut c_double, n: usize) -> c_int;
+    pub fn rcn_cuda_cnn_gradient_buffer(h: rcn_cuda_cnn_handle, device_ptr: *mut *mut c_double, n: *mut usize) -> c_int;
+    pub fn rcn_cuda_cnn_get_gradients(h: rcn_cuda_cnn_handle, flat: *mut c_double, n: usize) -> c_int;
+    pub fn rcn_cuda_cnn_get_layer_output(h: rcn_cuda_cnn_handle, layer: usize, out: *mut c_double) -> c_int;
+    pub fn rcn_cuda_cnn_get_input_gradient(h: rcn_cuda_cnn_handle, out: *mut c_double) -> c_int;
 }
