@@ -465,6 +465,21 @@ class ConvNet {
         check(rcn_cuda_cnn_classify_images(h_, images, pixel_format, B, H, W, out.data()));
         return out;
     }
+    /// Epoch mode over a dataset in DEVICE memory (rcn_cuda_cnn_epoch_* in rcn_cuda.h); perm may be null (identity).
+    void epoch_bind(const void* images, int pixel_format, const int64_t* labels, const int64_t* perm, size_t n_samples,
+                    size_t H, size_t W, size_t B) {
+        check(rcn_cuda_cnn_epoch_bind(h_, images, pixel_format, labels, perm, n_samples, H, W, B));
+    }
+    void epoch_seek(size_t position) { check(rcn_cuda_cnn_epoch_seek(h_, position)); }
+    size_t epoch_position() const {
+        size_t p = 0;
+        check(rcn_cuda_cnn_epoch_position(h_, &p));
+        return p;
+    }
+    void epoch_accumulate() { check(rcn_cuda_cnn_epoch_accumulate(h_)); }
+    void epoch_apply(double eta, size_t global_batch) { check(rcn_cuda_cnn_epoch_apply(h_, eta, global_batch)); }
+    void epoch_step(double eta) { check(rcn_cuda_cnn_epoch_step(h_, eta)); }
+    void epoch_run(double eta, size_t n_steps) { check(rcn_cuda_cnn_epoch_run(h_, eta, n_steps)); }
     rcn_cuda_cnn_handle handle() const { return h_; }
 
   private:

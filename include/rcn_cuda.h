@@ -323,7 +323,9 @@ int rcn_cuda_ext_gemm_f64(int device, void* cuda_stream, const double* A, size_t
  * is fixed at creation (it fixes L and so the parameter count): other H, W fail with RCN_ERR_SHAPE.
  * Pointers may be host or device memory as elsewhere; with device images, labels and outputs nothing synchronises, and
  * once a call with at least as many images has sized the buffers (rcn_cuda_allocation_generation), accumulate + apply can
- * be captured into a CUDA graph.  A NaN reaching a max pool is not reported (the cost turns NaN instead). */
+ * be captured into a CUDA graph.  A NaN reaching a max pool is not reported (the cost turns NaN instead).
+ * Epoch mode (rcn_cuda_cnn_epoch_*, below) trains over a dataset resident in device memory with a device-side cursor, like
+ * rcn_cuda_epoch_*; each step gathers its images and labels with one staging kernel. */
 enum { RCN_CNN_CONV = 0, RCN_CNN_POOL = 1 };
 #define RCN_CNN_LAYER_INTS 5
 /* Validates the whole spec before any device work (status codes and messages of the ext ops; a zero-width dense layer or
@@ -351,6 +353,30 @@ int rcn_cuda_cnn_train_batch(rcn_cuda_cnn_handle h, const void* images, int pixe
                              size_t H, size_t W, double eta);
 /* Quadratic cost and rcn.rs:153-157 hit count of the last accumulate, under the pre-update parameters. */
 int rcn_cuda_cnn_last_batch_stats(rcn_cuda_cnn_handle h, double* cost, uint64_t* hits);
+/* Epoch mode: `for batch in training_set.chunks_exact(B) { train_batch(batch, eta) }` (rcn.rs:144-149) over a dataset in
+ * DEVICE memory, with meaning, contract and status codes of rcn_cuda_epoch_*: step k trains on samples perm[pos .. pos+B)
+ * (perm == NULL: identity); pos advances by B with each apply and wraps to 0 once fewer than B samples remain.
+ *   bind        images (n_samples images in `pixel_format`, H x W as the network was created for: RCN_ERR_SHAPE otherwise),
+ *               labels (n_samples) and perm (n_samples, may be NULL) must be device pointers (RCN_ERR_INVALID otherwise)
+ *               and stay valid while bound; n_samples >= B > 0 (RCN_ERR_INVALID).  Every entry of perm must lie in
+ *               [0, n_samples): the caller's contract, not checked.  Reserves the step's buffers for B, sets the cursor
+ *               to 0 and drains the stream.  perm may be rewritten in place between steps (re-shuffle per epoch).
+ *   accumulate  one kernel gathers chunk perm[pos .. pos+B) and its labels (u8 images: with the f64 copy the first layer's
+ *               weight gradient reads), then rcn_cuda_cnn_accumulate's work on it; the cursor does not move, so two
+ *               accumulates without an apply see the same chunk.
+ *   apply       rcn_cuda_cnn_apply, and the cursor advances.
+ * Every step entry point before a bind fails with RCN_ERR_STATE.  After bind and one accumulate outside a capture a step
+ * neither allocates nor synchronises, so one captured step replays for every step of every epoch; re-capture when
+ * rcn_cuda_allocation_generation changed.  The layer buffers are shared with evaluate / classify: those calls on more than
+ * B images grow them (and move them), which a captured step notices only through that generation. */
+int rcn_cuda_cnn_epoch_bind(rcn_cuda_cnn_handle h, const void* images, int pixel_format, const int64_t* labels,
+                            const int64_t* perm, size_t n_samples, size_t H, size_t W, size_t B);
+int rcn_cuda_cnn_epoch_seek(rcn_cuda_cnn_handle h, size_t position);
+int rcn_cuda_cnn_epoch_position(rcn_cuda_cnn_handle h, size_t* position); /* synchronises the stream */
+int rcn_cuda_cnn_epoch_accumulate(rcn_cuda_cnn_handle h);
+int rcn_cuda_cnn_epoch_apply(rcn_cuda_cnn_handle h, double eta, size_t global_batch);
+int rcn_cuda_cnn_epoch_step(rcn_cuda_cnn_handle h, double eta); /* accumulate + apply with global_batch = B */
+int rcn_cuda_cnn_epoch_run(rcn_cuda_cnn_handle h, double eta, size_t n_steps); /* n_steps epoch steps in one call */
 /* Forward pass only: cost_out, accept_out as rcn_cuda_evaluate_images; labels_out (optional) the rcn.rs:92-97 argmax.
  * Leaves the gradients and the last-batch statistics untouched (the layer-output tap then shows this batch). */
 int rcn_cuda_cnn_evaluate_images(rcn_cuda_cnn_handle h, const void* images, int pixel_format, const int64_t* labels, size_t B,

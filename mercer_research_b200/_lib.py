@@ -109,6 +109,13 @@ SIGNATURES = {
     "rcn_cuda_cnn_apply": [_vp, _d, _sz],
     "rcn_cuda_cnn_train_batch": [_vp, _vp, _i, _vp, _sz, _sz, _sz, _d],
     "rcn_cuda_cnn_last_batch_stats": [_vp, C.POINTER(_d), C.POINTER(C.c_uint64)],
+    "rcn_cuda_cnn_epoch_bind": [_vp, _vp, _i, _vp, _vp, _sz, _sz, _sz, _sz],
+    "rcn_cuda_cnn_epoch_seek": [_vp, _sz],
+    "rcn_cuda_cnn_epoch_position": [_vp, _szp],
+    "rcn_cuda_cnn_epoch_accumulate": [_vp],
+    "rcn_cuda_cnn_epoch_apply": [_vp, _d, _sz],
+    "rcn_cuda_cnn_epoch_step": [_vp, _d],
+    "rcn_cuda_cnn_epoch_run": [_vp, _d, _sz],
     "rcn_cuda_cnn_evaluate_images": [_vp, _vp, _i, _vp, _sz, _sz, _sz, _vp, _vp, _vp],
     "rcn_cuda_cnn_classify_images": [_vp, _vp, _i, _sz, _sz, _sz, _vp],
     "rcn_cuda_cnn_bind_gradient_buffer": [_vp, _vp, _sz],

@@ -68,6 +68,7 @@ class ConvNet:
             _lib.check(self._lib.rcn_cuda_cnn_layer_shape(self._h, i, C.byref(a), C.byref(b), C.byref(c)))
             self._shapes.append((a.value, b.value, c.value))
         self._B_out = self._B_grad = 0
+        self._params_set = False
 
     # -- lifetime -----------------------------------------------------------------------------------------------------
     def close(self):
@@ -150,6 +151,7 @@ class ConvNet:
     def set_params(self, flat):
         flat = np.ascontiguousarray(flat, dtype=np.float64).ravel()
         _lib.check(self._lib.rcn_cuda_cnn_set_params(self._h, flat.ctypes.data, flat.size))
+        self._params_set = True
 
     def get_params(self) -> np.ndarray:
         buf = np.zeros(self.n_params)
@@ -206,6 +208,122 @@ class ConvNet:
         self._use_torch_stream(buf, lb)
         _lib.check(self._lib.rcn_cuda_cnn_train_batch(self._h, buf.ptr, fmt, lb.ptr, B, H, W, float(eta)))
         self._B_out = self._B_grad = B
+
+    # -- epoch mode (rcn.rs:144-149 on a dataset resident in HBM) -------------------------------------------------------
+    def epoch_bind(self, images, labels, batch: int, perm=None):
+        """Bind a device-resident dataset (torch CUDA tensors): images (N, H, W) uint8 or (N, H, W, C) float64, labels (N,)
+        int64, optional ``perm`` (N,) int64 shuffle with entries in [0, N) that may be rewritten in place between epochs.
+        Step k then trains on samples ``perm[pos:pos+batch]`` with ``pos`` kept on the device (chunks_exact semantics,
+        remainder dropped)."""
+        buf, fmt, (N, H, W) = self._images(images)
+        lb = _Buf(labels, np.int64)
+        pm = _Buf(perm, np.int64) if perm is not None else None
+        if not (buf.torch and lb.torch and (pm is None or pm.torch)):
+            raise ValueError("epoch mode needs torch CUDA tensors (the dataset stays resident in HBM)")
+        self._use_torch_stream(buf)
+        self._epoch_keepalive = (buf, lb, pm)
+        _lib.check(self._lib.rcn_cuda_cnn_epoch_bind(self._h, buf.ptr, fmt, lb.ptr, pm.ptr if pm else None, N, H, W,
+                                                     int(batch)))
+        self._epoch_B = int(batch)
+
+    def epoch_seek(self, position: int):
+        _lib.check(self._lib.rcn_cuda_cnn_epoch_seek(self._h, int(position)))
+
+    def epoch_position(self) -> int:
+        p = C.c_size_t()
+        _lib.check(self._lib.rcn_cuda_cnn_epoch_position(self._h, C.byref(p)))
+        return p.value
+
+    def _epoch_ran(self):
+        self._B_out = self._B_grad = getattr(self, "_epoch_B", 0)
+
+    def epoch_accumulate(self):
+        """Gradient sums of the current chunk; the cursor stays."""
+        _lib.check(self._lib.rcn_cuda_cnn_epoch_accumulate(self._h))
+        self._epoch_ran()
+
+    def epoch_apply(self, eta: float, global_batch: int):
+        """Update with the global batch, then advance the cursor."""
+        _lib.check(self._lib.rcn_cuda_cnn_epoch_apply(self._h, float(eta), int(global_batch)))
+
+    def epoch_step(self, eta: float):
+        _lib.check(self._lib.rcn_cuda_cnn_epoch_step(self._h, float(eta)))
+        self._epoch_ran()
+
+    def epoch_run(self, eta: float, n_steps: int):
+        """``n_steps`` iterations of ``for batch in training_set.chunks_exact(batch) { train_batch(batch, eta) }``
+        (rcn.rs:147-149) over the bound dataset, one library call."""
+        _lib.check(self._lib.rcn_cuda_cnn_epoch_run(self._h, float(eta), int(n_steps)))
+        if n_steps:
+            self._epoch_ran()
+
+    def train_arrays(self, train_images, train_labels, test_images, test_labels, batch_size: int, epochs: int,
+                     eta: float, seed: int = 0, log=print, cuda_graph: bool = True):
+        """``RCN::train`` (rcn.rs:126-167) for this network on in-memory images, both sets RESIDENT IN HBM: per epoch a
+        ``default_rng(seed)`` permutation written in place on the device, ``n // batch_size`` chunks_exact steps selected by
+        the device-side cursor (replays of one captured step with ``cuda_graph``, re-captured when a library buffer moved),
+        then the test set evaluated in chunks of at most ``batch_size`` (accept counts summed, costs added in chunk order)
+        and the reference's log line (rcn.rs:158-164).  Parameters that were never set are drawn with ``init_params`` from
+        the same generator before the first permutation.  Returns the per-epoch accept counts."""
+        import torch
+        dev = torch.device("cuda", self.device)
+        rng = np.random.default_rng(seed)
+        tr = torch.as_tensor(np.ascontiguousarray(train_images)).to(dev)
+        te = torch.as_tensor(np.ascontiguousarray(test_images)).to(dev)
+        if tr.dtype != torch.uint8:
+            tr, te = tr.to(torch.float64), te.to(torch.float64)
+        tr_y = torch.as_tensor(np.asarray(train_labels, dtype=np.int64)).to(dev)
+        te_y = torch.as_tensor(np.asarray(test_labels, dtype=np.int64)).to(dev)
+        n, n_test, bs = int(tr.shape[0]), int(te.shape[0]), int(batch_size)
+        stream = torch.cuda.current_stream(dev)
+        self.set_stream(stream.cuda_stream)
+        if not self._params_set:
+            self.init_params(rng)
+        history = []
+        n_steps = n // bs
+        perm = torch.arange(n, dtype=torch.int64, device=dev)
+        graph = None
+        if n_steps:
+            self.epoch_bind(tr, tr_y, bs, perm)
+            if cuda_graph:
+                side = torch.cuda.Stream(dev)
+                side.wait_stream(stream)
+                with torch.cuda.stream(side):
+                    self.set_stream(side.cuda_stream)
+                    self.epoch_accumulate()                   # warm-up launch outside capture (allocations, attributes)
+                stream.wait_stream(side)
+
+                def capture_step():
+                    torch.cuda.synchronize(dev)
+                    g = torch.cuda.CUDAGraph()
+                    with torch.cuda.graph(g):
+                        self.set_stream(torch.cuda.current_stream(dev).cuda_stream)
+                        self.epoch_step(eta)
+                    self.set_stream(stream.cuda_stream)
+                    return g, _lib.allocation_generation()
+
+                graph, graph_gen = capture_step()
+        for e in range(epochs):
+            if n_steps:
+                perm.copy_(torch.as_tensor(rng.permutation(n)), non_blocking=False)   # training_set.shuffle (rcn.rs:146)
+                self.epoch_seek(0)
+                if graph is not None and _lib.allocation_generation() != graph_gen:
+                    graph, graph_gen = capture_step()         # a library buffer moved since the capture
+                for _ in range(n_steps):                      # chunks_exact(batch_size) (rcn.rs:147-149)
+                    if graph is not None:
+                        graph.replay()
+                    else:
+                        self.epoch_step(eta)
+                self._epoch_ran()
+            accept = 0
+            for i in range(0, n_test, max(1, bs)):            # never more images than a training step: no buffer grows
+                a, _ = self.evaluate_images(te[i:i + bs], te_y[i:i + bs])
+                accept += a
+            history.append(accept)
+            if log:
+                log("Epoch {}: {}/{} [{:.2f}%]".format(e, accept, n_test, accept / max(1, n_test) * 100.0))
+        self.synchronize()
+        return history
 
     def last_batch_stats(self) -> Tuple[float, int]:
         """(quadratic cost, hits) of the last accumulated batch, evaluated with the pre-update parameters."""

@@ -6,7 +6,8 @@
 // The handle owns the conv parameters, the per-layer activations and a dense rcn_cuda_model (model.cu) created with an
 // empty convpool stack, whose gradient buffer is the tail of this handle's flat gradient buffer.  A step only launches
 // kernels that already exist as ops (conv.cu, extops.cu, dense.cu, smallnet.cu), plus the dense stack's input gradient
-// (launch_dense_input_grad) and, for u8 images, one widening copy for the first layer's weight gradient:
+// (launch_dense_input_grad) and cnn_stage_batch_kernel: for u8 images the widening copy the first layer's weight gradient
+// reads, and in epoch mode the gather of the step's images and labels from the bound dataset (that copy included):
 //   forward    per conv layer  conv2d forward, bias + ReLU in its epilogue (direct kernel / DMMA / tcgen05 implicit GEMM)
 //              per pool layer  ext_pool_forward_kernel (argmax bytes kept for the backward pass)
 //              dense stack     the model's accumulate on the last output (fused kernels A/B on narrow heads), delta0 kept
@@ -26,8 +27,59 @@
 
 namespace rcn {
 
-__global__ void cnn_u8_to_f64_kernel(const uint8_t* __restrict__ x, size_t n, double* __restrict__ y) {
-    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) y[i] = (double)x[i];
+template <int VEC> struct StageVec;
+template <> struct StageVec<16> { using T = uint4; };
+template <> struct StageVec<8> { using T = uint2; };
+template <> struct StageVec<4> { using T = unsigned; };
+template <> struct StageVec<1> { using T = uint8_t; };
+
+__device__ __forceinline__ unsigned stage_word(const uint4& v, int j) { return j == 0 ? v.x : j == 1 ? v.y : j == 2 ? v.z : v.w; }
+__device__ __forceinline__ unsigned stage_word(const uint2& v, int j) { return j == 0 ? v.x : v.y; }
+__device__ __forceinline__ unsigned stage_word(unsigned v, int) { return v; }
+
+// Builds a step's input from a dataset in device memory: chunk image b is dataset image perm[c + b] (perm == NULL: c + b)
+// with c = *cursor, read once (cursor == NULL: 0).  chunk (optional) receives the images as stored, x64 (optional, u8
+// images) their f64 widening, labels_batch (optional) labels[perm[c + b]].  Each thread copies one VEC-byte vector
+// (b, k) of the chunk per iteration, so every thread of the grid has a load in flight, whatever the image size; VEC
+// divides img_bytes and the alignment of `images` and `chunk` (launch_stage_batch picks it), and for VEC >= 2 the widened
+// copy goes out in 16-byte stores.  (b, k) advances by the grid stride without a division inside the loop.
+template <int VEC>
+__global__ void __launch_bounds__(256) cnn_stage_batch_kernel(const uint8_t* __restrict__ images, size_t img_bytes,
+                                                              const int64_t* __restrict__ perm,
+                                                              const long long* __restrict__ cursor, size_t B,
+                                                              const int64_t* __restrict__ labels,
+                                                              int64_t* __restrict__ labels_batch, uint8_t* __restrict__ chunk,
+                                                              double* __restrict__ x64) {
+    using V = typename StageVec<VEC>::T;
+    const long long c = cursor ? __ldcg(cursor) : 0;   // the previous step's update wrote it
+    const size_t nv = img_bytes / VEC;                 // vectors per image
+    const size_t stride = (size_t)gridDim.x * blockDim.x;
+    const size_t sb = stride / nv, sk = stride - sb * nv;
+    const size_t t = blockIdx.x * (size_t)blockDim.x + threadIdx.x;
+    size_t b = t / nv, k = t - b * nv;
+    while (b < B) {
+        const long long i = perm ? __ldg(perm + c + (long long)b) : c + (long long)b;
+        if (labels_batch && k == 0) labels_batch[b] = __ldg(labels + i);
+        const V v = __ldg(reinterpret_cast<const V*>(images + (size_t)i * img_bytes) + k);
+        if (chunk) reinterpret_cast<V*>(chunk + b * img_bytes)[k] = v;
+        if (x64) {
+            double* wide = x64 + b * img_bytes + k * VEC;
+            if constexpr (VEC == 1) {
+                wide[0] = (double)v;
+            } else {
+                double2* w2 = reinterpret_cast<double2*>(wide);
+#pragma unroll
+                for (int j = 0; j < VEC; j += 2) {
+                    const unsigned wd = stage_word(v, j >> 2);
+                    const int s = (j & 3) * 8;
+                    w2[j >> 1] = make_double2((double)((wd >> s) & 0xffu), (double)((wd >> (s + 8)) & 0xffu));
+                }
+            }
+        }
+        b += sb;
+        k += sk;
+        if (k >= nv) { k -= nv; ++b; }
+    }
 }
 
 struct CnnLayer {
@@ -60,6 +112,14 @@ struct rcn_cuda_cnn {
     OzakiWorkspace oz;
     size_t out_B = 0;                  // batch of the last forward (layer-output taps)
     size_t grad_B = 0;                 // batch of the last accumulate (input-gradient tap)
+    // epoch mode: the bound dataset (caller's device memory), the staged chunk and the state block
+    // ep_state = [cursor, padding, labels_batch[B]] (int64)
+    const void* ep_images = nullptr;
+    const int64_t* ep_labels = nullptr;
+    const int64_t* ep_perm = nullptr;
+    int ep_fmt = 0;
+    size_t ep_n = 0, ep_B = 0;
+    DevBuf ep_chunk, ep_state;
 };
 
 namespace {
@@ -84,18 +144,52 @@ int layer_shape(const CnnLayer& ly, size_t B, ConvShape* s) {
     return check_conv_shape(B, ly.Hi, ly.Wi, ly.Ci, ly.Co, ly.kh, ly.kw, ly.padding, s);
 }
 
-// Checks the call's images against the network and stages them (and the labels, when given) on the handle's stream.
-int stage_inputs(rcn_cuda_cnn* h, const void* images, int fmt, const int64_t* labels, size_t B, size_t H, size_t W,
-                 const void** img_dev, const int64_t** lab_dev, bool* host_in) {
+size_t image_bytes(const rcn_cuda_cnn* h, int fmt) { return h->H * h->W * h->Cin * (fmt == RCN_PIXELS_U8_ROWMAJOR ? 1 : 8); }
+
+// The pixel format and the image size of a call against the network.
+int check_images(const rcn_cuda_cnn* h, int fmt, size_t H, size_t W) {
     if (fmt != RCN_PIXELS_U8_ROWMAJOR && fmt != RCN_PIXELS_F64_NHWC)
         return fail(RCN_ERR_INVALID, "unknown pixel format %d (the network takes u8 row-major or f64 NHWC images)", fmt);
     if (fmt == RCN_PIXELS_U8_ROWMAJOR && h->Cin != 1)
         return fail(RCN_ERR_SHAPE, "u8 images have one channel, the network takes %zu", h->Cin);
     if (H != h->H || W != h->W)
         return fail(RCN_ERR_SHAPE, "the network was created for %zu x %zu images, got %zu x %zu", h->H, h->W, H, W);
+    return RCN_OK;
+}
+
+// cnn_stage_batch_kernel over B images of img_bytes each; the widest access that img_bytes and both byte pointers allow.
+int launch_stage_batch(rcn_cuda_cnn* h, const void* images, size_t img_bytes, const int64_t* perm, const long long* cursor,
+                       size_t B, const int64_t* labels, int64_t* labels_batch, void* chunk, double* x64) {
+    if (B == 0) return RCN_OK;
+    const uintptr_t align = (uintptr_t)images | (uintptr_t)chunk;
+    int vec = 1;
+    for (int v : {16, 8, 4})
+        if (img_bytes % v == 0 && align % v == 0) { vec = v; break; }
+    // one vector per thread, grid-stride beyond 8 CTAs per SM
+    const unsigned grid = (unsigned)std::min<size_t>((B * (img_bytes / vec) + 255) / 256, (size_t)kNumSMs * 8);
+    const uint8_t* src = (const uint8_t*)images;
+    uint8_t* dst = (uint8_t*)chunk;
+#define RCN_STAGE_LAUNCH(V)                                                                                                  \
+    RCN_LAUNCH("cnn_stage_batch_kernel", h->stream,                                                                          \
+               cnn_stage_batch_kernel<V><<<grid, 256, 0, h->stream>>>(src, img_bytes, perm, cursor, B, labels, labels_batch, \
+                                                                      dst, x64))
+    switch (vec) {
+        case 16: RCN_STAGE_LAUNCH(16); break;
+        case 8: RCN_STAGE_LAUNCH(8); break;
+        case 4: RCN_STAGE_LAUNCH(4); break;
+        default: RCN_STAGE_LAUNCH(1); break;
+    }
+#undef RCN_STAGE_LAUNCH
+    return RCN_OK;
+}
+
+// Checks the call's images against the network and stages them (and the labels, when given) on the handle's stream.
+int stage_inputs(rcn_cuda_cnn* h, const void* images, int fmt, const int64_t* labels, size_t B, size_t H, size_t W,
+                 const void** img_dev, const int64_t** lab_dev, bool* host_in) {
+    RCN_TRY(check_images(h, fmt, H, W));
     if (!images) return fail(RCN_ERR_INVALID, "null images");
     StagedIn in;
-    RCN_TRY(in.stage(images, B * H * W * h->Cin * (fmt == RCN_PIXELS_U8_ROWMAJOR ? 1 : 8), h->in_stage, h->stream, host_in));
+    RCN_TRY(in.stage(images, B * image_bytes(h, fmt), h->in_stage, h->stream, host_in));
     *img_dev = in.dev;
     if (lab_dev) {
         if (!labels) return fail(RCN_ERR_INVALID, "null labels");
@@ -107,8 +201,9 @@ int stage_inputs(rcn_cuda_cnn* h, const void* images, int fmt, const int64_t* la
 }
 
 // The conv / pool stack on device images.  `training`: keep the max-pool argmax bytes and an f64 copy of u8 images for the
-// first conv layer's weight gradient.  Returns the first layer's f64 input (NULL when u8 images were read directly).
-int forward_stack(rcn_cuda_cnn* h, const void* img, int fmt, size_t B, bool training, const double** x0) {
+// first conv layer's weight gradient (`x64_staged`: the epoch staging kernel already wrote that copy into x64).  Returns
+// the first layer's f64 input (NULL when u8 images were read directly).
+int forward_stack(rcn_cuda_cnn* h, const void* img, int fmt, size_t B, bool training, bool x64_staged, const double** x0) {
     const bool u8 = fmt == RCN_PIXELS_U8_ROWMAJOR;
     const CnnLayer& first = h->layers[0];
     ConvShape s0{};
@@ -116,12 +211,11 @@ int forward_stack(rcn_cuda_cnn* h, const void* img, int fmt, size_t B, bool trai
     const bool direct_u8 = u8 && first.kind == RCN_CNN_CONV && conv_direct_ok(s0);
     const double* x = u8 ? nullptr : (const double*)img;
     if (u8 && (!direct_u8 || (training && first.kind == RCN_CNN_CONV))) {
-        const size_t n = B * h->H * h->W;
-        RCN_TRY(h->x64.reserve(n * sizeof(double)));
-        unsigned grid = cdiv(n, 256);
-        if (grid > kNumSMs * 8) grid = kNumSMs * 8;
-        RCN_LAUNCH("cnn_u8_to_f64_kernel", h->stream,
-                   cnn_u8_to_f64_kernel<<<grid, 256, 0, h->stream>>>((const uint8_t*)img, n, h->x64.as<double>()));
+        if (!x64_staged) {
+            const size_t n = B * h->H * h->W;
+            RCN_TRY(h->x64.reserve(n * sizeof(double)));
+            RCN_TRY(launch_stage_batch(h, img, h->H * h->W, nullptr, nullptr, B, nullptr, nullptr, nullptr, h->x64.as<double>()));
+        }
         x = h->x64.as<double>();
     }
     *x0 = x;
@@ -152,13 +246,13 @@ int forward_stack(rcn_cuda_cnn* h, const void* img, int fmt, size_t B, bool trai
     return RCN_OK;
 }
 
-int accumulate_dev(rcn_cuda_cnn* h, const void* img, int fmt, const int64_t* labels, size_t B) {
+int accumulate_dev(rcn_cuda_cnn* h, const void* img, int fmt, const int64_t* labels, size_t B, bool x64_staged = false) {
     if (B == 0) {
         RCN_CUDA_TRY(cudaMemsetAsync(h->grads, 0, h->n_params * sizeof(double), h->stream));
         return RCN_OK;
     }
     const double* x0 = nullptr;
-    RCN_TRY(forward_stack(h, img, fmt, B, true, &x0));
+    RCN_TRY(forward_stack(h, img, fmt, B, true, x64_staged, &x0));
     const size_t n = h->layers.size();
     RCN_TRY(rcn_cuda_accumulate_gradients(h->dense, h->layers[n - 1].out.as<double>(), nullptr, labels, B));
     // dX = W0^T delta0, read before apply moves W0
@@ -229,6 +323,35 @@ int apply(rcn_cuda_cnn* h, double eta, size_t batch) {
     if (batch == 0) return RCN_OK;
     // (eta / batch) formed first, then the rounded product subtracted (rcn.rs:214); the dense part forms the same scale
     if (h->n_conv) RCN_TRY(launch_sgd_update(h->params.as<double>(), h->grads, h->n_conv, eta / (double)batch, h->stream));
+    return rcn_cuda_apply_gradients(h->dense, eta, batch);
+}
+
+// ---- epoch mode: rcn.rs:144-149 over a dataset resident in device memory ---------------------------------------------
+constexpr size_t kCnnEpSlots = 2;   // ep_state: cursor, padding; labels_batch follows
+
+int require_epoch(const rcn_cuda_cnn* h) {
+    if (!h->ep_images) return fail(RCN_ERR_STATE, "no dataset bound: call rcn_cuda_cnn_epoch_bind first");
+    return RCN_OK;
+}
+
+// Stages chunk perm[c .. c+B) (and for u8 images its f64 copy) and accumulates it; the cursor stays where it is.
+int epoch_accumulate(rcn_cuda_cnn* h) {
+    RCN_TRY(require_epoch(h));
+    const bool u8 = h->ep_fmt == RCN_PIXELS_U8_ROWMAJOR;
+    long long* st = h->ep_state.as<long long>();
+    int64_t* lab = reinterpret_cast<int64_t*>(st + kCnnEpSlots);
+    RCN_TRY(launch_stage_batch(h, h->ep_images, image_bytes(h, h->ep_fmt), h->ep_perm, st, h->ep_B, h->ep_labels, lab,
+                               h->ep_chunk.p, u8 ? h->x64.as<double>() : nullptr));
+    return accumulate_dev(h, h->ep_chunk.p, h->ep_fmt, lab, h->ep_B, u8);
+}
+
+// apply(), with the conv update also advancing the cursor by B (chunks_exact wrap-around, rcn.rs:147); with no conv
+// parameters the update kernel runs on zero of them and only advances the cursor.
+int epoch_apply(rcn_cuda_cnn* h, double eta, size_t batch) {
+    RCN_TRY(require_epoch(h));
+    if (batch == 0) return fail(RCN_ERR_INVALID, "global batch is zero");
+    RCN_TRY(launch_sgd_update(h->params.as<double>(), h->grads, h->n_conv, eta / (double)batch, h->stream,
+                              h->ep_state.as<long long>(), (long long)h->ep_B, (long long)h->ep_n));
     return rcn_cuda_apply_gradients(h->dense, eta, batch);
 }
 
@@ -334,7 +457,7 @@ int rcn_cuda_cnn_destroy(rcn_cuda_cnn_handle h) {
     if (h->own_stream) { cudaStreamSynchronize(h->own_stream); cudaStreamDestroy(h->own_stream); }
     for (CnnLayer& ly : h->layers) { ly.out.release(); ly.argmax.release(); }
     DevBuf* bufs[] = {&h->params, &h->grads_own, &h->in_stage, &h->lab_stage, &h->out_stage, &h->x64, &h->dx, &h->gbuf[0],
-                      &h->gbuf[1], &h->flip_ws, &h->wgrad_ws, &h->small, &h->rs.buf};
+                      &h->gbuf[1], &h->flip_ws, &h->wgrad_ws, &h->small, &h->rs.buf, &h->ep_chunk, &h->ep_state};
     for (DevBuf* b : bufs) b->release();
     h->oz.release();
     delete h;
@@ -401,6 +524,73 @@ int rcn_cuda_cnn_train_batch(rcn_cuda_cnn_handle h, const void* images, int pixe
     return apply(h, eta, B);
 }
 
+int rcn_cuda_cnn_epoch_bind(rcn_cuda_cnn_handle h, const void* images, int pixel_format, const int64_t* labels,
+                            const int64_t* perm, size_t n_samples, size_t H, size_t W, size_t B) {
+    RCN_CNN_ENTER(h);
+    if (!images || !labels || B == 0 || n_samples < B)
+        return fail(RCN_ERR_INVALID, "epoch_bind needs images, labels and n_samples >= B > 0");
+    if (!is_device_ptr(images) || !is_device_ptr(labels) || (perm && !is_device_ptr(perm)))
+        return fail(RCN_ERR_INVALID, "epoch mode needs a dataset resident in device memory");
+    RCN_TRY(check_images(h, pixel_format, H, W));
+    const size_t img_bytes = image_bytes(h, pixel_format);
+    RCN_TRY(h->ep_chunk.reserve(B * img_bytes));
+    if (pixel_format == RCN_PIXELS_U8_ROWMAJOR) RCN_TRY(h->x64.reserve(B * img_bytes * sizeof(double)));
+    RCN_TRY(h->ep_state.reserve((kCnnEpSlots + B) * sizeof(int64_t)));
+    RCN_CUDA_TRY(cudaMemsetAsync(h->ep_state.p, 0, (kCnnEpSlots + B) * sizeof(int64_t), h->stream));
+    h->ep_images = images; h->ep_labels = labels; h->ep_perm = perm; h->ep_fmt = pixel_format;
+    h->ep_n = n_samples; h->ep_B = B;
+    RCN_CUDA_TRY(cudaStreamSynchronize(h->stream));   // the cursor is zero before any step kernel can look at it
+    return RCN_OK;
+}
+
+int rcn_cuda_cnn_epoch_seek(rcn_cuda_cnn_handle h, size_t position) {
+    RCN_CNN_ENTER(h);
+    RCN_TRY(require_epoch(h));
+    if (position + h->ep_B > h->ep_n) return fail(RCN_ERR_INVALID, "position %zu leaves fewer than B samples", position);
+    const long long pos = (long long)position;
+    RCN_CUDA_TRY(cudaMemcpyAsync(h->ep_state.p, &pos, sizeof(pos), cudaMemcpyHostToDevice, h->stream));
+    RCN_CUDA_TRY(cudaStreamSynchronize(h->stream));
+    return RCN_OK;
+}
+
+int rcn_cuda_cnn_epoch_position(rcn_cuda_cnn_handle h, size_t* position) {
+    RCN_CNN_ENTER(h);
+    RCN_TRY(require_epoch(h));
+    if (!position) return fail(RCN_ERR_INVALID, "null output");
+    long long pos = 0;
+    RCN_CUDA_TRY(cudaMemcpyAsync(&pos, h->ep_state.p, sizeof(pos), cudaMemcpyDeviceToHost, h->stream));
+    RCN_CUDA_TRY(cudaStreamSynchronize(h->stream));
+    *position = (size_t)pos;
+    return RCN_OK;
+}
+
+int rcn_cuda_cnn_epoch_accumulate(rcn_cuda_cnn_handle h) {
+    RCN_CNN_ENTER(h);
+    return epoch_accumulate(h);
+}
+
+int rcn_cuda_cnn_epoch_apply(rcn_cuda_cnn_handle h, double eta, size_t global_batch) {
+    RCN_CNN_ENTER(h);
+    return epoch_apply(h, eta, global_batch);
+}
+
+int rcn_cuda_cnn_epoch_step(rcn_cuda_cnn_handle h, double eta) {
+    RCN_CNN_ENTER(h);
+    RCN_TRY(epoch_accumulate(h));
+    return epoch_apply(h, eta, h->ep_B);
+}
+
+int rcn_cuda_cnn_epoch_run(rcn_cuda_cnn_handle h, double eta, size_t n_steps) {
+    RCN_CNN_ENTER(h);
+    RCN_TRY(require_epoch(h));
+    if (n_steps > (size_t)1 << 30) return fail(RCN_ERR_INVALID, "too many steps in one call");
+    for (size_t k = 0; k < n_steps; ++k) {
+        RCN_TRY(epoch_accumulate(h));
+        RCN_TRY(epoch_apply(h, eta, h->ep_B));
+    }
+    return RCN_OK;
+}
+
 int rcn_cuda_cnn_last_batch_stats(rcn_cuda_cnn_handle h, double* cost, uint64_t* hits) {
     RCN_CNN_ENTER(h);
     return rcn_cuda_last_batch_stats(h->dense, cost, hits);
@@ -422,7 +612,7 @@ int rcn_cuda_cnn_evaluate_images(rcn_cuda_cnn_handle h, const void* images, int 
         const bool lab_host = labels_out && !is_device_ptr(labels_out);
         if (lab_host) { RCN_TRY(h->out_stage.reserve(B * sizeof(int64_t))); lab_dev = h->out_stage.as<int64_t>(); }
         const double* x0 = nullptr;
-        RCN_TRY(forward_stack(h, img, pixel_format, B, false, &x0));
+        RCN_TRY(forward_stack(h, img, pixel_format, B, false, false, &x0));
         RCN_TRY(model_evaluate_features(h->dense, h->layers.back().out.as<double>(), lab, B, st, lab_dev));
         if (lab_host) RCN_TRY(deliver(h, labels_out, lab_dev, B * sizeof(int64_t)));
         if (host_in) RCN_CUDA_TRY(cudaStreamSynchronize(h->stream));
@@ -443,7 +633,7 @@ int rcn_cuda_cnn_classify_images(rcn_cuda_cnn_handle h, const void* images, int 
     const bool lab_host = !is_device_ptr(labels_out);
     if (lab_host) { RCN_TRY(h->out_stage.reserve(B * sizeof(int64_t))); lab_dev = h->out_stage.as<int64_t>(); }
     const double* x0 = nullptr;
-    RCN_TRY(forward_stack(h, img, pixel_format, B, false, &x0));
+    RCN_TRY(forward_stack(h, img, pixel_format, B, false, false, &x0));
     RCN_TRY(model_evaluate_features(h->dense, h->layers.back().out.as<double>(), nullptr, B, nullptr, lab_dev));
     if (lab_host) RCN_TRY(deliver(h, labels_out, lab_dev, B * sizeof(int64_t)));
     if (host_in) RCN_CUDA_TRY(cudaStreamSynchronize(h->stream));

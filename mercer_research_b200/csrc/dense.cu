@@ -606,8 +606,8 @@ __global__ void sgd_update_kernel(double* __restrict__ p, const double* __restri
 
 int launch_sgd_update(double* params, const double* grads, size_t n, double scale, cudaStream_t stream,
                       long long* cursor, long long batch, long long n_samples, const double* stats, double* stats_ring) {
-    if (n == 0) return RCN_OK;
-    unsigned grid = cdiv(n, 256);
+    if (n == 0 && !cursor) return RCN_OK;
+    unsigned grid = n ? cdiv(n, 256) : 1;   // n == 0 with a cursor: only the cursor advances
     if (grid > kNumSMs * 8) grid = kNumSMs * 8;
     RCN_LAUNCH("sgd_update_kernel", stream,
                sgd_update_kernel<<<grid, 256, 0, stream>>>(params, grads, n, scale, cursor, batch, n_samples, stats, stats_ring));

@@ -40,7 +40,8 @@ int launch_reduce_splits(const double* partials, int splits, size_t n, double* o
 int launch_bias_grad(const double* delta, size_t M, size_t N, double* db, ReduceScratch& rs, cudaStream_t stream);
 
 // params -= scale * grads   (rcn.rs:210-222, scale = eta / batch formed first)
-// cursor (optional): device-side position of the epoch walk, advanced by `batch` with chunks_exact wrap-around.
+// cursor (optional): device-side position of the epoch walk, advanced by `batch` with chunks_exact wrap-around (also when
+// n == 0: one thread then only advances the cursor).
 // stats / stats_ring (optional, with cursor): the step's {cost, hits} pair is copied to stats_ring + 2 * (cursor / batch)
 // (pinned host memory in rcn_cuda_train_epoch_host) before the cursor advances.
 int launch_sgd_update(double* params, const double* grads, size_t n, double scale, cudaStream_t stream,

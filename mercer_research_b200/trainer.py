@@ -9,7 +9,7 @@ the single-GPU result only by summation order (SURVEY.md 8e). No other collectiv
 
 The compute backend is any object with ``n_params``, ``bind_gradient_buffer(t)``, ``accumulate_gradients_images``,
 ``accumulate_gradients``, ``apply_gradients`` and ``last_batch_stats`` (``evaluate`` also needs ``evaluate_images``) --
-in the product that is ``RCN`` (CUDA);
+in the product that is ``RCN`` (CUDA) or ``ConvNet`` (CUDA, NCCL exchange only);
 the gloo CPU tests plug in a checker-backed stand-in to exercise exactly this host logic without a GPU.
 
 Stream discipline: the library launches on the stream bound with ``set_stream``; the NCCL collective is ordered against
@@ -225,12 +225,14 @@ class DataParallelTrainer:
                 self._epoch_step_eager()
         self.graph = graph
         self._graph_generation = _lib.allocation_generation()
-        self._graph_scale = self.model.scale_set          # (mean, sd) travel by value in the captured kernel arguments
+        # (mean, sd) travel by value in the captured kernel arguments; a ConvNet has no scale_set
+        self._graph_scale = getattr(self.model, "scale_set", None)
         self._bind_stream()
 
     def _replay(self):
         from . import _lib
-        if _lib.allocation_generation() != self._graph_generation or self.model.scale_set != self._graph_scale:
+        if (_lib.allocation_generation() != self._graph_generation
+                or getattr(self.model, "scale_set", None) != self._graph_scale):
             self._capture_graph()
         self.graph.replay()
 

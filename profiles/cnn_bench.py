@@ -1,10 +1,17 @@
 """Times one training step of the convolutional network handle (mercer_research_b200.ConvNet) on device-resident data
-larger than the 126 MB L2, for the two shapes of BASELINE.json configs 3 and 4:
+larger than the 126 MB L2, for an MNIST-shaped network and the two shapes of BASELINE.json configs 3 and 4:
 
+  mnist   28x28 u8,    Conv(8)/Pool                                -> 1568-30-10,   B = 1024
   cifar   32x32x3 f64, Conv(32)/Pool/Conv(64)/Pool/Conv(128)/Pool -> 2048-256-10, B = 4096
   wide    64x64 u8,    Conv(64)/Conv(64)/Pool/Conv(128)/Pool       -> 32768-32-10,  B = 256
 
-Per shape: images/s (CUDA events over >= 0.3 s after warm-up, profiler off), per-kernel time shares from the library's
+Two ways to drive the same steps over the same data, alternated three times (median and spread of each): the eager loop,
+one train_batch_images call per host-sliced minibatch (step_ms / images_per_s), and the epoch mode, the data bound with a
+random perm and one captured epoch_step replayed per step (epoch_graph).  The epoch staging kernel's time per step comes
+from the library's launch profiler, its bytes from the shapes (images read and written, the f64 copy of u8 images, perm
+and labels); a torch device-to-device copy moving the same number of bytes, rotated through the dataset so it comes from
+HBM, is timed in the same call.
+Per shape also: per-kernel time shares of the eager step from the library's
 launch profiler (a separate pass), the conv engine each layer's forward / backward-data / backward-weight took, and for
 the GEMM-shaped kernels the achieved rate against the DGEMM peak (torch.matmul f64) or the int8 tensor-core peak
 (torch._int_mm) measured in the same call.  The tcgen05 conv kernels run 15 int8 plane products per f64 product, so their
@@ -26,6 +33,7 @@ from mercer_research_b200 import _lib, ext  # noqa: E402
 
 P, Q = m.Padding, m.Pooling
 SHAPES = {
+    "mnist": dict(shape=(28, 28, 1), u8=True, B=1024, ff=[30], layers=[m.Conv(8), m.Pool(Q.Max, P.Same)]),
     "cifar": dict(shape=(32, 32, 3), u8=False, B=4096, ff=[256],
                   layers=[m.Conv(32), m.Pool(Q.Max, P.Same), m.Conv(64), m.Pool(Q.Max, P.Same), m.Conv(128), m.Pool(Q.Max, P.Same)]),
     "wide": dict(shape=(64, 64, 1), u8=True, B=256, ff=[32],
@@ -130,7 +138,59 @@ def run_shape(name, cfg, pk):
     for _ in range(3):
         step()
     torch.cuda.synchronize()
-    ms, n = timed(step)
+    # the same data bound for epoch mode under a random perm; one captured step replayed per step
+    flat, flat_y = data.view((n_batches * B,) + data.shape[2:]), labels.view(-1)
+    perm = torch.randperm(n_batches * B, device="cuda", generator=g)
+    net.epoch_bind(flat, flat_y, B, perm)
+    net.epoch_accumulate()
+    torch.cuda.synchronize()
+    graph = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(graph):
+        net.set_stream(torch.cuda.current_stream().cuda_stream)
+        net.epoch_step(0.05)
+    net.set_stream(torch.cuda.current_stream().cuda_stream)
+    gen = _lib.allocation_generation()
+    eager_runs, graph_runs = [], []
+    for _ in range(3):
+        eager_runs.append(timed(step))
+        graph_runs.append(timed(graph.replay))
+    assert _lib.allocation_generation() == gen, "a library buffer moved under the captured step"
+    ms = float(np.median([r[0] for r in eager_runs]))
+    n = int(sum(r[1] for r in eager_runs))
+    g_ms = float(np.median([r[0] for r in graph_runs]))
+
+    def spread(runs):
+        v = [r[0] for r in runs]
+        return dict(median_ms=float(np.median(v)), min_ms=min(v), max_ms=max(v), runs_ms=v,
+                    spread=(max(v) - min(v)) / float(np.median(v)), steps=[r[1] for r in runs])
+
+    # staging kernel: time per step (event-bracketed launches, eager epoch steps) and bytes moved per step
+    img_bytes = int(np.prod(c["shape"])) * (1 if c["u8"] else 8)
+    stage_bytes = B * img_bytes * (2 + (8 if c["u8"] else 0)) + B * 8 * 3   # images in/out (+f64), perm, labels in/out
+    torch.cuda.synchronize()
+    _lib.profile_enable(True)
+    for _ in range(20):
+        net.epoch_step(0.05)
+    rep = _lib.profile_report()
+    _lib.profile_enable(False)
+    st = [v for kname, v in rep.items() if kname.startswith("cnn_stage_batch_kernel")]
+    stage_ms = sum(v["total_ms"] for v in st) / max(1, sum(v["launches"] for v in st))
+    raw = data.view(torch.uint8).view(-1)
+    half = stage_bytes // 2                                                  # a copy moves 2x its size
+    dst = torch.empty(half, dtype=torch.uint8, device="cuda")
+    off = [0]
+
+    def copy():
+        o = off[0]
+        off[0] = (o + half) % (raw.numel() - half)
+        dst.copy_(raw[o:o + half])
+
+    copy_ms, _ = timed(copy)
+    epoch = dict(graph_step=spread(graph_runs), eager_step=spread(eager_runs), step_ms=g_ms, images_per_s=B / (g_ms * 1e-3),
+                 replay_speedup=ms / g_ms, stage_kernel_ms_per_step=stage_ms, stage_bytes_per_step=stage_bytes,
+                 stage_bytes_per_s=stage_bytes / (stage_ms * 1e-3), torch_d2d_copy_ms=copy_ms,
+                 torch_d2d_copy_bytes_per_s=2 * half / (copy_ms * 1e-3),
+                 stage_launches_per_step=sum(v["launches"] for v in st) / 20)
     # profile pass (separate: the event pairs slow the host)
     torch.cuda.synchronize()
     _lib.profile_enable(True)
@@ -164,8 +224,8 @@ def run_shape(name, cfg, pk):
             rates[f"conv2d_{pas} ({'tcgen05' if tc else 'DMMA'})"] = r
     res = dict(batch=B, n_batches_resident=n_batches, resident_bytes=n_batches * per_batch, step_ms=ms, timed_steps=n,
                images_per_s=B / (ms * 1e-3), kernel_shares=shares, conv_engines=eng, gemm_rates=rates,
-               n_params=net.n_params, feature_len=net.feature_len)
-    del data, labels
+               n_params=net.n_params, feature_len=net.feature_len, epoch_graph=epoch)
+    del graph, data, labels, flat, flat_y, perm, raw, dst
     net.close()
     torch.cuda.empty_cache()
     return res
@@ -182,7 +242,10 @@ def main():
     for name, cfg in SHAPES.items():
         out["shapes"][name] = run_shape(name, cfg, pk)
         r = out["shapes"][name]
-        print(f"{name}: {r['images_per_s']:.0f} images/s ({r['step_ms']:.3f} ms/step, B={r['batch']})", flush=True)
+        e = r["epoch_graph"]
+        print(f"{name}: {r['images_per_s']:.0f} images/s ({r['step_ms']:.3f} ms/step, B={r['batch']}); epoch graph "
+              f"{e['step_ms']:.3f} ms/step (x{e['replay_speedup']:.2f}); staging {e['stage_kernel_ms_per_step'] * 1e3:.1f} us "
+              f"{e['stage_bytes_per_s'] / 1e9:.0f} GB/s, torch copy {e['torch_d2d_copy_bytes_per_s'] / 1e9:.0f} GB/s", flush=True)
     with open(os.path.join(args.out, "cnn_bench_b200.json"), "w") as f:
         json.dump(out, f, indent=1)
     print(json.dumps({k: v for k, v in out.items() if k != "shapes"}))

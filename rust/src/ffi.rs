@@ -156,6 +156,14 @@ extern "C" {
     pub fn rcn_cuda_cnn_train_batch(h: rcn_cuda_cnn_handle, images: *const c_void, pixel_format: c_int, labels: *const i64,
                                     B: usize, H: usize, W: usize, eta: c_double) -> c_int;
     pub fn rcn_cuda_cnn_last_batch_stats(h: rcn_cuda_cnn_handle, cost: *mut c_double, hits: *mut u64) -> c_int;
+    pub fn rcn_cuda_cnn_epoch_bind(h: rcn_cuda_cnn_handle, images: *const c_void, pixel_format: c_int, labels: *const i64,
+                                   perm: *const i64, n_samples: usize, H: usize, W: usize, B: usize) -> c_int;
+    pub fn rcn_cuda_cnn_epoch_seek(h: rcn_cuda_cnn_handle, position: usize) -> c_int;
+    pub fn rcn_cuda_cnn_epoch_position(h: rcn_cuda_cnn_handle, position: *mut usize) -> c_int;
+    pub fn rcn_cuda_cnn_epoch_accumulate(h: rcn_cuda_cnn_handle) -> c_int;
+    pub fn rcn_cuda_cnn_epoch_apply(h: rcn_cuda_cnn_handle, eta: c_double, global_batch: usize) -> c_int;
+    pub fn rcn_cuda_cnn_epoch_step(h: rcn_cuda_cnn_handle, eta: c_double) -> c_int;
+    pub fn rcn_cuda_cnn_epoch_run(h: rcn_cuda_cnn_handle, eta: c_double, n_steps: usize) -> c_int;
     pub fn rcn_cuda_cnn_evaluate_images(h: rcn_cuda_cnn_handle, images: *const c_void, pixel_format: c_int, labels: *const i64,
                                         B: usize, H: usize, W: usize, cost_out: *mut c_double, accept_out: *mut u64,
                                         labels_out: *mut i64) -> c_int;
