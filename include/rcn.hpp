@@ -399,6 +399,10 @@ class RCN {
     int device_ = 0;
 };
 
+/// Output head of a ConvNet's dense stack (RCN_HEAD_* in rcn_cuda.h): the reference's sigmoid layer with quadratic cost, or an
+/// affine output layer with softmax and cross-entropy.
+enum class Head : int { SigmoidQuadratic = RCN_HEAD_SIGMOID_QUADRATIC, SoftmaxCrossEntropy = RCN_HEAD_SOFTMAX_XENT };
+
 /// Learned conv / pool layers in front of the reference's dense stack (rcn_cuda_cnn_* in rcn_cuda.h): a thin owner of the
 /// handle.  Images are u8 (B, H, W) row-major or f64 (B, H, W, C) NHWC, host or device memory.
 class ConvNet {
@@ -412,11 +416,11 @@ class ConvNet {
     };
 
     ConvNet(size_t H, size_t W, size_t in_channels, const std::vector<Layer>& layers, const std::vector<size_t>& feedforward,
-            size_t classes, int device = 0) {
+            size_t classes, int device = 0, Head head = Head::SigmoidQuadratic) {
         std::vector<int32_t> spec;
         for (const Layer& l : layers) spec.insert(spec.end(), l.spec, l.spec + RCN_CNN_LAYER_INTS);
-        check(rcn_cuda_cnn_create(device, H, W, in_channels, spec.data(), layers.size(), feedforward.data(), feedforward.size(),
-                                  classes, &h_));
+        check(rcn_cuda_cnn_create_with_head(device, H, W, in_channels, spec.data(), layers.size(), feedforward.data(),
+                                            feedforward.size(), classes, (int)head, &h_));
     }
     ~ConvNet() { rcn_cuda_cnn_destroy(h_); }
     ConvNet(const ConvNet&) = delete;

@@ -308,7 +308,7 @@ int rcn_cuda_ext_gemm_f64(int device, void* cuda_stream, const double* A, size_t
 /* ---- convolutional network: learned conv / pool layers in front of the dense stack ---------------------------------
  * EXTENSION (BASELINE.json north_star configs 3 and 4; the reference has no learned convolution).  The network is
  *   input (B, H, W, C)  ->  conv / pool stack (NHWC)  ->  flatten  ->  the reference's dense stack (sigmoid layers,
- *   quadratic cost, W -= (eta/B) * sum dW).
+ *   quadratic cost, W -= (eta/B) * sum dW), or with RCN_HEAD_SOFTMAX_XENT the same stack with a softmax cross-entropy head.
  * layer_spec: n_layers records of RCN_CNN_LAYER_INTS int32 each:
  *   {RCN_CNN_CONV, Co, kh, kw, padding}   learned cross-correlation with bias, ALWAYS followed by ReLU; conventions and
  *                                         contract errors of rcn_cuda_ext_conv2d_forward (odd kernels for Same)
@@ -328,10 +328,26 @@ int rcn_cuda_ext_gemm_f64(int device, void* cuda_stream, const double* A, size_t
  * rcn_cuda_epoch_*; each step gathers its images and labels with one staging kernel. */
 enum { RCN_CNN_CONV = 0, RCN_CNN_POOL = 1 };
 #define RCN_CNN_LAYER_INTS 5
+/* Output head of the network's dense stack.
+ *   RCN_HEAD_SIGMOID_QUADRATIC  the reference's: sigmoid output layer, cost sum_b 0.5 |a_b - y_b|^2, delta_L = (a - y) a (1 - a),
+ *                               a hit when {i : a_i = max a} = {label} (rcn.rs:153-157), labels the last-max-wins argmax of a.
+ *   RCN_HEAD_SOFTMAX_XENT       hidden layers unchanged (sigmoid, delta_l = (W_{l+1}^T delta_{l+1}) a (1 - a)); the output
+ *                               layer is affine, z = W a + b, and p = softmax(z) per sample with rcn_cuda_ext_softmax_xent's
+ *                               arithmetic (m = max z, then s = sum exp(z - m), then log s).  Cost per sample
+ *                               (log s + m) - z_label, summed over the batch; delta_L = p - onehot(label).  Hits and labels
+ *                               are decided on z, not on p (exp rounding can make distinct logits equal probabilities): a hit
+ *                               when {i : z_i = max z} = {label}, labels the last-max-wins argmax of z.  A label outside
+ *                               [0, classes) has an all-zero target (cost 0, delta = p); a non-finite logit makes that
+ *                               sample's p, delta and cost NaN.
+ * Both heads update with W -= (eta / B) * sum dW. */
+enum { RCN_HEAD_SIGMOID_QUADRATIC = 0, RCN_HEAD_SOFTMAX_XENT = 1 };
 /* Validates the whole spec before any device work (status codes and messages of the ext ops; a zero-width dense layer or
- * zero classes is RCN_ERR_INVALID).  Parameters start at zero: set them with rcn_cuda_cnn_set_params. */
+ * zero classes is RCN_ERR_INVALID).  Parameters start at zero: set them with rcn_cuda_cnn_set_params.
+ * rcn_cuda_cnn_create is rcn_cuda_cnn_create_with_head with RCN_HEAD_SIGMOID_QUADRATIC; an unknown head is RCN_ERR_INVALID. */
 int rcn_cuda_cnn_create(int device, size_t H, size_t W, size_t in_channels, const int32_t* layer_spec, size_t n_layers,
                         const size_t* feedforward, size_t n_ff, size_t classes, rcn_cuda_cnn_handle* out);
+int rcn_cuda_cnn_create_with_head(int device, size_t H, size_t W, size_t in_channels, const int32_t* layer_spec, size_t n_layers,
+                                  const size_t* feedforward, size_t n_ff, size_t classes, int head, rcn_cuda_cnn_handle* out);
 int rcn_cuda_cnn_destroy(rcn_cuda_cnn_handle h);
 /* As rcn_cuda_set_stream: NULL is the legacy default stream, RCN_STREAM_OWN the handle's own stream. */
 int rcn_cuda_cnn_set_stream(rcn_cuda_cnn_handle h, void* cuda_stream);
@@ -351,7 +367,7 @@ int rcn_cuda_cnn_apply(rcn_cuda_cnn_handle h, double eta, size_t global_batch);
 /* accumulate + apply(eta, B) */
 int rcn_cuda_cnn_train_batch(rcn_cuda_cnn_handle h, const void* images, int pixel_format, const int64_t* labels, size_t B,
                              size_t H, size_t W, double eta);
-/* Quadratic cost and rcn.rs:153-157 hit count of the last accumulate, under the pre-update parameters. */
+/* The head's cost and the head's hit count (rule above) of the last accumulate, under the pre-update parameters. */
 int rcn_cuda_cnn_last_batch_stats(rcn_cuda_cnn_handle h, double* cost, uint64_t* hits);
 /* Epoch mode: `for batch in training_set.chunks_exact(B) { train_batch(batch, eta) }` (rcn.rs:144-149) over a dataset in
  * DEVICE memory, with meaning, contract and status codes of rcn_cuda_epoch_*: step k trains on samples perm[pos .. pos+B)
@@ -377,10 +393,12 @@ int rcn_cuda_cnn_epoch_accumulate(rcn_cuda_cnn_handle h);
 int rcn_cuda_cnn_epoch_apply(rcn_cuda_cnn_handle h, double eta, size_t global_batch);
 int rcn_cuda_cnn_epoch_step(rcn_cuda_cnn_handle h, double eta); /* accumulate + apply with global_batch = B */
 int rcn_cuda_cnn_epoch_run(rcn_cuda_cnn_handle h, double eta, size_t n_steps); /* n_steps epoch steps in one call */
-/* Forward pass only: cost_out, accept_out as rcn_cuda_evaluate_images; labels_out (optional) the rcn.rs:92-97 argmax.
+/* Forward pass only: cost_out the head's batch cost, accept_out the count of hits under the head's hit rule, labels_out
+ * (optional) the head's labels (the rcn.rs:92-97 last-max-wins argmax, of z with the softmax head).
  * Leaves the gradients and the last-batch statistics untouched (the layer-output tap then shows this batch). */
 int rcn_cuda_cnn_evaluate_images(rcn_cuda_cnn_handle h, const void* images, int pixel_format, const int64_t* labels, size_t B,
                                  size_t H, size_t W, double* cost_out, uint64_t* accept_out, int64_t* labels_out);
+/* The head's labels of B images, as evaluate's labels_out. */
 int rcn_cuda_cnn_classify_images(rcn_cuda_cnn_handle h, const void* images, int pixel_format, size_t B, size_t H, size_t W,
                                  int64_t* labels_out);
 /* As rcn_cuda_bind_gradient_buffer / rcn_cuda_gradient_buffer / rcn_cuda_get_gradients, over the whole flat buffer. */

@@ -98,6 +98,7 @@ SIGNATURES = {
     "rcn_cuda_ext_gemm_f64": [_i, _vp, _vp, _sz, _i, _vp, _sz, _i, _sz, _sz, _sz, _i, _vp],
     # convolutional network handle (learned conv / pool layers + the dense stack)
     "rcn_cuda_cnn_create": [_i, _sz, _sz, _sz, _vp, _sz, _vp, _sz, _sz, C.POINTER(_vp)],
+    "rcn_cuda_cnn_create_with_head": [_i, _sz, _sz, _sz, _vp, _sz, _vp, _sz, _sz, _i, C.POINTER(_vp)],
     "rcn_cuda_cnn_destroy": [_vp],
     "rcn_cuda_cnn_set_stream": [_vp, _vp],
     "rcn_cuda_cnn_synchronize": [_vp],

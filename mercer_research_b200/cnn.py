@@ -1,5 +1,6 @@
 """A trainable convolutional network: learned conv / pool layers in front of the reference's dense stack (sigmoid layers,
-quadratic cost, ``W -= (eta/B) * sum dW``), driving the ``rcn_cuda_cnn_*`` entry points of librcn_cuda.so.
+quadratic cost, ``W -= (eta/B) * sum dW``) or of the same stack with a softmax cross-entropy head (``Head``), driving the
+``rcn_cuda_cnn_*`` entry points of librcn_cuda.so.
 
 Images are numpy arrays (staged through the device) or torch CUDA tensors (used in place, on torch's current stream):
 ``(B, H, W)`` uint8 (one channel) or ``(B, H, W, C)`` float64 channels-last.  Labels are ``(B,)`` int64.  The flat
@@ -11,6 +12,7 @@ from __future__ import annotations
 
 import ctypes as C
 from dataclasses import dataclass
+from enum import IntEnum
 from typing import List, Sequence, Tuple
 
 import numpy as np
@@ -20,6 +22,17 @@ from .kernel import Padding, Pooling, _is_torch
 from .rcn import _Buf
 
 CNN_CONV, CNN_POOL, LAYER_INTS = 0, 1, 5
+
+
+class Head(IntEnum):
+    """Output head of the dense stack (``RCN_HEAD_*``, semantics in rcn_cuda.h).
+
+    ``SigmoidQuadratic``: the reference's sigmoid output layer, cost ``sum_b 0.5 |a_b - y_b|^2``.
+    ``SoftmaxCrossEntropy``: an affine output layer ``z = W a + b``, ``p = softmax(z)``, cost ``sum_b (log s + m) - z_label``
+    (``m = max z``, ``s = sum exp(z - m)``) and ``delta = p - onehot(label)``; hits and labels are decided on the logits.
+    Hidden layers stay sigmoid with either head."""
+    SigmoidQuadratic = 0
+    SoftmaxCrossEntropy = 1
 
 
 @dataclass(frozen=True)
@@ -45,9 +58,10 @@ class Pool:
 
 
 class ConvNet:
-    """``ConvNet((H, W, C), [Conv(16), Pool(), ...], feedforward=[64], classes=10)``."""
+    """``ConvNet((H, W, C), [Conv(16), Pool(), ...], feedforward=[64], classes=10, head=Head.SoftmaxCrossEntropy)``."""
 
-    def __init__(self, input_shape: Sequence[int], layers: Sequence, feedforward: Sequence[int], classes: int, device: int = 0):
+    def __init__(self, input_shape: Sequence[int], layers: Sequence, feedforward: Sequence[int], classes: int, device: int = 0,
+                 head: Head = Head.SigmoidQuadratic):
         self._lib = _lib.load()
         H, W, Cin = (int(x) for x in input_shape)
         self.input_shape = (H, W, Cin)
@@ -55,12 +69,13 @@ class ConvNet:
         self.feedforward = [int(x) for x in feedforward]
         self.classes = int(classes)
         self.device = int(device)
+        self.head = Head(head)
         spec = [v for l in self.layers for v in l.spec()]
         arr = (C.c_int32 * max(1, len(spec)))(*spec)
         ff = (C.c_size_t * max(1, len(self.feedforward)))(*self.feedforward)
         h = C.c_void_p()
-        _lib.check(self._lib.rcn_cuda_cnn_create(self.device, H, W, Cin, arr, len(self.layers), ff, len(self.feedforward),
-                                                 self.classes, C.byref(h)))
+        _lib.check(self._lib.rcn_cuda_cnn_create_with_head(self.device, H, W, Cin, arr, len(self.layers), ff,
+                                                           len(self.feedforward), self.classes, int(self.head), C.byref(h)))
         self._h = h
         self._shapes = []
         for i in range(len(self.layers)):
@@ -326,7 +341,8 @@ class ConvNet:
         return history
 
     def last_batch_stats(self) -> Tuple[float, int]:
-        """(quadratic cost, hits) of the last accumulated batch, evaluated with the pre-update parameters."""
+        """(cost, hits) of the last accumulated batch under the head's cost and hit rule, evaluated with the pre-update
+        parameters."""
         c, h = C.c_double(), C.c_uint64()
         _lib.check(self._lib.rcn_cuda_cnn_last_batch_stats(self._h, C.byref(c), C.byref(h)))
         return c.value, h.value
@@ -340,8 +356,9 @@ class ConvNet:
         return o, o.ctypes.data
 
     def evaluate_images(self, images, labels, want_labels: bool = False):
-        """``(accept, cost)`` of a labelled batch -- the rcn.rs:153-157 hit count and the quadratic cost -- and with
-        ``want_labels`` also the predicted labels, ``(accept, cost, labels)``.  Leaves the gradients untouched."""
+        """``(accept, cost)`` of a labelled batch -- the hit count and the batch cost under the head's rules (the
+        sigmoid head's are rcn.rs:153-157 and the quadratic cost) -- and with ``want_labels`` also the predicted labels,
+        ``(accept, cost, labels)``.  Leaves the gradients untouched."""
         buf, fmt, (B, H, W) = self._images(images)
         lb = _Buf(labels, np.int64)
         self._use_torch_stream(buf, lb)

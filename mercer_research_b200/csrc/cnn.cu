@@ -3,6 +3,11 @@
 //
 //   images -> [conv (+bias, ReLU) | pool]* -> flatten -> dense stack (sigmoid, quadratic cost) -> SGD on every parameter
 //
+// or, created with RCN_HEAD_SOFTMAX_XENT, the same dense stack with an affine output layer, softmax and cross-entropy
+// (semantics in rcn_cuda.h).  The head lives in the dense model (model_set_head): its last layer stores the logits and
+// softmax_xent_head_kernel turns them into p, delta_L = p - y and the batch statistics; the backward pass below is the same
+// for both heads.
+//
 // The handle owns the conv parameters, the per-layer activations and a dense rcn_cuda_model (model.cu) created with an
 // empty convpool stack, whose gradient buffer is the tail of this handle's flat gradient buffer.  A step only launches
 // kernels that already exist as ops (conv.cu, extops.cu, dense.cu, smallnet.cu), plus the dense stack's input gradient
@@ -403,8 +408,15 @@ extern "C" {
 
 int rcn_cuda_cnn_create(int device, size_t H, size_t W, size_t in_channels, const int32_t* layer_spec, size_t n_layers,
                         const size_t* feedforward, size_t n_ff, size_t classes, rcn_cuda_cnn_handle* out) {
+    return rcn_cuda_cnn_create_with_head(device, H, W, in_channels, layer_spec, n_layers, feedforward, n_ff, classes,
+                                         RCN_HEAD_SIGMOID_QUADRATIC, out);
+}
+
+int rcn_cuda_cnn_create_with_head(int device, size_t H, size_t W, size_t in_channels, const int32_t* layer_spec, size_t n_layers,
+                                  const size_t* feedforward, size_t n_ff, size_t classes, int head, rcn_cuda_cnn_handle* out) {
     if (!out) return fail(RCN_ERR_INVALID, "null out handle");
     *out = nullptr;
+    if (head != RCN_HEAD_SIGMOID_QUADRATIC && head != RCN_HEAD_SOFTMAX_XENT) return fail(RCN_ERR_INVALID, "unknown head %d", head);
     if (n_layers == 0 || !layer_spec) return fail(RCN_ERR_INVALID, "the network needs at least one conv / pool layer");
     if (n_ff && !feedforward) return fail(RCN_ERR_INVALID, "null feedforward");
     if (H == 0 || W == 0 || H > 32768 || W > 32768) return fail(RCN_ERR_INVALID, "bad image size %zu x %zu", H, W);
@@ -432,6 +444,7 @@ int rcn_cuda_cnn_create(int device, size_t H, size_t W, size_t in_channels, cons
         rc = fail(RCN_ERR_CUDA, "cudaStreamCreateWithFlags failed");
     h->stream = h->own_stream;
     if (rc == RCN_OK) rc = rcn_cuda_set_stream(m, h->stream);
+    if (rc == RCN_OK) rc = model_set_head(m, head);   // before the shapes: they pick the dense route
     if (rc == RCN_OK) rc = rcn_cuda_init_params_shapes(m, rows.data(), cols.data(), rows.size());
     if (rc == RCN_OK) rc = h->params.reserve(h->n_conv * sizeof(double));
     if (rc == RCN_OK) rc = h->grads_own.reserve(h->n_params * sizeof(double));

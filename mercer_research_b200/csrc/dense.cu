@@ -63,6 +63,10 @@ struct EpiForward {
         }
     }
 };
+struct EpiLogits {  // z = w * a + b with no activation: the softmax head's logits (softmax_xent_head_kernel follows)
+    const double* bias; double* z_out; int M;
+    __device__ __forceinline__ void operator()(int m, int n, double v) const { z_out[(size_t)n * M + m] = v + bias[m]; }
+};
 struct EpiBackData {
     const double* a; double* delta_out; int M;
     __device__ __forceinline__ void operator()(int m, int n, double v) const {
@@ -135,6 +139,8 @@ __device__ __forceinline__ void sk_dmma(double& c0, double& c1, double a, double
 // grid = ceil(N / 32); 256 threads: warp w contracts k in [w*K/8, (w+1)*K/8) for the CTA's 32 samples.  A lane loads
 // 4 consecutive k of one sample as two 16-byte loads (k = kb + 4t + j, j = 0..3): DMMA k-step j then uses element j of
 // every lane, i.e. the k set {kb + 4t + j}, and the W fragment is read at the same k.  Requires K % 128 == 0.
+// LOGITS: store z = w * a + b with no activation (the softmax head's logits; delta_out, onehot and labels are unused).
+template <bool LOGITS>
 __global__ void __launch_bounds__(256) skinny_forward_kernel(const double* __restrict__ W, const double* __restrict__ bias,
                                                              const double* __restrict__ A_in, int M, int K, int N,
                                                              double* __restrict__ A_out, double* __restrict__ delta_out,
@@ -213,6 +219,10 @@ __global__ void __launch_bounds__(256) skinny_forward_kernel(const double* __res
 #pragma unroll
         for (int q = 1; q < 8; ++q) v += part[q][s][m];          // K ranges in ascending order
         const double z = v + bias[m];                            // w * a + b           (rcn.rs:287)
+        if constexpr (LOGITS) {
+            A_out[(size_t)n * M + m] = z;
+            continue;
+        }
         const double act = sigmoid1(z);                          // sigmoid(&z)         (rcn.rs:289)
         const size_t idx = (size_t)n * M + m;
         A_out[idx] = act;
@@ -322,14 +332,28 @@ int launch_dense_forward(const double* W, const double* b, const double* A_in, s
                          cudaStream_t stream, OzakiWorkspace* oz) {
     if (N > 0 && skinny_layer(M, K)) {
         RCN_LAUNCH("skinny_forward_kernel", stream,
-                   skinny_forward_kernel<<<cdiv(N, SK_FWD_SAMPLES), 256, 0, stream>>>(W, b, A_in, (int)M, (int)K, (int)N, A_out, delta_out,
-                                                                                      onehot, labels));
+                   skinny_forward_kernel<false><<<cdiv(N, SK_FWD_SAMPLES), 256, 0, stream>>>(W, b, A_in, (int)M, (int)K, (int)N, A_out,
+                                                                                             delta_out, onehot, labels));
         return RCN_OK;
     }
     EpiForward epi{b, A_out, delta_out, onehot, labels, (int)M};
     const bool tc = use_tensor_cores(M, N, K, oz);
     return launch_gemm<false, true, EpiForward>(tc ? "dense_forward_gemm(tcgen05 int8 slices)" : "dense_forward_gemm", W, (int)M, A_in,
                                                 (int)K, M, N, K, 1, epi, stream, oz);
+}
+
+int launch_dense_logits(const double* W, const double* b, const double* A_in, size_t M, size_t K, size_t N, double* Z,
+                        cudaStream_t stream, OzakiWorkspace* oz) {
+    if (N > 0 && skinny_layer(M, K)) {
+        RCN_LAUNCH("skinny_forward_kernel(logits)", stream,
+                   skinny_forward_kernel<true><<<cdiv(N, SK_FWD_SAMPLES), 256, 0, stream>>>(W, b, A_in, (int)M, (int)K, (int)N, Z,
+                                                                                            nullptr, nullptr, nullptr));
+        return RCN_OK;
+    }
+    EpiLogits epi{b, Z, (int)M};
+    const bool tc = use_tensor_cores(M, N, K, oz);
+    return launch_gemm<false, true, EpiLogits>(tc ? "dense_logits_gemm(tcgen05 int8 slices)" : "dense_logits_gemm", W, (int)M, A_in,
+                                               (int)K, M, N, K, 1, epi, stream, oz);
 }
 
 int launch_dense_backward_data(const double* W_up, const double* delta_up, const double* A, size_t M, size_t K,
@@ -699,6 +723,104 @@ int launch_batch_stats(const double* acts, size_t n, size_t B, const double* one
     // ticket 1023 is reserved for this kernel
     RCN_LAUNCH("batch_stats_kernel", stream,
                batch_stats_kernel<<<grid, 256, 0, stream>>>(acts, (int)n, B, onehot, labels, stats_dev, rs.partials(), rs.tickets() + 1023));
+    return RCN_OK;
+}
+
+// Softmax cross-entropy head (launch_softmax_xent_head): one warp per sample (grid-stride), softmax_xent_warp's arithmetic,
+// in place over the logits.  Hits and labels are decided on z, not on p: exp rounding can make distinct logits equal
+// probabilities (z = (0, 2^-60) gives p = (0.5, 0.5)).  The argmax follows argmax_last_kernel's sequential rule exactly,
+// NaN included: after the last NaN q the scan restarts at q + 1 (the label is q itself when q = n - 1).  Each warp adds its
+// samples' costs in order, warp 0..7 sums are added in order per CTA, and the last CTA to arrive adds the per-CTA partials in
+// CTA order (batch_stats_kernel's scheme: deterministic for a given B) and resets the ticket for the next launch.
+__global__ void __launch_bounds__(256) softmax_xent_head_kernel(double* __restrict__ z, int n, size_t B,
+                                                               const int64_t* __restrict__ labels, double* __restrict__ delta,
+                                                               int64_t* __restrict__ labels_out, double* __restrict__ stats,
+                                                               double* __restrict__ partial, unsigned* __restrict__ ticket) {
+    __shared__ double sc[8];
+    __shared__ unsigned long long sh[8];
+    __shared__ bool s_last;
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const size_t warp = (blockIdx.x * (size_t)blockDim.x + threadIdx.x) >> 5;
+    const size_t n_warps = ((size_t)gridDim.x * blockDim.x) >> 5;
+    double cost = 0.0;
+    unsigned long long hits = 0;
+    for (size_t b = warp; b < B; b += n_warps) {
+        double* zb = z + b * n;
+        const int64_t lab = labels ? labels[b] : -1;
+        int q = -1;                                       // last NaN logit
+        int best = -1;
+        if (labels_out) {
+            for (int i = lane; i < n; i += 32) if (zb[i] != zb[i]) q = i;
+            q = __reduce_max_sync(0xffffffffu, q);
+            if (q >= 0 && q + 1 < n) {                    // last-max-wins over (q, n), which holds no NaN
+                double mx = -INFINITY;
+                for (int i = q + 1 + lane; i < n; i += 32) mx = fmax(mx, zb[i]);
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+                for (int i = q + 1 + lane; i < n; i += 32) if (zb[i] == mx) best = i;
+            } else if (q >= 0) {
+                best = q;
+            }
+        }
+        bool ok = true;
+        int at_max = -1;
+        const auto target = [&](int i) { return lab == (int64_t)i ? 1.0 : 0.0; };
+        const auto visit = [&](int i, double zi, double m, double p, double d) {
+            zb[i] = p;
+            if (delta) delta[b * n + i] = d;
+            ok = ok && ((zi == m) == (lab == (int64_t)i));   // {i : z_i = max z} == {label}
+            if (zi == m) at_max = i;
+        };
+        const double l = softmax_xent_warp(zb, n, lane, target, visit);
+        if (labels_out) {
+            if (q < 0) best = at_max;
+            best = __reduce_max_sync(0xffffffffu, best);
+            if (lane == 0) labels_out[b] = best;
+        }
+        const bool hit = __all_sync(0xffffffffu, ok);
+        cost += l;
+        hits += hit ? 1ull : 0ull;
+    }
+    if (!stats) return;
+    if (lane == 0) { sc[w] = cost; sh[w] = hits; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double ct = 0.0;
+        unsigned long long ht = 0;
+        for (int i = 0; i < 8; ++i) { ct += sc[i]; ht += sh[i]; }
+        partial[2 * blockIdx.x] = ct;
+        reinterpret_cast<unsigned long long*>(partial)[2 * blockIdx.x + 1] = ht;
+        __threadfence();
+        const unsigned t = atomicAdd(ticket, 1u);
+        s_last = (t == gridDim.x - 1);
+        if (s_last) *ticket = 0;
+    }
+    __syncthreads();
+    if (s_last && threadIdx.x == 0) {
+        __threadfence();
+        double ct = 0.0;
+        unsigned long long ht = 0;
+        for (unsigned i = 0; i < gridDim.x; ++i) {
+            ct += __ldcg(partial + 2 * i);
+            ht += __ldcg(reinterpret_cast<const unsigned long long*>(partial) + 2 * i + 1);
+        }
+        stats[0] = ct;
+        reinterpret_cast<unsigned long long*>(stats)[1] = ht;
+    }
+}
+
+int launch_softmax_xent_head(double* z, size_t n, size_t B, const int64_t* labels, double* delta, int64_t* labels_out,
+                             double* stats_dev, ReduceScratch& rs, cudaStream_t stream) {
+    if (n == 0 || n > 0x7fffffff) return fail(RCN_ERR_INVALID, "softmax head over %zu classes", n);
+    if (stats_dev && !labels) return fail(RCN_ERR_INVALID, "internal: head statistics need labels");
+    if (B == 0) return RCN_OK;
+    unsigned grid = cdiv(B, 8);
+    if (grid > kNumSMs * 8) grid = kNumSMs * 8;
+    // the partial region and ticket 1023 of batch_stats_kernel, which this kernel replaces on the softmax head
+    RCN_TRY(rs.ensure(((size_t)2 * grid + 2048) * sizeof(double), stream));
+    RCN_LAUNCH("softmax_xent_head_kernel", stream,
+               softmax_xent_head_kernel<<<grid, 256, 0, stream>>>(z, (int)n, B, labels, delta, labels_out, stats_dev, rs.partials(),
+                                                                  rs.tickets() + 1023));
     return RCN_OK;
 }
 

@@ -55,4 +55,48 @@ int launch_argmax_last(const double* acts, size_t n, size_t B, int64_t* labels, 
 int launch_batch_stats(const double* acts, size_t n, size_t B, const double* onehot, const int64_t* labels,
                        double* stats_dev, ReduceScratch& rs, cudaStream_t stream);
 
+// Z (M x N) = W (M x K) * A_in (K x N) + b 1^T with no activation: the logits of the softmax cross-entropy head, on the
+// engine launch_dense_forward would pick for the same shape.
+int launch_dense_logits(const double* W, const double* b, const double* A_in, size_t M, size_t K, size_t N, double* Z,
+                        cudaStream_t stream, OzakiWorkspace* oz = nullptr);
+
+// Softmax cross-entropy head over the logits z (n x B column-major), in place: z becomes p = softmax(z) per sample.
+// delta (optional, training): p - onehot(label).  labels_out (optional): the rcn.rs:92-97 last-max-wins argmax of z.
+// stats (optional, needs labels): stats[0] = sum_b of the per-sample cost (log s + m) - z_label, stats[1] = bit pattern of
+// the uint64 count of samples whose set {i : z_i = max z} is {label}.  Labels outside [0, n) have an all-zero target.
+int launch_softmax_xent_head(double* z, size_t n, size_t B, const int64_t* labels, double* delta, int64_t* labels_out,
+                             double* stats_dev, ReduceScratch& rs, cudaStream_t stream);
+
+#ifdef __CUDACC__
+// Softmax + cross-entropy of one sample's logits z[0..n) on one warp (lanes stride the classes); the reductions are warp
+// shuffles in a fixed order (deterministic): m = max z, then s = sum exp(z - m), then ls = log s.  Then for each of the
+// lane's classes i, in ascending order, with y = target(i): p = exp(z_i - m) / s and visit(i, z_i, m, p, p - y), where
+// z_i was read before visit is called (so visit may overwrite z in place).  Returns, on every lane, the sample's cost
+// sum_i y_i ((ls + m) - z_i) over the classes with y_i != 0.  ext_softmax_xent_kernel and softmax_xent_head_kernel share
+// this arithmetic.
+template <class Target, class Visit>
+__device__ __forceinline__ double softmax_xent_warp(const double* z, int n, int lane, const Target& target, const Visit& visit) {
+    double m = -INFINITY;
+    for (int i = lane; i < n; i += 32) m = fmax(m, z[i]);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) m = fmax(m, __shfl_xor_sync(0xffffffffu, m, o));
+    double s = 0.0;
+    for (int i = lane; i < n; i += 32) s += exp(z[i] - m);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    const double ls = log(s);
+    double l = 0.0;
+    for (int i = lane; i < n; i += 32) {
+        const double y = target(i);
+        const double zi = z[i];
+        const double p = exp(zi - m) / s;
+        visit(i, zi, m, p, p - y);
+        if (y != 0.0) l += y * ((ls + m) - zi);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) l += __shfl_xor_sync(0xffffffffu, l, o);
+    return l;
+}
+#endif
+
 }  // namespace rcn

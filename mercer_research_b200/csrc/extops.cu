@@ -10,6 +10,7 @@
 // output element with the channel index fastest, so every warp access is a contiguous run.  Checked against
 // oracle/ext_oracle.cpp ("parity unpinned").
 #include "conv.cuh"
+#include "dense.cuh"
 #include "opctx.cuh"
 
 namespace rcn {
@@ -69,7 +70,8 @@ __global__ void __launch_bounds__(256) ext_pool_backward_kernel(const double* __
 }
 
 // softmax + cross-entropy over column-major logits (n x B): one warp per sample, lanes stride the classes; the
-// max / sum reductions are warp shuffles in a fixed order (deterministic).
+// max / sum reductions are warp shuffles in a fixed order (deterministic).  The per-sample arithmetic is
+// softmax_xent_warp (dense.cuh), which the network's softmax head runs too.
 __global__ void __launch_bounds__(256) ext_softmax_xent_kernel(const double* __restrict__ z, int n, size_t B,
                                                                const double* __restrict__ onehot, const int64_t* __restrict__ labels,
                                                                double* __restrict__ probs, double* __restrict__ loss,
@@ -78,26 +80,12 @@ __global__ void __launch_bounds__(256) ext_softmax_xent_kernel(const double* __r
     const size_t warp = (blockIdx.x * (size_t)blockDim.x + threadIdx.x) >> 5;
     const size_t n_warps = ((size_t)gridDim.x * blockDim.x) >> 5;
     for (size_t b = warp; b < B; b += n_warps) {
-        const double* zb = z + b * n;
-        double m = -INFINITY;
-        for (int i = lane; i < n; i += 32) m = fmax(m, zb[i]);
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) m = fmax(m, __shfl_xor_sync(0xffffffffu, m, o));
-        double s = 0.0;
-        for (int i = lane; i < n; i += 32) s += exp(zb[i] - m);
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-        const double ls = log(s);
-        double l = 0.0;
-        for (int i = lane; i < n; i += 32) {
-            const double y = onehot ? onehot[b * n + i] : ((labels[b] == (int64_t)i) ? 1.0 : 0.0);
-            const double p = exp(zb[i] - m) / s;
+        const auto target = [&](int i) { return onehot ? onehot[b * n + i] : ((labels[b] == (int64_t)i) ? 1.0 : 0.0); };
+        const auto visit = [&](int i, double, double, double p, double d) {
             if (probs) probs[b * n + i] = p;
-            if (delta) delta[b * n + i] = p - y;
-            if (y != 0.0) l += y * ((ls + m) - zb[i]);
-        }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) l += __shfl_xor_sync(0xffffffffu, l, o);
+            if (delta) delta[b * n + i] = d;
+        };
+        const double l = softmax_xent_warp(z + b * n, n, lane, target, visit);
         if (loss && lane == 0) loss[b] = l;
     }
 }

@@ -213,6 +213,7 @@ struct rcn_cuda_model {
     double mean = 1.0, sd = 1.0;  // scale_set starts at (1, 1)  (rcn.rs:71)
     SmallNetDesc small_desc{};      // fused path for narrow networks (smallnet.cu)
     bool use_small = false;
+    int head = RCN_HEAD_SIGMOID_QUADRATIC;   // output layer and cost: only the convolutional network sets another (model_set_head)
 
     // feature plan cache
     bool plan_valid = false;
@@ -318,7 +319,8 @@ int features_into(rcn_cuda_model* h, const void* images, int fmt, size_t B, size
     return launch_features(h->plan, in.dev, fmt, B, H, W, standardise, h->mean, h->sd, out_dev, h->fscratch, h->stream);
 }
 
-// forward pass over device feats (cols[0] x B); fills acts; last layer also fills deltas when targets given
+// forward pass over device feats (cols[0] x B); fills acts; last layer also fills deltas when targets given.  With the
+// softmax head the last layer's activations are the logits z instead, and its deltas are left to the head kernel.
 int forward_dev(rcn_cuda_model* h, const double* feats, size_t B, const double* onehot, const int64_t* labels,
                 bool want_delta) {
     const size_t n = h->rows.size();
@@ -330,6 +332,11 @@ int forward_dev(rcn_cuda_model* h, const double* feats, size_t B, const double* 
     for (size_t l = 0; l < n; ++l) {
         const double* a_in = l == 0 ? feats : h->act(l - 1, B);
         const bool last = (l + 1 == n);
+        if (last && h->head == RCN_HEAD_SOFTMAX_XENT) {   // logits; the head kernel computes p and the output delta
+            RCN_TRY(launch_dense_logits(h->params.as<double>() + h->w_off[l], h->params.as<double>() + h->b_off[l], a_in, h->rows[l],
+                                        h->cols[l], B, h->act(l, B), h->stream, &h->oz));
+            break;
+        }
         RCN_TRY(launch_dense_forward(h->params.as<double>() + h->w_off[l], h->params.as<double>() + h->b_off[l], a_in,
                                      h->rows[l], h->cols[l], B, h->act(l, B),
                                      (last && want_delta) ? h->delta(l, B) : nullptr, onehot, labels, h->stream, &h->oz));
@@ -417,7 +424,13 @@ int accumulate_dev(rcn_cuda_model* h, const double* feats, const double* onehot,
         return RCN_OK;
     }
     if (front) return fail(RCN_ERR_STATE, "internal: fused front end requested on the generic path");
+    const bool softmax = h->head == RCN_HEAD_SOFTMAX_XENT;
+    if (softmax && !labels) return fail(RCN_ERR_INVALID, "the softmax head takes labels, not one-hot targets");
     RCN_TRY(forward_dev(h, feats, B, onehot, labels, true));
+    RCN_TRY(h->small.reserve(64));
+    if (softmax)   // p over z, delta_L = p - onehot(label), and the batch {cost, hits}
+        RCN_TRY(launch_softmax_xent_head(h->act(n - 1, B), h->rows[n - 1], B, labels, h->delta(n - 1, B), nullptr,
+                                         h->small.as<double>(), h->rs, h->stream));
     for (size_t l = n - 1; l-- > 0;)  // rcn.rs:305-311
         RCN_TRY(launch_dense_backward_data(h->params.as<double>() + h->w_off[l + 1], h->delta(l + 1, B), h->act(l, B),
                                            h->rows[l], h->rows[l + 1], B, h->delta(l, B), h->stream, &h->oz));
@@ -426,8 +439,8 @@ int accumulate_dev(rcn_cuda_model* h, const double* feats, const double* onehot,
         RCN_TRY(launch_dense_backward_weight(h->delta(l, B), a_prev, h->rows[l], h->cols[l], B, h->grads + h->w_off[l],
                                              h->grads + h->b_off[l], h->gemm_ws, h->rs, h->stream, &h->oz));
     }
-    RCN_TRY(h->small.reserve(64));
-    RCN_TRY(launch_batch_stats(h->act(n - 1, B), h->rows[n - 1], B, onehot, labels, h->small.as<double>(), h->rs, h->stream));
+    if (!softmax)
+        RCN_TRY(launch_batch_stats(h->act(n - 1, B), h->rows[n - 1], B, onehot, labels, h->small.as<double>(), h->rs, h->stream));
     h->stats_valid = true;
     h->last_B = B;
     return RCN_OK;
@@ -612,6 +625,7 @@ int install_shapes(rcn_cuda_model* h, const std::vector<size_t>& rows, const std
             for (size_t i = 0; i < n; ++i) { d.rows[i] = (int)h->rows[i]; d.w_off[i] = (int)h->w_off[i]; d.b_off[i] = (int)h->b_off[i]; }
             bool ok = true;
             for (size_t i = 0; i < n; ++i) ok = ok && h->rows[i] <= 32;
+            ok = ok && h->head == RCN_HEAD_SIGMOID_QUADRATIC;   // kernels A/B implement the sigmoid / quadratic head only
             if (ok && smallnet_eligible(d)) { h->small_desc = d; h->small_desc.tl = h->tl_on ? h->timeline.as<Timeline>() : nullptr; h->use_small = true; }
         }
     }
@@ -1650,8 +1664,18 @@ int model_evaluate_features(rcn_cuda_model* h, const double* feats, const int64_
     if (B == 0) return RCN_OK;
     RCN_TRY(forward_dev(h, feats, B, nullptr, nullptr, false));
     const size_t n = h->rows.size();
+    if (h->head == RCN_HEAD_SOFTMAX_XENT)
+        return launch_softmax_xent_head(h->act(n - 1, B), h->rows[n - 1], B, labels, nullptr, labels_out, labels ? stats : nullptr,
+                                        h->rs, h->stream);
     if (labels) RCN_TRY(launch_batch_stats(h->act(n - 1, B), h->rows[n - 1], B, nullptr, labels, stats, h->rs, h->stream));
     if (labels_out) RCN_TRY(launch_argmax_last(h->act(n - 1, B), h->rows[n - 1], B, labels_out, h->stream));
+    return RCN_OK;
+}
+
+int model_set_head(rcn_cuda_model* h, int head) {
+    if (head != RCN_HEAD_SIGMOID_QUADRATIC && head != RCN_HEAD_SOFTMAX_XENT) return fail(RCN_ERR_INVALID, "unknown head %d", head);
+    if (h->params_ready) return fail(RCN_ERR_STATE, "internal: the head is set before the layer shapes");
+    h->head = head;
     return RCN_OK;
 }
 

@@ -15,7 +15,11 @@ Per shape also: per-kernel time shares of the eager step from the library's
 launch profiler (a separate pass), the conv engine each layer's forward / backward-data / backward-weight took, and for
 the GEMM-shaped kernels the achieved rate against the DGEMM peak (torch.matmul f64) or the int8 tensor-core peak
 (torch._int_mm) measured in the same call.  The tcgen05 conv kernels run 15 int8 plane products per f64 product, so their
-int8 rate is 15 x 2MNK over the kernel time.  usage: python profiles/cnn_bench.py [--out DIR]"""
+int8 rate is 15 x 2MNK over the kernel time.
+Heads (run_heads, also alone with --heads-only -> cnn_heads_b200.json): per shape the sigmoid / quadratic head and the softmax
+cross-entropy head (ConvNet(head=...)) on the same parameters and data, alternated three times in the same process: the eager
+step and the replayed epoch step of each; and the per-step time of softmax_xent_head_kernel (and of every other kernel) from
+the launch profiler in a separate pass.  usage: python profiles/cnn_bench.py [--out DIR] [--heads-only]"""
 import argparse
 import json
 import os
@@ -231,17 +235,96 @@ def run_shape(name, cfg, pk):
     return res
 
 
+def run_heads(name, cfg):
+    """Both heads on the same parameters and resident data: eager and replayed epoch step times, alternated three times."""
+    c = cfg
+    B = c["B"]
+    per_batch = B * int(np.prod(c["shape"])) * (1 if c["u8"] else 8)
+    n_batches = max(2, -(-2 * L2_BYTES // per_batch))
+    g = torch.Generator(device="cuda"); g.manual_seed(2)
+    if c["u8"]:
+        data = torch.randint(0, 256, (n_batches, B) + c["shape"][:2], dtype=torch.uint8, device="cuda", generator=g)
+    else:
+        data = torch.randn((n_batches, B) + c["shape"], dtype=torch.float64, device="cuda", generator=g)
+    labels = torch.randint(0, 10, (n_batches, B), device="cuda", generator=g)
+    flat, flat_y = data.view((n_batches * B,) + data.shape[2:]), labels.view(-1)
+    perm = torch.randperm(n_batches * B, device="cuda", generator=g)
+    nets, steps, graphs = {}, {}, {}
+    for head in (m.Head.SigmoidQuadratic, m.Head.SoftmaxCrossEntropy):
+        net = m.ConvNet(c["shape"], c["layers"], c["ff"], 10, head=head)
+        net.init_params(np.random.default_rng(1))
+        k = [0]
+
+        def step(net=net, k=k):
+            i = k[0] % n_batches
+            k[0] += 1
+            net.train_batch_images(data[i], labels[i], 0.05)
+
+        for _ in range(3):
+            step()
+        net.epoch_bind(flat, flat_y, B, perm)
+        net.epoch_accumulate()
+        torch.cuda.synchronize()
+        graph = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(graph):
+            net.set_stream(torch.cuda.current_stream().cuda_stream)
+            net.epoch_step(0.05)
+        net.set_stream(torch.cuda.current_stream().cuda_stream)
+        nets[head.name], steps[head.name], graphs[head.name] = net, step, graph
+    gen = _lib.allocation_generation()
+    runs = {h: {"eager": [], "graph": []} for h in nets}
+    for _ in range(3):
+        for h in nets:
+            runs[h]["eager"].append(timed(steps[h])[0])
+            runs[h]["graph"].append(timed(graphs[h].replay)[0])
+    assert _lib.allocation_generation() == gen, "a library buffer moved under a captured step"
+    res = {"batch": B}
+    for h in nets:
+        torch.cuda.synchronize()
+        _lib.profile_enable(True)
+        for _ in range(5):
+            steps[h]()
+        rep = _lib.profile_report()
+        _lib.profile_enable(False)
+        kern = {kn: {"ms_per_step": v["total_ms"] / 5, "launches_per_step": v["launches"] / 5}
+                for kn, v in sorted(rep.items(), key=lambda kv: -kv[1]["total_ms"])}
+        r = {mode: dict(median_ms=float(np.median(v)), min_ms=min(v), max_ms=max(v), runs_ms=v) for mode, v in runs[h].items()}
+        r["kernels"] = kern
+        res[h] = r
+    s, x = res["SigmoidQuadratic"], res["SoftmaxCrossEntropy"]
+    res["softmax_over_sigmoid"] = {mode: x[mode]["median_ms"] / s[mode]["median_ms"] for mode in ("eager", "graph")}
+    res["head_kernel_ms_per_step"] = x["kernels"].get("softmax_xent_head_kernel", {}).get("ms_per_step")
+    for net in nets.values():
+        net.close()
+    del graphs, data, labels, flat, flat_y, perm
+    torch.cuda.empty_cache()
+    return res
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", default=".", help="directory that receives cnn_bench_b200.json")
+    ap.add_argument("--heads-only", action="store_true", help="only run_heads, into cnn_heads_b200.json")
     args = ap.parse_args()
     os.makedirs(args.out, exist_ok=True)
     info = gpu_info()
+    if args.heads_only:
+        out = dict(info, time=time.strftime("%Y-%m-%d %H:%M:%S"), shapes={})
+        for name, cfg in SHAPES.items():
+            r = out["shapes"][name] = run_heads(name, cfg)
+            print(f"{name}: sigmoid eager {r['SigmoidQuadratic']['eager']['median_ms']:.3f} graph "
+                  f"{r['SigmoidQuadratic']['graph']['median_ms']:.3f} ms; softmax eager {r['SoftmaxCrossEntropy']['eager']['median_ms']:.3f} "
+                  f"graph {r['SoftmaxCrossEntropy']['graph']['median_ms']:.3f} ms; head kernel {r['head_kernel_ms_per_step']} ms",
+                  flush=True)
+        with open(os.path.join(args.out, "cnn_heads_b200.json"), "w") as f:
+            json.dump(out, f, indent=1)
+        return
     pk = peaks()
     out = dict(info, measured_peaks=pk, time=time.strftime("%Y-%m-%d %H:%M:%S"), shapes={})
     for name, cfg in SHAPES.items():
         out["shapes"][name] = run_shape(name, cfg, pk)
         r = out["shapes"][name]
+        r["heads"] = run_heads(name, cfg)
         e = r["epoch_graph"]
         print(f"{name}: {r['images_per_s']:.0f} images/s ({r['step_ms']:.3f} ms/step, B={r['batch']}); epoch graph "
               f"{e['step_ms']:.3f} ms/step (x{e['replay_speedup']:.2f}); staging {e['stage_kernel_ms_per_step'] * 1e3:.1f} us "

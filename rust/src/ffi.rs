@@ -143,6 +143,9 @@ extern "C" {
     // ---- convolutional network handle (learned conv / pool layers + the dense stack) -------------------------------
     pub fn rcn_cuda_cnn_create(device: c_int, H: usize, W: usize, in_channels: usize, layer_spec: *const i32, n_layers: usize,
                                feedforward: *const usize, n_ff: usize, classes: usize, out: *mut rcn_cuda_cnn_handle) -> c_int;
+    pub fn rcn_cuda_cnn_create_with_head(device: c_int, H: usize, W: usize, in_channels: usize, layer_spec: *const i32,
+                                         n_layers: usize, feedforward: *const usize, n_ff: usize, classes: usize, head: c_int,
+                                         out: *mut rcn_cuda_cnn_handle) -> c_int;
     pub fn rcn_cuda_cnn_destroy(h: rcn_cuda_cnn_handle) -> c_int;
     pub fn rcn_cuda_cnn_set_stream(h: rcn_cuda_cnn_handle, stream: *mut c_void) -> c_int;
     pub fn rcn_cuda_cnn_synchronize(h: rcn_cuda_cnn_handle) -> c_int;
