@@ -403,6 +403,33 @@ class RCN {
 /// affine output layer with softmax and cross-entropy.
 enum class Head : int { SigmoidQuadratic = RCN_HEAD_SIGMOID_QUADRATIC, SoftmaxCrossEntropy = RCN_HEAD_SOFTMAX_XENT };
 
+/// Optimizer of a ConvNet's update (rcn_cuda_cnn_set_optimizer in rcn_cuda.h gives the formulas); the other kind's fields are
+/// ignored.  Optimizer{} is plain SGD, the default update.
+struct Optimizer {
+    int kind = RCN_OPTIMIZER_SGD;
+    double momentum = 0.0;
+    bool nesterov = false;
+    double weight_decay = 0.0;
+    double beta1 = 0.9, beta2 = 0.999, eps = 1e-8;
+
+    static Optimizer sgd(double momentum = 0.0, bool nesterov = false, double weight_decay = 0.0) {
+        Optimizer o;
+        o.momentum = momentum;
+        o.nesterov = nesterov;
+        o.weight_decay = weight_decay;
+        return o;
+    }
+    static Optimizer adamw(double beta1 = 0.9, double beta2 = 0.999, double eps = 1e-8, double weight_decay = 0.0) {
+        Optimizer o;
+        o.kind = RCN_OPTIMIZER_ADAMW;
+        o.beta1 = beta1;
+        o.beta2 = beta2;
+        o.eps = eps;
+        o.weight_decay = weight_decay;
+        return o;
+    }
+};
+
 /// Learned conv / pool layers in front of the reference's dense stack (rcn_cuda_cnn_* in rcn_cuda.h): a thin owner of the
 /// handle.  Images are u8 (B, H, W) row-major or f64 (B, H, W, C) NHWC, host or device memory.
 class ConvNet {
@@ -484,6 +511,19 @@ class ConvNet {
     void epoch_apply(double eta, size_t global_batch) { check(rcn_cuda_cnn_epoch_apply(h_, eta, global_batch)); }
     void epoch_step(double eta) { check(rcn_cuda_cnn_epoch_step(h_, eta)); }
     void epoch_run(double eta, size_t n_steps) { check(rcn_cuda_cnn_epoch_run(h_, eta, n_steps)); }
+    /// Selects the update of apply / epoch_apply and resets its state (captured steps must be re-captured).
+    void set_optimizer(const Optimizer& o) {
+        check(rcn_cuda_cnn_set_optimizer(h_, o.kind, o.momentum, o.nesterov ? 1 : 0, o.weight_decay, o.beta1, o.beta2, o.eps));
+    }
+    /// The optimizer's state as a flat vector (empty for plain SGD), to resume training in another network.
+    std::vector<double> optimizer_state() const {
+        size_t n = 0;
+        check(rcn_cuda_cnn_optimizer_state_size(h_, &n));
+        std::vector<double> s(n);
+        check(rcn_cuda_cnn_get_optimizer_state(h_, s.data(), n));
+        return s;
+    }
+    void set_optimizer_state(const std::vector<double>& s) { check(rcn_cuda_cnn_set_optimizer_state(h_, s.data(), s.size())); }
     rcn_cuda_cnn_handle handle() const { return h_; }
 
   private:

@@ -362,7 +362,8 @@ int rcn_cuda_cnn_get_params(rcn_cuda_cnn_handle h, double* flat, size_t n);
  * backward, ReLU', conv weight and bias gradients, and conv input gradients except for the first conv layer. */
 int rcn_cuda_cnn_accumulate(rcn_cuda_cnn_handle h, const void* images, int pixel_format, const int64_t* labels, size_t B,
                             size_t H, size_t W);
-/* p <- p - (eta / global_batch) * g over every parameter (rcn.rs:210-222 rounding). */
+/* p <- p - (eta / global_batch) * g over every parameter (rcn.rs:210-222 rounding), or the step of the optimizer set with
+ * rcn_cuda_cnn_set_optimizer (below). */
 int rcn_cuda_cnn_apply(rcn_cuda_cnn_handle h, double eta, size_t global_batch);
 /* accumulate + apply(eta, B) */
 int rcn_cuda_cnn_train_batch(rcn_cuda_cnn_handle h, const void* images, int pixel_format, const int64_t* labels, size_t B,
@@ -409,6 +410,34 @@ int rcn_cuda_cnn_get_gradients(rcn_cuda_cnn_handle h, double* flat, size_t n);
  * for a pool; B x H x W x C), and the dense stack's input gradient dX (L x B) of the last accumulate. */
 int rcn_cuda_cnn_get_layer_output(rcn_cuda_cnn_handle h, size_t layer, double* out);
 int rcn_cuda_cnn_get_input_gradient(rcn_cuda_cnn_handle h, double* out);
+/* Optimizer of the network's apply / epoch_apply (the update above is the default; RCN has no optimizer choice).
+ * Let g be a parameter's gradient sum (the flat buffer, after any all-reduce), B the global batch, eta the learning rate
+ * and lambda the weight decay, which applies to every parameter.  Every product, sum, quotient and square root is rounded
+ * on its own (no fused multiply-add), in this order:
+ *   RCN_OPTIMIZER_SGD     momentum mu in [0, 1), nesterov 0 / 1 (needs mu > 0), weight_decay lambda >= 0.  The default.
+ *                         mu = lambda = 0 is the plain update W -= (eta / B) * g, unchanged.  Otherwise (torch.optim.SGD
+ *                         without dampening; v starts at 0):
+ *                           gh = g / B;  d = gh + lambda * p;  v = mu * v + d;  u = nesterov ? d + mu * v : v;  p = p - eta * u
+ *                         (with mu = 0 there is no v and u = d).
+ *   RCN_OPTIMIZER_ADAMW   beta1, beta2 in [0, 1), eps > 0, weight_decay lambda >= 0 (torch.optim.AdamW).  The device keeps
+ *                         t and the running products beta1^t, beta2^t (from 0, 1, 1).  Per step t += 1, b1 = beta1^t * beta1,
+ *                         b2 = beta2^t * beta2 (stored back as the new beta1^t, beta2^t), then per parameter
+ *                           p = p * (1 - eta * lambda)            (the factor formed once on the host)
+ *                           gh = g / B;  m = beta1 * m + (1 - beta1) * gh;  v = beta2 * v + (1 - beta2) * (gh * gh)
+ *                           p = p - eta * ((m / (1 - b1)) / (sqrt(v / (1 - b2)) + eps))
+ * apply with global_batch 0 changes nothing, t included.  set_optimizer checks the hyperparameters of `kind` (those of the
+ * other kind are ignored; an unknown kind, a value out of range or a non-finite one is RCN_ERR_INVALID before any device
+ * work), allocates and resets the state and bumps rcn_cuda_allocation_generation, so a captured step must be re-captured
+ * (it also holds eta and the hyperparameters by value).  A step itself never allocates.
+ * The state is a flat f64 vector with the layout of the gradient buffer: v (n_params) for SGD with mu > 0, m | v | t,
+ * beta1^t, beta2^t (2 n_params + 3) for AdamW, empty otherwise.  get / set copy it (n must be the state size:
+ * RCN_ERR_INVALID otherwise); set moves no buffer, so the allocation generation stays. */
+enum { RCN_OPTIMIZER_SGD = 0, RCN_OPTIMIZER_ADAMW = 1 };
+int rcn_cuda_cnn_set_optimizer(rcn_cuda_cnn_handle h, int kind, double momentum, int nesterov, double weight_decay, double beta1,
+                               double beta2, double eps);
+int rcn_cuda_cnn_optimizer_state_size(rcn_cuda_cnn_handle h, size_t* n);
+int rcn_cuda_cnn_get_optimizer_state(rcn_cuda_cnn_handle h, double* state, size_t n);
+int rcn_cuda_cnn_set_optimizer_state(rcn_cuda_cnn_handle h, const double* state, size_t n);
 
 #ifdef __cplusplus
 }

@@ -8,7 +8,7 @@ from ._lib import RcnCudaError, load as load_library  # noqa: F401
 from .kernel import (Padding, Pooling, SeparableOperator, convolve_2d, convolve_2d_separated, pool_2d, relu,  # noqa: F401
                      sobel_separated)
 from .rcn import RCN, RCNLayer  # noqa: F401
-from .cnn import Conv, ConvNet, Head, Pool  # noqa: F401
+from .cnn import SGD, AdamW, Conv, ConvNet, Head, Pool  # noqa: F401
 
-__all__ = ["RCN", "RCNLayer", "ConvNet", "Conv", "Pool", "Head", "Padding", "Pooling", "SeparableOperator", "convolve_2d", "convolve_2d_separated",
+__all__ = ["RCN", "RCNLayer", "ConvNet", "Conv", "Pool", "Head", "SGD", "AdamW", "Padding", "Pooling", "SeparableOperator", "convolve_2d", "convolve_2d_separated",
            "relu", "pool_2d", "sobel_separated", "RcnCudaError", "load_library"]

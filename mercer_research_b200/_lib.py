@@ -124,6 +124,10 @@ SIGNATURES = {
     "rcn_cuda_cnn_get_gradients": [_vp, _vp, _sz],
     "rcn_cuda_cnn_get_layer_output": [_vp, _sz, _vp],
     "rcn_cuda_cnn_get_input_gradient": [_vp, _vp],
+    "rcn_cuda_cnn_set_optimizer": [_vp, _i, _d, _i, _d, _d, _d, _d],
+    "rcn_cuda_cnn_optimizer_state_size": [_vp, _szp],
+    "rcn_cuda_cnn_get_optimizer_state": [_vp, _vp, _sz],
+    "rcn_cuda_cnn_set_optimizer_state": [_vp, _vp, _sz],
 }
 _RESTYPES = {"rcn_cuda_last_error": C.c_char_p}
 

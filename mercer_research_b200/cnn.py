@@ -36,6 +36,28 @@ class Head(IntEnum):
 
 
 @dataclass(frozen=True)
+class SGD:
+    """``ConvNet.set_optimizer(SGD(momentum=0.9, nesterov=False, weight_decay=5e-4))``: torch's SGD without dampening, with
+    the exact operation order of rcn_cuda.h.  ``SGD()`` is the default update ``p -= (eta / B) * g``."""
+    momentum: float = 0.0
+    nesterov: bool = False
+    weight_decay: float = 0.0
+
+
+@dataclass(frozen=True)
+class AdamW:
+    """``ConvNet.set_optimizer(AdamW(beta1, beta2, eps, weight_decay))``: torch's AdamW with bias correction from running
+    products of the betas kept on the device, with the exact operation order of rcn_cuda.h."""
+    beta1: float = 0.9
+    beta2: float = 0.999
+    eps: float = 1e-8
+    weight_decay: float = 0.0
+
+
+OPTIMIZER_SGD, OPTIMIZER_ADAMW = 0, 1
+
+
+@dataclass(frozen=True)
 class Conv:
     """Learned cross-correlation with bias, always followed by ReLU (odd kernels for ``Padding.Same``)."""
     out_channels: int
@@ -178,6 +200,33 @@ class ConvNet:
         _lib.check(self._lib.rcn_cuda_cnn_get_gradients(self._h, buf.ctypes.data, buf.size))
         return buf
 
+    # -- optimizer ------------------------------------------------------------------------------------------------------
+    def set_optimizer(self, opt):
+        """Selects the update of ``apply_gradients`` / ``epoch_apply`` (``SGD`` or ``AdamW``) and resets its state.  A
+        captured step must be re-captured afterwards (``_lib.allocation_generation()`` changes); ``train_arrays`` and
+        ``DataParallelTrainer`` do that themselves."""
+        if isinstance(opt, SGD):
+            args = (OPTIMIZER_SGD, float(opt.momentum), int(bool(opt.nesterov)), float(opt.weight_decay), 0.0, 0.0, 0.0)
+        elif isinstance(opt, AdamW):
+            args = (OPTIMIZER_ADAMW, 0.0, 0, float(opt.weight_decay), float(opt.beta1), float(opt.beta2), float(opt.eps))
+        else:
+            raise TypeError(f"expected SGD or AdamW, got {type(opt).__name__}")
+        _lib.check(self._lib.rcn_cuda_cnn_set_optimizer(self._h, *args))
+
+    def optimizer_state(self) -> np.ndarray:
+        """The optimizer's state, flat f64: ``v`` for SGD with momentum, ``m | v | t, beta1^t, beta2^t`` for AdamW (each
+        with the flat parameter layout), empty for plain SGD."""
+        n = C.c_size_t()
+        _lib.check(self._lib.rcn_cuda_cnn_optimizer_state_size(self._h, C.byref(n)))
+        buf = np.zeros(n.value)
+        _lib.check(self._lib.rcn_cuda_cnn_get_optimizer_state(self._h, buf.ctypes.data, buf.size))
+        return buf
+
+    def load_optimizer_state(self, state):
+        """Restores a state from ``optimizer_state()`` of a network with the same shape and optimizer."""
+        state = np.ascontiguousarray(state, dtype=np.float64).ravel()
+        _lib.check(self._lib.rcn_cuda_cnn_set_optimizer_state(self._h, state.ctypes.data, state.size))
+
     def bind_gradient_buffer(self, tensor):
         """Use a caller-owned torch CUDA float64 tensor (n_params) as the flat gradient buffer (all-reduce target)."""
         if tensor is None:
@@ -214,7 +263,8 @@ class ConvNet:
         self._B_out = self._B_grad = B
 
     def apply_gradients(self, eta: float, batch: int):
-        """p <- p - (eta / batch) * g over every parameter; ``batch`` is the global minibatch."""
+        """p <- p - (eta / batch) * g over every parameter, or the step of the optimizer set with ``set_optimizer``;
+        ``batch`` is the global minibatch."""
         _lib.check(self._lib.rcn_cuda_cnn_apply(self._h, float(eta), int(batch)))
 
     def train_batch_images(self, images, labels, eta: float):

@@ -3,6 +3,8 @@
 //
 //   images -> [conv (+bias, ReLU) | pool]* -> flatten -> dense stack (sigmoid, quadratic cost) -> SGD on every parameter
 //
+// (or momentum SGD / AdamW, rcn_cuda_cnn_set_optimizer: one optim.cu launch over the conv and the dense parameters)
+//
 // or, created with RCN_HEAD_SOFTMAX_XENT, the same dense stack with an affine output layer, softmax and cross-entropy
 // (semantics in rcn_cuda.h).  The head lives in the dense model (model_set_head): its last layer stores the logits and
 // softmax_xent_head_kernel turns them into p, delta_L = p - y and the batch statistics; the backward pass below is the same
@@ -28,6 +30,7 @@
 #include "cnn.cuh"
 #include "conv.cuh"
 #include "dense.cuh"
+#include "optim.cuh"
 #include "ozaki.cuh"
 
 namespace rcn {
@@ -125,6 +128,9 @@ struct rcn_cuda_cnn {
     int ep_fmt = 0;
     size_t ep_n = 0, ep_B = 0;
     DevBuf ep_chunk, ep_state;
+    // optimizer (rcn_cuda_cnn_set_optimizer): opt_state = [state (optim_state_len doubles) | AdamW's CTA ticket]
+    OptimConfig opt;
+    DevBuf opt_state;
 };
 
 namespace {
@@ -324,8 +330,20 @@ int accumulate(rcn_cuda_cnn* h, const void* images, int fmt, const int64_t* labe
     return RCN_OK;
 }
 
+// The optimizer step of a non-default optimizer over the conv parameters and the dense model's, in one launch.
+int optim_step(rcn_cuda_cnn* h, double eta, size_t batch, long long* cursor = nullptr) {
+    double* dense = nullptr;
+    size_t n_dense = 0;
+    RCN_TRY(model_params(h->dense, &dense, &n_dense));
+    double* st = h->opt_state.as<double>();
+    unsigned* ticket = st ? reinterpret_cast<unsigned*>(st + optim_state_len(h->opt, h->n_params)) : nullptr;
+    return launch_optim_update(h->opt, h->params.as<double>(), h->n_conv, dense, n_dense, h->grads, st, ticket, eta, batch,
+                               h->stream, cursor, (long long)h->ep_B, (long long)h->ep_n);
+}
+
 int apply(rcn_cuda_cnn* h, double eta, size_t batch) {
     if (batch == 0) return RCN_OK;
+    if (!optim_is_plain(h->opt)) return optim_step(h, eta, batch);
     // (eta / batch) formed first, then the rounded product subtracted (rcn.rs:214); the dense part forms the same scale
     if (h->n_conv) RCN_TRY(launch_sgd_update(h->params.as<double>(), h->grads, h->n_conv, eta / (double)batch, h->stream));
     return rcn_cuda_apply_gradients(h->dense, eta, batch);
@@ -355,6 +373,7 @@ int epoch_accumulate(rcn_cuda_cnn* h) {
 int epoch_apply(rcn_cuda_cnn* h, double eta, size_t batch) {
     RCN_TRY(require_epoch(h));
     if (batch == 0) return fail(RCN_ERR_INVALID, "global batch is zero");
+    if (!optim_is_plain(h->opt)) return optim_step(h, eta, batch, h->ep_state.as<long long>());
     RCN_TRY(launch_sgd_update(h->params.as<double>(), h->grads, h->n_conv, eta / (double)batch, h->stream,
                               h->ep_state.as<long long>(), (long long)h->ep_B, (long long)h->ep_n));
     return rcn_cuda_apply_gradients(h->dense, eta, batch);
@@ -470,7 +489,7 @@ int rcn_cuda_cnn_destroy(rcn_cuda_cnn_handle h) {
     if (h->own_stream) { cudaStreamSynchronize(h->own_stream); cudaStreamDestroy(h->own_stream); }
     for (CnnLayer& ly : h->layers) { ly.out.release(); ly.argmax.release(); }
     DevBuf* bufs[] = {&h->params, &h->grads_own, &h->in_stage, &h->lab_stage, &h->out_stage, &h->x64, &h->dx, &h->gbuf[0],
-                      &h->gbuf[1], &h->flip_ws, &h->wgrad_ws, &h->small, &h->rs.buf, &h->ep_chunk, &h->ep_state};
+                      &h->gbuf[1], &h->flip_ws, &h->wgrad_ws, &h->small, &h->rs.buf, &h->ep_chunk, &h->ep_state, &h->opt_state};
     for (DevBuf* b : bufs) b->release();
     h->oz.release();
     delete h;
@@ -690,6 +709,51 @@ int rcn_cuda_cnn_get_input_gradient(rcn_cuda_cnn_handle h, double* out) {
     if (!out) return fail(RCN_ERR_INVALID, "null destination");
     if (!h->grad_B) return fail(RCN_ERR_STATE, "no batch has been accumulated yet");
     return deliver(h, out, h->dx.p, h->L * h->grad_B * sizeof(double));
+}
+
+int rcn_cuda_cnn_set_optimizer(rcn_cuda_cnn_handle h, int kind, double momentum, int nesterov, double weight_decay, double beta1,
+                               double beta2, double eps) {
+    if (!h) return fail(RCN_ERR_INVALID, "null network handle");
+    OptimConfig c;
+    c.kind = kind; c.momentum = momentum; c.nesterov = nesterov; c.weight_decay = weight_decay;
+    c.beta1 = beta1; c.beta2 = beta2; c.eps = eps;
+    RCN_TRY(optim_validate(c));
+    RCN_CUDA_TRY(cudaSetDevice(h->device));
+    RCN_CUDA_TRY(cudaStreamSynchronize(h->stream));   // no queued step still reads the old state
+    h->opt_state.release();
+    h->opt = OptimConfig{};
+    const size_t len = optim_state_len(c, h->n_params);
+    if (len) {
+        RCN_TRY(h->opt_state.reserve(len * sizeof(double) + 16));
+        RCN_CUDA_TRY(cudaMemsetAsync(h->opt_state.p, 0, len * sizeof(double) + 16, h->stream));
+        RCN_TRY(optim_reset_state(c, h->opt_state.as<double>(), h->n_params, h->stream));
+        RCN_CUDA_TRY(cudaStreamSynchronize(h->stream));
+    }
+    h->opt = c;
+    alloc_generation().fetch_add(1, std::memory_order_relaxed);   // a captured step holds the old update and its arguments
+    return RCN_OK;
+}
+
+int rcn_cuda_cnn_optimizer_state_size(rcn_cuda_cnn_handle h, size_t* n) {
+    if (!h || !n) return fail(RCN_ERR_INVALID, "null network handle / output");
+    *n = optim_state_len(h->opt, h->n_params);
+    return RCN_OK;
+}
+
+int rcn_cuda_cnn_get_optimizer_state(rcn_cuda_cnn_handle h, double* state, size_t n) {
+    RCN_CNN_ENTER(h);
+    const size_t len = optim_state_len(h->opt, h->n_params);
+    if (n != len) return fail(RCN_ERR_INVALID, "the optimizer state holds %zu doubles, got %zu", len, n);
+    if (len && !state) return fail(RCN_ERR_INVALID, "null destination");
+    return deliver(h, state, h->opt_state.p, len * sizeof(double));
+}
+
+int rcn_cuda_cnn_set_optimizer_state(rcn_cuda_cnn_handle h, const double* state, size_t n) {
+    RCN_CNN_ENTER(h);
+    const size_t len = optim_state_len(h->opt, h->n_params);
+    if (n != len) return fail(RCN_ERR_INVALID, "the optimizer state holds %zu doubles, got %zu", len, n);
+    if (len && !state) return fail(RCN_ERR_INVALID, "null source");
+    return copy_in(h, h->opt_state.as<double>(), state, len);
 }
 
 }  // extern "C"

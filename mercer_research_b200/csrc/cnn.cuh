@@ -16,5 +16,8 @@ int model_set_head(rcn_cuda_model* h, int head);
 // Device pointers of the first layer's weights W0 (rows0 x cols0, column-major) and of the first layer's deltas of the last
 // accumulate (rows0 x B).
 int model_first_layer(rcn_cuda_model* h, const double** W0, const double** delta0, size_t* rows0, size_t* cols0);
+// Device pointer of the model's flat parameters [W0|b0|W1|b1|...] and their count: the optimizer step of the handle updates
+// them in place (optim.cu).
+int model_params(rcn_cuda_model* h, double** params, size_t* n);
 
 }  // namespace rcn

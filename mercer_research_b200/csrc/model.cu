@@ -1688,4 +1688,11 @@ int model_first_layer(rcn_cuda_model* h, const double** W0, const double** delta
     return RCN_OK;
 }
 
+int model_params(rcn_cuda_model* h, double** params, size_t* n) {
+    RCN_TRY(require_params(h));
+    *params = h->params.as<double>();
+    *n = h->n_params;
+    return RCN_OK;
+}
+
 }  // namespace rcn

@@ -193,11 +193,13 @@ class DataParallelTrainer:
         tens of microseconds long.
 
         The warm-up (buffer sizing, kernel attributes, NCCL channel set-up) runs ``warmup`` real steps on a side stream and
-        then RESTORES parameters and cursor: capture() leaves the training state exactly as it found it, so the step-for-
-        step sequence of rcn.rs:144-149 is not advanced by it."""
+        then RESTORES parameters, cursor and optimizer state (momentum, AdamW's moments and step count; a model without
+        ``optimizer_state`` has none): capture() leaves the training state exactly as it found it, so the step-for-step
+        sequence of rcn.rs:144-149 is not advanced by it."""
         import torch
         position = self.model.epoch_position()
         params = self.model.get_params()
+        opt_state = self.model.optimizer_state() if hasattr(self.model, "optimizer_state") else None
         side = torch.cuda.Stream()
         side.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(side):
@@ -207,6 +209,8 @@ class DataParallelTrainer:
         torch.cuda.synchronize()
         self.check()
         self.model.set_params(params)
+        if opt_state is not None:
+            self.model.load_optimizer_state(opt_state)
         self.model.epoch_seek(position)
         self.steps_per_graph = max(1, int(steps_per_graph))
         self._capture_graph()

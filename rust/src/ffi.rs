@@ -27,6 +27,8 @@ pub const RCN_PIXELS_F64_NHWC: c_int = 2;
 pub const RCN_CNN_CONV: i32 = 0;
 pub const RCN_CNN_POOL: i32 = 1;
 pub const RCN_CNN_LAYER_INTS: usize = 5;
+pub const RCN_OPTIMIZER_SGD: c_int = 0;
+pub const RCN_OPTIMIZER_ADAMW: c_int = 1;
 
 extern "C" {
     pub fn rcn_cuda_last_error() -> *const c_char;
@@ -177,4 +179,9 @@ extern "C" {
     pub fn rcn_cuda_cnn_get_gradients(h: rcn_cuda_cnn_handle, flat: *mut c_double, n: usize) -> c_int;
     pub fn rcn_cuda_cnn_get_layer_output(h: rcn_cuda_cnn_handle, layer: usize, out: *mut c_double) -> c_int;
     pub fn rcn_cuda_cnn_get_input_gradient(h: rcn_cuda_cnn_handle, out: *mut c_double) -> c_int;
+    pub fn rcn_cuda_cnn_set_optimizer(h: rcn_cuda_cnn_handle, kind: c_int, momentum: c_double, nesterov: c_int,
+                                      weight_decay: c_double, beta1: c_double, beta2: c_double, eps: c_double) -> c_int;
+    pub fn rcn_cuda_cnn_optimizer_state_size(h: rcn_cuda_cnn_handle, n: *mut usize) -> c_int;
+    pub fn rcn_cuda_cnn_get_optimizer_state(h: rcn_cuda_cnn_handle, state: *mut c_double, n: usize) -> c_int;
+    pub fn rcn_cuda_cnn_set_optimizer_state(h: rcn_cuda_cnn_handle, state: *const c_double, n: usize) -> c_int;
 }
