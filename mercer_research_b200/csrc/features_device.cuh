@@ -4,6 +4,8 @@
 #pragma once
 #include "features.cuh"
 
+#include <cuda_fp16.h>
+
 namespace rcn {
 
 // ------------------------------------------------------------------------------------------------
@@ -334,6 +336,118 @@ __device__ __forceinline__ void cp_item(const CpStage& st, const int* __restrict
         o[nxt_map] = l;
         o[2 * nxt_map] = r;
         nxt[sB * nxt_map + (x + 2) * nxt_hp + y + 2] = b;
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
+// Packed form of a ONE-stage plan: the two fp16 lanes of a tile word hold the same pixel of two images.  From u8 pixels, every
+// intermediate of the closed form above is an integer of magnitude <= 255 * 4 = 1020 and fp16 holds every integer up to 2048
+// exactly, so HADD2 / HFMA2 (tap 2) / HMNMX2 compute both images' values exactly, one instruction for the pair.  (A second
+// stage would reach 255 * 16: more stages keep the int32 tiles.)
+// ------------------------------------------------------------------------------------------------
+__device__ __forceinline__ __half2 cp_h2(uint32_t u) { return *reinterpret_cast<const __half2*>(&u); }
+__device__ __forceinline__ uint32_t cp_u32(__half2 h) { return *reinterpret_cast<const uint32_t*>(&h); }
+
+// cp_item<true, true> over packed tiles: the four features of the pair's image in lane .x go to sink_x, those of lane .y to
+// sink_y (skipped when `live_y` is false: that lane is a zero image).
+template <typename Sink>
+__device__ __forceinline__ void cp_item_pair(const CpStage& st, const uint32_t* __restrict__ in, int it, const Sink& sink_x,
+                                             const Sink& sink_y, bool live_y) {
+    const int hw_out = st.h_out * st.w_out;
+    const int hp = st.hp;
+    const int x = cp_div(it, st.magic_h);
+    const int y = it - x * st.h_out;
+    const uint32_t* f = in + (2 * x) * hp + 2 * y;
+    __half2 p[4][4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        const uint2 a = *reinterpret_cast<const uint2*>(f + k * hp);
+        const uint2 b = *reinterpret_cast<const uint2*>(f + k * hp + 2);
+        p[0][k] = cp_h2(a.x); p[1][k] = cp_h2(a.y); p[2][k] = cp_h2(b.x); p[3][k] = cp_h2(b.y);
+    }
+    const bool rok0 = y > 0, rok1 = 2 * y + 1 < st.h;
+    const bool cok1 = 2 * x + 1 < st.w;
+    const __half2 zero = __float2half2_rn(0.0f), two = __float2half2_rn(2.0f);
+    __half2 tmax = zero, tmin = zero, lmax = zero, lmin = zero;
+#pragma unroll
+    for (int a = 0; a < 2; ++a) {
+        __half2 vT[4], vS[4];
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            vT[k] = __hsub2(p[a][k], p[a + 2][k]);
+            vS[k] = __hfma2(two, p[a + 1][k], __hadd2(p[a][k], p[a + 2][k]));
+        }
+        const bool rok = a ? rok1 : rok0;
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+            const bool ok = rok && (e ? cok1 : true);
+            const __half2 T = ok ? __hfma2(two, vT[e + 1], __hadd2(vT[e], vT[e + 2])) : zero;
+            const __half2 L = ok ? __hsub2(vS[e], vS[e + 2]) : zero;
+            tmax = __hmax2(tmax, T); tmin = __hmin2(tmin, T);
+            lmax = __hmax2(lmax, L); lmin = __hmin2(lmin, L);
+        }
+    }
+    // t = tmax, b = -tmin, l = lmax, r = -lmin, each in [0, 1020]: 1024 + v is exact and its fp16 mantissa field is v
+    const __half2 k1024 = __float2half2_rn(1024.0f);
+    const uint32_t t = cp_u32(__hadd2(k1024, tmax)), b = cp_u32(__hsub2(k1024, tmin));
+    const uint32_t l = cp_u32(__hadd2(k1024, lmax)), r = cp_u32(__hsub2(k1024, lmin));
+    sink_x(it, (int)(t & 0x3FF));
+    sink_x(it + hw_out, (int)(l & 0x3FF));
+    sink_x(it + 2 * hw_out, (int)(r & 0x3FF));
+    sink_x(it + 3 * hw_out, (int)(b & 0x3FF));
+    if (live_y) {
+        sink_y(it, (int)((t >> 16) & 0x3FF));
+        sink_y(it + hw_out, (int)((l >> 16) & 0x3FF));
+        sink_y(it + 2 * hw_out, (int)((r >> 16) & 0x3FF));
+        sink_y(it + 3 * hw_out, (int)((b >> 16) & 0x3FF));
+    }
+}
+
+// u8 row-major staging buffers -> packed fp16 tiles of a one-stage plan for n_img images: pair q holds image q in lane .x and
+// image q + y_off in lane .y (staging at stg + image * stg_stride bytes, tiles at tiles + q * tile_stride words); lanes of images
+// >= n_img are zero.  Byte k of both images' words is placed in the low byte of each half by one byte permute, given the
+// exponent of 1024 (0x6400: the half 1024 + byte, exact) and shifted back by 1024 with one HSUB2.  Task geometry and bank
+// pattern as cp_transpose_images below, over the pairs.
+__device__ __forceinline__ void cp_transpose_pairs(const uint8_t* __restrict__ stg, int stg_stride, int y_off,
+                                                   uint32_t* __restrict__ tiles, int tile_stride, int n_img, int H, int W,
+                                                   const CpPlan& cp, int tid, int nt) {
+    const int W4 = W >> 2;
+    const int hp = cp.s[0].hp;
+    const int chunks = (W4 + kCpWordsPerTask - 1) / kCpWordsPerTask;
+    const int tpi = cp.tasks_per_image;
+    const int lane = tid & 31, warp = tid >> 5, nwarps = nt >> 5;
+    const int n_pairs = min(y_off, n_img);
+    const __half2 k1024 = __float2half2_rn(1024.0f);
+    for (int task = warp; task < n_pairs * tpi; task += nwarps) {
+        const int q = cp_div1(task, tpi, cp.magic_tasks);
+        const int tl = task - q * tpi;
+        const int rg = cp_div1(tl, chunks, cp.magic_chunks);
+        const int it0 = (tl - rg * chunks) * kCpWordsPerTask;
+        const int r = rg * 32 + lane;
+        if (r >= H) continue;
+        int j = lane + it0;
+        if (W4 > 1) j -= cp_div(j, cp.magic_w4) * W4; else j = 0;
+        const uint32_t* row_x = reinterpret_cast<const uint32_t*>(stg + (size_t)q * stg_stride) + r * W4;
+        const uint32_t* row_y = reinterpret_cast<const uint32_t*>(stg + (size_t)(q + y_off) * stg_stride) + r * W4;
+        const bool live_y = q + y_off < n_img;
+        uint32_t* col0 = tiles + q * tile_stride + 2 * hp + r + 2;
+        const int n = min(kCpWordsPerTask, W4 - it0);
+#pragma unroll
+        for (int u = 0; u < kCpWordsPerTask; ++u) {
+            if (u < n) {
+                const uint32_t vx = row_x[j];
+                const uint32_t vy = live_y ? row_y[j] : 0u;
+                uint32_t* dst = col0 + 4 * j * hp;
+#pragma unroll
+                for (int k = 0; k < 4; ++k) {
+                    if (k == 3 && j == W4 - 1) break;   // column W-1 is never read downstream and stays zero
+                    // selector nibble n picks result byte n: byte k of vx -> byte 0, byte k of vy (index 4 + k) -> byte 2
+                    const uint32_t w = (__byte_perm(vx, vy, (unsigned)(k | ((k + 4) << 8))) & 0x00FF00FFu) | 0x64006400u;
+                    dst[k * hp] = cp_u32(__hsub2(cp_h2(w), k1024));
+                }
+                j = (j + 1 == W4) ? 0 : j + 1;
+            }
+        }
     }
 }
 

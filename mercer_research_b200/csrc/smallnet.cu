@@ -248,40 +248,62 @@ __device__ __forceinline__ void sn_phase_a(const SmallNetDesc& d, const double* 
     if (FUSED == 2) {
         // ---- staged front end: the 8 images arrive by bulk-async copies while the tiles' zero frames are written; then
         // all 16 warps transpose and run the conv+pool stages over the 8 images together (features_device.cuh) ---------
+        // (fr.cp_pairs: SN_TB / 2 packed tiles, pair q = images q and q + SN_TB / 2, see cp_item_pair)
         int* tiles = reinterpret_cast<int*>(stg + SN_TB * fr.cp.stage_bytes);
         const int n_live = min(SN_TB, B - s0);
+        const int n_tiles = fr.cp_pairs ? SN_TB / 2 : SN_TB;
         SN_PHASE(10);
-        for (int i = tid; i < SN_TB * fr.cp.tile_ints; i += SNA_THREADS) tiles[i] = 0;
+        for (int i = tid; i < n_tiles * fr.cp.tile_ints; i += SNA_THREADS) tiles[i] = 0;
         for (int i = n_live * pitch + tid; i < SN_TB * pitch; i += SNA_THREADS) tile[i] = 0.0;   // absent samples
         SN_PHASE(11);
         __syncthreads();
         SN_PHASE(12);
         cpbulk::mbar_wait(&s_bar, 0u);
         SN_PHASE(1);
-        cp_transpose_images(stg, fr.cp.stage_bytes, tiles, fr.cp.tile_ints, n_live, fr.H, fr.W, fr.cp, tid, SNA_THREADS);
+        if (fr.cp_pairs)
+            cp_transpose_pairs(stg, fr.cp.stage_bytes, SN_TB / 2, reinterpret_cast<uint32_t*>(tiles), fr.cp.tile_ints, n_live,
+                               fr.H, fr.W, fr.cp, tid, SNA_THREADS);
+        else
+            cp_transpose_images(stg, fr.cp.stage_bytes, tiles, fr.cp.tile_ints, n_live, fr.H, fr.W, fr.cp, tid, SNA_THREADS);
         __syncthreads();
         SN_PHASE(2);
-        for (int q = 0; q < fr.cp.n; ++q) {
-            const CpStage& st = fr.cp.s[q];
-            const int items = st.n_in * st.h_out * st.w_out;
-            const bool last = q == fr.cp.n - 1;
-            const CpStage& nx = fr.cp.s[last ? q : q + 1];
-            for (int it = tid; it < n_live * items; it += SNA_THREADS) {
-                const int gi = cp_div(it, st.magic_items);
-                const int itl = it - gi * items;
-                const int* in = tiles + gi * fr.cp.tile_ints + st.off;
-                int* nxt = tiles + gi * fr.cp.tile_ints + nx.off;
-                CpSinkTile<PREWAIT || INFER> sink{tile + (size_t)gi * pitch,
-                                                  (INFER || (PREWAIT && fr.prewait == 2)) ? nullptr : feats + (size_t)(s0 + gi) * L, fr.sc};
-                if (last) {
-                    if (q == 0) cp_item<true, true>(st, in, itl, nullptr, 0, 0, sink);
-                    else cp_item<true, false>(st, in, itl, nullptr, 0, 0, sink);
-                } else {
-                    if (q == 0) cp_item<false, true>(st, in, itl, nxt, nx.hp, nx.map_elems, sink);
-                    else cp_item<false, false>(st, in, itl, nxt, nx.hp, nx.map_elems, sink);
-                }
+        if (fr.cp_pairs) {
+            const CpStage& st = fr.cp.s[0];
+            const int items = st.h_out * st.w_out;
+            for (int it = tid; it < min(SN_TB / 2, n_live) * items; it += SNA_THREADS) {
+                const int q = cp_div(it, st.magic_items);   // one input map: magic_items divides by h_out * w_out
+                const int itl = it - q * items;
+                const int qy = q + SN_TB / 2;
+                const bool live_y = qy < n_live;
+                const bool hbm = !(INFER || (PREWAIT && fr.prewait == 2));
+                CpSinkTile<PREWAIT || INFER> sx{tile + (size_t)q * pitch, hbm ? feats + (size_t)(s0 + q) * L : nullptr, fr.sc};
+                CpSinkTile<PREWAIT || INFER> sy{tile + (size_t)qy * pitch, hbm && live_y ? feats + (size_t)(s0 + qy) * L : nullptr,
+                                                fr.sc};
+                cp_item_pair(st, reinterpret_cast<const uint32_t*>(tiles) + q * fr.cp.tile_ints, itl, sx, sy, live_y);
             }
             __syncthreads();
+        } else {
+            for (int q = 0; q < fr.cp.n; ++q) {
+                const CpStage& st = fr.cp.s[q];
+                const int items = st.n_in * st.h_out * st.w_out;
+                const bool last = q == fr.cp.n - 1;
+                const CpStage& nx = fr.cp.s[last ? q : q + 1];
+                for (int it = tid; it < n_live * items; it += SNA_THREADS) {
+                    const int gi = cp_div(it, st.magic_items);
+                    const int itl = it - gi * items;
+                    const int* in = tiles + gi * fr.cp.tile_ints + st.off;
+                    int* nxt = tiles + gi * fr.cp.tile_ints + nx.off;
+                    CpSinkTile<PREWAIT || INFER> sink{tile + (size_t)gi * pitch,
+                                                      (INFER || (PREWAIT && fr.prewait == 2)) ? nullptr : feats + (size_t)(s0 + gi) * L, fr.sc};
+                    if (last) {   // q > 0: one-stage plans take the packed path above
+                        cp_item<true, false>(st, in, itl, nullptr, 0, 0, sink);
+                    } else {
+                        if (q == 0) cp_item<false, true>(st, in, itl, nxt, nx.hp, nx.map_elems, sink);
+                        else cp_item<false, false>(st, in, itl, nxt, nx.hp, nx.map_elems, sink);
+                    }
+                }
+                __syncthreads();
+            }
         }
     } else if (FUSED == 1) {
         // ---- fused front end: two warps per image --------------------------------------------------------------
@@ -1011,7 +1033,8 @@ static size_t kernel_a_smem(const SmallNetDesc& d, const SmallNetFront* fr) {
     size_t bytes = ((size_t)SNA_WARPS * SN_TB * SN_ZPITCH + SN_MAX_SMALL) * sizeof(double);
     if (fr) {
         bytes += (size_t)SN_TB * (d.n_in + SN_TILE_PAD) * sizeof(double);
-        if (fr->use_cp) bytes += 128 + (size_t)SN_TB * ((size_t)fr->cp.stage_bytes + (size_t)fr->cp.tile_ints * sizeof(int));
+        if (fr->use_cp) bytes += 128 + (size_t)SN_TB * (size_t)fr->cp.stage_bytes +
+                                 (size_t)(fr->cp_pairs ? SN_TB / 2 : SN_TB) * (size_t)fr->cp.tile_ints * sizeof(int);
         else bytes += (size_t)SN_TB * 2 * fr->max_elems * sizeof(int);
     }
     return bytes;
@@ -1022,8 +1045,13 @@ bool smallnet_front_fits(const SmallNetDesc& d, const SmallNetFront& fr) { retur
 void smallnet_front_select(const FeaturePlan& plan, SmallNetFront* fr) {
     static const bool off = []() { const char* e = getenv("RCN_CUDA_FEATURES_STAGED"); return e && e[0] == '0'; }();
     fr->use_cp = 0;
+    fr->cp_pairs = 0;
     if (off || (reinterpret_cast<uintptr_t>(fr->images) & 15) != 0 || ((size_t)fr->H * fr->W) % 16 != 0) return;
-    if (make_cp_plan(plan, (size_t)fr->H, (size_t)fr->W, &fr->cp)) fr->use_cp = 1;
+    if (!make_cp_plan(plan, (size_t)fr->H, (size_t)fr->W, &fr->cp)) return;
+    fr->use_cp = 1;
+    long long bound = 255;   // largest magnitude of an intermediate after the plan's stages
+    for (int q = 0; q < fr->cp.n; ++q) bound *= 4;
+    fr->cp_pairs = bound <= 2048;   // one stage (1020; two reach 4080): the form cp_item_pair and kernel A's int32 loop assume
 }
 
 static int launch_kernel_a(const SmallNetDesc& d, const double* params, double* feats, size_t B, const double* onehot,

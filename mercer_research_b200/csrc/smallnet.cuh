@@ -33,9 +33,11 @@ struct SmallNetFront {
                                        // 2: one GPU, under the tail of the previous step's kernel B, which still reads the
                                        // feature buffer -- the features stay in the tile until the wait has passed
     int use_cp;                        // staged front end (bulk-async image loads, zero-framed tiles): see CpPlan
+    int cp_pairs;                      // ... on image pairs in exact fp16 lanes (cp_item_pair): every intermediate is an integer of
+                                       // magnitude <= 255 * 4^n_stages, which must not exceed 2048 -- one stage
     CpPlan cp;
 };
-// Fills use_cp / cp: the staged front end needs a qualifying plan, 16-byte aligned images and H*W % 16 == 0.
+// Fills use_cp / cp_pairs / cp: the staged front end needs a qualifying plan, 16-byte aligned images and H*W % 16 == 0.
 void smallnet_front_select(const FeaturePlan& plan, SmallNetFront* fr);
 
 // `params` may be null with `cursor` set: the kernel then only advances the cursor / writes the result ring (data-parallel

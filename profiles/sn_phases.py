@@ -1,7 +1,9 @@
 """Where kernel A (smallnet_fwd_bwd_kernel) spends its time on config c2: per-CTA clock64() stamps at the phase boundaries
 (library built by profiles/build_phases.sh with -DRCN_SN_PHASES).  Usage on the GPU box:
-    profiles/build_phases.sh && RCN_CUDA_LIB=profiles/_build/librcn_cuda_phases.so python profiles/sn_phases.py
+    profiles/build_phases.sh && RCN_CUDA_LIB=profiles/_build/librcn_cuda_phases.so python profiles/sn_phases.py [B] [--json PATH]
+(--json: also write the per-phase means of the front end and of the whole kernel, in ns, to PATH.)
 """
+import json
 import ctypes as C
 import os
 import sys
@@ -17,8 +19,7 @@ NAMES = ["image loads (bulk) + zero frames", "transpose", "conv+pool stages", "l
          "partial sums + narrow forward", "output delta + backward chain + writes", "small-parameter partials"]
 
 
-def main():
-    B = int(sys.argv[1]) if len(sys.argv) > 1 else 1024
+def main(B=1024, json_path=None):
     dev = torch.device("cuda", 0)
     model = RCN(10, [RCNLayer.Convolve2D(Padding.Same), RCNLayer.Pool2D(Pooling.Max)], [30])
     model.load_weights_and_bias(784)
@@ -49,6 +50,15 @@ def main():
         print(f"  {name:45s} {d[:, k].mean():8.0f} {d[:, k].min():8.0f} {d[:, k].max():8.0f}")
     tot = (out[:n, 7] - out[:n, 0]) / 1.965
     print(f"  {'thread-0 lifetime':45s} {tot.mean():8.0f} {tot.min():8.0f} {tot.max():8.0f}")
+    if json_path:
+        rec = {"B": B, "ctas": n, "clock_mhz_assumed": 1965,
+               "head_ns": {nm: float(ds[:, k].mean()) for k, nm in enumerate(
+                   ["bulk-load issue + labels", "W fragment loads issued", "small params staged", "zero frames", "barrier",
+                    "mbarrier wait"])},
+               "phases_ns": {nm: float(d[:, k].mean()) for k, nm in enumerate(NAMES)},
+               "thread0_lifetime_ns": float(tot.mean())}
+        with open(json_path, "w") as f:
+            json.dump(rec, f, indent=1)
 
 
 def timeline(B=1024, steps=40):
@@ -104,4 +114,10 @@ if __name__ == "__main__":
         timeline(int(sys.argv[2]) if len(sys.argv) > 2 else 1024)
         sys.exit(0)
 
-    main()
+    args = sys.argv[1:]
+    jp = None
+    if "--json" in args:
+        k = args.index("--json")
+        jp = args[k + 1]
+        del args[k:k + 2]
+    main(int(args[0]) if args else 1024, jp)
