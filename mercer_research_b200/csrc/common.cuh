@@ -35,7 +35,7 @@ int fail(int code, const char* fmt, ...);
 
 #define RCN_LAUNCH_CHECK()                                                                         \
     do {                                                                                           \
-        cudaError_t _e = cudaPeekAtLastError();                                                    \
+        cudaError_t _e = cudaGetLastError(); /* read and clear: a failed launch is reported once */ \
         if (_e != cudaSuccess)                                                                     \
             return ::rcn::fail(RCN_ERR_CUDA, "kernel launch failed: %s (%s:%d)", cudaGetErrorString(_e), \
                                __FILE__, __LINE__);                                                \
@@ -146,5 +146,7 @@ __device__ __forceinline__ double sgd_apply(double p, double scale, double g) { 
 constexpr int kNumSMs = 148;  // B200
 
 inline unsigned cdiv(size_t a, size_t b) { return (unsigned)((a + b - 1) / b); }
+// Largest gridDim.y / gridDim.z: a launch whose y or z extent grows with the batch caps it and loops, or launches slabs.
+constexpr unsigned kMaxGridYZ = 65535;
 
 }  // namespace rcn

@@ -181,66 +181,70 @@ __global__ void activation_backward_kernel(const double* __restrict__ y, const d
 // One CTA = a 16 x 16 tile of output pixels of one image, all output channels.  The input halo tile
 // ((16+kh-1) x (16+kw-1) x Ci) and the whole weight tensor are staged in shared memory (coalesced row runs); each
 // thread owns one pixel and produces the output channels eight at a time (weights are warp-uniform broadcasts).
+// gridDim.z = min(B, kMaxGridYZ): a CTA loops over images blockIdx.z, blockIdx.z + gridDim.z, ... with the weights
+// staged once; each output's sum runs in the same order whatever the batch.
 // The pixel type is a template parameter: u8 images (one channel) are read as they are stored.
 constexpr int DT = 16;
 template <typename Px>
 __device__ __forceinline__ void conv2d_direct_small(const Px* __restrict__ x, int H, int W, int Ci, const double* __restrict__ w,
                                                     const double* __restrict__ bias, int Co, int kh, int kw, int ph, int pw, int Ho,
-                                                    int Wo, int act, double* __restrict__ y) {
+                                                    int Wo, int act, int B, double* __restrict__ y) {
     extern __shared__ __align__(16) double sm_direct[];
     const int th = DT + kh - 1, tw = DT + kw - 1;
     const int kk = kh * kw * Ci;
     double* sx = sm_direct;                 // [th][tw][Ci]
     double* sw = sm_direct + th * tw * Ci;  // [Co][kh][kw][Ci]
     const int tid = threadIdx.x;
-    const int b = blockIdx.z;
     const int oy0 = blockIdx.y * DT, ox0 = blockIdx.x * DT;
     for (int i = tid; i < Co * kk; i += DT * DT) sw[i] = __ldg(w + i);
     const int row_len = tw * Ci;
-    for (int i = tid; i < th * row_len; i += DT * DT) {
-        const int ry = i / row_len, rx = i - ry * row_len;
-        const int iy = oy0 + ry - ph;
-        const int ix = ox0 - pw + rx / Ci;
-        const bool ok = (unsigned)iy < (unsigned)H && (unsigned)ix < (unsigned)W;
-        sx[i] = ok ? (double)__ldg(x + (((long long)b * H + iy) * W + (ox0 - pw)) * Ci + rx) : 0.0;
-    }
-    __syncthreads();
     const int ty = tid / DT, tx = tid % DT;
     const int oy = oy0 + ty, ox = ox0 + tx;
-    if (oy >= Ho || ox >= Wo) return;
-    double* yo = y + (((size_t)b * Ho + oy) * Wo + ox) * Co;
-    for (int co0 = 0; co0 < Co; co0 += 8) {
-        double acc[8];
+    for (int b = blockIdx.z; b < B; b += gridDim.z) {
+        if (b != (int)blockIdx.z) __syncthreads();   // everyone is done reading the previous image's tile
+        for (int i = tid; i < th * row_len; i += DT * DT) {
+            const int ry = i / row_len, rx = i - ry * row_len;
+            const int iy = oy0 + ry - ph;
+            const int ix = ox0 - pw + rx / Ci;
+            const bool ok = (unsigned)iy < (unsigned)H && (unsigned)ix < (unsigned)W;
+            sx[i] = ok ? (double)__ldg(x + (((long long)b * H + iy) * W + (ox0 - pw)) * Ci + rx) : 0.0;
+        }
+        __syncthreads();
+        if (oy >= Ho || ox >= Wo) continue;
+        double* yo = y + (((size_t)b * Ho + oy) * Wo + ox) * Co;
+        for (int co0 = 0; co0 < Co; co0 += 8) {
+            double acc[8];
 #pragma unroll
-        for (int j = 0; j < 8; ++j) acc[j] = 0.0;
-        for (int ky = 0; ky < kh; ++ky)
-            for (int q = 0; q < kw * Ci; ++q) {       // (kx, ci) run is contiguous in both the tile row and the weights
-                const double xv = sx[((ty + ky) * tw + tx) * Ci + q];
-                const double* wp = sw + (size_t)co0 * kk + ky * kw * Ci + q;
+            for (int j = 0; j < 8; ++j) acc[j] = 0.0;
+            for (int ky = 0; ky < kh; ++ky)
+                for (int q = 0; q < kw * Ci; ++q) {       // (kx, ci) run is contiguous in both the tile row and the weights
+                    const double xv = sx[((ty + ky) * tw + tx) * Ci + q];
+                    const double* wp = sw + (size_t)co0 * kk + ky * kw * Ci + q;
 #pragma unroll
-                for (int j = 0; j < 8; ++j)
-                    if (co0 + j < Co) acc[j] = fma(xv, wp[j * kk], acc[j]);
-            }
+                    for (int j = 0; j < 8; ++j)
+                        if (co0 + j < Co) acc[j] = fma(xv, wp[j * kk], acc[j]);
+                }
 #pragma unroll
-        for (int j = 0; j < 8; ++j)
-            if (co0 + j < Co) {
-                double v = acc[j];
-                if (bias) v += __ldg(bias + co0 + j);
-                yo[co0 + j] = act_forward(v, act);
-            }
+            for (int j = 0; j < 8; ++j)
+                if (co0 + j < Co) {
+                    double v = acc[j];
+                    if (bias) v += __ldg(bias + co0 + j);
+                    yo[co0 + j] = act_forward(v, act);
+                }
+        }
     }
 }
 __global__ void __launch_bounds__(DT * DT) conv2d_direct_small_kernel(const double* __restrict__ x, int H, int W, int Ci,
                                                                        const double* __restrict__ w, const double* __restrict__ bias,
                                                                        int Co, int kh, int kw, int ph, int pw, int Ho, int Wo,
-                                                                       int act, double* __restrict__ y) {
-    conv2d_direct_small(x, H, W, Ci, w, bias, Co, kh, kw, ph, pw, Ho, Wo, act, y);
+                                                                       int act, int B, double* __restrict__ y) {
+    conv2d_direct_small(x, H, W, Ci, w, bias, Co, kh, kw, ph, pw, Ho, Wo, act, B, y);
 }
 __global__ void __launch_bounds__(DT * DT) conv2d_direct_small_u8_kernel(const uint8_t* __restrict__ x, int H, int W, int Ci,
                                                                           const double* __restrict__ w, const double* __restrict__ bias,
                                                                           int Co, int kh, int kw, int ph, int pw, int Ho, int Wo,
-                                                                          int act, double* __restrict__ y) {
-    conv2d_direct_small(x, H, W, Ci, w, bias, Co, kh, kw, ph, pw, Ho, Wo, act, y);
+                                                                          int act, int B, double* __restrict__ y) {
+    conv2d_direct_small(x, H, W, Ci, w, bias, Co, kh, kw, ph, pw, Ho, Wo, act, B, y);
 }
 
 // ---- host side --------------------------------------------------------------------------------------------------------
@@ -304,16 +308,15 @@ int launch_conv2d_forward_u8(const uint8_t* x, const double* w, const double* bi
                              cudaStream_t stream) {
     if (s.B == 0) return RCN_OK;
     if (!use_direct(s) || s.Ci != 1) return fail(RCN_ERR_STATE, "internal: u8 convolution outside the direct kernel");
-    if (s.B > 65535) return fail(RCN_ERR_INVALID, "batch too large for the direct convolution kernel");
     const size_t smem = ((DT + s.kh - 1) * (DT + s.kw - 1) * s.Ci + s.Co * s.kh * s.kw * s.Ci) * sizeof(double);
     static SmemAttrCache attr;
     if (smem > 48 * 1024 && attr.need(smem))
         RCN_CUDA_TRY(cudaFuncSetAttribute(conv2d_direct_small_u8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    dim3 grid(cdiv(s.Wo, DT), cdiv(s.Ho, DT), (unsigned)s.B);
+    const dim3 grid(cdiv(s.Wo, DT), cdiv(s.Ho, DT), (unsigned)std::min<size_t>(s.B, kMaxGridYZ));
     RCN_LAUNCH("conv2d_direct_small_u8_kernel", stream,
                conv2d_direct_small_u8_kernel<<<grid, DT * DT, smem, stream>>>(x, (int)s.H, (int)s.W, (int)s.Ci, w, bias, (int)s.Co,
                                                                              (int)s.kh, (int)s.kw, s.ph, s.pw, (int)s.Ho, (int)s.Wo,
-                                                                             act, y));
+                                                                             act, (int)s.B, y));
     return RCN_OK;
 }
 
@@ -335,12 +338,11 @@ int launch_conv2d_forward(const double* x, const double* w, const double* bias, 
         static SmemAttrCache attr;
         if (smem > 48 * 1024 && attr.need(smem))
             RCN_CUDA_TRY(cudaFuncSetAttribute(conv2d_direct_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        if (s.B > 65535) return fail(RCN_ERR_INVALID, "batch too large for the direct convolution kernel");
-        dim3 grid(cdiv(s.Wo, DT), cdiv(s.Ho, DT), (unsigned)s.B);
+        const dim3 grid(cdiv(s.Wo, DT), cdiv(s.Ho, DT), (unsigned)std::min<size_t>(s.B, kMaxGridYZ));
         RCN_LAUNCH("conv2d_direct_small_kernel", stream,
                    conv2d_direct_small_kernel<<<grid, DT * DT, smem, stream>>>(x, (int)s.H, (int)s.W, (int)s.Ci, w, bias, (int)s.Co,
                                                                                 (int)s.kh, (int)s.kw, s.ph, s.pw, (int)s.Ho,
-                                                                                (int)s.Wo, act, y));
+                                                                                (int)s.Wo, act, (int)s.B, y));
         return RCN_OK;
     }
     const int M = (int)s.Co, N = (int)(s.B * s.Ho * s.Wo), K = (int)(s.kh * s.kw * s.Ci);

@@ -103,7 +103,7 @@ static int launch_gemm(const char* name, const double* A, int lda, const double*
     int k_per_split;
     split_plan(K, splits, k_per_split);
     if (gemm_impl() == GEMM_SIMT) {
-        dim3 grid(cdiv(M, 32), cdiv(N, 8), splits);
+        const dim3 grid(cdiv(M, 32), min(cdiv(N, 8), kMaxGridYZ), splits);
         RCN_LAUNCH(name, stream, gemm_f64_simt_kernel<AK, BKc, Epi><<<grid, 256, 0, stream>>>(A, lda, B, ldb, M, N, K, k_per_split, epi));
         return RCN_OK;
     }
@@ -233,16 +233,17 @@ __global__ void __launch_bounds__(256) skinny_forward_kernel(const double* __res
     }
 }
 
-// delta_out[k, n] = (sum_m W_up[m, k] delta_up[m, n]) * a (1 - a), a = A[k, n].  grid (ceil(K / 256), ceil(N / 16)).
-template <int MR>
+// delta_out[k, n] = (sum_m W_up[m, k] delta_up[m, n]) * a (1 - a), a = A[k, n].  grid (ceil(K / 256), chunks of 16
+// samples), sample chunks from n_chunk0 on when SLAB (a batch of more chunks than gridDim.y holds is several launches).
+template <int MR, bool SLAB>
 __global__ void __launch_bounds__(256) skinny_backward_data_kernel(const double* __restrict__ W_up, const double* __restrict__ delta_up,
-                                                                   const double* __restrict__ A, int K, int N,
+                                                                   const double* __restrict__ A, int K, int N, int n_chunk0,
                                                                    double* __restrict__ delta_out) {
     constexpr int NS = 16;
     constexpr int MP = (MR + 1) & ~1;               // rows padded to an even count: 16-byte shared loads
     __shared__ __align__(16) double sd[NS][MP];
     const int k = blockIdx.x * 256 + threadIdx.x;
-    const int n0 = blockIdx.y * NS;
+    const int n0 = ((SLAB ? n_chunk0 : 0) + blockIdx.y) * NS;
     for (int i = threadIdx.x; i < NS * MP; i += 256) {
         const int s = i / MP, m = i - s * MP;
         sd[s][m] = (m < MR && n0 + s < N) ? delta_up[(size_t)(n0 + s) * MR + m] : 0.0;
@@ -319,8 +320,17 @@ static bool skinny_layer(size_t M, size_t K) {
 template <int MR>
 static int launch_skinny_bwd_t(const double* W_up, const double* delta_up, const double* A, size_t M, size_t K, size_t N,
                                double* delta_out, cudaStream_t stream) {
-    RCN_LAUNCH("skinny_backward_data_kernel", stream,
-               skinny_backward_data_kernel<MR><<<dim3(cdiv(M, 256), cdiv(N, 16)), 256, 0, stream>>>(W_up, delta_up, A, (int)M, (int)N, delta_out));
+    const unsigned chunks = cdiv(N, 16);
+    if (chunks <= kMaxGridYZ) {
+        RCN_LAUNCH("skinny_backward_data_kernel", stream,
+                   skinny_backward_data_kernel<MR, false><<<dim3(cdiv(M, 256), chunks), 256, 0, stream>>>(W_up, delta_up, A, (int)M,
+                                                                                                      (int)N, 0, delta_out));
+        return RCN_OK;
+    }
+    for (unsigned c0 = 0; c0 < chunks; c0 += kMaxGridYZ)   // one launch per slab of at most kMaxGridYZ sample chunks
+        RCN_LAUNCH("skinny_backward_data_kernel", stream,
+                   skinny_backward_data_kernel<MR, true><<<dim3(cdiv(M, 256), min(chunks - c0, kMaxGridYZ)), 256, 0, stream>>>(
+                       W_up, delta_up, A, (int)M, (int)N, (int)c0, delta_out));
     return RCN_OK;
 }
 

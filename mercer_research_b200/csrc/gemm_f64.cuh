@@ -65,9 +65,11 @@ __device__ __forceinline__ void dmma_8x8x4(double& c0, double& c1, double a, dou
                  : "d"(a), "d"(b));
 }
 
-template <int BM, int BN, int WM, int WN, class ALoad, class BLoad, typename Epi>
+// SLAB: one of several launches over the column tiles, starting at column n_base (unused otherwise, so a grid within the
+// gridDim.y limit runs the same code as before slabs existed).
+template <int BM, int BN, int WM, int WN, class ALoad, class BLoad, typename Epi, bool SLAB>
 __global__ void __launch_bounds__(GEMM_THREADS) gemm_f64_dmma_kernel(const ALoad la, const BLoad lb, int M, int N, int K,
-                                                                      int k_per_split, Epi epi) {
+                                                                      int k_per_split, int n_base, Epi epi) {
     static_assert((BM / WM) * (BN / WN) == GEMM_THREADS / 32, "warp grid must use all warps");
     using TA = TileLayout<BM, ALoad::KCONTIG>;
     using TB = TileLayout<BN, BLoad::KCONTIG>;
@@ -81,7 +83,7 @@ __global__ void __launch_bounds__(GEMM_THREADS) gemm_f64_dmma_kernel(const ALoad
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int g = lane >> 2, t = lane & 3;
     const int wm = warp % (BM / WM), wn = warp / (BM / WM);
-    const int m0 = blockIdx.x * BM, n0 = blockIdx.y * BN;
+    const int m0 = blockIdx.x * BM, n0 = (SLAB ? n_base : 0) + blockIdx.y * BN;
     const int k_begin = blockIdx.z * k_per_split;
     const int k_end = min(K, k_begin + k_per_split);
     const int ntiles = (k_end - k_begin + KT - 1) / KT;
@@ -149,20 +151,22 @@ __global__ void __launch_bounds__(GEMM_THREADS) gemm_f64_dmma_kernel(const ALoad
 }
 
 // Plain one-thread-per-output kernel: slow, obviously correct; cross-checks the DMMA path (RCN_CUDA_GEMM=simt).
+// gridDim.y is capped at kMaxGridYZ; the rows of 8 columns beyond it are looped over.
 template <bool AK, bool BKc, typename Epi>
 __global__ void gemm_f64_simt_kernel(const double* __restrict__ A, int lda, const double* __restrict__ B, int ldb, int M,
                                      int N, int K, int k_per_split, Epi epi) {
     const int m = blockIdx.x * 32 + (threadIdx.x & 31);
-    const int n = blockIdx.y * 8 + (threadIdx.x >> 5);
-    if (m >= M || n >= N) return;
+    if (m >= M) return;
     const int k_begin = blockIdx.z * k_per_split, k_end = min(K, k_begin + k_per_split);
-    double acc = 0.0;
-    for (int k = k_begin; k < k_end; ++k) {
-        const double a = AK ? A[(size_t)m * lda + k] : A[(size_t)k * lda + m];
-        const double b = BKc ? B[(size_t)n * ldb + k] : B[(size_t)k * ldb + n];
-        acc = fma(a, b, acc);
+    for (int n = blockIdx.y * 8 + (threadIdx.x >> 5); n < N; n += gridDim.y * 8) {
+        double acc = 0.0;
+        for (int k = k_begin; k < k_end; ++k) {
+            const double a = AK ? A[(size_t)m * lda + k] : A[(size_t)k * lda + m];
+            const double b = BKc ? B[(size_t)n * ldb + k] : B[(size_t)k * ldb + n];
+            acc = fma(a, b, acc);
+        }
+        epi(m, n, acc);
     }
-    epi(m, n, acc);
 }
 
 template <int BM, int BN, int WM, int WN, class ALoad, class BLoad, typename Epi>
@@ -172,11 +176,24 @@ static int launch_dmma(const char* name, const ALoad& la, const BLoad& lb, int M
     using TB = TileLayout<BN, BLoad::KCONTIG>;
     constexpr size_t smem = (size_t)STAGES * (TA::ELEMS + TB::ELEMS) * sizeof(double) +
                             (size_t)(BM * ALoad::kPrepInts + BN * BLoad::kPrepInts) * sizeof(int);
-    auto kern = gemm_f64_dmma_kernel<BM, BN, WM, WN, ALoad, BLoad, Epi>;
-    static SmemAttrCache attr;  // per instantiation
+    const unsigned n_tiles = cdiv(N, BN);
+    if (n_tiles <= kMaxGridYZ) {
+        auto kern = gemm_f64_dmma_kernel<BM, BN, WM, WN, ALoad, BLoad, Epi, false>;
+        static SmemAttrCache attr;  // per instantiation
+        if (attr.need(smem)) RCN_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        const dim3 grid(cdiv(M, BM), n_tiles, splits);
+        RCN_LAUNCH(name, stream, kern<<<grid, GEMM_THREADS, smem, stream>>>(la, lb, M, N, K, k_per_split, 0, epi));
+        return RCN_OK;
+    }
+    // More column tiles than gridDim.y holds (a conv layer's columns are its B*Ho*Wo output pixels): one launch per slab
+    // of at most kMaxGridYZ tiles.
+    auto kern = gemm_f64_dmma_kernel<BM, BN, WM, WN, ALoad, BLoad, Epi, true>;
+    static SmemAttrCache attr;
     if (attr.need(smem)) RCN_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    dim3 grid(cdiv(M, BM), cdiv(N, BN), splits);
-    RCN_LAUNCH(name, stream, kern<<<grid, GEMM_THREADS, smem, stream>>>(la, lb, M, N, K, k_per_split, epi));
+    for (unsigned t0 = 0; t0 < n_tiles; t0 += kMaxGridYZ) {
+        const dim3 grid(cdiv(M, BM), min(n_tiles - t0, kMaxGridYZ), splits);
+        RCN_LAUNCH(name, stream, kern<<<grid, GEMM_THREADS, smem, stream>>>(la, lb, M, N, K, k_per_split, (int)t0 * BN, epi));
+    }
     return RCN_OK;
 }
 
