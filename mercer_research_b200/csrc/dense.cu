@@ -340,7 +340,9 @@ static int launch_skinny_bwd_t(const double* W_up, const double* delta_up, const
 int launch_dense_forward(const double* W, const double* b, const double* A_in, size_t M, size_t K, size_t N,
                          double* A_out, double* delta_out, const double* onehot, const int64_t* labels,
                          cudaStream_t stream, OzakiWorkspace* oz) {
-    if (N > 0 && skinny_layer(M, K)) {
+    // the skinny kernel reads A_in as double2: a layer's activations start at an odd double when the rows below it times B
+    // are odd, and those take the GEMM, whose cp.async copies are 8 bytes
+    if (N > 0 && skinny_layer(M, K) && ((uintptr_t)A_in & 15) == 0) {
         RCN_LAUNCH("skinny_forward_kernel", stream,
                    skinny_forward_kernel<false><<<cdiv(N, SK_FWD_SAMPLES), 256, 0, stream>>>(W, b, A_in, (int)M, (int)K, (int)N, A_out,
                                                                                              delta_out, onehot, labels));
@@ -354,7 +356,7 @@ int launch_dense_forward(const double* W, const double* b, const double* A_in, s
 
 int launch_dense_logits(const double* W, const double* b, const double* A_in, size_t M, size_t K, size_t N, double* Z,
                         cudaStream_t stream, OzakiWorkspace* oz) {
-    if (N > 0 && skinny_layer(M, K)) {
+    if (N > 0 && skinny_layer(M, K) && ((uintptr_t)A_in & 15) == 0) {   // 16-byte loads, as in launch_dense_forward
         RCN_LAUNCH("skinny_forward_kernel(logits)", stream,
                    skinny_forward_kernel<true><<<cdiv(N, SK_FWD_SAMPLES), 256, 0, stream>>>(W, b, A_in, (int)M, (int)K, (int)N, Z,
                                                                                             nullptr, nullptr, nullptr));
